@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the slam_recognition filter-pipeline hot path on B200 (contract: see the driver's prompt / DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path (pyramid -> S1-S7 fused stack -> feature-point emit) over one batch of synthetic
 1080p uint8 BGR frames (BASELINE config C3: 1920x1080, scale sqrt(2) -> 6 levels of 192x288, batch 64 per GPU; frames of
@@ -20,6 +20,9 @@ crosses NVLink). Prints ONE JSON line on rank 0.
             restated in numpy; real TensorFlow-1 cannot be installed here), for C1 and C3 frames
   ranks     per-rank device ms (min / median / max), host enqueue time per step, wait for the last point gather
   gather_check  (N > 1) rank 0 recomputes rank 1's frames locally and compares them with the rows NCCL delivered
+
+--dump-outputs DIR writes what the last timed step handed its caller on rank 0 as DIR/<name>.npy (see dump_outputs), so
+that two builds run with the same arguments (hence the same seeded frames) can be compared output for output.
 """
 import argparse
 import concurrent.futures
@@ -35,6 +38,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the tree may be read-only and the bench writes nothing into it: no bytecode caches, in this process or its CPU workers
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 METRIC = "frames/sec (1080p RGB, full pyramid)"
 CENTER = (288, 192)
@@ -339,6 +345,35 @@ def link_probe(dev, world):
     return {"h2d_and_d2h_concurrent_gbs_each": nbytes / dt / 1e9, "bytes_each_way": nbytes}
 
 
+DUMP_SAMPLE = 1 << 22   # elements kept of each [B*L,h,w,3] result tensor: 16 MB of float32, 32 MB for the two
+DUMP_LIMIT = 64 << 20   # bytes of one dump in all
+
+
+def dump_outputs(out_dir, orient, padded_line_end, points, gathered=None):
+    """Write the arrays the timed path handed its caller as ``out_dir/<name>.npy``: ``orient`` and ``padded_line_end``
+    (float32; beyond DUMP_SAMPLE elements, the elements at the sorted unique flat indices of
+    ``RandomState(0).randint(0, numel, DUMP_SAMPLE)``, which depend on the shape alone), ``points`` (the valid feature-point
+    rows (level, y, x, 0), float64: exact for these integers) and, on several GPUs, ``gathered_points`` (every rank's rows
+    as the point gather delivered them)."""
+    import torch
+    arrays = {}
+    numel = orient.numel()
+    if numel > DUMP_SAMPLE:
+        index = np.unique(np.random.RandomState(0).randint(0, numel, size=DUMP_SAMPLE))
+        index = torch.from_numpy(index).to(orient.device)
+    for name, t in (("orient", orient), ("padded_line_end", padded_line_end)):
+        arrays[name] = (t.reshape(-1)[index] if numel > DUMP_SAMPLE else t).cpu().numpy().astype(np.float32)
+    arrays["points"] = points.cpu().numpy().astype(np.float64)
+    if gathered is not None:
+        arrays["gathered_points"] = gathered.cpu().numpy().astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args, rank, local_rank, world):
     import ctypes
     import torch
@@ -417,6 +452,9 @@ def run_ours(args, rank, local_rank, world):
                 int(counts.sum().item()) == int(pts.shape[0]) and bool((pts[1:, 0] >= pts[:-1, 0]).all())
             gather_check = "ok" if ok else "MISMATCH"
             del other
+    if args.dump_outputs and rank == 0:   # before the passes below run the step again into the same buffers
+        dump_outputs(args.dump_outputs, bufs[0], bufs[1], bufs[2][:count_points],
+                     pts if gatherer is not None else None)
 
     # per-stage device time (separate, untimed pass with the library's event hooks)
     _lib.check(_lib.lib().silent_plan_enable_timing(plan.handle, 1))
@@ -590,7 +628,13 @@ def main():
     ap.add_argument("--no-natural", dest="natural", action="store_false")
     ap.add_argument("--native-gather", action="store_true",
                     help="point gather through silent_gather_points (ncclAllGather behind the C ABI) instead of torch's")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's results to DIR/<name>.npy (at most 64 MB, see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the CPU arm keeps only point counts")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
