@@ -83,6 +83,22 @@ typedef struct silent_bank_weights {
     int32_t border;
 } silent_bank_weights;
 
+/* Orientation bank of any fused width: `orientations` = 4, 8, 12 or 16 (SILENT_E_SHAPE otherwise), n below. Each HWIO
+ * array is sized for SILENT_BANK_MAX and holds the n-wide filter packed densely at its front ([3,3,3,n] for the stripe
+ * bank, [7,7,n,n] blur, [3,3,n,n] end); the rest is ignored. orientation_bank_filters(n) (pipeline.py) builds them with
+ * the generators named at silent_bank_weights. Same structure requirements as silent_bank_weights (SILENT_E_STRUCTURE). */
+#define SILENT_BANK_MAX 16
+typedef struct silent_orientation_bank {
+    int32_t orientations;
+    float rgc[3 * 3 * 3 * 3];
+    float rgby[3 * 3 * 3 * 3];
+    float stripe[3 * 3 * 3 * SILENT_BANK_MAX];                  /* identical over the 3 input channels */
+    float blur[7 * 7 * SILENT_BANK_MAX * SILENT_BANK_MAX];      /* every slice identical */
+    float end[3 * 3 * SILENT_BANK_MAX * SILENT_BANK_MAX];       /* depthwise */
+    float regulation_value, regulation_root, clip_max;
+    int32_t border;
+} silent_orientation_bank;
+
 int silent_abi_version(void);
 const char *silent_last_error(void);
 /* Number of CUDA kernels this library has launched in this process so far (bench.py reports the delta per step). */
@@ -243,6 +259,15 @@ int silent_stack_fused(const float *pyramid_dev, int n, int h, int w, const sile
                        float *orient_dev, float *line_end_dev, float *gray_dev, void *workspace_dev,
                        size_t workspace_bytes, silent_stream stream);
 
+/* The orientation bank's stack on an NHWC pyramid: pyramid_dev [n,h,w,3] -> rgc -> rgby -> stripe bank -> regulator ->
+ * end bank -> mask -> mean, orient_dev / line_end_dev [n,h,w,nb], gray_dev [n,h,w,1] (nb = bank_host->orientations; any
+ * output may be NULL). Two kernels: stack_a (as in silent_stack_fused) and stack_bank_kernel. Workspace size and the
+ * finite-input PRECONDITION as for silent_stack_fused. The width and structure checks (SILENT_E_SHAPE,
+ * SILENT_E_STRUCTURE) run on the host before any CUDA call. */
+int silent_stack_bank(const float *pyramid_dev, int n, int h, int w, const silent_orientation_bank *bank_host,
+                      float *orient_dev, float *line_end_dev, float *gray_dev, void *workspace_dev, size_t workspace_bytes,
+                      silent_stream stream);
+
 /* The whole hot path for a batch resident in HBM: frames -> pyramid -> S1-S7 -> feature points (S8, region =
  * (h/2, w/2), recognition_testing.py:40,90-91). Uses the plan workspace (silent_plan_reserve(batch) first).
  * Outputs as in silent_stack_fused / silent_max_value_indices_region; pyramid_dev may be NULL (plan scratch is used). */
@@ -252,17 +277,27 @@ int silent_pipeline_run(silent_plan *plan, const silent_stack_weights *weights_h
 
 /* The same path with the 8-orientation bank (config C4): frames -> pyramid -> rgc -> rgby -> stripe bank -> regulator ->
  * end bank -> mask -> mean -> feature points; orient_dev / line_end_dev are [batch*L, h, w, 8]. uint8 frames with 3 colours
- * only; SILENT_E_STRUCTURE when the bank lacks the generators' structure (use the per-operator calls then). */
+ * only; SILENT_E_STRUCTURE when the bank lacks the generators' structure (use the per-operator calls then). Equal to
+ * silent_pipeline_run_orientations with the same 8-wide bank. */
 int silent_pipeline_run_bank(silent_plan *plan, const silent_bank_weights *weights_host, const void *frames_dev, int batch,
                              float *orient_dev, float *line_end_dev, int64_t *points_dev, int64_t capacity,
                              int64_t *count_dev, silent_stream stream);
 
-/* Measurement hook: when enabled, silent_pipeline_run brackets its stages with CUDA events on the launching stream.
+/* The same path for a bank of 4, 8, 12 or 16 orientations: orient_dev / line_end_dev are [batch*L, h, w, nb]. Same
+ * preconditions as silent_pipeline_run_bank (uint8 frames, 3 colours, frame-pair pyramid path). The bank's width and
+ * structure are checked on the host before any CUDA call (SILENT_E_SHAPE, SILENT_E_STRUCTURE). */
+int silent_pipeline_run_orientations(silent_plan *plan, const silent_orientation_bank *bank_host, const void *frames_dev,
+                                     int batch, float *orient_dev, float *line_end_dev, int64_t *points_dev,
+                                     int64_t capacity, int64_t *count_dev, silent_stream stream);
+
+/* Measurement hook: when enabled, silent_pipeline_run (and the two bank entries above) brackets its stages with CUDA
+ * events on the launching stream.
  * silent_plan_stage_ms synchronises those events and returns the device time of the LAST run's pyramid, fused-stack and
  * emit stages in milliseconds. */
 int silent_plan_enable_timing(silent_plan *plan, int enable);
 int silent_plan_stage_ms(silent_plan *plan, float *pyramid_ms, float *stack_ms, float *emit_ms);
-/* the fused stack's two kernels separately: x -> channel sum (stack_a) and channel sum -> outputs (stack_b) */
+/* the fused stack's two kernels separately: x -> channel sum (stack_a) and channel sum -> outputs (stack_b, or
+ * stack_bank_kernel on the bank entries) */
 int silent_plan_stack_split_ms(silent_plan *plan, float *stack_a_ms, float *stack_b_ms);
 
 /* Same, with HOST buffers on both sides: the drop-in for LineEndDisplayer.callback (recognition_testing.py:136-144):

@@ -24,7 +24,7 @@ SYMBOLS = (
     "silent_plan_level_tables", "silent_plan_algorithmic_bytes", "silent_pyramid_build", "silent_conv2d",
     "silent_regulate", "silent_pad_inwards", "silent_value_from_color", "silent_selection_workspace_bytes",
     "silent_max_value_indices_region", "silent_top_value_points", "silent_stack_workspace_bytes", "silent_stack_fused", "silent_pipeline_run",
-    "silent_pipeline_run_host", "silent_pipeline_run_bank", "silent_get_centroids", "silent_resize_nearest", "silent_get_boosting", "silent_pointwise", "silent_display_tensors", "silent_pack_points",
+    "silent_pipeline_run_host", "silent_pipeline_run_bank", "silent_pipeline_run_orientations", "silent_stack_bank", "silent_get_centroids", "silent_resize_nearest", "silent_get_boosting", "silent_pointwise", "silent_display_tensors", "silent_pack_points",
     "silent_comm_unique_id", "silent_comm_create", "silent_comm_destroy", "silent_comm_check", "silent_gather_points",
 )
 
@@ -47,6 +47,19 @@ class SilentBankWeights(ctypes.Structure):
                 ("blur", ctypes.c_float * (49 * 64)), ("end", ctypes.c_float * (9 * 64)),
                 ("regulation_value", ctypes.c_float), ("regulation_root", ctypes.c_float), ("clip_max", ctypes.c_float),
                 ("border", ctypes.c_int32)]
+
+
+BANK_MAX = 16                  # SILENT_BANK_MAX
+FUSED_BANK_WIDTHS = (4, 8, 12, 16)   # orientation counts with fused kernels (silent_pipeline_run_orientations)
+
+
+class SilentOrientationBank(ctypes.Structure):
+    """silent_orientation_bank: a bank of ``orientations`` = 4, 8, 12 or 16; each filter packed densely at the front of
+    an array sized for ``BANK_MAX``."""
+    _fields_ = [("orientations", ctypes.c_int32), ("rgc", ctypes.c_float * 81), ("rgby", ctypes.c_float * 81),
+                ("stripe", ctypes.c_float * (9 * 3 * BANK_MAX)), ("blur", ctypes.c_float * (49 * BANK_MAX * BANK_MAX)),
+                ("end", ctypes.c_float * (9 * BANK_MAX * BANK_MAX)), ("regulation_value", ctypes.c_float),
+                ("regulation_root", ctypes.c_float), ("clip_max", ctypes.c_float), ("border", ctypes.c_int32)]
 
 
 _lib = None
@@ -93,6 +106,8 @@ def lib():
         "silent_pipeline_run": (i, [p, ctypes.POINTER(SilentStackWeights), p, i, p, p, p, p, i64, p, p]),
         "silent_pipeline_run_host": (i, [p, ctypes.POINTER(SilentStackWeights), p, i, p, p, p, i64, p, p]),
         "silent_pipeline_run_bank": (i, [p, ctypes.POINTER(SilentBankWeights), p, i, p, p, p, i64, p, p]),
+        "silent_pipeline_run_orientations": (i, [p, ctypes.POINTER(SilentOrientationBank), p, i, p, p, p, i64, p, p]),
+        "silent_stack_bank": (i, [p, i, i, i, ctypes.POINTER(SilentOrientationBank), p, p, p, p, sz, p]),
         "silent_get_centroids": (i, [p, i, i, i, i, i, p, p, p, p]),
         "silent_resize_nearest": (i, [p, i, i, i, i, i, i, p, p]),
         "silent_get_boosting": (i, [p, p, i, i, i, f, f, i, p, p, p]),
@@ -143,6 +158,30 @@ def make_bank_weights(rgc, rgby, stripe, blur, end, regulation_value=1.0, regula
         a = np.ascontiguousarray(np.asarray(arr), dtype=np.float32)
         if a.shape != shape:
             raise ValueError("the fused orientation bank needs %s of shape %s, got %s" % (name, shape, a.shape))
+        ctypes.memmove(getattr(w, name), a.ctypes.data, a.nbytes)
+    w.regulation_value, w.regulation_root, w.clip_max, w.border = regulation_value, regulation_root, clip_max, border
+    return w
+
+
+def make_orientation_bank(rgc, rgby, stripe, blur, end, regulation_value=1.0, regulation_root=.1, clip_max=255.0,
+                          border=2):
+    """Pack an orientation bank (HWIO, any float dtype) into ``silent_orientation_bank``. The width n is the stripe
+    bank's output count; blur must be [7,7,n,n] and end [3,3,n,n]. Whether the library has fused kernels for n (4, 8, 12,
+    16) is checked by the library itself."""
+    arrays = {k: np.ascontiguousarray(np.asarray(a), dtype=np.float32)
+              for k, a in (("rgc", rgc), ("rgby", rgby), ("stripe", stripe), ("blur", blur), ("end", end))}
+    st = arrays["stripe"].shape
+    if len(st) != 4 or st[:3] != (3, 3, 3) or not 1 <= st[3] <= BANK_MAX:
+        raise ValueError("an orientation bank needs a stripe bank of shape (3, 3, 3, n) with 1 <= n <= %d, got %s"
+                         % (BANK_MAX, st))
+    n = st[3]
+    w = SilentOrientationBank()
+    w.orientations = n
+    for name, shape in (("rgc", (3, 3, 3, 3)), ("rgby", (3, 3, 3, 3)), ("stripe", (3, 3, 3, n)), ("blur", (7, 7, n, n)),
+                        ("end", (3, 3, n, n))):
+        a = arrays[name]
+        if a.shape != shape:
+            raise ValueError("a %d-orientation bank needs %s of shape %s, got %s" % (n, name, shape, a.shape))
         ctypes.memmove(getattr(w, name), a.ctypes.data, a.nbytes)
     w.regulation_value, w.regulation_root, w.clip_max, w.border = regulation_value, regulation_root, clip_max, border
     return w

@@ -251,3 +251,23 @@ def stack_fused(pyramid, weights, want_orient=True, want_line_end=True, want_gra
         _lib.check(_lib.lib().silent_stack_fused(ptr(x), n, h, w, ctypes.byref(weights), ptr(orient), ptr(line_end),
                                                  ptr(gray), ptr(ws), nbytes, stream_ptr()), "silent_stack_fused")
     return orient, line_end, gray
+
+
+def stack_bank(pyramid, bank, want_orient=True, want_line_end=True, want_gray=True):
+    """The orientation bank's stack (``silent_stack_bank``) on a finite NHWC pyramid ``[n, h, w, 3]``: returns orient and
+    padded_line_end ``[n, h, w, bank.orientations]`` and gray ``[n, h, w, 1]``."""
+    x = as_device_tensor(pyramid)
+    n, h, w, c = _nhwc(x, "stack_bank")
+    if c != 3:
+        raise ValueError("the fused orientation bank needs 3-channel pyramids")
+    nb = int(bank.orientations)
+    mk = lambda ch: torch.empty((n, h, w, ch), dtype=torch.float32, device=x.device)  # noqa: E731
+    orient = mk(nb) if want_orient else None
+    line_end = mk(nb) if want_line_end else None
+    gray = mk(1) if want_gray else None
+    nbytes = _lib.lib().silent_stack_workspace_bytes(n, h, w)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().silent_stack_bank(ptr(x), n, h, w, ctypes.byref(bank), ptr(orient), ptr(line_end),
+                                                ptr(gray), ptr(ws), nbytes, stream_ptr()), "silent_stack_bank")
+    return orient, line_end, gray

@@ -3,6 +3,7 @@
 // LineEndDisplayer.callback (reference recognition_testing.py:136-144) with host buffers on both sides.
 #include <algorithm>
 #include <cstring>
+#include <memory>
 
 #include <nvtx3/nvToolsExt.h>
 
@@ -232,15 +233,17 @@ int silent_pipeline_run(silent_plan *plan, const silent_stack_weights *weights_h
     return rc;
 }
 
-int silent_pipeline_run_bank(silent_plan *plan, const silent_bank_weights *weights_host, const void *frames_dev, int batch,
-                             float *orient_dev, float *line_end_dev, int64_t *points_dev, int64_t capacity,
-                             int64_t *count_dev, silent_stream stream)
+int silent_pipeline_run_orientations(silent_plan *plan, const silent_orientation_bank *bank_host, const void *frames_dev,
+                                     int batch, float *orient_dev, float *line_end_dev, int64_t *points_dev,
+                                     int64_t capacity, int64_t *count_dev, silent_stream stream)
 {
-    if (!plan || !weights_host || !frames_dev) return fail(SILENT_E_INVAL, "silent_pipeline_run_bank: null argument");
+    int rc = check_bank(bank_host, "silent_pipeline_run_orientations");
+    if (rc != SILENT_OK) return rc;
+    if (!plan || !frames_dev) return fail(SILENT_E_INVAL, "silent_pipeline_run_orientations: null argument");
     if (batch <= 0) return fail(SILENT_E_INVAL, "batch must be positive");
     if (plan->levels == 0) return fail(SILENT_E_SHAPE, "frame is not larger than the pyramid centre: 0 levels");
     if (!pyramid_pair_supported(plan))
-        return fail(SILENT_E_SHAPE, "silent_pipeline_run_bank needs uint8 frames with 3 colours (frame-pair pyramid path)");
+        return fail(SILENT_E_SHAPE, "the fused orientation bank needs uint8 frames with 3 colours (frame-pair pyramid path)");
     if ((plan->h % 2) || (plan->w % 2))
         return fail(SILENT_E_SHAPE, "Ambiguous dimension: region shape (h/2, w/2) must be integral (h=%d, w=%d)", plan->h,
                     plan->w);
@@ -250,21 +253,37 @@ int silent_pipeline_run_bank(silent_plan *plan, const silent_bank_weights *weigh
     cudaStream_t s = (cudaStream_t)stream;
     const int n = batch * plan->levels;
     if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[0], s));
-    int rc = pyramid_pair_build(plan, frames_dev, batch, ws.d_pyramid, s);
+    rc = pyramid_pair_build(plan, frames_dev, batch, ws.d_pyramid, s);
     if (rc != SILENT_OK) return rc;
     if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[1], s));
-    rc = stack_bank(ws.d_pyramid, n, plan->h, plan->w, plan->levels, weights_host, orient_dev, line_end_dev, ws.d_gray,
-                    ws.d_stack, ws.stack_bytes, s);
+    rc = stack_bank(ws.d_pyramid, n, plan->h, plan->w, plan->levels, bank_host, orient_dev, line_end_dev, ws.d_gray,
+                    ws.d_stack, ws.stack_bytes, s, plan->timing ? plan->ev_mid : nullptr);
     if (rc != SILENT_OK) return rc;
-    if (plan->timing) {
-        SILENT_CUDA(cudaEventRecord(plan->ev_mid, s));
-        SILENT_CUDA(cudaEventRecord(plan->ev[2], s));
-    }
+    if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[2], s));
     if (count_dev)
         rc = max_value_indices_region(ws.d_gray, n, plan->h, plan->w, plan->h / 2, plan->w / 2, points_dev, capacity,
                                       count_dev, ws.d_select, ws.select_bytes, nullptr, nullptr, s);
     if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[3], s));
     return rc;
+}
+
+int silent_pipeline_run_bank(silent_plan *plan, const silent_bank_weights *weights_host, const void *frames_dev, int batch,
+                             float *orient_dev, float *line_end_dev, int64_t *points_dev, int64_t capacity,
+                             int64_t *count_dev, silent_stream stream)
+{
+    if (!weights_host) return fail(SILENT_E_INVAL, "silent_pipeline_run_bank: null argument");
+    std::unique_ptr<silent_orientation_bank> bank(new silent_orientation_bank());
+    const silent_bank_weights &W = *weights_host;
+    bank->orientations = SILENT_BANK;
+    std::memcpy(bank->rgc, W.rgc, sizeof(W.rgc));
+    std::memcpy(bank->rgby, W.rgby, sizeof(W.rgby));
+    std::memcpy(bank->stripe, W.stripe, sizeof(W.stripe));
+    std::memcpy(bank->blur, W.blur, sizeof(W.blur));
+    std::memcpy(bank->end, W.end, sizeof(W.end));
+    bank->regulation_value = W.regulation_value, bank->regulation_root = W.regulation_root, bank->clip_max = W.clip_max;
+    bank->border = W.border;
+    return silent_pipeline_run_orientations(plan, bank.get(), frames_dev, batch, orient_dev, line_end_dev, points_dev,
+                                            capacity, count_dev, stream);
 }
 
 int silent_plan_enable_timing(silent_plan *plan, int enable)

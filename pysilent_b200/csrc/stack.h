@@ -28,9 +28,14 @@ struct TileMaxima {
     int tile_h = 0, tile_w = 0, nty = 0, ntx = 0;
 };
 
-// orientation bank (config C4): xpair (pyramid_pair_kernel layout) -> orient / line_end [n,h,w,8], gray [n,h,w]
-int stack_bank(const void *xpair, int n, int h, int w, int pair_levels, const silent_bank_weights *W, float *orient,
-               float *line_end, float *gray, void *workspace, size_t workspace_bytes, cudaStream_t stream);
+// orientation bank of W->orientations = 4, 8, 12 or 16 (config C4: 8): pyr -> orient / line_end [n,h,w,nb], gray [n,h,w].
+// pyr as in stack_fused: NHWC [n][h][w][3] when pair_levels == 0, else the pyramid_pair_kernel layout. between_kernels
+// (optional) is recorded between stack_a and stack_bank_kernel. The caller has passed W through check_bank.
+int stack_bank(const void *pyr, int n, int h, int w, int pair_levels, const silent_orientation_bank *W, float *orient,
+               float *line_end, float *gray, void *workspace, size_t workspace_bytes, cudaStream_t stream,
+               cudaEvent_t between_kernels = nullptr);
+// width (SILENT_E_SHAPE) and structure (SILENT_E_STRUCTURE) checks of a bank; host only, no CUDA call
+int check_bank(const silent_orientation_bank *W, const char *who);
 
 // pyramid.cu
 int pyramid_build(const silent_plan *plan, const void *frames_dev, int batch, float *pyramid_dev, cudaStream_t stream);

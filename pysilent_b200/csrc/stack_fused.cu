@@ -1272,8 +1272,9 @@ stack_b_kernel(const f2 *__restrict__ bsum2, const __grid_constant__ ParamsB P, 
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// kernel BANK: stack_b for an orientation BANK (BASELINE config C4: 8 orientations through the reference's per-vector
-// generators, stripe_tensor.py:21-70 / oriented_end_detector.py:13-55 / gaussian_blur.py:13-54):
+// kernel BANK: stack_b for an orientation BANK of NB = 4, 8, 12 or 16 orientations (BASELINE config C4: 8 orientations)
+// through the reference's per-vector generators, stripe_tensor.py:21-70 / oriented_end_detector.py:13-55 /
+// gaussian_blur.py:13-54:
 //   bsum2 -> stripe bank 1 -> NB (identical over the rgby channels, so it runs on the channel sum like S3) -> regulator
 //   (one 7x7 blur of the NB-channel sum, all NB x NB slices identical) -> end bank, DEPTHWISE (orientation k only feeds
 //   orientation k) + relu + clip -> border mask -> mean. Outputs orient / padded_line_end [n, h, w, NB], gray [n, h, w].
@@ -1281,22 +1282,24 @@ stack_b_kernel(const f2 *__restrict__ bsum2, const __grid_constant__ ParamsB P, 
 // pitches, staged NHWC rows leaving through bulk stores, the quad-sum early-out of the blur) with runs of 4 pixels, so
 // that 4 orientations x 4 pixels of results fit in registers at a time. Chains run in the canonical (ky, kx) order of
 // the per-operator kernels: skipping the end bank's exact-zero cross-orientation weights is a no-op for finite data.
+// Orientations are handled in groups of 4 (one float4 per pixel in the NHWC restage, NB / 4 groups in S5), hence NB % 4 == 0.
 // ---------------------------------------------------------------------------------------------------------------------
 
-constexpr int kNB = 8;   // orientations of the bank
 constexpr int kRun = 4;  // pixels per run
 
+template <int NB>
 struct ParamsBank {
-    f2 w3[9][kNB];   // stripe [tap][orientation]
+    static_assert(NB % 4 == 0, "orientations are processed in groups of four");
+    f2 w3[9][NB];   // stripe [tap][orientation]
     f2 wb[49];       // blur
-    f2 w5[9][kNB];   // end, depthwise [tap][orientation]
+    f2 w5[9][NB];   // end, depthwise [tap][orientation]
     float reg_value, reg_root, clip_max, quick_thr;
     int border, h, w, n;
     unsigned long long pair_levels;   // pack_pair_levels()
     int tma_store;   // orient / line_end leave as TMA tile stores (StoreMaps valid)
 };
 
-template <int TH, int TW>
+template <int NB, int TH, int TW>
 struct TileBank {
     static constexpr int C_RUNS = (TW + 9 + kRun - 1) / kRun;   // stripe runs start at column -5 (need -4 .. TW + 3)
     static constexpr int D_RUNS = (TW + 2 + kRun - 1) / kRun;   // regulator runs start at column -1
@@ -1309,10 +1312,10 @@ struct TileBank {
                                                                                        : kRun * (E_RUNS - 1) + 6);   // -1
     static constexpr int Q_PITCH = C_RUNS | 1;                                     // one quad sum per stripe run
     static constexpr int B_PLANE = B_ROWS * B_PITCH, CS_PLANE = CS_ROWS * CS_PITCH, CD_PLANE = CD_ROWS * CD_PITCH;
-    static constexpr int ST_PITCH = TW * kNB + 4;                    // floats per staged NHWC row (odd multiple of 16 B)
+    static constexpr int ST_PITCH = TW * NB + 4;                    // floats per staged NHWC row (odd multiple of 16 B)
     static constexpr int STAGE_F2 = 2 * TH * ST_PITCH / 2;
     static constexpr int FRONT_F2 = B_PLANE + CS_PLANE > STAGE_F2 ? B_PLANE + CS_PLANE : STAGE_F2;
-    static constexpr size_t kSmemBytes = (size_t)(FRONT_F2 + kNB * CD_PLANE + CS_ROWS * Q_PITCH) * sizeof(f2) + 64;
+    static constexpr size_t kSmemBytes = (size_t)(FRONT_F2 + NB * CD_PLANE + CS_ROWS * Q_PITCH) * sizeof(f2) + 64;
     static_assert(TW % kRun == 0 && TW % 4 == 0, "tile width must be a multiple of the run length");
 };
 
@@ -1323,18 +1326,22 @@ __device__ __forceinline__ void store_cols4(f2 *__restrict__ dst, const f2 (&v)[
     p[1] = make_float4(v[2].x, v[2].y, v[3].x, v[3].y);
 }
 
-template <int TH, int TW, int NT>
-__global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict__ bsum2, const __grid_constant__ ParamsBank P,
+template <int NB, int TH, int TW, int NT>
+__global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict__ bsum2, const __grid_constant__ ParamsBank<NB> P,
                                                            const __grid_constant__ StoreMaps M, float *__restrict__ orient, float *__restrict__ line_end,
                                                            float *__restrict__ gray)
 {
-    using T = TileBank<TH, TW>;
+    using T = TileBank<NB, TH, TW>;
+    // loops over the orientations, unrolled whole up to 8 orientations. Wider banks walk them in chunks (4 orientations
+    // in S3 / S4, one group of 4 in the restage and S5) that are not unrolled into each other: unrolled whole, the
+    // compiler hoists every orientation's weights into registers and spills.
+    constexpr int kChunkO = NB <= 8 ? NB : 4, kChunkG = NB <= 8 ? NB / 4 : 1;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     pdl_enter();
     f2 *sB = reinterpret_cast<f2 *>(smem_raw);   // [B_ROWS][B_PITCH]      rgby channel sum, origin (-5, -6)
     f2 *sCs = sB + T::B_PLANE;                   // [CS_ROWS][CS_PITCH]    sum of the stripe bank, origin (-4, -5)
     f2 *sCD = sB + T::FRONT_F2;                  // [NB][CD_ROWS][CD_PITCH] stripe bank, regulated in place, origin (-1, -1)
-    f2 *sQ = sCD + kNB * T::CD_PLANE;            // [CS_ROWS][Q_PITCH]     quad sums of sCs
+    f2 *sQ = sCD + NB * T::CD_PLANE;            // [CS_ROWS][Q_PITCH]     quad sums of sCs
     float *sStage = reinterpret_cast<float *>(sB);   // [2][TH][ST_PITCH] NHWC staging, valid after the S4 barrier
 
     const int tid = threadIdx.x;
@@ -1369,8 +1376,10 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
 #pragma unroll
         for (int p = 0; p < kRun; ++p) cs[p] = zero2();
         const int rd = r - 3;   // row in the CD planes
+#pragma unroll 1
+        for (int o0 = 0; o0 < NB; o0 += kChunkO)
 #pragma unroll
-        for (int o = 0; o < kNB; ++o) {
+        for (int o = o0; o < o0 + kChunkO; ++o) {
             f2 acc[kRun];
 #pragma unroll
             for (int p = 0; p < kRun; ++p) acc[p] = zero2();
@@ -1430,8 +1439,10 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
             for (int p = 0; p < kRun; ++p)
                 gain[p] = make_float2(slow_gain(m[p].x, P.reg_value, P.reg_root), slow_gain(m[p].y, P.reg_value, P.reg_root));
         }
+#pragma unroll 1
+        for (int o0 = 0; o0 < NB; o0 += kChunkO)
 #pragma unroll
-        for (int o = 0; o < kNB; ++o) {
+        for (int o = o0; o < o0 + kChunkO; ++o) {
             f2 *cd = sCD + o * T::CD_PLANE + r * T::CD_PITCH + kRun * j;
             f2 c[4];
             load_cols<2>(cd, c);
@@ -1453,15 +1464,17 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
     if (orient) {
         for (int t = tid; t < TH * T::E_RUNS; t += NT) {
             const int r = t % TH, k = t / TH;
+#pragma unroll 1
+            for (int g0 = 0; g0 < NB / 4; g0 += kChunkG)
 #pragma unroll
-            for (int g = 0; g < kNB / 4; ++g) {
+            for (int g = g0; g < g0 + kChunkG; ++g) {
                 f2 d[4][6];
 #pragma unroll
                 for (int oo = 0; oo < 4; ++oo) load_cols<3>(sCD + (4 * g + oo) * T::CD_PLANE + (r + 1) * T::CD_PITCH + kRun * k, d[oo]);
 #pragma unroll
                 for (int p = 0; p < kRun; ++p) {
-                    float *a = sStage + (size_t)r * T::ST_PITCH + (kRun * k + p) * kNB + 4 * g;
-                    float *b = sStage + (size_t)(TH + r) * T::ST_PITCH + (kRun * k + p) * kNB + 4 * g;
+                    float *a = sStage + (size_t)r * T::ST_PITCH + (kRun * k + p) * NB + 4 * g;
+                    float *b = sStage + (size_t)(TH + r) * T::ST_PITCH + (kRun * k + p) * NB + 4 * g;
                     *reinterpret_cast<float4 *>(a) = make_float4(d[0][p + 1].x, d[1][p + 1].x, d[2][p + 1].x, d[3][p + 1].x);
                     *reinterpret_cast<float4 *>(b) = make_float4(d[0][p + 1].y, d[1][p + 1].y, d[2][p + 1].y, d[3][p + 1].y);
                 }
@@ -1476,13 +1489,13 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
                 issued = true;
             }
         } else if (bulk_ok) {
-            issued = bulk_rows<TH>(sStage, T::ST_PITCH, orient, img0, img1, has_b, ty0, h, (size_t)w * kNB, (size_t)tx0 * kNB,
-                                   (uint32_t)(min(TW, w - tx0) * kNB), warp_u, 0, NT / 32, leader);
+            issued = bulk_rows<TH>(sStage, T::ST_PITCH, orient, img0, img1, has_b, ty0, h, (size_t)w * NB, (size_t)tx0 * NB,
+                                   (uint32_t)(min(TW, w - tx0) * NB), warp_u, 0, NT / 32, leader);
         } else {
-            for (int i = tid; i < 2 * TH * TW * kNB; i += NT) {
-                const int e = i % (TW * kNB), row = i / (TW * kNB), lane = row / TH, gy = ty0 + row % TH;
-                if (gy < h && tx0 + e / kNB < w && (lane == 0 || has_b))
-                    orient[(((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * kNB + e] = sStage[(size_t)row * T::ST_PITCH + e];
+            for (int i = tid; i < 2 * TH * TW * NB; i += NT) {
+                const int e = i % (TW * NB), row = i / (TW * NB), lane = row / TH, gy = ty0 + row % TH;
+                if (gy < h && tx0 + e / NB < w && (lane == 0 || has_b))
+                    orient[(((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * NB + e] = sStage[(size_t)row * T::ST_PITCH + e];
             }
         }
         if (issued) bulk_wait_read();
@@ -1490,14 +1503,16 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
     }
 
     // ---- S5-S7: depthwise end bank + relu + clip, border mask, mean over the orientations --------------------------------
-    const float inv_nb = __fdiv_rn(1.0f, (float)kNB);
+    const float inv_nb = __fdiv_rn(1.0f, (float)NB);
     for (int t = tid; t < TH * T::E_RUNS; t += NT) {
         const int r = t % TH, k = t / TH;
         const int gy = ty0 + r, gx0 = tx0 + kRun * k;
         const bool row_in = gy >= P.border && gy < h - P.border;
         f2 g[kRun];
+#pragma unroll 1
+        for (int gq0 = 0; gq0 < NB / 4; gq0 += kChunkG)
 #pragma unroll
-        for (int gq = 0; gq < kNB / 4; ++gq) {
+        for (int gq = gq0; gq < gq0 + kChunkG; ++gq) {
             f2 e[4][kRun];
 #pragma unroll
             for (int oo = 0; oo < 4; ++oo) {
@@ -1525,8 +1540,8 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
             }
 #pragma unroll
             for (int p = 0; p < kRun; ++p) {
-                float *a = sStage + (size_t)r * T::ST_PITCH + (kRun * k + p) * kNB + 4 * gq;
-                float *b = sStage + (size_t)(TH + r) * T::ST_PITCH + (kRun * k + p) * kNB + 4 * gq;
+                float *a = sStage + (size_t)r * T::ST_PITCH + (kRun * k + p) * NB + 4 * gq;
+                float *b = sStage + (size_t)(TH + r) * T::ST_PITCH + (kRun * k + p) * NB + 4 * gq;
                 *reinterpret_cast<float4 *>(a) = make_float4(e[0][p].x, e[1][p].x, e[2][p].x, e[3][p].x);
                 *reinterpret_cast<float4 *>(b) = make_float4(e[0][p].y, e[1][p].y, e[2][p].y, e[3][p].y);
             }
@@ -1559,13 +1574,13 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
                 issued = true;
             }
         } else if (bulk_ok) {
-            issued = bulk_rows<TH>(sStage, T::ST_PITCH, line_end, img0, img1, has_b, ty0, h, (size_t)w * kNB, (size_t)tx0 * kNB,
-                                   (uint32_t)(min(TW, w - tx0) * kNB), warp_u, 0, NT / 32, leader);
+            issued = bulk_rows<TH>(sStage, T::ST_PITCH, line_end, img0, img1, has_b, ty0, h, (size_t)w * NB, (size_t)tx0 * NB,
+                                   (uint32_t)(min(TW, w - tx0) * NB), warp_u, 0, NT / 32, leader);
         } else {
-            for (int i = tid; i < 2 * TH * TW * kNB; i += NT) {
-                const int e = i % (TW * kNB), row = i / (TW * kNB), lane = row / TH, gy = ty0 + row % TH;
-                if (gy < h && tx0 + e / kNB < w && (lane == 0 || has_b))
-                    line_end[(((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * kNB + e] = sStage[(size_t)row * T::ST_PITCH + e];
+            for (int i = tid; i < 2 * TH * TW * NB; i += NT) {
+                const int e = i % (TW * NB), row = i / (TW * NB), lane = row / TH, gy = ty0 + row % TH;
+                if (gy < h && tx0 + e / NB < w && (lane == 0 || has_b))
+                    line_end[(((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * NB + e] = sStage[(size_t)row * T::ST_PITCH + e];
             }
         }
     }
@@ -1980,43 +1995,62 @@ int stack_fused(const void *pyr, int n, int h, int w, int pair_levels, const sil
 }
 
 
-// ---- orientation bank (config C4): S1-S2 through stack_a, then stack_bank_kernel ------------------------------------------
-constexpr int kBankTH = 16, kBankTW = 32;
+// ---- orientation banks (config C4 and its 4-, 12- and 16-wide variants): S1-S2 through stack_a, then stack_bank_kernel ---
 
-int stack_bank(const void *xpair, int n, int h, int w, int pair_levels, const silent_bank_weights *W, float *orient,
-               float *line_end, float *gray, void *workspace, size_t workspace_bytes, cudaStream_t stream)
+// Tile per width, 16 rows x 32 columns up to 8 orientations, 16 x 16 beyond: wider banks on 32 columns fit one CTA per SM
+// (115 / 152 KB of shared memory) and, at NB = 16, a tile row outgrows the 256-element TMA store box; on 16 columns
+// they run 2 CTAs/SM with tile stores, 15 % (NB = 12) and 18 % (NB = 16) faster on C4 frames (DESIGN §4).
+template <int NB>
+struct BankTile {
+    static constexpr int TH = 16;
+    static constexpr int TW = NB <= 8 ? 32 : 16;
+    using T = TileBank<NB, TH, TW>;
+    static constexpr int NT = (T::CS_ROWS * T::C_RUNS + 31) / 32 * 32;   // one warp-rounded round of S3
+};
+
+static bool bank_width_supported(int nb) { return nb == 4 || nb == 8 || nb == 12 || nb == 16; }
+
+int check_bank(const silent_orientation_bank *W, const char *who)
 {
-    if (!xpair || !W) return fail(SILENT_E_INVAL, "silent_pipeline_run_bank: null argument");
-    if (pair_levels <= 0 || n % pair_levels != 0) return fail(SILENT_E_INVAL, "bank stack: n must be whole frames");
-    const int pairs = ((n / pair_levels + 1) / 2) * pair_levels;
-    if (pairs > 65535) return fail(SILENT_E_SHAPE, "bank stack: at most 65535 image pairs per call");
-    if (!workspace || workspace_bytes < stack_workspace_bytes(n, h, w))
-        return fail(SILENT_E_CAPACITY, "bank stack: workspace too small");
-    // structure the kernel relies on (what the reference's per-vector generators produce, SURVEY 8(d) config C4)
-    for (int t = 0; t < 9; ++t)
-        for (int o = 0; o < kNB; ++o) {
-            for (int ci = 1; ci < 3; ++ci)
-                if (!bits_equal(W->stripe[(t * 3 + ci) * kNB + o], W->stripe[(t * 3) * kNB + o]))
-                    return fail(SILENT_E_STRUCTURE, "stripe bank differs across input channels at tap %d", t);
-            for (int ci = 0; ci < kNB; ++ci)
-                if (ci != o && W->end[(t * kNB + ci) * kNB + o] != 0.0f)
+    if (!W) return fail(SILENT_E_INVAL, "%s: null bank", who);
+    const int nb = W->orientations;
+    if (!bank_width_supported(nb))
+        return fail(SILENT_E_SHAPE, "%s: %d orientations; the fused bank supports 4, 8, 12 or 16", who, nb);
+    // structure the kernel relies on (what the reference's per-vector generators produce, SURVEY 8(d) config C4); runs
+    // on every call, so the bitwise comparisons go by memcmp over contiguous runs
+    for (int t = 0; t < 9; ++t) {
+        const float *s0 = W->stripe + t * 3 * nb;
+        if (std::memcmp(s0 + nb, s0, nb * sizeof(float)) != 0 || std::memcmp(s0 + 2 * nb, s0, nb * sizeof(float)) != 0)
+            return fail(SILENT_E_STRUCTURE, "stripe bank differs across input channels at tap %d", t);
+        for (int ci = 0; ci < nb; ++ci)
+            for (int o = 0; o < nb; ++o)
+                if (ci != o && W->end[(t * nb + ci) * nb + o] != 0.0f)
                     return fail(SILENT_E_STRUCTURE, "end bank couples orientations %d -> %d (needs a depthwise bank)", ci, o);
-        }
-    ParamsBank B;
+    }
+    for (int t = 0; t < 49; ++t) {   // all nb * nb slices equal <=> every element equals its successor
+        const float *b = W->blur + t * nb * nb;
+        if (std::memcmp(b + 1, b, (nb * nb - 1) * sizeof(float)) != 0)
+            return fail(SILENT_E_STRUCTURE, "blur bank slices differ at tap %d", t);
+    }
+    return SILENT_OK;
+}
+
+template <int NB>
+static int launch_bank(const silent_orientation_bank *W, int n, int h, int w, int levels, int pairs, const f2 *bsum2,
+                       float *orient, float *line_end, float *gray, cudaStream_t stream)
+{
+    ParamsBank<NB> B;
     float blur_min = INFINITY;
     for (int t = 0; t < 49; ++t) {
-        for (int sl = 0; sl < kNB * kNB; ++sl)
-            if (!bits_equal(W->blur[t * kNB * kNB + sl], W->blur[t * kNB * kNB]))
-                return fail(SILENT_E_STRUCTURE, "blur bank slices differ at tap %d", t);
-        const float b = W->blur[t * kNB * kNB];
+        const float b = W->blur[t * NB * NB];
         B.wb[t] = dup(b);
         blur_min = b < blur_min ? b : blur_min;
         if (!(b > 0.0f) || std::isinf(b)) blur_min = -1.0f;
     }
     for (int t = 0; t < 9; ++t)
-        for (int o = 0; o < kNB; ++o) {
-            B.w3[t][o] = dup(W->stripe[(t * 3) * kNB + o]);
-            B.w5[t][o] = dup(W->end[(t * kNB + o) * kNB + o]);
+        for (int o = 0; o < NB; ++o) {
+            B.w3[t][o] = dup(W->stripe[(t * 3) * NB + o]);
+            B.w5[t][o] = dup(W->end[(t * NB + o) * NB + o]);
         }
     B.quick_thr = 0.0f;
     if (blur_min > 0.0f && blur_min < INFINITY) {
@@ -2025,9 +2059,42 @@ int stack_bank(const void *xpair, int n, int h, int w, int pair_levels, const si
         if ((double)blur_min * (double)T >= 1.0001 && T < 1.0e20f) B.quick_thr = T;
     }
     B.reg_value = W->regulation_value, B.reg_root = W->regulation_root, B.clip_max = W->clip_max, B.border = W->border;
-    B.h = h, B.w = w, B.n = n, B.pair_levels = pack_pair_levels(pair_levels);
+    B.h = h, B.w = w, B.n = n, B.pair_levels = pack_pair_levels(levels);
 
-    // S1 + S2 -> channel sum, exactly as in the three-orientation pipeline
+    using Tile = BankTile<NB>;
+    using T = typename Tile::T;
+    auto kern = stack_bank_kernel<NB, Tile::TH, Tile::TW, Tile::NT>;
+    SILENT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::kSmemBytes));
+    const dim3 grid(ceil_div(w, Tile::TW), ceil_div(h, Tile::TH), pairs);
+    StoreMaps maps;   // tile rows of up to 388 floats: described in 8-byte elements (a box holds at most 256 of them)
+    std::memset(&maps, 0, sizeof(maps));
+    const int pad = T::ST_PITCH - NB * Tile::TW;
+    B.tma_store = (!orient || make_tile_store_map(&maps.orient, orient, n, h, w, NB, Tile::TW, pad, kTileStoreRows, 2)) &&
+                  (!line_end || make_tile_store_map(&maps.line_end, line_end, n, h, w, NB, Tile::TW, pad, kTileStoreRows, 2));
+    if (const char *e = std::getenv("SILENT_B_TILE_STORE")) B.tma_store = B.tma_store && std::atoi(e) != 0;   // tuning knob
+    SILENT_CUDA(launch_dependent(kern, grid, dim3(Tile::NT), T::kSmemBytes, stream, bsum2, B, maps, orient, line_end, gray));
+    SILENT_LAUNCH_CHECK("stack_bank_kernel");
+    return SILENT_OK;
+}
+
+int stack_bank(const void *pyr, int n, int h, int w, int pair_levels, const silent_orientation_bank *W, float *orient,
+               float *line_end, float *gray, void *workspace, size_t workspace_bytes, cudaStream_t stream,
+               cudaEvent_t between_kernels)
+{
+    if (!pyr || !W) return fail(SILENT_E_INVAL, "bank stack: null argument");
+    if (n <= 0 || h <= 0 || w <= 0) return fail(SILENT_E_INVAL, "bank stack: bad shape %dx%dx%d", n, h, w);
+    const bool paired_in = pair_levels > 0;
+    const int levels = paired_in ? pair_levels : 1;
+    if (n % levels != 0) return fail(SILENT_E_INVAL, "bank stack: n must be whole frames");
+    const int pairs = ((n / levels + 1) / 2) * levels;
+    if (pairs > 65535) return fail(SILENT_E_SHAPE, "bank stack: at most 65535 image pairs per call");
+    if (!workspace || workspace_bytes < stack_workspace_bytes(n, h, w))
+        return fail(SILENT_E_CAPACITY, "bank stack: workspace too small (%zu < %zu bytes)", workspace_bytes,
+                    stack_workspace_bytes(n, h, w));
+    for (const void *p : {(const void *)pyr, (const void *)orient, (const void *)line_end, (const void *)gray})
+        if (((uintptr_t)p & 15) != 0) return fail(SILENT_E_INVAL, "bank stack: tensors must be 16-byte aligned");
+
+    // S1 + S2 -> channel sum, exactly as in the three-orientation stack
     silent_stack_weights tmp;
     std::memset(&tmp, 0, sizeof(tmp));
     std::memcpy(tmp.rgc, W->rgc, sizeof(tmp.rgc));
@@ -2037,26 +2104,20 @@ int stack_bank(const void *xpair, int n, int h, int w, int pair_levels, const si
     StackPlanHost S;
     int rc = pack_stack_params(&tmp, n, h, w, &S);
     if (rc != SILENT_OK) return rc;
-    S.a.pair_levels = pack_pair_levels(pair_levels);
+    S.a.pair_levels = pack_pair_levels(levels);
     f2 *bsum2 = reinterpret_cast<f2 *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    rc = pick_tile_w(w) == 48 ? launch_stack_a<48>(xpair, S, true, pairs, bsum2, stream)
-                              : launch_stack_a<64>(xpair, S, true, pairs, bsum2, stream);
+    rc = pick_tile_w(w) == 48 ? launch_stack_a<48>(pyr, S, paired_in, pairs, bsum2, stream)
+                              : launch_stack_a<64>(pyr, S, paired_in, pairs, bsum2, stream);
     if (rc != SILENT_OK) return rc;
-
-    using T = TileBank<kBankTH, kBankTW>;
-    constexpr int NT = (T::CS_ROWS * T::C_RUNS + 31) / 32 * 32;
-    auto kern = stack_bank_kernel<kBankTH, kBankTW, NT>;
-    SILENT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::kSmemBytes));
-    const dim3 grid(ceil_div(w, kBankTW), ceil_div(h, kBankTH), pairs);
-    StoreMaps maps;   // tile rows are 256 floats: described in 8-byte elements (a box holds at most 256 of them)
-    std::memset(&maps, 0, sizeof(maps));
-    B.tma_store = (!orient || make_tile_store_map(&maps.orient, orient, n, h, w, kNB, kBankTW, T::ST_PITCH - kNB * kBankTW, kTileStoreRows, 2)) &&
-                  (!line_end || make_tile_store_map(&maps.line_end, line_end, n, h, w, kNB, kBankTW, T::ST_PITCH - kNB * kBankTW, kTileStoreRows, 2));
-    if (const char *e = std::getenv("SILENT_B_TILE_STORE")) B.tma_store = B.tma_store && std::atoi(e) != 0;   // tuning knob
-    SILENT_CUDA(launch_dependent(kern, grid, dim3(NT), T::kSmemBytes, stream, (const f2 *)bsum2, B, maps, orient, line_end, gray));
-    SILENT_LAUNCH_CHECK("stack_bank_kernel");
-    return SILENT_OK;
+    if (between_kernels) SILENT_CUDA(cudaEventRecord(between_kernels, stream));   // stage timing hook
+    switch (W->orientations) {
+    case 4: return launch_bank<4>(W, n, h, w, levels, pairs, bsum2, orient, line_end, gray, stream);
+    case 8: return launch_bank<8>(W, n, h, w, levels, pairs, bsum2, orient, line_end, gray, stream);
+    case 12: return launch_bank<12>(W, n, h, w, levels, pairs, bsum2, orient, line_end, gray, stream);
+    default: return launch_bank<16>(W, n, h, w, levels, pairs, bsum2, orient, line_end, gray, stream);
+    }
 }
+
 }  // namespace silent
 
 extern "C" {
@@ -2073,6 +2134,16 @@ int silent_stack_fused(const float *pyramid_dev, int n, int h, int w, const sile
 {
     return silent::stack_fused(pyramid_dev, n, h, w, 0, weights_host, orient_dev, line_end_dev, gray_dev, workspace_dev,
                                workspace_bytes, nullptr, nullptr, nullptr, (cudaStream_t)stream, nullptr, false);
+}
+
+int silent_stack_bank(const float *pyramid_dev, int n, int h, int w, const silent_orientation_bank *bank_host,
+                      float *orient_dev, float *line_end_dev, float *gray_dev, void *workspace_dev, size_t workspace_bytes,
+                      silent_stream stream)
+{
+    const int rc = silent::check_bank(bank_host, "silent_stack_bank");
+    if (rc != SILENT_OK) return rc;
+    return silent::stack_bank(pyramid_dev, n, h, w, 0, bank_host, orient_dev, line_end_dev, gray_dev, workspace_dev,
+                              workspace_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -51,7 +51,9 @@ class LineEndPipeline:
 
     def __init__(self, n_dimensions=2, output_size=(288, 192), output_colors=3, zoom_ratio=math.e ** .5, device=None,
                  orientations=None):
-        self.orientations = orientations   # None: the reference's 3 simplex orientations (fused kernels); n: config C4
+        # None: the reference's 3 simplex orientations; n: a bank of n orientations (config C4: 8). Fused kernels for n = 4,
+        # 8, 12 and 16; other n up to 8 run operator by operator
+        self.orientations = orientations
         self._bank = None
         self._bank_weights = None
         self.output_size = tuple(output_size)
@@ -127,20 +129,44 @@ class LineEndPipeline:
             self._bank = orientation_bank_filters(self.orientations)
         return self._bank
 
+    def _bank_width(self):
+        """``orientations``, after rejecting the widths no path runs (before anything touches the GPU)."""
+        nb = int(self.orientations)
+        if nb > 16 or (nb > 8 and nb % 4):
+            raise ValueError("orientations=%d is not supported: a bank has up to 8 orientations, or 12 or 16 (fused "
+                             "kernels exist for 4, 8, 12 and 16)" % nb)
+        return nb
+
+    def orientation_bank(self):
+        """The bank's filters packed for the fused kernels (``silent_orientation_bank``)."""
+        if self._bank_weights is None:
+            f = self.bank_filters()
+            self._bank_weights = _lib.make_orientation_bank(f["rgc"], f["rgby"], f["stripe"], f["blur"], f["end"])
+        return self._bank_weights
+
     def run_bank(self, pyramid_tensor, want_points=True):
-        """Config C4: S1-S2 on 3 channels, S3-S7 on an ``orientations``-channel bank, through the per-operator kernels
-        (same composition as ``compile()``, ``recognition_testing.py:69-77``)."""
+        """Config C4: S1-S2 on 3 channels, S3-S7 on an ``orientations``-channel bank (same composition as ``compile()``,
+        ``recognition_testing.py:69-77``). Up to 8 orientations through the per-operator kernels; 12 and 16 through the
+        fused bank stack (``silent_stack_bank``), which needs a finite pyramid."""
         from .util.selection import pad_inwards, max_value_indices_region
         from .util.color import get_value_from_color
         from .util.regulator import regulate_tensor
-        f = self.bank_filters()
+        nb = self._bank_width()
         x = _ops.as_device_tensor(pyramid_tensor)
+        region = [1, self.region_shape[1], self.region_shape[2], nb]
+        if nb > 8:
+            if not bool((x.abs() <= _ops.FUSED_INPUT_MAX).all()):
+                raise ValueError("a pyramid with NaN, Inf or values beyond 1e30 goes operator by operator, which supports "
+                                 "at most 8 orientations (got %d)" % nb)
+            orient, padded, gray = _ops.stack_bank(x, self.orientation_bank())
+            points = max_value_indices_region(padded, region, gray) if want_points else None
+            return LineEndResult(orient, padded, gray, points)
+        f = self.bank_filters()
         x = _ops.conv2d(_ops.conv2d(x, f["rgc"], post=_lib.POST_RELU), f["rgby"], post=_lib.POST_RELU)
         orient = regulate_tensor(_ops.conv2d(x, f["stripe"], post=_lib.POST_RELU), f["blur"], 1.0, .1)
         line_end = _ops.conv2d(orient, f["end"], post=_lib.POST_RELU_CLIP, clip_max=255.0)
         padded = pad_inwards(line_end, [[0, 0], [2, 2], [2, 2], [0, 0]])
         gray = get_value_from_color(padded)
-        region = [1, self.region_shape[1], self.region_shape[2], self.orientations]
         points = max_value_indices_region(padded, region, gray) if want_points else None
         return LineEndResult(orient, padded, gray, points)
 
@@ -166,13 +192,14 @@ class LineEndPipeline:
         ``out`` may carry preallocated ``(orient, padded_line_end, points, count)`` tensors to avoid allocation in a
         steady-state loop; ``points`` then holds ``count`` valid rows (no host sync is performed in that case).
         """
+        nb = self._bank_width() if self.orientations is not None else None
         frames = frames if frames.dim() == 4 else frames.unsqueeze(0)
         frames = frames.contiguous()
-        if self.orientations is not None:   # config C4
-            if self.orientations == 8 and frames.dtype == torch.uint8 and frames.shape[3] >= 3 and self.blur_size == 7 \
-                    and self.output_colors == 3 and (frames.shape[2] * frames.shape[3]) % 16 == 0:
+        if nb is not None:   # config C4 and its variants
+            if nb in _lib.FUSED_BANK_WIDTHS and frames.dtype == torch.uint8 and frames.shape[3] >= 3 \
+                    and self.blur_size == 7 and self.output_colors == 3 and (frames.shape[2] * frames.shape[3]) % 16 == 0:
                 return self._run_frames_bank(frames, want_points, points_capacity)   # fused: 4 kernels + emit
-            from .util.zoom.from_image import image_to_zoom_tensor   # any other bank: operator by operator
+            from .util.zoom.from_image import image_to_zoom_tensor   # other frames: pyramid, then run_bank
             return self.run_bank(image_to_zoom_tensor(frames, self.output_colors, self.output_size, self.zoom_ratio),
                                  want_points)
         plan = self.plan_for(frames)
@@ -204,25 +231,23 @@ class LineEndPipeline:
         return LineEndResult(orient, line_end, None, points[:total])
 
     def _run_frames_bank(self, frames, want_points=True, points_capacity=None):
-        """Config C4 fused: pyramid_pair_kernel -> stack_a (rgc, rgby) -> stack_bank_kernel (8-orientation stripe bank,
-        regulator, depthwise end bank, mask, mean) -> emit, through ``silent_pipeline_run_bank``."""
+        """Config C4 fused: pyramid_pair_kernel -> stack_a (rgc, rgby) -> stack_bank_kernel (stripe bank, regulator,
+        depthwise end bank, mask, mean) -> emit, through ``silent_pipeline_run_orientations``."""
         plan = self.plan_for(frames)
         b = int(frames.shape[0])
         plan.reserve(b)
         n, dev = b * plan.levels, frames.device
-        if self._bank_weights is None:
-            f = self.bank_filters()
-            self._bank_weights = _lib.make_bank_weights(f["rgc"], f["rgby"], f["stripe"], f["blur"], f["end"])
-        orient = torch.empty((n, plan.h, plan.w, 8), dtype=torch.float32, device=dev)
+        bank = self.orientation_bank()
+        orient = torch.empty((n, plan.h, plan.w, bank.orientations), dtype=torch.float32, device=dev)
         line_end = torch.empty_like(orient)
         cap = int(points_capacity) if points_capacity else max(64 * n, 1024)
         points = torch.empty((cap, 4), dtype=torch.int64, device=dev)
         count = torch.zeros(1, dtype=torch.int64, device=dev)
         with torch.cuda.device(dev):
-            _lib.check(_lib.lib().silent_pipeline_run_bank(
-                plan.handle, ctypes.byref(self._bank_weights), _ops.ptr(frames), b, _ops.ptr(orient), _ops.ptr(line_end),
+            _lib.check(_lib.lib().silent_pipeline_run_orientations(
+                plan.handle, ctypes.byref(bank), _ops.ptr(frames), b, _ops.ptr(orient), _ops.ptr(line_end),
                 _ops.ptr(points), cap, _ops.ptr(count) if want_points else None, _ops.stream_ptr()),
-                "silent_pipeline_run_bank")
+                "silent_pipeline_run_orientations")
         if not want_points:
             return LineEndResult(orient, line_end, None, None)
         total = int(count.item())
@@ -232,13 +257,18 @@ class LineEndPipeline:
 
     # -- host buffers on both sides (LineEndDisplayer.callback) -----------------------------------------------------------
     def run_host(self, frames, orient_out=None, line_end_out=None, points_capacity=4096):
-        """frames: host numpy ``[B, H, W, 3]`` (ideally page-locked) -> host numpy results via the C-ABI host call."""
+        """frames: host numpy ``[B, H, W, 3]`` (ideally page-locked) -> host numpy results via the C-ABI host call (with
+        ``orientations`` set: through ``run_frames`` and page-locked buffers, results ``[B * L, h, w, orientations]``)."""
+        if self.orientations is not None:
+            self._bank_width()
         frames = np.ascontiguousarray(frames)
         if frames.ndim == 3:
             frames = frames[np.newaxis]
         if frames.dtype != np.uint8:
             frames = frames.astype(np.float32)
         dev = self._device()
+        if self.orientations is not None:
+            return self._run_host_bank(frames, dev, orient_out, line_end_out, points_capacity)
         tdtype = torch.uint8 if frames.dtype == np.uint8 else torch.float32
         plan = self._plan(frames.shape[1:], tdtype, dev)
         b = frames.shape[0]
@@ -259,6 +289,27 @@ class LineEndPipeline:
             # run_frames does -- feature points are never silently truncated
             return self.run_host(frames, orient_out, line_end_out, points_capacity=int(count.value))
         return LineEndResult(orient_out, line_end_out, None, points[:count.value])
+
+    def _run_host_bank(self, frames, dev, orient_out, line_end_out, points_capacity):
+        """run_host for a bank: the frames go up from a page-locked copy, and the results come back with asynchronous
+        copies into page-locked buffers and one synchronisation, as ``LineEndDisplayer.callback`` does."""
+        staged = torch.from_numpy(frames).pin_memory()
+        with torch.cuda.device(dev):
+            res = self.run_frames(staged.to(dev, non_blocking=True), points_capacity=points_capacity)
+            host = []
+            for t in (res.orient, res.padded_line_end, res.points):
+                h = torch.empty(tuple(t.shape), dtype=t.dtype).pin_memory()
+                h.copy_(t, non_blocking=True)
+                host.append(h)
+            torch.cuda.current_stream().synchronize()
+        orient, line_end, points = (h.numpy() for h in host)
+        if orient_out is not None:
+            orient_out[...] = orient
+            orient = orient_out
+        if line_end_out is not None:
+            line_end_out[...] = line_end
+            line_end = line_end_out
+        return LineEndResult(orient, line_end, None, points)
 
     def callback(self, frame, cam_id=None, depth=2):
         """Per-frame entry point with the reference's signature (``recognition_testing.py:136-144``).

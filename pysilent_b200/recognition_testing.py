@@ -90,6 +90,8 @@ class LineEndDisplayer(LineEndPipeline):
 
     def callback(self, frame, cam_id=None, depth=2):
         """``recognition_testing.py:136-144``: ``[frame] + [[tensors[x][y] for y in levels] for x in range(6)]``."""
+        if self.orientations is not None:
+            self._bank_width()
         z = np.asarray(frame)
         z = np.ascontiguousarray(z if z.dtype == np.uint8 else z.astype(np.float32))
         dev = self._device()
