@@ -137,30 +137,32 @@ def check(rc, what=""):
     return rc
 
 
-def make_stack_weights(rgc, rgby, stripe, blur, end, regulation_value=1.0, regulation_root=.1, clip_max=255.0, border=2):
-    """Pack HWIO filters (any float dtype) into the C struct, rounding to float32 like ``tf.constant(..., tf.float32)``."""
-    w = SilentStackWeights()
-    for name, arr, shape in (("rgc", rgc, (3, 3, 3, 3)), ("rgby", rgby, (3, 3, 3, 3)), ("stripe", stripe, (3, 3, 3, 3)),
-                             ("blur", blur, (7, 7, 3, 3)), ("end", end, (3, 3, 3, 3))):
+def _pack(w, who, filters, regulation_value, regulation_root, clip_max, border):
+    """Copy ``(name, array, shape)`` HWIO filters into the struct ``w``, rounded to float32 like ``tf.constant(...,
+    tf.float32)``; a filter of another shape raises ValueError ("<who> needs <name> of shape ...")."""
+    for name, arr, shape in filters:
         a = np.ascontiguousarray(np.asarray(arr), dtype=np.float32)
         if a.shape != shape:
-            raise ValueError("fused stack needs %s of shape %s, got %s" % (name, shape, a.shape))
+            raise ValueError("%s needs %s of shape %s, got %s" % (who, name, shape, a.shape))
         ctypes.memmove(getattr(w, name), a.ctypes.data, a.nbytes)
     w.regulation_value, w.regulation_root, w.clip_max, w.border = regulation_value, regulation_root, clip_max, border
     return w
+
+
+def make_stack_weights(rgc, rgby, stripe, blur, end, regulation_value=1.0, regulation_root=.1, clip_max=255.0, border=2):
+    """Pack HWIO filters (any float dtype) into the C struct, rounding to float32 like ``tf.constant(..., tf.float32)``."""
+    return _pack(SilentStackWeights(), "fused stack",
+                 (("rgc", rgc, (3, 3, 3, 3)), ("rgby", rgby, (3, 3, 3, 3)), ("stripe", stripe, (3, 3, 3, 3)),
+                  ("blur", blur, (7, 7, 3, 3)), ("end", end, (3, 3, 3, 3))),
+                 regulation_value, regulation_root, clip_max, border)
 
 
 def make_bank_weights(rgc, rgby, stripe, blur, end, regulation_value=1.0, regulation_root=.1, clip_max=255.0, border=2):
     """Pack the 8-orientation bank (HWIO, any float dtype) into ``silent_bank_weights``."""
-    w = SilentBankWeights()
-    for name, arr, shape in (("rgc", rgc, (3, 3, 3, 3)), ("rgby", rgby, (3, 3, 3, 3)), ("stripe", stripe, (3, 3, 3, 8)),
-                             ("blur", blur, (7, 7, 8, 8)), ("end", end, (3, 3, 8, 8))):
-        a = np.ascontiguousarray(np.asarray(arr), dtype=np.float32)
-        if a.shape != shape:
-            raise ValueError("the fused orientation bank needs %s of shape %s, got %s" % (name, shape, a.shape))
-        ctypes.memmove(getattr(w, name), a.ctypes.data, a.nbytes)
-    w.regulation_value, w.regulation_root, w.clip_max, w.border = regulation_value, regulation_root, clip_max, border
-    return w
+    return _pack(SilentBankWeights(), "the fused orientation bank",
+                 (("rgc", rgc, (3, 3, 3, 3)), ("rgby", rgby, (3, 3, 3, 3)), ("stripe", stripe, (3, 3, 3, 8)),
+                  ("blur", blur, (7, 7, 8, 8)), ("end", end, (3, 3, 8, 8))),
+                 regulation_value, regulation_root, clip_max, border)
 
 
 def make_orientation_bank(rgc, rgby, stripe, blur, end, regulation_value=1.0, regulation_root=.1, clip_max=255.0,
@@ -168,20 +170,14 @@ def make_orientation_bank(rgc, rgby, stripe, blur, end, regulation_value=1.0, re
     """Pack an orientation bank (HWIO, any float dtype) into ``silent_orientation_bank``. The width n is the stripe
     bank's output count; blur must be [7,7,n,n] and end [3,3,n,n]. Whether the library has fused kernels for n (4, 8, 12,
     16) is checked by the library itself."""
-    arrays = {k: np.ascontiguousarray(np.asarray(a), dtype=np.float32)
-              for k, a in (("rgc", rgc), ("rgby", rgby), ("stripe", stripe), ("blur", blur), ("end", end))}
-    st = arrays["stripe"].shape
+    st = np.asarray(stripe).shape
     if len(st) != 4 or st[:3] != (3, 3, 3) or not 1 <= st[3] <= BANK_MAX:
         raise ValueError("an orientation bank needs a stripe bank of shape (3, 3, 3, n) with 1 <= n <= %d, got %s"
                          % (BANK_MAX, st))
     n = st[3]
     w = SilentOrientationBank()
     w.orientations = n
-    for name, shape in (("rgc", (3, 3, 3, 3)), ("rgby", (3, 3, 3, 3)), ("stripe", (3, 3, 3, n)), ("blur", (7, 7, n, n)),
-                        ("end", (3, 3, n, n))):
-        a = arrays[name]
-        if a.shape != shape:
-            raise ValueError("a %d-orientation bank needs %s of shape %s, got %s" % (n, name, shape, a.shape))
-        ctypes.memmove(getattr(w, name), a.ctypes.data, a.nbytes)
-    w.regulation_value, w.regulation_root, w.clip_max, w.border = regulation_value, regulation_root, clip_max, border
-    return w
+    return _pack(w, "a %d-orientation bank" % n,
+                 (("rgc", rgc, (3, 3, 3, 3)), ("rgby", rgby, (3, 3, 3, 3)), ("stripe", stripe, (3, 3, 3, n)),
+                  ("blur", blur, (7, 7, n, n)), ("end", end, (3, 3, n, n))),
+                 regulation_value, regulation_root, clip_max, border)

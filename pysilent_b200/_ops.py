@@ -25,6 +25,11 @@ def _require_cuda():
 FUSED_INPUT_MAX = 1.0e30
 
 
+def fused_input_ok(x):
+    """Whether the fused stacks may take the tensor ``x``: no NaN, no Inf and no magnitude beyond FUSED_INPUT_MAX."""
+    return bool((x.abs() <= FUSED_INPUT_MAX).all())
+
+
 def as_device_tensor(t, dtype=torch.float32):
     """torch CUDA / numpy -> contiguous CUDA tensor of ``dtype``."""
     _require_cuda()
@@ -236,38 +241,29 @@ def display_tensors(gray, energy, region_h, region_w, half_h, half_w, exhaustion
     return cent, cent2, fired, update
 
 
-def stack_fused(pyramid, weights, want_orient=True, want_line_end=True, want_gray=True):
+def _stack(symbol, noun, pyramid, weights, channels, want_orient, want_line_end, want_gray):
     x = as_device_tensor(pyramid)
-    n, h, w, c = _nhwc(x, "stack_fused")
+    n, h, w, c = _nhwc(x, symbol[len("silent_"):])
     if c != 3:
-        raise ValueError("the fused stack needs 3-channel pyramids")
+        raise ValueError("%s needs 3-channel pyramids" % noun)
     mk = lambda ch: torch.empty((n, h, w, ch), dtype=torch.float32, device=x.device)  # noqa: E731
-    orient = mk(3) if want_orient else None
-    line_end = mk(3) if want_line_end else None
+    orient = mk(channels) if want_orient else None
+    line_end = mk(channels) if want_line_end else None
     gray = mk(1) if want_gray else None
     nbytes = _lib.lib().silent_stack_workspace_bytes(n, h, w)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
     with torch.cuda.device(x.device):
-        _lib.check(_lib.lib().silent_stack_fused(ptr(x), n, h, w, ctypes.byref(weights), ptr(orient), ptr(line_end),
-                                                 ptr(gray), ptr(ws), nbytes, stream_ptr()), "silent_stack_fused")
+        _lib.check(getattr(_lib.lib(), symbol)(ptr(x), n, h, w, ctypes.byref(weights), ptr(orient), ptr(line_end),
+                                               ptr(gray), ptr(ws), nbytes, stream_ptr()), symbol)
     return orient, line_end, gray
+
+
+def stack_fused(pyramid, weights, want_orient=True, want_line_end=True, want_gray=True):
+    return _stack("silent_stack_fused", "the fused stack", pyramid, weights, 3, want_orient, want_line_end, want_gray)
 
 
 def stack_bank(pyramid, bank, want_orient=True, want_line_end=True, want_gray=True):
     """The orientation bank's stack (``silent_stack_bank``) on a finite NHWC pyramid ``[n, h, w, 3]``: returns orient and
     padded_line_end ``[n, h, w, bank.orientations]`` and gray ``[n, h, w, 1]``."""
-    x = as_device_tensor(pyramid)
-    n, h, w, c = _nhwc(x, "stack_bank")
-    if c != 3:
-        raise ValueError("the fused orientation bank needs 3-channel pyramids")
-    nb = int(bank.orientations)
-    mk = lambda ch: torch.empty((n, h, w, ch), dtype=torch.float32, device=x.device)  # noqa: E731
-    orient = mk(nb) if want_orient else None
-    line_end = mk(nb) if want_line_end else None
-    gray = mk(1) if want_gray else None
-    nbytes = _lib.lib().silent_stack_workspace_bytes(n, h, w)
-    ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
-    with torch.cuda.device(x.device):
-        _lib.check(_lib.lib().silent_stack_bank(ptr(x), n, h, w, ctypes.byref(bank), ptr(orient), ptr(line_end),
-                                                ptr(gray), ptr(ws), nbytes, stream_ptr()), "silent_stack_bank")
-    return orient, line_end, gray
+    return _stack("silent_stack_bank", "the fused orientation bank", pyramid, bank, int(bank.orientations), want_orient,
+                  want_line_end, want_gray)

@@ -140,10 +140,11 @@ static TileMaxima tile_maxima(const silent_plan *plan)
 
 // K1 + K2 for frames [frame0, frame0 + nb) of a batch: the outputs, gray and the region maxima of these frames land at
 // their place in the whole-batch tensors, so that the emit stage can run once over the batch afterwards. frame0 must be
-// even on the frame-pair path (pairs never straddle a chunk).
-static int run_stack_stages(silent_plan *plan, const silent_stack_weights *W, const void *frames_dev, int frame0, int nb,
-                            float *pyramid_dev, float *orient_dev, float *line_end_dev, const WindowGeom *geo,
-                            cudaStream_t s, const PairClear *also_clear = nullptr)
+// even on the frame-pair path (pairs never straddle a chunk). K2 is the three-orientation stack (W) or, when bank is set,
+// the orientation bank's stack (frame-pair path only; no tile flags, geo must be null).
+static int run_stack_stages(silent_plan *plan, const silent_stack_weights *W, const silent_orientation_bank *bank,
+                            const void *frames_dev, int frame0, int nb, float *pyramid_dev, float *orient_dev,
+                            float *line_end_dev, const WindowGeom *geo, cudaStream_t s, const PairClear *also_clear = nullptr)
 {
     Workspace &ws = plan->ws;
     const bool pair_path = pyramid_pair_supported(plan);
@@ -155,11 +156,11 @@ static int run_stack_stages(silent_plan *plan, const silent_stack_weights *W, co
     // the caller adds in also_clear), so that no memset sits between the previous step's last kernel and this launch;
     // without that kernel a memset ahead of the launches does it
     int rc = SILENT_OK;
-    PairClear clear;
-    if (pair_path) {
+    PairClear clear;   // (the bank's kernel keeps no tile flags: nothing to clear)
+    if (!bank && pair_path) {
         stack_flag_region(ws.d_stack, n, plan->h, plan->w, &clear.a, &clear.a_bytes);
         if (also_clear) clear.b = also_clear->b, clear.b_bytes = also_clear->b_bytes;
-    } else {
+    } else if (!bank) {
         rc = stack_clear_flags(ws.d_stack, n, plan->h, plan->w, s);
         if (rc != SILENT_OK) return rc;
         if (also_clear && also_clear->b) SILENT_CUDA(cudaMemsetAsync(also_clear->b, 0, also_clear->b_bytes, s));
@@ -182,17 +183,23 @@ static int run_stack_stages(silent_plan *plan, const silent_stack_weights *W, co
     const void *pyr = pair_path ? (const void *)ws.d_pyramid
                                 : (const void *)(pyramid_dev ? pyramid_dev + img0 * level_elems * 3 : ws.d_pyramid);
     if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[1], s));
+    const size_t ch = bank ? bank->orientations : 3;
+    float *orient = orient_dev ? orient_dev + img0 * level_elems * ch : nullptr;
+    float *line_end = line_end_dev ? line_end_dev + img0 * level_elems * ch : nullptr;
+    cudaEvent_t mid = plan->timing ? plan->ev_mid : nullptr;
+    if (bank)
+        return stack_bank(pyr, n, plan->h, plan->w, plan->levels, bank, orient, line_end, ws.d_gray + img0 * level_elems,
+                          ws.d_stack, ws.stack_bytes, s, mid);
     const TileMaxima tm = tile_maxima(plan);
-    return stack_fused(pyr, n, plan->h, plan->w, pair_path ? plan->levels : 0, W,
-                       orient_dev ? orient_dev + img0 * level_elems * 3 : nullptr,
-                       line_end_dev ? line_end_dev + img0 * level_elems * 3 : nullptr, ws.d_gray + img0 * level_elems,
-                       ws.d_stack, ws.stack_bytes, geo, geo ? ws.d_winmax + img0 * geo->count : nullptr,
-                       ws.d_tilemax + img0 * tm.nty * tm.ntx, s, plan->timing ? plan->ev_mid : nullptr, true);
+    return stack_fused(pyr, n, plan->h, plan->w, pair_path ? plan->levels : 0, W, orient, line_end,
+                       ws.d_gray + img0 * level_elems, ws.d_stack, ws.stack_bytes, geo,
+                       geo ? ws.d_winmax + img0 * geo->count : nullptr, ws.d_tilemax + img0 * tm.nty * tm.ntx, s, mid, true);
 }
 
-static int check_pipeline_args(const silent_plan *plan, const silent_stack_weights *W, const void *frames, int batch)
+// checks shared by the pipeline entry points (`who` names the entry point); weights: the entry point's weight struct
+static int check_pipeline_args(const char *who, const silent_plan *plan, const void *weights, const void *frames, int batch)
 {
-    if (!plan || !W || !frames) return fail(SILENT_E_INVAL, "silent_pipeline_run: null argument");
+    if (!plan || !weights || !frames) return fail(SILENT_E_INVAL, "%s: null argument", who);
     if (batch <= 0) return fail(SILENT_E_INVAL, "batch must be positive");
     if (plan->params.num_colors != 3) return fail(SILENT_E_SHAPE, "the fused stack needs num_colors == 3");
     if (plan->levels == 0) return fail(SILENT_E_SHAPE, "frame is not larger than the pyramid centre: 0 levels");
@@ -202,69 +209,59 @@ static int check_pipeline_args(const silent_plan *plan, const silent_stack_weigh
     return SILENT_OK;
 }
 
-int silent_pipeline_run(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_dev, int batch,
-                        float *pyramid_dev, float *orient_dev, float *line_end_dev, int64_t *points_dev,
-                        int64_t capacity, int64_t *count_dev, silent_stream stream)
+// pyramid -> stack -> emit of a batch resident in HBM, with the three-orientation stack (W) or an orientation bank
+// (bank). The bank's kernel reduces neither region nor tile maxima: its emit scans gray on its own.
+static int run_pipeline(silent_plan *plan, const silent_stack_weights *W, const silent_orientation_bank *bank,
+                        const void *frames_dev, int batch, float *pyramid_dev, float *orient_dev, float *line_end_dev,
+                        int64_t *points_dev, int64_t capacity, int64_t *count_dev, cudaStream_t s)
 {
-    int rc = check_pipeline_args(plan, weights_host, frames_dev, batch);
-    if (rc != SILENT_OK) return rc;
     Workspace &ws = plan->ws;
     if (ws.batch < batch)
         return fail(SILENT_E_CAPACITY, "plan workspace holds %d frames, need %d: call silent_plan_reserve", ws.batch, batch);
-    cudaStream_t s = (cudaStream_t)stream;
     const int n = batch * plan->levels;
     const bool timing = plan->timing;
     if (timing) SILENT_CUDA(cudaEventRecord(plan->ev[0], s));
     WindowGeom geo;
-    const bool fuse_windows = count_dev && window_geometry(plan->h, plan->w, plan->h / 2, plan->w / 2, &geo);
+    const bool fuse_windows = !bank && count_dev && window_geometry(plan->h, plan->w, plan->h / 2, plan->w / 2, &geo);
     PairClear winmax_clear;   // the region maxima start at 0: cleared together with the tile flags (see run_stack_stages)
     if (fuse_windows) winmax_clear.b = ws.d_winmax, winmax_clear.b_bytes = (size_t)n * geo.count * sizeof(int);
-    rc = run_stack_stages(plan, weights_host, frames_dev, 0, batch, pyramid_dev, orient_dev, line_end_dev,
-                          fuse_windows ? &geo : nullptr, s, &winmax_clear);
+    int rc = run_stack_stages(plan, W, bank, frames_dev, 0, batch, pyramid_dev, orient_dev, line_end_dev,
+                              fuse_windows ? &geo : nullptr, s, &winmax_clear);
     if (rc != SILENT_OK) return rc;
     if (timing) SILENT_CUDA(cudaEventRecord(plan->ev[2], s));
     if (count_dev) {
         StageRange range("silent:emit");
         const TileMaxima tm = tile_maxima(plan);
         rc = max_value_indices_region(ws.d_gray, n, plan->h, plan->w, plan->h / 2, plan->w / 2, points_dev, capacity,
-                                      count_dev, ws.d_select, ws.select_bytes, fuse_windows ? ws.d_winmax : nullptr, &tm, s);
+                                      count_dev, ws.d_select, ws.select_bytes, fuse_windows ? ws.d_winmax : nullptr,
+                                      bank ? nullptr : &tm, s);
     }
     if (timing) SILENT_CUDA(cudaEventRecord(plan->ev[3], s));
     return rc;
+}
+
+int silent_pipeline_run(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_dev, int batch,
+                        float *pyramid_dev, float *orient_dev, float *line_end_dev, int64_t *points_dev,
+                        int64_t capacity, int64_t *count_dev, silent_stream stream)
+{
+    const int rc = check_pipeline_args("silent_pipeline_run", plan, weights_host, frames_dev, batch);
+    if (rc != SILENT_OK) return rc;
+    return run_pipeline(plan, weights_host, nullptr, frames_dev, batch, pyramid_dev, orient_dev, line_end_dev, points_dev,
+                        capacity, count_dev, (cudaStream_t)stream);
 }
 
 int silent_pipeline_run_orientations(silent_plan *plan, const silent_orientation_bank *bank_host, const void *frames_dev,
                                      int batch, float *orient_dev, float *line_end_dev, int64_t *points_dev,
                                      int64_t capacity, int64_t *count_dev, silent_stream stream)
 {
-    int rc = check_bank(bank_host, "silent_pipeline_run_orientations");
+    const char *who = "silent_pipeline_run_orientations";
+    int rc = check_bank(bank_host, who);
+    if (rc == SILENT_OK) rc = check_pipeline_args(who, plan, bank_host, frames_dev, batch);
     if (rc != SILENT_OK) return rc;
-    if (!plan || !frames_dev) return fail(SILENT_E_INVAL, "silent_pipeline_run_orientations: null argument");
-    if (batch <= 0) return fail(SILENT_E_INVAL, "batch must be positive");
-    if (plan->levels == 0) return fail(SILENT_E_SHAPE, "frame is not larger than the pyramid centre: 0 levels");
     if (!pyramid_pair_supported(plan))
         return fail(SILENT_E_SHAPE, "the fused orientation bank needs uint8 frames with 3 colours (frame-pair pyramid path)");
-    if ((plan->h % 2) || (plan->w % 2))
-        return fail(SILENT_E_SHAPE, "Ambiguous dimension: region shape (h/2, w/2) must be integral (h=%d, w=%d)", plan->h,
-                    plan->w);
-    Workspace &ws = plan->ws;
-    if (ws.batch < batch)
-        return fail(SILENT_E_CAPACITY, "plan workspace holds %d frames, need %d: call silent_plan_reserve", ws.batch, batch);
-    cudaStream_t s = (cudaStream_t)stream;
-    const int n = batch * plan->levels;
-    if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[0], s));
-    rc = pyramid_pair_build(plan, frames_dev, batch, ws.d_pyramid, s);
-    if (rc != SILENT_OK) return rc;
-    if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[1], s));
-    rc = stack_bank(ws.d_pyramid, n, plan->h, plan->w, plan->levels, bank_host, orient_dev, line_end_dev, ws.d_gray,
-                    ws.d_stack, ws.stack_bytes, s, plan->timing ? plan->ev_mid : nullptr);
-    if (rc != SILENT_OK) return rc;
-    if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[2], s));
-    if (count_dev)
-        rc = max_value_indices_region(ws.d_gray, n, plan->h, plan->w, plan->h / 2, plan->w / 2, points_dev, capacity,
-                                      count_dev, ws.d_select, ws.select_bytes, nullptr, nullptr, s);
-    if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[3], s));
-    return rc;
+    return run_pipeline(plan, nullptr, bank_host, frames_dev, batch, nullptr, orient_dev, line_end_dev, points_dev, capacity,
+                        count_dev, (cudaStream_t)stream);
 }
 
 int silent_pipeline_run_bank(silent_plan *plan, const silent_bank_weights *weights_host, const void *frames_dev, int batch,
@@ -332,7 +329,7 @@ int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weig
                              int batch, float *orient_host, float *line_end_host, int64_t *points_host,
                              int64_t capacity, int64_t *count_host, silent_stream stream)
 {
-    int rc = check_pipeline_args(plan, weights_host, frames_host, batch);
+    int rc = check_pipeline_args("silent_pipeline_run_host", plan, weights_host, frames_host, batch);
     if (rc != SILENT_OK) return rc;
     if (capacity < 0) return fail(SILENT_E_INVAL, "capacity must be >= 0");
     rc = silent_plan_reserve(plan, batch);
@@ -399,7 +396,7 @@ int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weig
             SILENT_CUDA(cudaMemcpyAsync((char *)ws.d_frames + fbytes * f0, src, fbytes * nb, cudaMemcpyHostToDevice, ws.s_in));
             SILENT_CUDA(cudaEventRecord(ws.ev_in[chunk], ws.s_in));
             SILENT_CUDA(cudaStreamWaitEvent(s, ws.ev_in[chunk], 0));
-            const int rcs = run_stack_stages(plan, weights_host, ws.d_frames, f0, nb, nullptr,
+            const int rcs = run_stack_stages(plan, weights_host, nullptr, ws.d_frames, f0, nb, nullptr,
                                              orient_host ? ws.d_orient : nullptr, line_end_host ? ws.d_line_end : nullptr,
                                              fuse_windows ? &geo : nullptr, s);
             if (rcs != SILENT_OK) return rcs;

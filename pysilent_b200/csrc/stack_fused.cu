@@ -28,7 +28,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <initializer_list>
 #include <mutex>
@@ -159,14 +158,14 @@ __device__ __forceinline__ void store_nhwc8(float *__restrict__ dst, const f2 (&
     }
 }
 
-// Write a staged tile ([2 images][TH][TW*3 (+4 pad)] floats, NHWC) to global memory with coalesced 128-bit stores.
-template <int TH, int TW, int NT>
+// Write a staged tile ([2 images][TH][TW*CH (+4 pad)] floats, NHWC) to global memory with coalesced 128-bit stores.
+template <int TH, int TW, int CH, int NT>
 __device__ __forceinline__ void copy_out_tile(const float *__restrict__ stage, float *__restrict__ out, int img0, int img1,
                                               bool has_b, int ty0, int tx0, int h, int w, int tid)
 {
     if (!out) return;
-    constexpr int QUADS = TW * 3 / 4, PITCH = TW * 3 + 4;
-    const int valid_floats = min(TW, w - tx0) * 3;
+    constexpr int QUADS = TW * CH / 4, PITCH = TW * CH + 4;
+    const int valid_floats = min(TW, w - tx0) * CH;
     const bool vec_ok = (w % 4) == 0;
     for (int i = tid; i < 2 * TH * QUADS; i += NT) {
         const int q = i % QUADS, rest = i / QUADS;
@@ -174,7 +173,7 @@ __device__ __forceinline__ void copy_out_tile(const float *__restrict__ stage, f
         const int gy = ty0 + r;
         if (gy >= h || (lane == 1 && !has_b) || 4 * q >= valid_floats) continue;
         const float4 v = *reinterpret_cast<const float4 *>(stage + (size_t)(lane * TH + r) * PITCH + 4 * q);
-        float *dst = out + (((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * 3 + 4 * q;
+        float *dst = out + (((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * CH + 4 * q;
         if (vec_ok && 4 * q + 4 <= valid_floats) {
             *reinterpret_cast<float4 *>(dst) = v;
         } else {
@@ -231,6 +230,30 @@ __device__ __forceinline__ void tile_store_images(const CUtensorMap *map, const 
         tma_store_tile(map, stage + (size_t)part * kTileStoreRows * pitch, bx, y, img0);
         if (has_b) tma_store_tile(map, stage + (size_t)(TH + part * kTileStoreRows) * pitch, bx, y, img1);
     }
+}
+
+// A staged tile ([2][TH][pitch] floats: image A's rows, then image B's; CH floats per pixel) leaves shared memory by one
+// of three routes: TMA tile stores issued by thread `issuer` (tile_store), one bulk copy per row from the warps of the
+// threads [first, first + NTHREADS) (bulk_ok: 16-byte aligned global rows), or coalesced element-wise copies by those
+// threads. The caller fences and synchronises the participants before. Returns true for a thread that issued bulk
+// copies: it must bulk_wait_read() before the staging buffer is reused.
+template <int TH, int TW, int CH, int NTHREADS>
+__device__ __forceinline__ bool store_staged_tile(const CUtensorMap *map, const float *stage, int pitch, float *out,
+                                                  bool tile_store, bool bulk_ok, int tid, int issuer, int first, int warp,
+                                                  bool leader, int bx, int ty0, int tx0, int h, int w, int img0, int img1,
+                                                  bool has_b)
+{
+    if (tile_store) {
+        if (tid != issuer) return false;
+        tile_store_images<TH>(map, stage, pitch, bx, ty0, h, img0, img1, has_b);
+        bulk_commit();
+        return true;
+    }
+    if (bulk_ok)
+        return bulk_rows<TH>(stage, pitch, out, img0, img1, has_b, ty0, h, (size_t)w * CH, (size_t)tx0 * CH,
+                             (uint32_t)(min(TW, w - tx0) * CH), warp, first / 32, NTHREADS / 32, leader);
+    copy_out_tile<TH, TW, CH, NTHREADS>(stage, out, img0, img1, has_b, ty0, tx0, h, w, tid - first);
+    return false;
 }
 
 __device__ __forceinline__ void store_cols8(f2 *__restrict__ dst, const f2 (&v)[kPX])
@@ -1011,19 +1034,10 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
         } else {
             __syncthreads();
         }
-        if (tile_store) {
-            if (tid == kRestageFirst) {   // two tile stores per 16 rows (one per image) instead of a bulk copy per row
-                tile_store_images<TH>(&M.orient, sStage, T::ST_PITCH, bx, ty0, h, img0, img1, has_b);
-                bulk_commit();
-                issued_orient = true;
-            }
-        } else if (bulk_ok) {
-            issued_orient = bulk_rows<TH>(sStage, T::ST_PITCH, orient, img0, img1, has_b, ty0, h, (size_t)w * 3, (size_t)tx0 * 3,
-                                          (uint32_t)(min(TW, w - tx0) * 3), warp_u, kRestageFirst / 32, kRestageThreads / 32,
-                                          leader);
-        } else {
-            copy_out_tile<TH, TW, kRestageThreads>(sStage, orient, img0, img1, has_b, ty0, tx0, h, w, tid - kRestageFirst);
-        }
+        // (tile stores: two per 16 rows, one per image, instead of a bulk copy per row)
+        issued_orient = store_staged_tile<TH, TW, 3, kRestageThreads>(&M.orient, sStage, T::ST_PITCH, orient, tile_store,
+                                                                      bulk_ok, tid, kRestageFirst, kRestageFirst, warp_u,
+                                                                      leader, bx, ty0, tx0, h, w, img0, img1, has_b);
     }
 
     // ---- S5-S7: e = clip(relu(conv3x3(d, end))); p = mask * e; g = mean(p)                 recognition_testing.py:73-77
@@ -1177,29 +1191,13 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
     // ---- copy-out: staged rows -> global NHWC, one bulk store per row ---------------------------------------------------
     fence_async_smem();
     __syncthreads();
-    if (gray && tile_store && kGrayTileStore) {
-        if (tid == 32) {
-            tile_store_images<TH>(&M.gray, sGray, T::G_PITCH, bx, ty0, h, img0, img1, has_b);
-            bulk_commit();
-            issued_line_end = true;
-        }
-    } else if (gray && bulk_ok)   // 2 * TH rows of TW floats, dealt like the line_end rows
-        issued_line_end |= bulk_rows<TH>(sGray, T::G_PITCH, gray, img0, img1, has_b, ty0, h, (size_t)w, (size_t)tx0,
-                                         (uint32_t)min(TW, w - tx0), warp_u, 0, NT / 32, leader);
-    if (line_end) {
-        if (tile_store) {
-            if (tid == 0) {
-                tile_store_images<TH>(&M.line_end, sStage, T::ST_PITCH, bx, ty0, h, img0, img1, has_b);
-                bulk_commit();
-                issued_line_end = true;
-            }
-        } else if (bulk_ok) {
-            issued_line_end |= bulk_rows<TH>(sStage, T::ST_PITCH, line_end, img0, img1, has_b, ty0, h, (size_t)w * 3,
-                                             (size_t)tx0 * 3, (uint32_t)(min(TW, w - tx0) * 3), warp_u, 0, NT / 32, leader);
-        } else {
-            copy_out_tile<TH, TW, NT>(sStage, line_end, img0, img1, has_b, ty0, tx0, h, w, tid);
-        }
-    }
+    const bool gray_tile_store = tile_store && kGrayTileStore;
+    if (gray && (gray_tile_store || bulk_ok))   // (without bulk_ok, gray left straight from registers in S5)
+        issued_line_end |= store_staged_tile<TH, TW, 1, NT>(&M.gray, sGray, T::G_PITCH, gray, gray_tile_store, true, tid, 32,
+                                                            0, warp_u, leader, bx, ty0, tx0, h, w, img0, img1, has_b);
+    if (line_end)
+        issued_line_end |= store_staged_tile<TH, TW, 3, NT>(&M.line_end, sStage, T::ST_PITCH, line_end, tile_store, bulk_ok,
+                                                            tid, 0, 0, warp_u, leader, bx, ty0, tx0, h, w, img0, img1, has_b);
     if (P.win.count) {
         if (tid < 8) {
             const int lane = tid >> 2, win = tid & 3;
@@ -1482,22 +1480,8 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
         }
         fence_async_smem();
         __syncthreads();
-        if (tile_store) {
-            if (tid == 0) {
-                tile_store_images<TH>(&M.orient, sStage, T::ST_PITCH, blockIdx.x, ty0, h, img0, img1, has_b);
-                bulk_commit();
-                issued = true;
-            }
-        } else if (bulk_ok) {
-            issued = bulk_rows<TH>(sStage, T::ST_PITCH, orient, img0, img1, has_b, ty0, h, (size_t)w * NB, (size_t)tx0 * NB,
-                                   (uint32_t)(min(TW, w - tx0) * NB), warp_u, 0, NT / 32, leader);
-        } else {
-            for (int i = tid; i < 2 * TH * TW * NB; i += NT) {
-                const int e = i % (TW * NB), row = i / (TW * NB), lane = row / TH, gy = ty0 + row % TH;
-                if (gy < h && tx0 + e / NB < w && (lane == 0 || has_b))
-                    orient[(((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * NB + e] = sStage[(size_t)row * T::ST_PITCH + e];
-            }
-        }
+        issued = store_staged_tile<TH, TW, NB, NT>(&M.orient, sStage, T::ST_PITCH, orient, tile_store, bulk_ok, tid, 0, 0,
+                                                   warp_u, leader, blockIdx.x, ty0, tx0, h, w, img0, img1, has_b);
         if (issued) bulk_wait_read();
         __syncthreads();   // the staging buffer is free again
     }
@@ -1565,25 +1549,9 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
     }
     fence_async_smem();
     __syncthreads();
-    issued = false;
-    if (line_end) {
-        if (tile_store) {
-            if (tid == 0) {
-                tile_store_images<TH>(&M.line_end, sStage, T::ST_PITCH, blockIdx.x, ty0, h, img0, img1, has_b);
-                bulk_commit();
-                issued = true;
-            }
-        } else if (bulk_ok) {
-            issued = bulk_rows<TH>(sStage, T::ST_PITCH, line_end, img0, img1, has_b, ty0, h, (size_t)w * NB, (size_t)tx0 * NB,
-                                   (uint32_t)(min(TW, w - tx0) * NB), warp_u, 0, NT / 32, leader);
-        } else {
-            for (int i = tid; i < 2 * TH * TW * NB; i += NT) {
-                const int e = i % (TW * NB), row = i / (TW * NB), lane = row / TH, gy = ty0 + row % TH;
-                if (gy < h && tx0 + e / NB < w && (lane == 0 || has_b))
-                    line_end[(((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * NB + e] = sStage[(size_t)row * T::ST_PITCH + e];
-            }
-        }
-    }
+    issued = line_end && store_staged_tile<TH, TW, NB, NT>(&M.line_end, sStage, T::ST_PITCH, line_end, tile_store, bulk_ok,
+                                                           tid, 0, 0, warp_u, leader, blockIdx.x, ty0, tx0, h, w, img0,
+                                                           img1, has_b);
     if (issued) bulk_wait_read();
 }
 
@@ -1597,9 +1565,8 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-// float32 view [planes][rows][2 * w] of a pair-interleaved tensor, boxes of [bp][br][2 * pitch]. False if TMA cannot be used.
-static bool make_pair_map(CUtensorMap *map, const void *base, int w, int rows, long long planes, int pitch, int box_rows,
-                          int box_planes)
+// the driver's cuTensorMapEncodeTiled, looked up on first use; null if the driver does not provide it
+static EncodeTiledFn encode_tiled()
 {
     static EncodeTiledFn encode = nullptr;
     if (!encode) {
@@ -1607,10 +1574,19 @@ static bool make_pair_map(CUtensorMap *map, const void *base, int w, int rows, l
         cudaDriverEntryPointQueryResult q;
         if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess || !fn) {
             (void)cudaGetLastError();
-            return false;
+            return nullptr;
         }
         encode = (EncodeTiledFn)fn;
     }
+    return encode;
+}
+
+// float32 view [planes][rows][2 * w] of a pair-interleaved tensor, boxes of [bp][br][2 * pitch]. False if TMA cannot be used.
+static bool make_pair_map(CUtensorMap *map, const void *base, int w, int rows, long long planes, int pitch, int box_rows,
+                          int box_planes)
+{
+    const EncodeTiledFn encode = encode_tiled();
+    if (!encode) return false;
     if ((w % 2) != 0 || 2 * pitch > 256 || box_rows > 256 || ((uintptr_t)base & 15) != 0) return false;
     const cuuint64_t dims[3] = {(cuuint64_t)2 * w, (cuuint64_t)rows, (cuuint64_t)planes};
     const cuuint64_t strides[2] = {(cuuint64_t)2 * w * 4, (cuuint64_t)2 * w * 4 * rows};
@@ -1625,16 +1601,8 @@ static bool make_pair_map(CUtensorMap *map, const void *base, int w, int rows, l
 static bool make_tile_store_map(CUtensorMap *map, const void *base, int n, int h, int w, int ch, int tw, int pad, int box_rows,
                                 int elem_floats = 1)   // 2: 8-byte elements (tile rows of more than 252 floats: boxes hold <= 256 elements)
 {
-    static EncodeTiledFn encode = nullptr;
-    if (!encode) {
-        void *fn = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess || !fn) {
-            (void)cudaGetLastError();
-            return false;
-        }
-        encode = (EncodeTiledFn)fn;
-    }
+    const EncodeTiledFn encode = encode_tiled();
+    if (!encode) return false;
     const int tile_floats = tw * ch;
     if (!base || ((uintptr_t)base & 15) != 0 || w % tw != 0 || tile_floats % 4 != 0 || (tile_floats + pad) % 4 != 0 ||
         (tile_floats + pad) / elem_floats > 256 || box_rows > 256)
@@ -1650,6 +1618,14 @@ static bool make_tile_store_map(CUtensorMap *map, const void *base, int n, int h
 }
 static f2 dup(float v) { return make_float2(v, v); }
 
+// multiprocessors of the current device (148 on a B200, assumed if the query fails)
+static int sm_count()
+{
+    int dev = 0, sms = 148;
+    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return sms;
+}
+
 struct StackPlanHost {
     ParamsA a;
     ParamsB b;
@@ -1658,28 +1634,38 @@ struct StackPlanHost {
     bool s3_sym, s5_ownoth;   // structure of the stripe / end filters (see stack_b_kernel)
 };
 
-// Validate the structure the fused kernels rely on and repack the HWIO filters as (w, w) pairs.
-int pack_stack_params(const silent_stack_weights *W, int n, int h, int w, StackPlanHost *S)
+// S4 early-out threshold from the 49 blur taps taps[0], taps[stride], ...: the smallest float T with rn(w_min * T) >= 1,
+// w_min * T >= 1.0001 in exact arithmetic (see S4 in stack_b_tile); 0 (early-out off) unless every tap is positive.
+static float quick_threshold(const float *taps, int stride)
 {
-    if (!W) return fail(SILENT_E_INVAL, "null weights");
-    if (W->border < 0) return fail(SILENT_E_INVAL, "border must be >= 0");
+    float blur_min = INFINITY;
+    for (int t = 0; t < 49; ++t) {
+        const float b = taps[t * stride];
+        blur_min = b < blur_min ? b : blur_min;                 // (a NaN weight leaves blur_min alone ...)
+        if (!(b > 0.0f) || std::isinf(b)) blur_min = -1.0f;   // ... and lands here
+    }
+    if (!(blur_min > 0.0f && blur_min < INFINITY)) return 0.0f;
+    float T = (float)(1.0001 / (double)blur_min);
+    for (int guard = 0; guard < 8 && !((double)blur_min * (double)T >= 1.0001); ++guard) T = std::nextafterf(T, INFINITY);
+    return (double)blur_min * (double)T >= 1.0001 && T < 1.0e20f ? T : 0.0f;
+}
+
+// stack_a's part (S1, S2): repack rgc and rgby ([3][3][3][3] HWIO) as (w, w) pairs and detect the structures its kernel
+// variants exploit. Any weights are accepted (the dense variant takes the rest).
+static void pack_stack_a(const float *rgc, const float *rgby, int n, int h, int w, StackPlanHost *S)
+{
     S->s1_depthwise = S->s2_rgby = true;
     for (int t = 0; t < 9; ++t)
         for (int ci = 0; ci < 3; ++ci)
             for (int co = 0; co < 3; ++co) {
                 const int i = (t * 3 + ci) * 3 + co;
-                S->a.w1[t][ci][co] = dup(W->rgc[i]);
-                S->a.w2[t][ci][co] = dup(W->rgby[i]);
-                S->b.w5[t][ci][co] = dup(W->end[i]);
-                if (ci != co && W->rgc[i] != 0.0f) S->s1_depthwise = false;
-                if (!rgby_nonzero(t, ci, co) && W->rgby[i] != 0.0f) S->s2_rgby = false;
-                if (!bits_equal(W->stripe[i], W->stripe[(t * 3) * 3 + co]))
-                    return fail(SILENT_E_STRUCTURE, "stripe filter differs across input channels at tap %d; the fused "
-                                                    "stack needs identical input slices (use the per-operator calls)", t);
-                S->b.w3[t][co] = dup(W->stripe[(t * 3) * 3 + co]);
+                S->a.w1[t][ci][co] = dup(rgc[i]);
+                S->a.w2[t][ci][co] = dup(rgby[i]);
+                if (ci != co && rgc[i] != 0.0f) S->s1_depthwise = false;
+                if (!rgby_nonzero(t, ci, co) && rgby[i] != 0.0f) S->s2_rgby = false;
             }
     {   // rgby_3 shared-surround structure (all comparisons bitwise; 2 * S is exact in float32)
-        const float *R = W->rgby;
+        const float *R = rgby;
         auto at = [&](int t, int ci, int co) { return R[(t * 3 + ci) * 3 + co]; };
         bool ok = bits_equal(at(4, 0, 1), 0.0f);
         for (int t = 0; t < 9 && ok; ++t) {
@@ -1694,23 +1680,33 @@ int pack_stack_params(const silent_stack_weights *W, int n, int h, int w, StackP
         S->a.s2c[0] = dup(at(4, 0, 0)), S->a.s2c[1] = dup(at(4, 1, 1)), S->a.s2c[2] = dup(at(4, 2, 2));
         S->a.s2c[3] = dup(at(4, 1, 2)), S->a.s2c[4] = dup(at(4, 2, 1)), S->a.s2c[5] = dup(2.0f);
     }
-    float blur_min = INFINITY;
+    S->a.h = h, S->a.w = w, S->a.n = n;
+}
+
+// stack_b's part (S3-S7): validate the structure the fused kernel needs (one stripe kernel over the input channels, one
+// blur kernel in every slice), repack stripe, blur and end as (w, w) pairs and detect the structured variant.
+static int pack_stack_b(const silent_stack_weights *W, int n, int h, int w, StackPlanHost *S)
+{
+    if (!W) return fail(SILENT_E_INVAL, "null weights");
+    if (W->border < 0) return fail(SILENT_E_INVAL, "border must be >= 0");
+    for (int t = 0; t < 9; ++t)
+        for (int ci = 0; ci < 3; ++ci)
+            for (int co = 0; co < 3; ++co) {
+                const int i = (t * 3 + ci) * 3 + co;
+                S->b.w5[t][ci][co] = dup(W->end[i]);
+                if (!bits_equal(W->stripe[i], W->stripe[(t * 3) * 3 + co]))
+                    return fail(SILENT_E_STRUCTURE, "stripe filter differs across input channels at tap %d; the fused "
+                                                    "stack needs identical input slices (use the per-operator calls)", t);
+                S->b.w3[t][co] = dup(W->stripe[(t * 3) * 3 + co]);
+            }
     for (int t = 0; t < 49; ++t) {
         for (int s = 0; s < 9; ++s)
             if (!bits_equal(W->blur[t * 9 + s], W->blur[t * 9]))
                 return fail(SILENT_E_STRUCTURE, "blur filter slices differ at tap %d; the fused stack needs one 7x7 "
                                                 "kernel in every slice (use the per-operator calls)", t);
         S->b.wb[t] = dup(W->blur[t * 9]);
-        blur_min = W->blur[t * 9] < blur_min ? W->blur[t * 9] : blur_min;   // (a NaN weight leaves blur_min alone ...)
-        if (!(W->blur[t * 9] > 0.0f) || std::isinf(W->blur[t * 9])) blur_min = -1.0f;   // ... and lands here
     }
-    // S4 early-out threshold: the smallest float T with rn(w_min * T) >= 1 (only when every blur weight is positive)
-    S->b.quick_thr = 0.0f;
-    if (blur_min > 0.0f && blur_min < INFINITY) {   // w_min * T >= 1.0001 in exact arithmetic (see S4 in stack_b_kernel)
-        float T = (float)(1.0001 / (double)blur_min);
-        for (int guard = 0; guard < 8 && !((double)blur_min * (double)T >= 1.0001); ++guard) T = std::nextafterf(T, INFINITY);
-        if ((double)blur_min * (double)T >= 1.0001 && T < 1.0e20f) S->b.quick_thr = T;
-    }
+    S->b.quick_thr = quick_threshold(W->blur, 9);
     // stripe kernels symmetric under a 180-degree rotation: w3[0..4] already are the five distinct taps
     S->s3_sym = true;
     for (int t = 0; t < 4; ++t)
@@ -1731,9 +1727,7 @@ int pack_stack_params(const silent_stack_weights *W, int n, int h, int w, StackP
                 S->b.w5[t][ci][1] = dup(W->end[(t * 3 + ci) * 3 + (ci + 1) % 3]);
                 S->b.w5[t][ci][2] = dup(0.0f);
             }
-    S->a.h = S->b.h = h;
-    S->a.w = S->b.w = w;
-    S->a.n = S->b.n = n;
+    S->b.h = h, S->b.w = w, S->b.n = n;
     S->b.reg_value = W->regulation_value;
     S->b.reg_root = W->regulation_root;
     S->b.clip_max = W->clip_max;
@@ -1873,17 +1867,12 @@ static int launch_b(StackPlanHost &S, int pairs, f2 *bsum2, float *orient, float
     S.b.tma_store = (!orient || make_tile_store_map(&maps.orient, orient, S.b.n, h, w, 3, TW, TB::ST_PITCH - 3 * TW, kTileStoreRows)) &&
                     (!line_end || make_tile_store_map(&maps.line_end, line_end, S.b.n, h, w, 3, TW, TB::ST_PITCH - 3 * TW, kTileStoreRows)) &&
                     (!gray || make_tile_store_map(&maps.gray, gray, S.b.n, h, w, 1, TW, TB::G_PITCH - TW, kTileStoreRows));
-    if (const char *e = std::getenv("SILENT_B_TILE_STORE")) S.b.tma_store = S.b.tma_store && std::atoi(e) != 0;   // tuning knob
     S.b.pairs = pairs;
-    S.b.prefetch_pairs = 4;   // measured: 2 / 4 / 8 alike (-5 % on the quick pass), 0 = off
-    if (const char *e = std::getenv("SILENT_B_PREFETCH")) S.b.prefetch_pairs = std::atoi(e);   // tuning knob
+    S.b.prefetch_pairs = 4;   // measured: 2 / 4 / 8 alike (-5 % on the quick pass against 0 = off)
     const int nbx = ceil_div(w, TW), nby = ceil_div(h, TH);
     dim3 grid(nbx, nby, pairs);
-    if (!LITE && tile_flag) {   // fix-up pass: two CTAs per SM walk the flagged tiles
-        int dev = 0, sms = 148;
-        if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        grid = dim3((unsigned)std::min<long long>((long long)nbx * nby * pairs, 2LL * sms));
-    }
+    if (!LITE && tile_flag)   // fix-up pass: two CTAs per SM walk the flagged tiles
+        grid = dim3((unsigned)std::min<long long>((long long)nbx * nby * pairs, 2LL * sm_count()));
     static_assert(TH % kTileHB == 0, "a launch's tiles are whole multiples of the emit grid's tile rows");
     SILENT_CUDA(launch_dependent(kern, grid, dim3(NT), TB::kSmemBytes, stream, (const f2 *)bsum2, S.b, map_b, maps, orient, line_end,
                                  gray, winmax, tilemax, tile_flag, nbx, nby, pairs, TH / kTileHB));
@@ -1899,7 +1888,6 @@ static int launch_stack_a(const void *pyr, StackPlanHost &S, bool paired_in, int
     std::memset(&map_x, 0, sizeof(map_x));
     using TA = TileA<kTileHA, TWA>;
     S.a.prefetch_pairs = 8;   // ~ the image pairs whose tiles are resident on the chip at once
-    if (const char *e = std::getenv("SILENT_A_PREFETCH")) S.a.prefetch_pairs = std::atoi(e);   // tuning knob
     S.a.use_tma = paired_in && make_pair_map(&map_x, pyr, w, h, 3LL * pairs, TA::X_PITCH, TA::X_ROWS, 3);
     return paired_in ? dispatch_a<TWA, true>(S.s1_depthwise, S.s2_rgby, S.s2_shared, pyr, S.a, map_x, bsum2, pairs, stream)
                      : dispatch_a<TWA, false>(S.s1_depthwise, S.s2_rgby, S.s2_shared, pyr, S.a, map_x, bsum2, pairs, stream);
@@ -1917,8 +1905,7 @@ static int launch_stack(const void *pyr, StackPlanHost &S, bool paired_in, int p
         return launch_b<kTileHB, TW, false, false>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, nullptr, stream);
     // a grid that fits the device in about one wave (single frames, config C2) gains nothing from the quick variant's
     // higher occupancy and would pay for a second launch: the full variant does it alone
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = sm_count();
     const long long tiles = (long long)pairs * ceil_div(S.b.h, kTileHB) * ceil_div(S.b.w, TW);
     if (tiles <= 3LL * sms && (S.b.h % (2 * kTileHB)) == 0)   // ... on tiles twice as tall (half as many CTAs, one wave)
         return launch_b<2 * kTileHB, TW, true, false>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, nullptr, stream);
@@ -1964,27 +1951,41 @@ int stack_clear_flags(void *workspace, int n, int h, int w, cudaStream_t stream)
     return SILENT_OK;
 }
 
+// Argument checks shared by the stack entry points (`who` names the entry point in the messages); *pairs: the image
+// pairs of n images with pair_levels levels per frame (0: NHWC input, images paired (2p, 2p + 1)).
+static int check_stack_args(const char *who, const void *pyr, int n, int h, int w, int pair_levels, const float *orient,
+                            const float *line_end, const float *gray, const void *workspace, size_t workspace_bytes,
+                            int *pairs)
+{
+    if (!pyr) return fail(SILENT_E_INVAL, "%s: null pyramid", who);
+    if (n <= 0 || h <= 0 || w <= 0) return fail(SILENT_E_INVAL, "%s: bad shape %dx%dx%d", who, n, h, w);
+    const int levels = pair_levels > 0 ? pair_levels : 1;
+    if (n % levels != 0) return fail(SILENT_E_INVAL, "%s: n must be a multiple of the levels per frame", who);
+    *pairs = ((n / levels + 1) / 2) * levels;
+    if (*pairs > 65535) return fail(SILENT_E_SHAPE, "%s: at most 65535 image pairs per call", who);
+    if (!workspace || workspace_bytes < stack_workspace_bytes(n, h, w))
+        return fail(SILENT_E_CAPACITY, "%s: workspace too small (%zu < %zu bytes)", who, workspace_bytes,
+                    stack_workspace_bytes(n, h, w));
+    for (const void *p : {(const void *)pyr, (const void *)orient, (const void *)line_end, (const void *)gray})
+        if (((uintptr_t)p & 15) != 0) return fail(SILENT_E_INVAL, "%s: tensors must be 16-byte aligned", who);
+    return SILENT_OK;
+}
+
 int stack_fused(const void *pyr, int n, int h, int w, int pair_levels, const silent_stack_weights *W, float *orient,
                 float *line_end, float *gray, void *workspace, size_t workspace_bytes, const WindowGeom *geo,
                 int *winmax, int *tilemax, cudaStream_t stream, cudaEvent_t between_kernels, bool flags_clean)
 {
-    if (!pyr) return fail(SILENT_E_INVAL, "silent_stack_fused: null pyramid");
-    if (n <= 0 || h <= 0 || w <= 0) return fail(SILENT_E_INVAL, "silent_stack_fused: bad shape %dx%dx%d", n, h, w);
-    const bool paired_in = pair_levels > 0;
-    const int levels = paired_in ? pair_levels : 1;
-    if (n % levels != 0) return fail(SILENT_E_INVAL, "silent_stack_fused: n must be a multiple of the levels per frame");
-    const int pairs = ((n / levels + 1) / 2) * levels;
-    if (pairs > 65535) return fail(SILENT_E_SHAPE, "silent_stack_fused: at most 65535 image pairs per call");
-    if (!workspace || workspace_bytes < stack_workspace_bytes(n, h, w))
-        return fail(SILENT_E_CAPACITY, "silent_stack_fused: workspace too small (%zu < %zu bytes)", workspace_bytes,
-                    stack_workspace_bytes(n, h, w));
-    for (const void *p : {(const void *)pyr, (const void *)orient, (const void *)line_end, (const void *)gray})
-        if (((uintptr_t)p & 15) != 0) return fail(SILENT_E_INVAL, "silent_stack_fused: tensors must be 16-byte aligned");
-    StackPlanHost S;
-    int rc = pack_stack_params(W, n, h, w, &S);
+    int pairs = 0;
+    int rc = check_stack_args("silent_stack_fused", pyr, n, h, w, pair_levels, orient, line_end, gray, workspace,
+                              workspace_bytes, &pairs);
     if (rc != SILENT_OK) return rc;
+    StackPlanHost S;
+    rc = pack_stack_b(W, n, h, w, &S);
+    if (rc != SILENT_OK) return rc;
+    pack_stack_a(W->rgc, W->rgby, n, h, w, &S);
     if (geo && winmax) S.b.win = *geo;
-    S.a.pair_levels = S.b.pair_levels = pack_pair_levels(levels);
+    const bool paired_in = pair_levels > 0;
+    S.a.pair_levels = S.b.pair_levels = pack_pair_levels(paired_in ? pair_levels : 1);
     f2 *bsum2 = reinterpret_cast<f2 *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
     unsigned char *tile_flag = reinterpret_cast<unsigned char *>(bsum2) + stack_plane_bytes(n, h, w) + 16;   // [-4]: counter
     if (pick_tile_w(w) == 48)
@@ -2040,24 +2041,13 @@ static int launch_bank(const silent_orientation_bank *W, int n, int h, int w, in
                        float *orient, float *line_end, float *gray, cudaStream_t stream)
 {
     ParamsBank<NB> B;
-    float blur_min = INFINITY;
-    for (int t = 0; t < 49; ++t) {
-        const float b = W->blur[t * NB * NB];
-        B.wb[t] = dup(b);
-        blur_min = b < blur_min ? b : blur_min;
-        if (!(b > 0.0f) || std::isinf(b)) blur_min = -1.0f;
-    }
+    for (int t = 0; t < 49; ++t) B.wb[t] = dup(W->blur[t * NB * NB]);
     for (int t = 0; t < 9; ++t)
         for (int o = 0; o < NB; ++o) {
             B.w3[t][o] = dup(W->stripe[(t * 3) * NB + o]);
             B.w5[t][o] = dup(W->end[(t * NB + o) * NB + o]);
         }
-    B.quick_thr = 0.0f;
-    if (blur_min > 0.0f && blur_min < INFINITY) {
-        float T = (float)(1.0001 / (double)blur_min);
-        for (int guard = 0; guard < 8 && !((double)blur_min * (double)T >= 1.0001); ++guard) T = std::nextafterf(T, INFINITY);
-        if ((double)blur_min * (double)T >= 1.0001 && T < 1.0e20f) B.quick_thr = T;
-    }
+    B.quick_thr = quick_threshold(W->blur, NB * NB);
     B.reg_value = W->regulation_value, B.reg_root = W->regulation_root, B.clip_max = W->clip_max, B.border = W->border;
     B.h = h, B.w = w, B.n = n, B.pair_levels = pack_pair_levels(levels);
 
@@ -2071,7 +2061,6 @@ static int launch_bank(const silent_orientation_bank *W, int n, int h, int w, in
     const int pad = T::ST_PITCH - NB * Tile::TW;
     B.tma_store = (!orient || make_tile_store_map(&maps.orient, orient, n, h, w, NB, Tile::TW, pad, kTileStoreRows, 2)) &&
                   (!line_end || make_tile_store_map(&maps.line_end, line_end, n, h, w, NB, Tile::TW, pad, kTileStoreRows, 2));
-    if (const char *e = std::getenv("SILENT_B_TILE_STORE")) B.tma_store = B.tma_store && std::atoi(e) != 0;   // tuning knob
     SILENT_CUDA(launch_dependent(kern, grid, dim3(Tile::NT), T::kSmemBytes, stream, bsum2, B, maps, orient, line_end, gray));
     SILENT_LAUNCH_CHECK("stack_bank_kernel");
     return SILENT_OK;
@@ -2081,29 +2070,16 @@ int stack_bank(const void *pyr, int n, int h, int w, int pair_levels, const sile
                float *line_end, float *gray, void *workspace, size_t workspace_bytes, cudaStream_t stream,
                cudaEvent_t between_kernels)
 {
-    if (!pyr || !W) return fail(SILENT_E_INVAL, "bank stack: null argument");
-    if (n <= 0 || h <= 0 || w <= 0) return fail(SILENT_E_INVAL, "bank stack: bad shape %dx%dx%d", n, h, w);
+    int pairs = 0;
+    int rc = check_stack_args("bank stack", pyr, n, h, w, pair_levels, orient, line_end, gray, workspace, workspace_bytes,
+                              &pairs);
+    if (rc != SILENT_OK) return rc;
+    if (W->border < 0) return fail(SILENT_E_INVAL, "border must be >= 0");
+    // S1 + S2 -> channel sum, exactly as in the three-orientation stack
+    StackPlanHost S;
+    pack_stack_a(W->rgc, W->rgby, n, h, w, &S);
     const bool paired_in = pair_levels > 0;
     const int levels = paired_in ? pair_levels : 1;
-    if (n % levels != 0) return fail(SILENT_E_INVAL, "bank stack: n must be whole frames");
-    const int pairs = ((n / levels + 1) / 2) * levels;
-    if (pairs > 65535) return fail(SILENT_E_SHAPE, "bank stack: at most 65535 image pairs per call");
-    if (!workspace || workspace_bytes < stack_workspace_bytes(n, h, w))
-        return fail(SILENT_E_CAPACITY, "bank stack: workspace too small (%zu < %zu bytes)", workspace_bytes,
-                    stack_workspace_bytes(n, h, w));
-    for (const void *p : {(const void *)pyr, (const void *)orient, (const void *)line_end, (const void *)gray})
-        if (((uintptr_t)p & 15) != 0) return fail(SILENT_E_INVAL, "bank stack: tensors must be 16-byte aligned");
-
-    // S1 + S2 -> channel sum, exactly as in the three-orientation stack
-    silent_stack_weights tmp;
-    std::memset(&tmp, 0, sizeof(tmp));
-    std::memcpy(tmp.rgc, W->rgc, sizeof(tmp.rgc));
-    std::memcpy(tmp.rgby, W->rgby, sizeof(tmp.rgby));
-    for (float &b : tmp.blur) b = 1.0f;
-    tmp.regulation_value = 1.0f, tmp.regulation_root = 0.1f, tmp.clip_max = W->clip_max, tmp.border = W->border;
-    StackPlanHost S;
-    int rc = pack_stack_params(&tmp, n, h, w, &S);
-    if (rc != SILENT_OK) return rc;
     S.a.pair_levels = pack_pair_levels(levels);
     f2 *bsum2 = reinterpret_cast<f2 *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
     rc = pick_tile_w(w) == 48 ? launch_stack_a<48>(pyr, S, paired_in, pairs, bsum2, stream)

@@ -102,7 +102,7 @@ class LineEndPipeline:
         x = _ops.as_device_tensor(pyramid_tensor)
         # the fused kernels skip exact-zero weights and shortcut the regulator where the blur is provably >= 1: valid for
         # finite input only (include/silent_b200.h). NaN / Inf / huge values go operator by operator, like the graph.
-        if not bool((x.abs() <= _ops.FUSED_INPUT_MAX).all()):
+        if not _ops.fused_input_ok(x):
             return self.run_unfused(x, want_points)
         orient, line_end, gray = _ops.stack_fused(x, self.stack_weights())
         points = None
@@ -155,7 +155,7 @@ class LineEndPipeline:
         x = _ops.as_device_tensor(pyramid_tensor)
         region = [1, self.region_shape[1], self.region_shape[2], nb]
         if nb > 8:
-            if not bool((x.abs() <= _ops.FUSED_INPUT_MAX).all()):
+            if not _ops.fused_input_ok(x):
                 raise ValueError("a pyramid with NaN, Inf or values beyond 1e30 goes operator by operator, which supports "
                                  "at most 8 orientations (got %d)" % nb)
             orient, padded, gray = _ops.stack_bank(x, self.orientation_bank())
@@ -190,15 +190,15 @@ class LineEndPipeline:
         """frames: CUDA ``[B, H, W, 3]`` uint8/float32 -> LineEndResult over ``B * L`` levels (pyramid + S1-S8).
 
         ``out`` may carry preallocated ``(orient, padded_line_end, points, count)`` tensors to avoid allocation in a
-        steady-state loop; ``points`` then holds ``count`` valid rows (no host sync is performed in that case).
+        steady-state loop; ``points`` then holds ``count`` valid rows (no host sync is performed in that case). With
+        ``orientations`` set, orient and padded_line_end have ``orientations`` channels instead of 3.
         """
         nb = self._bank_width() if self.orientations is not None else None
         frames = frames if frames.dim() == 4 else frames.unsqueeze(0)
         frames = frames.contiguous()
-        if nb is not None:   # config C4 and its variants
-            if nb in _lib.FUSED_BANK_WIDTHS and frames.dtype == torch.uint8 and frames.shape[3] >= 3 \
-                    and self.blur_size == 7 and self.output_colors == 3 and (frames.shape[2] * frames.shape[3]) % 16 == 0:
-                return self._run_frames_bank(frames, want_points, points_capacity)   # fused: 4 kernels + emit
+        if nb is not None and not (nb in _lib.FUSED_BANK_WIDTHS and frames.dtype == torch.uint8 and frames.shape[3] >= 3
+                                   and self.blur_size == 7 and self.output_colors == 3
+                                   and (frames.shape[2] * frames.shape[3]) % 16 == 0):
             from .util.zoom.from_image import image_to_zoom_tensor   # other frames: pyramid, then run_bank
             return self.run_bank(image_to_zoom_tensor(frames, self.output_colors, self.output_size, self.zoom_ratio),
                                  want_points)
@@ -208,7 +208,7 @@ class LineEndPipeline:
         n = b * plan.levels
         dev = frames.device
         if out is None:
-            orient = torch.empty((n, plan.h, plan.w, 3), dtype=torch.float32, device=dev)
+            orient = torch.empty((n, plan.h, plan.w, nb or 3), dtype=torch.float32, device=dev)
             line_end = torch.empty_like(orient)
             cap = int(points_capacity) if points_capacity else max(64 * n, 1024)
             points = torch.empty((cap, 4), dtype=torch.int64, device=dev)
@@ -216,11 +216,16 @@ class LineEndPipeline:
         else:
             orient, line_end, points, count = out
             cap = int(points.shape[0])
+        # the 3-orientation stack (silent_pipeline_run, no pyramid output) or the fused bank (config C4 and its variants:
+        # pyramid_pair_kernel -> stack_a -> stack_bank_kernel -> emit)
+        if nb is None:
+            name, args = "silent_pipeline_run", (ctypes.byref(self.stack_weights()), _ops.ptr(frames), b, None)
+        else:
+            name, args = "silent_pipeline_run_orientations", (ctypes.byref(self.orientation_bank()), _ops.ptr(frames), b)
         with torch.cuda.device(dev):
-            _lib.check(_lib.lib().silent_pipeline_run(
-                plan.handle, ctypes.byref(self.stack_weights()), _ops.ptr(frames), b, None, _ops.ptr(orient),
-                _ops.ptr(line_end), _ops.ptr(points), cap, _ops.ptr(count) if want_points else None,
-                _ops.stream_ptr()), "silent_pipeline_run")
+            _lib.check(getattr(_lib.lib(), name)(
+                plan.handle, *args, _ops.ptr(orient), _ops.ptr(line_end), _ops.ptr(points), cap,
+                _ops.ptr(count) if want_points else None, _ops.stream_ptr()), name)
         if out is not None:
             return LineEndResult(orient, line_end, None, points)
         if not want_points:
@@ -228,31 +233,6 @@ class LineEndPipeline:
         total = int(count.item())
         if total > cap:   # rare (e.g. an all-black level emits every pixel): redo the emit with room for everything
             return self.run_frames(frames, want_points, points_capacity=total)
-        return LineEndResult(orient, line_end, None, points[:total])
-
-    def _run_frames_bank(self, frames, want_points=True, points_capacity=None):
-        """Config C4 fused: pyramid_pair_kernel -> stack_a (rgc, rgby) -> stack_bank_kernel (stripe bank, regulator,
-        depthwise end bank, mask, mean) -> emit, through ``silent_pipeline_run_orientations``."""
-        plan = self.plan_for(frames)
-        b = int(frames.shape[0])
-        plan.reserve(b)
-        n, dev = b * plan.levels, frames.device
-        bank = self.orientation_bank()
-        orient = torch.empty((n, plan.h, plan.w, bank.orientations), dtype=torch.float32, device=dev)
-        line_end = torch.empty_like(orient)
-        cap = int(points_capacity) if points_capacity else max(64 * n, 1024)
-        points = torch.empty((cap, 4), dtype=torch.int64, device=dev)
-        count = torch.zeros(1, dtype=torch.int64, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(_lib.lib().silent_pipeline_run_orientations(
-                plan.handle, ctypes.byref(bank), _ops.ptr(frames), b, _ops.ptr(orient), _ops.ptr(line_end),
-                _ops.ptr(points), cap, _ops.ptr(count) if want_points else None, _ops.stream_ptr()),
-                "silent_pipeline_run_orientations")
-        if not want_points:
-            return LineEndResult(orient, line_end, None, None)
-        total = int(count.item())
-        if total > cap:
-            return self._run_frames_bank(frames, want_points, points_capacity=total)
         return LineEndResult(orient, line_end, None, points[:total])
 
     # -- host buffers on both sides (LineEndDisplayer.callback) -----------------------------------------------------------

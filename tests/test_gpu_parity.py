@@ -247,6 +247,29 @@ def test_fused_stack_bit_exact_random(seed, n, h, w, c_oracle, default_filters):
     assert_close(line_end, ref_lit["padded"], "padded literal")
 
 
+@pytest.mark.parametrize("seed,n,h,w", [(35, 2, 64, 96), (36, 3, 37, 53), (37, 2, 30, 100)])
+def test_fused_stack_dense_variants_bit_exact(seed, n, h, w, c_oracle, default_filters):
+    """Weights without the generators' structure run the dense variants of both kernels (stack_a without the depthwise /
+    zero-pattern / shared-surround forms, stack_b without SYM3 / OWNOTH): bitwise against the oracle, which takes the
+    same dispatch. The widths cover the three routes a staged tile leaves by: tile stores, bulk rows, element-wise."""
+    from pysilent_b200 import _lib, _ops
+    f = {k: np.array(v, copy=True) for k, v in default_filters.items()}
+    f["rgc"][1, 1, 0, 1] = 0.05          # not depthwise
+    f["rgby"][0, 0, 1, 2] *= 1.5         # not the shared surround (as in test_c_oracle_fused_order_uses_the_structures) ...
+    f["rgby"][0, 0, 1, 1] = 0.05         # ... nor the zero pattern
+    f["end"][2, 1, 0, 1] += 0.01         # not own / other
+    W = {k: np.ascontiguousarray(v, np.float32) for k, v in f.items()}
+    L = c_oracle.lib()
+    assert not L.so_depthwise3(W["rgc"]) and not L.so_rgby_shared(W["rgby"]) and not L.so_end_ownoth(W["end"])
+    pyr = _pyr(seed, n, h, w)
+    orient, line_end, gray = _ops.stack_fused(pyr, _lib.make_stack_weights(f["rgc"], f["rgby"], f["stripe"], f["blur"],
+                                                                           f["end"]))
+    ref = c_oracle.line_end_stack(pyr, f)
+    assert_bits(orient, ref["orient"], "orient")
+    assert_bits(line_end, ref["padded"], "padded_line_end")
+    assert_bits(gray, ref["gray"], "gray")
+
+
 def test_fused_stack_rejects_unstructured_weights():
     from pysilent_b200 import LineEndPipeline, _lib, _ops
     pipe = LineEndPipeline()

@@ -232,6 +232,26 @@ def test_bank16_at_4k(cuda, c_oracle):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("n", [8, 16])
+def test_bank_run_frames_into_caller_buffers(n, cuda):
+    """run_frames(frames, out=bufs) with orientations set fills the caller's (orient, padded_line_end, points, count), as
+    for the 3-orientation stack, bit for bit what the call without out returns."""
+    from pysilent_b200 import LineEndPipeline
+    pipe = LineEndPipeline(output_size=(96, 64), zoom_ratio=SQRT2, orientations=n)
+    frames = cuda.from_numpy(np.stack([structured_frame(90 + i, 300, 432) for i in range(3)])).cuda()
+    ref = pipe.run_frames(frames)
+    bufs = (cuda.full_like(ref.orient, -7.0), cuda.full_like(ref.padded_line_end, -7.0),
+            cuda.full((64 * ref.orient.shape[0], 4), -1, dtype=cuda.int64, device="cuda"),
+            cuda.zeros(1, dtype=cuda.int64, device="cuda"))
+    res = pipe.run_frames(frames, out=bufs)
+    assert res.orient is bufs[0] and res.padded_line_end is bufs[1] and res.points is bufs[2]
+    assert cuda.equal(bufs[0].view(cuda.int32), ref.orient.view(cuda.int32))
+    assert cuda.equal(bufs[1].view(cuda.int32), ref.padded_line_end.view(cuda.int32))
+    count = int(bufs[3].item())
+    assert count == ref.points.shape[0] and cuda.equal(bufs[2][:count], ref.points)
+
+
+@pytest.mark.gpu
 def test_bank8_new_entry_equals_old_entry(cuda):
     """At n = 8, silent_pipeline_run_orientations, silent_pipeline_run_bank and run_frames agree bit for bit."""
     from pysilent_b200 import LineEndPipeline, _ops
