@@ -216,6 +216,21 @@ int silent_display_tensors(const float *gray_dev, int n, int h, int w, int regio
                            float centerer, float *centroids_disp_dev, float *centroids2_disp_dev, float *fired_disp_dev,
                            float *update_disp_dev, float *scratch_dev, silent_stream stream);
 
+/* silent_display_tensors over a clip: `steps` consecutive time steps of n images each, time-major (gray_dev
+ * [steps*n,h,w,1], image t*n + e is step t of energy slice e). energy_dev [n,oh,ow,1] is updated in place and the four
+ * outputs hold steps*n images each, shaped as in silent_display_tensors: the result equals `steps` calls of
+ * silent_display_tensors on the consecutive slices of n images, bit for bit. Two launches: the centroid images and block
+ * importance of every step at once, then the boosting recurrence of the whole clip in one thread-block cluster per
+ * energy slice, its state on chip. A grid no cluster can hold (a band of more than 8192 cells on 16 CTAs: levels far
+ * beyond a megapixel at 3 x 3 blocks) takes 2 launches per step instead. scratch_dev: at least
+ * silent_display_sequence_scratch_bytes(steps, n, h, w, region_h, region_w) bytes (0 for a non-positive argument). */
+size_t silent_display_sequence_scratch_bytes(int steps, int n, int h, int w, int region_h, int region_w);
+int silent_display_sequence(const float *gray_dev, int steps, int n, int h, int w, int region_h, int region_w,
+                            int half_h, int half_w, float *energy_dev, float exhaustion_max, float excitation_max,
+                            int recovery_mode, float normer, float centerer, float *centroids_disp_dev,
+                            float *centroids2_disp_dev, float *fired_disp_dev, float *update_disp_dev, void *scratch_dev,
+                            size_t scratch_bytes, silent_stream stream);
+
 /* ---- multi-GPU: the path's only exchange is the feature-point gather (SURVEY 8(e)) ------------------------------------- */
 
 /* Packs one rank's points for a single fixed-size all-gather: packed_dev [capacity + 1][4] int64 = the first

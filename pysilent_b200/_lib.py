@@ -24,7 +24,8 @@ SYMBOLS = (
     "silent_plan_level_tables", "silent_plan_algorithmic_bytes", "silent_pyramid_build", "silent_conv2d",
     "silent_regulate", "silent_pad_inwards", "silent_value_from_color", "silent_selection_workspace_bytes",
     "silent_max_value_indices_region", "silent_top_value_points", "silent_stack_workspace_bytes", "silent_stack_fused", "silent_pipeline_run",
-    "silent_pipeline_run_host", "silent_pipeline_run_bank", "silent_pipeline_run_orientations", "silent_stack_bank", "silent_get_centroids", "silent_resize_nearest", "silent_get_boosting", "silent_pointwise", "silent_display_tensors", "silent_pack_points",
+    "silent_pipeline_run_host", "silent_pipeline_run_bank", "silent_pipeline_run_orientations", "silent_stack_bank", "silent_get_centroids", "silent_resize_nearest", "silent_get_boosting", "silent_pointwise", "silent_display_tensors",
+    "silent_display_sequence_scratch_bytes", "silent_display_sequence", "silent_pack_points",
     "silent_comm_unique_id", "silent_comm_create", "silent_comm_destroy", "silent_comm_check", "silent_gather_points",
 )
 
@@ -113,6 +114,8 @@ def lib():
         "silent_get_boosting": (i, [p, p, i, i, i, f, f, i, p, p, p]),
         "silent_pointwise": (i, [p, p, sz, i, p, p]),
         "silent_display_tensors": (i, [p, i, i, i, i, i, i, i, p, f, f, i, f, f, p, p, p, p, p, p]),
+        "silent_display_sequence_scratch_bytes": (sz, [i, i, i, i, i, i]),
+        "silent_display_sequence": (i, [p, i, i, i, i, i, i, i, i, p, f, f, i, f, f, p, p, p, p, p, sz, p]),
         "silent_pack_points": (i, [p, p, i64, i64, p, p]),
         "silent_comm_unique_id": (i, [p]),
         "silent_comm_create": (i, [p, i, i, ctypes.POINTER(p)]),

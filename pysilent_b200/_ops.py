@@ -241,6 +241,44 @@ def display_tensors(gray, energy, region_h, region_w, half_h, half_w, exhaustion
     return cent, cent2, fired, update
 
 
+def display_sequence(gray, energy, steps, region_h, region_w, half_h, half_w, exhaustion_max, excitation_max,
+                     recovery_mode):
+    """``display_tensors`` over a clip (``silent_display_sequence``): ``gray`` ``[steps * n, h, w, 1]`` is time-major
+    (image ``t * n + e`` is step t of slice e of ``energy`` ``[n, oh, ow, 1]``). Returns the four display tensors over
+    all ``steps * n`` images, equal to ``steps`` successive ``display_tensors`` calls, and leaves ``energy`` where the
+    last of them would."""
+    g = as_device_tensor(gray)
+    total, h, w, c = _nhwc(g, "display_sequence")
+    steps = int(steps)
+    n = total // steps if steps > 0 else 0
+    oh, ow = -(-h // region_h), -(-w // region_w)
+    if c != 1 or n <= 0 or total != steps * n or tuple(energy.shape) != (n, oh, ow, 1) or not energy.is_cuda \
+            or energy.dtype != torch.float32 or not energy.is_contiguous():
+        raise ValueError("display_sequence needs a one-channel gray tensor of steps * n images and a contiguous CUDA "
+                         "float32 energy tensor [n, ceil(h / region_h), ceil(w / region_w), 1]")
+    dev = g.device
+    cent = torch.empty((total, h, w, 1), dtype=torch.float32, device=dev)
+    cent2 = torch.empty((total, int(half_h), int(half_w), 1), dtype=torch.float32, device=dev)
+    fired = torch.empty((total, oh, ow, 3), dtype=torch.float32, device=dev)
+    update = torch.empty((total, oh, ow, 3), dtype=torch.float32, device=dev)
+    nbytes = display_sequence_scratch_bytes(steps, n, h, w, region_h, region_w)
+    scratch = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
+    normer = 255.0 / (exhaustion_max + excitation_max)                                   # boosting.py:37-38
+    centerer = (excitation_max / (exhaustion_max + excitation_max)) * 255.0
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().silent_display_sequence(
+            ptr(g), steps, n, h, w, int(region_h), int(region_w), int(half_h), int(half_w), ptr(energy),
+            float(exhaustion_max), float(excitation_max), int(recovery_mode), float(normer), float(centerer), ptr(cent),
+            ptr(cent2), ptr(fired), ptr(update), ptr(scratch), nbytes, stream_ptr()), "silent_display_sequence")
+    return cent, cent2, fired, update
+
+
+def display_sequence_scratch_bytes(steps, n, h, w, region_h, region_w):
+    """Bytes of device scratch ``display_sequence`` allocates for one call."""
+    return int(_lib.lib().silent_display_sequence_scratch_bytes(int(steps), int(n), int(h), int(w), int(region_h),
+                                                                int(region_w)))
+
+
 def _stack(symbol, noun, pyramid, weights, channels, want_orient, want_line_end, want_gray):
     x = as_device_tensor(pyramid)
     n, h, w, c = _nhwc(x, symbol[len("silent_"):])

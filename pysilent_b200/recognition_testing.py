@@ -56,11 +56,7 @@ class LineEndDisplayer(LineEndPipeline):
         shape = tuple(orient.shape)
         half = (np.asarray(shape[1:3], dtype=np.float32) / np.float32(m.e ** .5)).astype(np.int32)   # :82
         if fused:
-            rh, rw = region_dims(self.centroid_region_shape)
-            state_shape = (shape[0], -(-shape[1] // rh), -(-shape[2] // rw), 1)
-            if self.pyramid_tensor_shape != shape or self.energy_values is None:                  # pre_compile, :45-57
-                self.pyramid_tensor_shape = shape
-                self.energy_values = torch.full(state_shape, 8.0, dtype=torch.float32, device=gray.device)
+            rh, rw = self._boosting_state(shape, gray.device)
             cent, cent2, fired, update = _ops.display_tensors(gray, self.energy_values, rh, rw, int(half[0]), int(half[1]),
                                                               1, 1, recovery_mode(False, True))   # :79-87
             return [orient, cent, cent2, fired, update, padded_line_end]                          # :98-100
@@ -77,6 +73,16 @@ class LineEndDisplayer(LineEndPipeline):
         return [orient, _ops.pointwise(centroids, _lib.PW_INVERT255), _ops.pointwise(centroids2, _lib.PW_INVERT255),
                 _ops.pointwise(fired_importants, _lib.PW_MUL255), update_importances, padded_line_end]   # :98-100
 
+    def _boosting_state(self, shape, device):
+        """Re-initialise ``energy_values`` to 8 when the per-step shape ``(levels, h, w, C)`` changes (pre_compile,
+        ``:45-57``); returns the centroid region ``(rh, rw)``."""
+        rh, rw = region_dims(self.centroid_region_shape)
+        if self.pyramid_tensor_shape != shape or self.energy_values is None:
+            self.pyramid_tensor_shape = shape
+            self.energy_values = torch.full((shape[0], -(-shape[1] // rh), -(-shape[2] // rw), 1), 8.0,
+                                            dtype=torch.float32, device=device)
+        return rh, rw
+
     def run(self, pyramid_tensor):
         """``pyramid_tensor`` ``[L, h, w, 3]`` -> the six fetched tensors as host arrays (``session.run``, ``:132``)."""
         res = LineEndPipeline.run(self, pyramid_tensor, want_points=False)
@@ -87,6 +93,55 @@ class LineEndDisplayer(LineEndPipeline):
         ``B`` > 1 every frame is an independent camera stream with its own slice of the boosting state."""
         res = self.run_frames(frames, want_points=False)
         return self.display_tensors(res.orient, res.padded_line_end)
+
+    def run_clip(self, frames):
+        """A clip of consecutive frames resident in HBM -> the six display tensors on the device, in the order of
+        ``run_frames_display``. ``frames`` is ``[T, H, W, 3]`` (one camera) or ``[T, S, H, W, 3]`` (S cameras),
+        time-major; step t's images are ``[t * S * L, (t + 1) * S * L)`` and equal, bit for bit, what
+        ``run_frames_display(frames[t])`` returns when called for t = 0 ... T-1 in turn. ``energy_values`` ends where
+        those calls leave it, so ``callback``, ``run_clip`` and ``callback`` on one camera continue one state. The
+        pipeline runs once over all T * S frames, and the boosting recurrence over the whole clip in one launch."""
+        rank = frames.dim() if isinstance(frames, torch.Tensor) else np.ndim(frames)
+        if rank not in (4, 5) or frames.shape[0] < 1:
+            raise ValueError("run_clip takes frames [T, H, W, 3] or [T, S, H, W, 3] with T >= 1, got shape %s"
+                             % (tuple(frames.shape),))
+        steps = int(frames.shape[0])
+        res = self.run_frames(frames.reshape((-1,) + tuple(frames.shape[-3:])), want_points=False)
+        orient, padded = res.orient, res.padded_line_end
+        gray = get_value_from_color(padded)                                                       # :77
+        step_shape = (orient.shape[0] // steps,) + tuple(orient.shape[1:])
+        half = (np.asarray(step_shape[1:3], dtype=np.float32) / np.float32(m.e ** .5)).astype(np.int32)   # :82
+        rh, rw = self._boosting_state(step_shape, gray.device)
+        cent, cent2, fired, update = _ops.display_sequence(gray, self.energy_values, steps, rh, rw, int(half[0]),
+                                                           int(half[1]), 1, 1, recovery_mode(False, True))
+        return [orient, cent, cent2, fired, update, padded]
+
+    def callback_clip(self, frames, cam_id=None):
+        """``callback`` over a host clip ``[T, H, W, 3]`` of one camera: a list of T results, each
+        ``[frames[t]] + six lists of per-level images`` like ``callback``'s, with the state carried from step to step.
+        The clip goes up through a page-locked buffer, runs through ``run_clip`` and comes back with asynchronous
+        copies and one synchronisation. The arrays handed out stay untouched for the next ``host_slots - 1`` calls of
+        ``callback`` or ``callback_clip``."""
+        z = np.asarray(frames)
+        if z.ndim != 4 or z.shape[0] < 1:
+            raise ValueError("callback_clip takes host frames [T, H, W, 3] with T >= 1, got shape %s" % (z.shape,))
+        if self.orientations is not None:
+            self._bank_width()
+        z = np.ascontiguousarray(z if z.dtype == np.uint8 else z.astype(np.float32))
+        dev = self._device()
+        self._slot = (self._slot + 1) % self.host_slots
+        staged = self._host_buffer(("clip", self._slot), z.shape, torch.uint8 if z.dtype == np.uint8 else torch.float32)
+        staged.numpy()[...] = z
+        with torch.cuda.device(dev):
+            tensors = self.run_clip(staged.to(dev, non_blocking=True))
+            outs = []
+            for i, t in enumerate(tensors):
+                host = self._host_buffer(("clip_out", self._slot, i), tuple(t.shape), t.dtype)
+                host.copy_(t, non_blocking=True)
+                outs.append(host.numpy())
+            torch.cuda.current_stream().synchronize()
+        L = outs[0].shape[0] // z.shape[0]
+        return [[frames[t]] + [[outs[x][t * L + y] for y in range(L)] for x in range(6)] for t in range(z.shape[0])]
 
     def callback(self, frame, cam_id=None, depth=2):
         """``recognition_testing.py:136-144``: ``[frame] + [[tensors[x][y] for y in levels] for x in range(6)]``."""
