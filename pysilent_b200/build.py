@@ -11,7 +11,7 @@ NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-fmad=false",                      # canonical order: every FMA in the library is an explicit fmaf()
     "-Xcompiler", "-fPIC,-ffp-contract=off", "-Xptxas", "-v",
-] + ["-D%s=%s" % (k, os.environ[k]) for k in ("SILENT_PAIR_THREADS", "SILENT_TILE_HA", "SILENT_TILE_HB", "SILENT_ABLATE") if os.environ.get(k)]   # tuning knobs
+]
 
 
 def _nvcc():

@@ -84,7 +84,6 @@ silent_plan::~silent_plan()
     if (d_pair_ytab) cudaFree(d_pair_ytab);
     for (FrameTexture &ft : frame_textures)
         if (ft.tex) cudaDestroyTextureObject(ft.tex);
-    if (ytab_tex) cudaDestroyTextureObject(ytab_tex);
     if (htab_tex) cudaDestroyTextureObject(htab_tex);
 }
 

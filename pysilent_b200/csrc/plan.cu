@@ -1,6 +1,5 @@
 // Plan: the geometry of zoom.from_image (reference util/zoom/from_image.py:43-51) and the order-5 spline tap tables
 // of scipy.ndimage.zoom(prefilter=False, mode='constant'), computed once on the host in float64 and uploaded.
-#include <cstdlib>
 #include <stdarg.h>
 
 #include <algorithm>
@@ -173,7 +172,6 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
         const int waste = ceil_div(w, tw) * tw - w;
         if (waste <= best_waste) best_waste = waste, kPairTileW = tw;
     }
-    if (const char *e = std::getenv("SILENT_PAIR_TILEW")) kPairTileW = std::max(8, std::min(kPairTileWMax, std::atoi(e)));   // tuning knob
     plan->pair_tile_w = kPairTileW;
     plan->pair_ok = L > 0 && L <= kPairMaxLevels && ceil_div(w, kPairTileW) <= kPairMaxTiles && p->frame_c >= 3 &&
                     (int64_t)p->frame_h * p->frame_w * p->frame_c < INT32_MAX;   // row offsets inside a frame are 32-bit
@@ -211,9 +209,6 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
         }
         if ((size_t)pl.th * pl.vpitch * 8 > 190 * 1024) plan->pair_ok = false;
     }
-
-    if (const char *e = std::getenv("SILENT_PYRAMID_TEX")) plan->pair_tex_enabled = std::atoi(e) != 0;   // A/B knobs
-    if (const char *e = std::getenv("SILENT_PYRAMID_TEXTAB")) plan->pair_tex_tables = std::atoi(e);
 
     if (L > 0) {
         int ndev = 0;
@@ -306,22 +301,24 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
                 if (e == cudaSuccess) e = cudaMalloc(&plan->d_pair_ytab, ytab.size() * sizeof(int32_t));
                 if (e == cudaSuccess)
                     e = cudaMemcpy(plan->d_pair_ytab, ytab.data(), ytab.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
-                if (e == cudaSuccess) {   // both tables as linear textures of int4 texels (a failure only disables the option)
-                    void *ptrs[2] = {plan->d_pair_ytab, plan->d_pair_htab};
-                    size_t bytes[2] = {ytab.size() * sizeof(int32_t), htab.size() * sizeof(int32_t)};
-                    cudaTextureObject_t *objs[2] = {&plan->ytab_tex, &plan->htab_tex};
-                    for (int i = 0; i < 2; ++i) {
-                        cudaResourceDesc rd = {};
-                        rd.resType = cudaResourceTypeLinear;
-                        rd.res.linear.devPtr = ptrs[i];
-                        rd.res.linear.desc = cudaCreateChannelDesc<int4>();
-                        rd.res.linear.sizeInBytes = bytes[i];
-                        cudaTextureDesc td = {};
-                        td.readMode = cudaReadModeElementType;
-                        if (cudaCreateTextureObject(objs[i], &rd, &td, nullptr) != cudaSuccess) {
-                            (void)cudaGetLastError();
-                            *objs[i] = 0;
-                        }
+                if (e == cudaSuccess) {   // the phase-H table as a linear texture of int4 texels, and the alignment a
+                    // linear texture's devPtr needs (either failing only keeps the frame-pair kernel on its LDG variant)
+                    cudaResourceDesc rd = {};
+                    rd.resType = cudaResourceTypeLinear;
+                    rd.res.linear.devPtr = plan->d_pair_htab;
+                    rd.res.linear.desc = cudaCreateChannelDesc<int4>();
+                    rd.res.linear.sizeInBytes = htab.size() * sizeof(int32_t);
+                    cudaTextureDesc td = {};
+                    td.readMode = cudaReadModeElementType;
+                    if (cudaCreateTextureObject(&plan->htab_tex, &rd, &td, nullptr) != cudaSuccess) {
+                        (void)cudaGetLastError();
+                        plan->htab_tex = 0;
+                    }
+                    int dev = 0;
+                    if (cudaGetDevice(&dev) != cudaSuccess ||
+                        cudaDeviceGetAttribute(&plan->texture_alignment, cudaDevAttrTextureAlignment, dev) != cudaSuccess) {
+                        (void)cudaGetLastError();
+                        plan->texture_alignment = 0;
                     }
                 }
                 if (e != cudaSuccess) {

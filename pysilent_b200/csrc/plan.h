@@ -16,11 +16,8 @@ struct LevelInfo {
 // aligned 32-bit words of a frame row that its x-taps touch.
 constexpr int kPairTileWMax = 85;   // phase H deals the (column, channel) items of a tile over the CTA's threads
 constexpr int kPairMaxTiles = 64, kPairMaxLevels = 16;
-#ifndef SILENT_PAIR_THREADS
-#define SILENT_PAIR_THREADS 128
-#endif
 constexpr int kPairVGroup = 18;   // float2 slots per group of 16 byte-columns in the column-sum buffer (16 + 2 of padding)
-constexpr int kPairThreads = SILENT_PAIR_THREADS;   // threads per CTA of pyramid_pair_kernel (measured: 64 / 96 / 192 / 256 slower)
+constexpr int kPairThreads = 128;   // threads per CTA of pyramid_pair_kernel (measured: 64 / 96 / 192 / 256 slower)
 struct PairLevel {
     int ntx = 0, th = 0, vpitch = 0;
     int word_lo[kPairMaxTiles], nwords[kPairMaxTiles];
@@ -71,9 +68,8 @@ struct silent_plan {
     int *d_pair_words = nullptr;           // [L][kPairMaxTiles][4]: (word_lo, nwords, 2^32 / groups + 1, 0) per level and x tile
     int32_t *d_pair_htab = nullptr;        // [L][w][3][12]: phase-H tap offsets in the tile's column-sum row (6 ints) and weights (6 floats)
     int32_t *d_pair_ytab = nullptr;        // [L][h][12]: phase-V table: first tap row's byte offset ([0] < 0: zero row), step, six weights, other offsets (plan.cu)
-    int pair_tex_tables = 2;               // bit 0 / 1: the phase-V / phase-H table entries take the texture path too
-    cudaTextureObject_t ytab_tex = 0, htab_tex = 0;   // d_pair_ytab / d_pair_htab as linear textures of int4 texels
-    bool pair_tex_enabled = true;          // phase V of pyramid_pair_kernel reads the frames through the texture path
+    cudaTextureObject_t htab_tex = 0;      // d_pair_htab as a linear texture of int4 texels
+    int texture_alignment = 0;             // cudaDevAttrTextureAlignment of the plan's device (0: unknown, no textures)
     // linear textures over the callers' frame buffers, keyed by (pointer, bytes). An object may still be read by a
     // kernel in flight, so none is destroyed while the plan lives unless the table is full (then after a device
     // synchronisation): the host-buffer path cycles through its <= kMaxChunks staging slices, callers through a few buffers

@@ -136,7 +136,7 @@ constexpr int kVGroup = kPairVGroup;   // float2 slots per group of 16 byte-colu
 struct PairParams {
     const uint8_t *frames;
     cudaTextureObject_t frames_tex;   // TEX variant: the same frames as a linear texture of 128-bit texels
-    cudaTextureObject_t ytab_tex, htab_tex;   // the two tables as textures of int4 texels
+    cudaTextureObject_t htab_tex;     // TEX variant: htab as a texture of int4 texels
     f2 *xpair;
     const int4 *ytab;     // [L][h][3]: phase-V table (first tap row's byte offset, step, six weights | other offsets; plan.cu)
     const int4 *words;    // [L][kPairMaxTiles]: (first 32-bit word of a frame row, word count, 2^32 / groups + 1, 0) per x tile
@@ -165,9 +165,9 @@ __device__ __forceinline__ float magic_byte(uint32_t word, uint32_t selector)
 // were 28 % of the kernel's total, the table loads another 14 %): the texture path returns its data through the TEX
 // pipe's own write-back and leaves the LSU pipe to the shared-memory traffic of both phases (measured: 0.262 -> 0.250 ms
 // with the rows, 0.245 ms with the phase-H table entries too; the phase-V table entries gain nothing -- their latency
-// sits in front of every task's row loads). Same bits either way.
-template <int TEX, bool TEXY, bool TEXH>   // TEX: how many of a task's 12 row loads take the texture path; TEXY / TEXH: the
-                                           // phase-V / phase-H table entries too
+// sits in front of every task's row loads, so they always take LDG). Same bits either way: TEX = false is the variant for
+// frame buffers the texture unit cannot address.
+template <bool TEX>
 __global__ void __launch_bounds__(kPairThreads, 768 / kPairThreads) pyramid_pair_kernel(const __grid_constant__ PairParams P)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -220,11 +220,7 @@ __global__ void __launch_bounds__(kPairThreads, 768 / kPairThreads) pyramid_pair
         const int r = nq > 1 ? (int)__umulhi((uint32_t)t, magic) : t, qi = t - r * nq;
         // the row's table entry: two 128-bit words (first offset, step, six weights); a third one only for the few rows
         // whose tap rows are not consecutive (mirrored at the crop's edge)
-        auto ytab_word = [&](int k) {
-            if constexpr (TEXY) return tex1Dfetch<int4>(P.ytab_tex, (level * h + oy0 + r) * 3 + k);
-            else return __ldg(ytab + 3 * r + k);
-        };
-        const int4 y0 = ytab_word(0), y1 = ytab_word(1);
+        const int4 y0 = __ldg(ytab + 3 * r), y1 = __ldg(ytab + 3 * r + 1);
         f2 acc[16];
         if (y0.x < 0) {
 #pragma unroll
@@ -235,7 +231,7 @@ __global__ void __launch_bounds__(kPairThreads, 768 / kPairThreads) pyramid_pair
 #pragma unroll
                 for (int j = 0; j < kTaps; ++j) yoff[j] = y0.x + j * y0.y;
             } else {
-                const int4 y2 = ytab_word(2);
+                const int4 y2 = __ldg(ytab + 3 * r + 2);
                 yoff[0] = y0.x, yoff[1] = y2.x, yoff[2] = y2.y, yoff[3] = y2.z, yoff[4] = y2.w, yoff[5] = -y0.y - 1;
             }
             const float wyv[kTaps] = {__int_as_float(y0.z), __int_as_float(y0.w), __int_as_float(y1.x),
@@ -243,10 +239,13 @@ __global__ void __launch_bounds__(kPairThreads, 768 / kPairThreads) pyramid_pair
             uint4 qa[kTaps], qb[kTaps];
 #pragma unroll
             for (int j = 0; j < kTaps; ++j) {
-                if (2 * j < TEX) qa[j] = tex1Dfetch<uint4>(P.frames_tex, texA + (yoff[j] >> 4) + qi);
-                else qa[j] = __ldg(reinterpret_cast<const uint4 *>(frameA + yoff[j]) + qi);
-                if (2 * j + 1 < TEX) qb[j] = tex1Dfetch<uint4>(P.frames_tex, texB + (yoff[j] >> 4) + qi);
-                else qb[j] = __ldg(reinterpret_cast<const uint4 *>(frameB + yoff[j]) + qi);
+                if constexpr (TEX) {
+                    qa[j] = tex1Dfetch<uint4>(P.frames_tex, texA + (yoff[j] >> 4) + qi);
+                    qb[j] = tex1Dfetch<uint4>(P.frames_tex, texB + (yoff[j] >> 4) + qi);
+                } else {
+                    qa[j] = __ldg(reinterpret_cast<const uint4 *>(frameA + yoff[j]) + qi);
+                    qb[j] = __ldg(reinterpret_cast<const uint4 *>(frameB + yoff[j]) + qi);
+                }
             }
             // The first tap is a plain product: fma(w, v, +0) and w * v differ only when the product is -0 (a negative
             // weight on a zero byte), and a -0 column sum cannot change any output bit (phase H adds every term to +0).
@@ -283,7 +282,7 @@ __global__ void __launch_bounds__(kPairThreads, 768 / kPairThreads) pyramid_pair
         const int ox = bx * P.tile_w + item / 3;
         if (ox >= w) break;
         int4 t0, t1, t2;
-        if constexpr (TEXH) {
+        if constexpr (TEX) {
             const int ht = (level * w + ox) * 9 + 3 * c;
             t0 = tex1Dfetch<int4>(P.htab_tex, ht), t1 = tex1Dfetch<int4>(P.htab_tex, ht + 1), t2 = tex1Dfetch<int4>(P.htab_tex, ht + 2);
         } else {
@@ -328,10 +327,13 @@ int pyramid_pair_build(const silent_plan *plan, const void *frames_dev, int batc
     const silent_params &p = plan->params;
     const int pairs = (batch + 1) / 2;
     if (pairs > 65535) return fail(SILENT_E_SHAPE, "at most 131070 frames per call");
-    // frames as a texture of 128-bit texels (cached per plan: same pointer and size -> same object); the texel index is
-    // a 32-bit int and 1-D linear textures hold at most 2^27 texels
+    // frames as a texture of 128-bit texels (cached per plan: same pointer and size -> same object). The texture variant
+    // needs a pointer at the device's texture alignment (CUDA requires it of a linear texture's devPtr), fewer than 2^27
+    // texels (1-D linear textures; the texel index is a 32-bit int) and the phase-H table's texture; any other buffer
+    // takes the LDG variant, which computes the same bits
     const size_t total_bytes = (size_t)batch * p.frame_h * p.frame_w * p.frame_c;
-    bool use_tex = plan->pair_tex_enabled && (total_bytes >> 4) < ((size_t)1 << 27);
+    bool use_tex = plan->texture_alignment > 0 && (uintptr_t)frames_dev % (uintptr_t)plan->texture_alignment == 0 &&
+                   (total_bytes >> 4) < ((size_t)1 << 27) && plan->htab_tex != 0;
     cudaTextureObject_t tex = 0;
     if (use_tex) {
         silent_plan *mp = const_cast<silent_plan *>(plan);   // (the cache is plan-owned scratch, like the workspace)
@@ -358,24 +360,19 @@ int pyramid_pair_build(const silent_plan *plan, const void *frames_dev, int batc
                 mp->frame_textures.push_back(ft);
                 tex = obj;
             } else {
-                (void)cudaGetLastError();   // e.g. a pointer below the texture alignment: the LDG variant computes the
-                use_tex = false;            // same bits
+                (void)cudaGetLastError();   // the LDG variant computes the same bits
+                use_tex = false;
             }
         }
     }
-    auto kernel = pyramid_pair_kernel<0, false, false>;
-    if (use_tex) {
-        const bool ty = plan->ytab_tex != 0 && (plan->pair_tex_tables & 1), th = plan->htab_tex != 0 && (plan->pair_tex_tables & 2);
-        kernel = ty ? (th ? pyramid_pair_kernel<12, true, true> : pyramid_pair_kernel<12, true, false>)
-                    : (th ? pyramid_pair_kernel<12, false, true> : pyramid_pair_kernel<12, false, false>);
-    }
+    const auto kernel = use_tex ? pyramid_pair_kernel<true> : pyramid_pair_kernel<false>;
     // per launch, not once per process: the attribute belongs to the CURRENT device's context, and one process may
     // drive several GPUs (one LineEndPipeline per camera thread and device)
     SILENT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     PairParams P;
     P.frames = (const uint8_t *)frames_dev;
     P.frames_tex = tex;
-    P.ytab_tex = plan->ytab_tex, P.htab_tex = plan->htab_tex;
+    P.htab_tex = plan->htab_tex;
     P.xpair = (f2 *)xpair_dev;
     P.ytab = reinterpret_cast<const int4 *>(plan->d_pair_ytab);
     P.words = reinterpret_cast<const int4 *>(plan->d_pair_words);

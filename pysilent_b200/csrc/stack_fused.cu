@@ -95,12 +95,8 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
 // ---- bulk stores (cp.async.bulk shared -> global): one instruction moves a whole staged row; the TMA unit does the
 //      address arithmetic that a per-float4 copy loop spent ~30 instructions on
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-#ifndef SILENT_ABLATE
-#define SILENT_ABLATE 0   // experiments only: 1 no output stores, 2 no S5 arithmetic, 4 no S3 arithmetic (bit mask)
-#endif
 __device__ __forceinline__ void bulk_store(void *gdst, const void *ssrc, uint32_t bytes)
 {
-    if (SILENT_ABLATE & 1) return;
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(smem_u32(ssrc)), "r"(bytes)
                  : "memory");
 }
@@ -115,7 +111,6 @@ struct StoreMaps {
 };
 __device__ __forceinline__ void tma_store_tile(const CUtensorMap *map, const void *ssrc, int tile_x, int y, int img)
 {
-    if (SILENT_ABLATE & 1) return;
     asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.tile.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(map),
                  "r"(smem_u32(ssrc)), "r"(0), "r"(tile_x), "r"(y), "r"(img)
                  : "memory");
@@ -270,8 +265,8 @@ __device__ __forceinline__ void store_cols8(f2 *__restrict__ dst, const f2 (&v)[
 struct ParamsA {
     f2 w1[9][3][3];   // rgc  [tap][ci][co] as (w, w)
     f2 w2[9][3][3];   // rgby
-    f2 s2s[9];        // S2 mode 2: the shared surround kernel S (centre tap unused)
-    f2 s2c[6];        // S2 mode 2: centre taps d0, d1, d2 (ci -> ci), e12 (1 -> 2), e21 (2 -> 1), and the constant 2
+    f2 s2s[9];        // STRUCTURED S2: the shared surround kernel S (centre tap unused)
+    f2 s2c[6];        // STRUCTURED S2: centre taps d0, d1, d2 (ci -> ci), e12 (1 -> 2), e21 (2 -> 1), and the constant 2
     int h, w, n;      // level shape, number of images
     unsigned long long pair_levels;  // image pairing: pair p holds images (a, a + levels), packed by pack_pair_levels()
     int use_tma;      // PAIRED_IN only: load the tile with one TMA box copy
@@ -335,21 +330,15 @@ struct TileA {
     static_assert(TW % kPX == 0 && TW % 4 == 0, "tile width must be a multiple of the run length");
 };
 
-// rgby_3 structure (SURVEY Appendix A): off-centre taps couple only DIFFERENT channels; the centre tap couples each
-// channel with itself and channels 1 <-> 2. Anything else is structurally zero (28 of 81 weights).
-__host__ __device__ constexpr bool rgby_nonzero(int tap, int ci, int co)
-{
-    return tap == 4 ? (ci == co || (ci == 1 && co == 2) || (ci == 2 && co == 1)) : (ci != co);
-}
-
 // PAIRED_IN: the input is xpair[pair][c][y][x] float2 written by pyramid_pair_kernel (a verbatim 128-bit copy into the
 // planes); otherwise it is an NHWC float32 pyramid [n][h][w][3] (stand-alone silent_stack_fused).
-// S2 modes: 0 dense; 1 rgby_3 zero pattern (28 structural zeros skipped, 53 FFMA2 per pixel pair); 2 rgby_3 SHARED
-// surround (SURVEY Appendix A): off-centre taps couple every channel pair (i != j) through ONE kernel S, doubled for the
-// pair (1, 2), and the centre tap carries d_i on the diagonal plus e between channels 1 and 2. Then
+// STRUCTURED: rgc is depthwise (S1 computes the diagonal only) and rgby has rgby_3's SHARED surround (SURVEY Appendix A):
+// off-centre taps couple every channel pair (i != j) through ONE kernel S, doubled for the pair (1, 2), and the centre tap
+// carries d_i on the diagonal plus e between channels 1 and 2. Then
 //   T_i = S * a_i  (8 taps each),   u0 = d0 a0 + (T1 + T2),   u1 = d1 a1 + (e21 a2 + (2 T2 + T0)),   u2 likewise:
-// 24 + 8 FFMA2/FADD2 instead of 53. Part of the canonical FUSED order (oracle/silent_oracle.c: so_rgby_shared).
-template <int TH, int TW, int NT, bool S1_DEPTHWISE, int S2_MODE, bool PAIRED_IN>
+// 24 + 8 FFMA2/FADD2 instead of 81. Part of the canonical FUSED order (oracle/silent_oracle.c: so_rgby_shared).
+// Otherwise both stages run dense.
+template <int TH, int TW, int NT, bool STRUCTURED, bool PAIRED_IN>
 __global__ void __launch_bounds__(NT) stack_a_kernel(const void *__restrict__ input, const __grid_constant__ ParamsA P,
                                                      const __grid_constant__ CUtensorMap tmap, f2 *__restrict__ bsum2,
                                                      const unsigned char *__restrict__ s1_deal)
@@ -457,7 +446,7 @@ __global__ void __launch_bounds__(NT) stack_a_kernel(const void *__restrict__ in
     __syncthreads();
 
     // ---- S1: a = relu(conv3x3(x, rgc))   rows -1..TH, runs of 8 columns from -1               filters/rgc.py:13-16
-    if constexpr (S1_DEPTHWISE) {
+    if constexpr (STRUCTURED) {
         // depthwise weights (midget_rgc): a task is ONE channel of THREE output rows x 8 columns. Its five input rows are
         // loaded once (25 LDS.128 for 216 FFMA2, against 45 for a one-row three-channel task: this kernel is bound by
         // shared-memory bandwidth). Input rows are visited in ascending order, so every output still sees its taps in
@@ -532,9 +521,7 @@ __global__ void __launch_bounds__(NT) stack_a_kernel(const void *__restrict__ in
 #pragma unroll
                             for (int p = 0; p < kPX; ++p)
 #pragma unroll
-                                for (int co = 0; co < 3; ++co)
-                                    if (!S1_DEPTHWISE || ci == co)
-                                        acc[p][co] = fma2(P.w1[ky * 3 + kx][ci][co], v[p + kx], acc[p][co]);
+                                for (int co = 0; co < 3; ++co) acc[p][co] = fma2(P.w1[ky * 3 + kx][ci][co], v[p + kx], acc[p][co]);
                     }
                 }
             }
@@ -558,7 +545,7 @@ __global__ void __launch_bounds__(NT) stack_a_kernel(const void *__restrict__ in
         const int gy = ty0 + r, gx0 = tx0 + kPX * k;
         if (gy >= h || gx0 >= w) continue;
         f2 s[kPX];
-        if constexpr (S2_MODE == 2) {
+        if constexpr (STRUCTURED) {
             f2 T[3][kPX], ctr[3][kPX];
 #pragma unroll
             for (int ci = 0; ci < 3; ++ci) {
@@ -602,9 +589,7 @@ __global__ void __launch_bounds__(NT) stack_a_kernel(const void *__restrict__ in
 #pragma unroll
                         for (int p = 0; p < kPX; ++p)
 #pragma unroll
-                            for (int co = 0; co < 3; ++co)
-                                if (S2_MODE == 0 || rgby_nonzero(ky * 3 + kx, ci, co))
-                                    acc[p][co] = fma2(P.w2[ky * 3 + kx][ci][co], v[p + kx], acc[p][co]);
+                            for (int co = 0; co < 3; ++co) acc[p][co] = fma2(P.w2[ky * 3 + kx][ci][co], v[p + kx], acc[p][co]);
                 }
             }
 #pragma unroll
@@ -641,9 +626,9 @@ __global__ void __launch_bounds__(NT) stack_a_kernel(const void *__restrict__ in
 // ---------------------------------------------------------------------------------------------------------------------
 
 struct ParamsB {
-    f2 w3[9][3];      // stripe [tap][co]  (identical over ci); SYM3: taps 0..4 = the five distinct weights, see S3
+    f2 w3[9][3];      // stripe [tap][co]  (identical over ci); STRUCTURED: taps 0..4 = the five distinct weights, see S3
     f2 wb[49];        // blur   [tap]      (identical over ci, co)
-    f2 w5[9][3][3];   // end    [tap][ci][co]; OWNOTH: [tap][ci][0] = ci -> ci, [tap][ci][1] = ci -> each other channel
+    f2 w5[9][3][3];   // end    [tap][ci][co]; STRUCTURED: [tap][ci][0] = ci -> ci, [tap][ci][1] = ci -> each other channel
     float reg_value, reg_root, clip_max;
     float quick_thr;  // S4 early-out: a channel sum >= quick_thr under ANY blur tap proves m >= 1 (0: early-out disabled)
     int border;
@@ -692,15 +677,16 @@ struct TileB {
     static_assert(TW % kPX == 0, "tile width must be a multiple of the run length");
 };
 
-// SYM3: every stripe kernel is symmetric under a 180-degree rotation (K[ky][kx] == K[2-ky][2-kx], true for
-// rgb_2d_stripe_tensors): opposite taps are added first, 4 FADD2 + 15 FFMA2 per pixel pair instead of 27 FFMA2.
-// OWNOTH: an input channel of the end filter feeds the two OTHER output channels with one and the same 3x3 kernel (true
-// for rgb_2d_end_tensors): per input channel one "own" and one "other" chain, 54 FFMA2 + 6 FADD2 instead of 81 FFMA2.
+// STRUCTURED, both of:
+//  * every stripe kernel is symmetric under a 180-degree rotation (K[ky][kx] == K[2-ky][2-kx], true for
+//    rgb_2d_stripe_tensors): opposite taps are added first, 4 FADD2 + 15 FFMA2 per pixel pair instead of 27 FFMA2;
+//  * an input channel of the end filter feeds the two OTHER output channels with one and the same 3x3 kernel (true for
+//    rgb_2d_end_tensors): per input channel one "own" and one "other" chain, 54 FFMA2 + 6 FADD2 instead of 81 FFMA2.
 // Both orders are part of the canonical FUSED evaluation order (oracle/silent_oracle.c: so_line_end_stack_fused).
 // tile_flag [pairs][tile rows][tile cols] bytes: the LITE variant sets the flag of a tile it could not finish; the
 // full variant, given the flags, only works on flagged tiles (null: every tile).
 // One tile (bx, by) of image pair bz in a grid of nbx x nby tiles per pair.
-template <int TH, int TW, int NT, bool SYM3, bool OWNOTH, bool LITE>
+template <int TH, int TW, int NT, bool STRUCTURED, bool LITE>
 __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const int bz, const int nbx, const int nby,
                                              const f2 *__restrict__ bsum2, const ParamsB &P, const CUtensorMap &tmap,
                                              const StoreMaps &M, float *__restrict__ orient, float *__restrict__ line_end,
@@ -786,11 +772,8 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
         f2 acc[kPX][3];
 #pragma unroll
         for (int p = 0; p < kPX; ++p) acc[p][0] = acc[p][1] = acc[p][2] = zero2();
-        if ((SILENT_ABLATE & 4) && gy >= 0 && gy < h) {
-#pragma unroll
-            for (int p = 0; p < kPX; ++p) acc[p][0] = acc[p][1] = acc[p][2] = sB[(r + 1) * T::B_PITCH + kPX * k + p + 1];
-        } else if (gy >= 0 && gy < h) {
-            if constexpr (SYM3) {
+        if (gy >= 0 && gy < h) {
+            if constexpr (STRUCTURED) {
                 // chain over (b[-1,-1] + b[1,1]), (b[-1,0] + b[1,0]), (b[-1,1] + b[1,-1]), (b[0,-1] + b[0,1]), b[0,0]
                 {
                     f2 v0[10], v2[10];
@@ -1046,11 +1029,8 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
     const int gy = ty0 + r5, gx0 = tx0 + kPX * k5;
     const bool active = tid < TH * T::E_RUNS && gy < h && gx0 < w;
     f2 acc[kPX][3];
-    if ((SILENT_ABLATE & 2) && active) {
-#pragma unroll
-        for (int p = 0; p < kPX; ++p) acc[p][0] = acc[p][1] = acc[p][2] = sCD[(r5 + p) * T::CD_PITCH + kPX * k5];
-    } else if (active) {
-        if constexpr (OWNOTH) {
+    if (active) {
+        if constexpr (STRUCTURED) {
             // per input channel: own = its kernel into its own output channel, oth = the ONE kernel it feeds both other
             // output channels with; e_co = (t_0 + t_1) + t_2 with t_ci = (ci == co ? own_ci : oth_ci)
 #pragma unroll
@@ -1220,7 +1200,7 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
 // finish. The full variant without flags works on every tile (one CTA per tile); WITH flags it is the fix-up pass: a
 // small 1-D grid of CTAs walks the tile list and redoes the flagged tiles (none on textured input: the pass then costs
 // a few microseconds instead of a full grid of early exits).
-template <int TH, int TW, int NT, bool SYM3, bool OWNOTH, bool LITE>
+template <int TH, int TW, int NT, bool STRUCTURED, bool LITE>
 __global__ void __launch_bounds__(NT, LITE ? (TH <= 16 ? 5 : 3) : 2)
 stack_b_kernel(const f2 *__restrict__ bsum2, const __grid_constant__ ParamsB P, const __grid_constant__ CUtensorMap tmap,
                const __grid_constant__ StoreMaps M, float *__restrict__ orient, float *__restrict__ line_end, float *__restrict__ gray, int *__restrict__ winmax,
@@ -1258,14 +1238,14 @@ stack_b_kernel(const f2 *__restrict__ bsum2, const __grid_constant__ ParamsB P, 
                 const int bz = t / per_pair, rest = t - bz * per_pair;
                 if (again) __syncthreads();   // every thread is done with the previous tile's shared memory
                 again = true;
-                stack_b_tile<TH, TW, NT, SYM3, OWNOTH, LITE>(rest % nbx, rest / nbx, bz, nbx, nby, bsum2, P, tmap, M, orient,
-                                                             line_end, gray, winmax, tilemax, tile_flag, tm_split);
+                stack_b_tile<TH, TW, NT, STRUCTURED, LITE>(rest % nbx, rest / nbx, bz, nbx, nby, bsum2, P, tmap, M, orient,
+                                                       line_end, gray, winmax, tilemax, tile_flag, tm_split);
             }
             again = true;
         }
     } else {
-        stack_b_tile<TH, TW, NT, SYM3, OWNOTH, LITE>(blockIdx.x, blockIdx.y, blockIdx.z, gridDim.x, gridDim.y, bsum2, P, tmap,
-                                                     M, orient, line_end, gray, winmax, tilemax, tile_flag, tm_split);
+        stack_b_tile<TH, TW, NT, STRUCTURED, LITE>(blockIdx.x, blockIdx.y, blockIdx.z, gridDim.x, gridDim.y, bsum2, P, tmap,
+                                               M, orient, line_end, gray, winmax, tilemax, tile_flag, tm_split);
     }
 }
 
@@ -1629,9 +1609,8 @@ static int sm_count()
 struct StackPlanHost {
     ParamsA a;
     ParamsB b;
-    bool s1_depthwise, s2_rgby;
-    bool s2_shared;           // rgby_3's shared-surround structure (stack_a_kernel, S2 mode 2)
-    bool s3_sym, s5_ownoth;   // structure of the stripe / end filters (see stack_b_kernel)
+    bool a_structured;   // depthwise rgc and rgby_3's shared surround (stack_a_kernel)
+    bool b_structured;   // symmetric stripe and own / other end filters (stack_b_tile)
 };
 
 // S4 early-out threshold from the 49 blur taps taps[0], taps[stride], ...: the smallest float T with rn(w_min * T) >= 1,
@@ -1650,19 +1629,18 @@ static float quick_threshold(const float *taps, int stride)
     return (double)blur_min * (double)T >= 1.0001 && T < 1.0e20f ? T : 0.0f;
 }
 
-// stack_a's part (S1, S2): repack rgc and rgby ([3][3][3][3] HWIO) as (w, w) pairs and detect the structures its kernel
-// variants exploit. Any weights are accepted (the dense variant takes the rest).
+// stack_a's part (S1, S2): repack rgc and rgby ([3][3][3][3] HWIO) as (w, w) pairs and detect the structure of its
+// structured variant. Any weights are accepted (the dense variant takes the rest).
 static void pack_stack_a(const float *rgc, const float *rgby, int n, int h, int w, StackPlanHost *S)
 {
-    S->s1_depthwise = S->s2_rgby = true;
+    bool depthwise = true;
     for (int t = 0; t < 9; ++t)
         for (int ci = 0; ci < 3; ++ci)
             for (int co = 0; co < 3; ++co) {
                 const int i = (t * 3 + ci) * 3 + co;
                 S->a.w1[t][ci][co] = dup(rgc[i]);
                 S->a.w2[t][ci][co] = dup(rgby[i]);
-                if (ci != co && rgc[i] != 0.0f) S->s1_depthwise = false;
-                if (!rgby_nonzero(t, ci, co) && rgby[i] != 0.0f) S->s2_rgby = false;
+                if (ci != co && rgc[i] != 0.0f) depthwise = false;
             }
     {   // rgby_3 shared-surround structure (all comparisons bitwise; 2 * S is exact in float32)
         const float *R = rgby;
@@ -1676,7 +1654,7 @@ static void pack_stack_a(const float *rgc, const float *rgby, int n, int h, int 
                      bits_equal(at(t, 0, 0), 0.0f) && bits_equal(at(t, 1, 1), 0.0f) && bits_equal(at(t, 2, 2), 0.0f);
             S->a.s2s[t] = dup(sv);
         }
-        S->s2_shared = ok && S->s2_rgby;
+        S->a_structured = depthwise && ok;
         S->a.s2c[0] = dup(at(4, 0, 0)), S->a.s2c[1] = dup(at(4, 1, 1)), S->a.s2c[2] = dup(at(4, 2, 2));
         S->a.s2c[3] = dup(at(4, 1, 2)), S->a.s2c[4] = dup(at(4, 2, 1)), S->a.s2c[5] = dup(2.0f);
     }
@@ -1707,20 +1685,18 @@ static int pack_stack_b(const silent_stack_weights *W, int n, int h, int w, Stac
         S->b.wb[t] = dup(W->blur[t * 9]);
     }
     S->b.quick_thr = quick_threshold(W->blur, 9);
-    // stripe kernels symmetric under a 180-degree rotation: w3[0..4] already are the five distinct taps
-    S->s3_sym = true;
+    // structured: stripe kernels symmetric under a 180-degree rotation (w3[0..4] already are the five distinct taps) and
+    // an end filter whose input channel ci feeds both other output channels with the same kernel
+    S->b_structured = true;
     for (int t = 0; t < 4; ++t)
         for (int co = 0; co < 3; ++co)
-            if (!bits_equal(W->stripe[(t * 3) * 3 + co], W->stripe[((8 - t) * 3) * 3 + co])) S->s3_sym = false;
-    // end filter: input channel ci feeds both other output channels with the same kernel
-    S->s5_ownoth = true;
+            if (!bits_equal(W->stripe[(t * 3) * 3 + co], W->stripe[((8 - t) * 3) * 3 + co])) S->b_structured = false;
     for (int t = 0; t < 9; ++t)
         for (int ci = 0; ci < 3; ++ci) {
             const int o1 = (ci + 1) % 3, o2 = (ci + 2) % 3;
-            if (!bits_equal(W->end[(t * 3 + ci) * 3 + o1], W->end[(t * 3 + ci) * 3 + o2])) S->s5_ownoth = false;
+            if (!bits_equal(W->end[(t * 3 + ci) * 3 + o1], W->end[(t * 3 + ci) * 3 + o2])) S->b_structured = false;
         }
-    if (!(S->s3_sym && S->s5_ownoth)) S->s3_sym = S->s5_ownoth = false;   // two kernel variants: structured or dense
-    if (S->s5_ownoth)
+    if (S->b_structured)
         for (int t = 0; t < 9; ++t)
             for (int ci = 0; ci < 3; ++ci) {
                 S->b.w5[t][ci][0] = dup(W->end[(t * 3 + ci) * 3 + ci]);
@@ -1737,14 +1713,9 @@ static int pack_stack_b(const silent_stack_weights *W, int n, int h, int w, Stac
     return SILENT_OK;
 }
 
-#ifndef SILENT_TILE_HB
-#define SILENT_TILE_HB 16
-#endif
-#ifndef SILENT_TILE_HA
-#define SILENT_TILE_HA 16
-#endif
-// stack_a tile rows: TH + 2 must be a multiple of 3 (S1 row triples); with 22 the 8 triples of a tile fill a quarter-warp
-constexpr int kTileHA = SILENT_TILE_HA, kTileHB = SILENT_TILE_HB;   // stack_b tile rows (quick and full variant share the tile grid)
+// stack_a tile rows: TH + 2 must be a multiple of 3 (S1 row triples)
+constexpr int kTileHA = 16;
+constexpr int kTileHB = 16;   // stack_b tile rows (quick and full variant share the tile grid)
 
 // Tile width: the candidate that wastes the fewest columns of the last tile (288-wide levels: 6 x 48 instead of 4.5 x 64).
 static int pick_tile_w(int w) { return ceil_div(w, 48) * 48 < ceil_div(w, 64) * 64 ? 48 : 64; }
@@ -1816,15 +1787,15 @@ static const unsigned char *s1_deal_table()
     return d;
 }
 
-template <int TW, bool DW, int RGBY, bool PAIRED>
+template <int TW, bool STRUCTURED, bool PAIRED>
 static int launch_a(const void *pyr, const ParamsA &P, const CUtensorMap &tmap, f2 *bsum2, int pairs, cudaStream_t stream)
 {
     using T = TileA<kTileHA, TW>;
     constexpr int kThreadsA = ThreadsA<TW>::value;
-    auto kern = stack_a_kernel<kTileHA, TW, kThreadsA, DW, RGBY, PAIRED>;
+    auto kern = stack_a_kernel<kTileHA, TW, kThreadsA, STRUCTURED, PAIRED>;
     SILENT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::kSmemBytes));
     const dim3 grid(ceil_div(P.w, TW), ceil_div(P.h, kTileHA), pairs);
-    const unsigned char *deal = DW ? s1_deal_table<TW>() : nullptr;
+    const unsigned char *deal = STRUCTURED ? s1_deal_table<TW>() : nullptr;
     SILENT_CUDA(launch_dependent(kern, grid, dim3(kThreadsA), T::kSmemBytes, stream, pyr, P, tmap, bsum2, deal));
     SILENT_LAUNCH_CHECK("stack_a_kernel");
     return SILENT_OK;
@@ -1839,16 +1810,6 @@ static size_t stack_flag_bytes(int n, int h, int w)
 static size_t stack_plane_bytes(int n, int h, int w) { return ((size_t)(n / 2 + 8) * h * (w + 2) * sizeof(f2) + 255) / 256 * 256; }
 size_t stack_workspace_bytes(int n, int h, int w) { return stack_plane_bytes(n, h, w) + stack_flag_bytes(n, h, w) + 256; }
 
-// three variants: the reference's filters (depthwise rgc + shared-surround rgby), their zero patterns only, dense
-template <int TW, bool PAIRED>
-static int dispatch_a(bool dw, bool rgby, bool shared, const void *in, const ParamsA &P, const CUtensorMap &tmap, f2 *bsum2,
-                      int pairs, cudaStream_t stream)
-{
-    if (dw && shared) return launch_a<TW, true, 2, PAIRED>(in, P, tmap, bsum2, pairs, stream);
-    if (dw && rgby) return launch_a<TW, true, 1, PAIRED>(in, P, tmap, bsum2, pairs, stream);
-    return launch_a<TW, false, 0, PAIRED>(in, P, tmap, bsum2, pairs, stream);
-}
-
 template <int TH, int TW, bool STRUCTURED, bool LITE>
 static int launch_b(StackPlanHost &S, int pairs, f2 *bsum2, float *orient, float *line_end, float *gray, int *winmax,
                     int *tilemax, unsigned char *tile_flag, cudaStream_t stream)
@@ -1858,7 +1819,7 @@ static int launch_b(StackPlanHost &S, int pairs, f2 *bsum2, float *orient, float
     std::memset(&map_b, 0, sizeof(map_b));
     using TB = TileB<TH, TW, LITE>;
     constexpr int NT = ThreadsB<TH, TW, LITE>::value;
-    auto kern = stack_b_kernel<TH, TW, NT, STRUCTURED, STRUCTURED, LITE>;
+    auto kern = stack_b_kernel<TH, TW, NT, STRUCTURED, LITE>;
     SILENT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TB::kSmemBytes));
     S.b.use_tma = (w % 2) == 0 && make_pair_map(&map_b, bsum2, w + 2, h, pairs, TB::B_PITCH, TB::B_ROWS, 1);
     // outputs as TMA tile stores (one per 16 rows and image instead of one bulk copy per row) when every tile is whole in x
@@ -1889,8 +1850,12 @@ static int launch_stack_a(const void *pyr, StackPlanHost &S, bool paired_in, int
     using TA = TileA<kTileHA, TWA>;
     S.a.prefetch_pairs = 8;   // ~ the image pairs whose tiles are resident on the chip at once
     S.a.use_tma = paired_in && make_pair_map(&map_x, pyr, w, h, 3LL * pairs, TA::X_PITCH, TA::X_ROWS, 3);
-    return paired_in ? dispatch_a<TWA, true>(S.s1_depthwise, S.s2_rgby, S.s2_shared, pyr, S.a, map_x, bsum2, pairs, stream)
-                     : dispatch_a<TWA, false>(S.s1_depthwise, S.s2_rgby, S.s2_shared, pyr, S.a, map_x, bsum2, pairs, stream);
+    // two variants: the reference's filters (depthwise rgc + shared-surround rgby) or dense
+    if (S.a_structured)
+        return paired_in ? launch_a<TWA, true, true>(pyr, S.a, map_x, bsum2, pairs, stream)
+                         : launch_a<TWA, true, false>(pyr, S.a, map_x, bsum2, pairs, stream);
+    return paired_in ? launch_a<TWA, false, true>(pyr, S.a, map_x, bsum2, pairs, stream)
+                     : launch_a<TWA, false, false>(pyr, S.a, map_x, bsum2, pairs, stream);
 }
 
 template <int TW>
@@ -1901,7 +1866,7 @@ static int launch_stack(const void *pyr, StackPlanHost &S, bool paired_in, int p
     int rc = launch_stack_a<TW>(pyr, S, paired_in, pairs, bsum2, stream);   // (96-wide stack_a tiles: measured 8 % slower)
     if (rc != SILENT_OK) return rc;
     if (between_kernels) SILENT_CUDA(cudaEventRecord(between_kernels, stream));   // stage timing hook
-    if (!(S.s3_sym && S.s5_ownoth))
+    if (!S.b_structured)
         return launch_b<kTileHB, TW, false, false>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, nullptr, stream);
     // a grid that fits the device in about one wave (single frames, config C2) gains nothing from the quick variant's
     // higher occupancy and would pay for a second launch: the full variant does it alone

@@ -249,25 +249,34 @@ def test_fused_stack_bit_exact_random(seed, n, h, w, c_oracle, default_filters):
 
 @pytest.mark.parametrize("seed,n,h,w", [(35, 2, 64, 96), (36, 3, 37, 53), (37, 2, 30, 100)])
 def test_fused_stack_dense_variants_bit_exact(seed, n, h, w, c_oracle, default_filters):
-    """Weights without the generators' structure run the dense variants of both kernels (stack_a without the depthwise /
-    zero-pattern / shared-surround forms, stack_b without SYM3 / OWNOTH): bitwise against the oracle, which takes the
-    same dispatch. The widths cover the three routes a staged tile leaves by: tile stores, bulk rows, element-wise."""
+    """Weights without the generators' structure run the dense variants of both kernels (stack_a without its depthwise
+    rgc + shared-surround rgby form, stack_b without its symmetric-stripe + own / other end form): bitwise against the
+    oracle, which takes the same dispatch. The second weight set keeps the depthwise rgc, rgby_3's zero pattern and
+    stack_b's structure and breaks only the shared surround: stack_a runs dense there, like the oracle. The widths cover
+    the three routes a staged tile leaves by: tile stores, bulk rows, element-wise."""
     from pysilent_b200 import _lib, _ops
-    f = {k: np.array(v, copy=True) for k, v in default_filters.items()}
-    f["rgc"][1, 1, 0, 1] = 0.05          # not depthwise
-    f["rgby"][0, 0, 1, 2] *= 1.5         # not the shared surround (as in test_c_oracle_fused_order_uses_the_structures) ...
-    f["rgby"][0, 0, 1, 1] = 0.05         # ... nor the zero pattern
-    f["end"][2, 1, 0, 1] += 0.01         # not own / other
-    W = {k: np.ascontiguousarray(v, np.float32) for k, v in f.items()}
     L = c_oracle.lib()
-    assert not L.so_depthwise3(W["rgc"]) and not L.so_rgby_shared(W["rgby"]) and not L.so_end_ownoth(W["end"])
+    f32 = lambda a: np.ascontiguousarray(a, np.float32)
+    dense = {k: np.array(v, copy=True) for k, v in default_filters.items()}
+    dense["rgc"][1, 1, 0, 1] = 0.05          # not depthwise
+    dense["rgby"][0, 0, 1, 2] *= 1.5         # not the shared surround (as in test_c_oracle_fused_order_uses_the_structures) ...
+    dense["rgby"][0, 0, 1, 1] = 0.05         # ... nor the zero pattern
+    dense["end"][2, 1, 0, 1] += 0.01         # not own / other
+    assert not L.so_depthwise3(f32(dense["rgc"])) and not L.so_rgby_shared(f32(dense["rgby"]))
+    assert not L.so_end_ownoth(f32(dense["end"]))
+    zeros = {k: np.array(v, copy=True) for k, v in default_filters.items()}
+    zeros["rgby"][0, 0, 1, 2] *= 1.5         # not the shared surround; every structural zero of rgby_3 stays zero
+    assert np.array_equal(zeros["rgby"] == 0, default_filters["rgby"] == 0)
+    assert L.so_depthwise3(f32(zeros["rgc"])) and not L.so_rgby_shared(f32(zeros["rgby"]))
+    assert L.so_stripe_sym180(f32(zeros["stripe"])) and L.so_end_ownoth(f32(zeros["end"]))
     pyr = _pyr(seed, n, h, w)
-    orient, line_end, gray = _ops.stack_fused(pyr, _lib.make_stack_weights(f["rgc"], f["rgby"], f["stripe"], f["blur"],
-                                                                           f["end"]))
-    ref = c_oracle.line_end_stack(pyr, f)
-    assert_bits(orient, ref["orient"], "orient")
-    assert_bits(line_end, ref["padded"], "padded_line_end")
-    assert_bits(gray, ref["gray"], "gray")
+    for name, f in (("dense", dense), ("rgby_3 zero pattern", zeros)):
+        orient, line_end, gray = _ops.stack_fused(pyr, _lib.make_stack_weights(f["rgc"], f["rgby"], f["stripe"],
+                                                                               f["blur"], f["end"]))
+        ref = c_oracle.line_end_stack(pyr, f)
+        assert_bits(orient, ref["orient"], "orient, " + name)
+        assert_bits(line_end, ref["padded"], "padded_line_end, " + name)
+        assert_bits(gray, ref["gray"], "gray, " + name)
 
 
 def test_fused_stack_rejects_unstructured_weights():
@@ -914,43 +923,58 @@ def test_pipeline_low_contrast_frames(c_oracle, default_filters):
     _check_stack(host, ref, None, "low contrast, host")
 
 
-@pytest.mark.parametrize("knobs", [{"SILENT_PYRAMID_TEX": "0"}, {"SILENT_PYRAMID_TEXTAB": "3"}, {"SILENT_PYRAMID_TEXTAB": "0"}])
-def test_pyramid_texture_and_ldg_variants_bit_identical(knobs, monkeypatch, c_oracle, default_filters):
-    """pyramid_pair_kernel fetches frame rows (and its phase-H table) through the texture path by default; the LDG
-    variant and the other table routings are the same arithmetic: bitwise equal to the default and to the oracle, on a
-    batch whose frames differ (texel indices of frame B) and an odd batch (frame B = frame A in the last pair)."""
-    from pysilent_b200 import LineEndPipeline
-    frames = np.stack([synthetic_frame(2, i, 360, 640) for i in range(5)])
-    dev = torch.from_numpy(frames).cuda()
-    base = LineEndPipeline(zoom_ratio=1.5).run_frames(dev)
-    for k, v in knobs.items():
-        monkeypatch.setenv(k, v)   # read at plan creation: a fresh pipeline makes a fresh plan
-    other = LineEndPipeline(zoom_ratio=1.5).run_frames(dev)
-    for name in ("orient", "padded_line_end"):
-        a, b = getattr(base, name).cpu().numpy(), getattr(other, name).cpu().numpy()
-        assert np.array_equal(a.view(np.uint32), b.view(np.uint32)), "%s differs with %s" % (name, knobs)
-    assert np.array_equal(base.points.cpu().numpy(), other.points.cpu().numpy())
-    _, ref = _oracle_pipeline(c_oracle, frames, (288, 192), 1.5, default_filters)
-    _check_stack(other, ref, None, "pyramid variant %s" % (knobs,))
+def _texture_alignment():
+    """cudaDevAttrTextureAlignment of the current device, from the CUDA runtime torch has loaded (torch does not expose
+    it): a linear texture's devPtr must be a multiple of it, so pyramid_pair_kernel reads other frame pointers by LDG."""
+    import ctypes
+    rt = ctypes.CDLL("libcudart.so.%s" % torch.version.cuda.split(".")[0])
+    value = ctypes.c_int()
+    assert rt.cudaDeviceGetAttribute(ctypes.byref(value), 14, torch.cuda.current_device()) == 0   # 14: TextureAlignment
+    return value.value
 
 
 def test_pyramid_texture_path_unaligned_frame_pointer(c_oracle, default_filters):
-    """Frames handed over as a slice of a larger device buffer: the pointer is 16-byte aligned (required) but not aligned
-    to the texture alignment (672000-byte frames). Whether the driver accepts the linear texture or the launch falls back
-    to the LDG variant, the results are the oracle's; many different slices cycle through the plan's texture table."""
+    """Frames handed over as a slice of a larger device buffer: the pointer is 16-byte aligned (required) but need not be
+    aligned to the device's texture alignment. pyramid_pair_kernel reads frames at that alignment through the texture path
+    and any others through its LDG variant, which is the same arithmetic; the code picks the route from the pointer.
+     * a buffer at byte offset 16 (LDG), on a batch whose frames differ (texel indices of frame B) and that is odd (frame
+       B = frame A in the last pair): bitwise equal to the run from an aligned buffer (texture) and to the oracle;
+     * slices of a batch of 672000-byte frames: frame 1 starts off the alignment (LDG), frames 0 and 2 on it (texture);
+     * 70 texture-aligned buffers, more than the plan's table of frame textures holds: the table is flushed (after a
+       synchronisation) and refilled, and every result is the oracle's."""
     from pysilent_b200 import LineEndPipeline
+    align = _texture_alignment()
+    assert align > 16 and 672000 % align != 0, "the LDG cases below need a texture alignment above 16 bytes, got %d" % align
+    frames = np.stack([synthetic_frame(2, i, 360, 640) for i in range(5)])
+    dev = torch.from_numpy(frames).cuda()
+    assert dev.data_ptr() % align == 0
+    base = LineEndPipeline(zoom_ratio=1.5).run_frames(dev)
+    buf = torch.zeros(frames.size + 16, dtype=torch.uint8, device="cuda")
+    shifted = buf[16:].view(frames.shape)
+    assert shifted.data_ptr() % align != 0
+    shifted.copy_(dev)
+    other = LineEndPipeline(zoom_ratio=1.5).run_frames(shifted)
+    for name in ("orient", "padded_line_end"):
+        a, b = getattr(base, name).cpu().numpy(), getattr(other, name).cpu().numpy()
+        assert np.array_equal(a.view(np.uint32), b.view(np.uint32)), "%s differs at byte offset 16" % name
+    assert np.array_equal(base.points.cpu().numpy(), other.points.cpu().numpy())
+    _, ref = _oracle_pipeline(c_oracle, frames, (288, 192), 1.5, default_filters)
+    _check_stack(other, ref, None, "frames at byte offset 16")
+
     frames = np.stack([synthetic_frame(7, i, 2000, 112) for i in range(4)])
     dev = torch.from_numpy(frames).cuda()
     pipe = LineEndPipeline(zoom_ratio=1.5)
     for lo, hi in ((1, 3), (1, 4), (2, 4), (0, 4)):
         _, ref = _oracle_pipeline(c_oracle, frames[lo:hi], (288, 192), 1.5, default_filters)
         _check_stack(pipe.run_frames(dev[lo:hi]), ref, None, "frames[%d:%d]" % (lo, hi))
-    big = torch.zeros(70 * 4 * 96 * 160 * 3 + 16, dtype=torch.uint8, device="cuda")
     small = np.stack([synthetic_frame(3, i, 96, 160) for i in range(2)])
+    assert small.size % align == 0
+    big = torch.zeros(70 * small.size, dtype=torch.uint8, device="cuda")
     _, ref = _oracle_pipeline(c_oracle, small, (32, 24), 1.5, default_filters)
     pipe2 = LineEndPipeline(output_size=(32, 24), zoom_ratio=1.5)
     for i in range(70):   # more distinct buffers than the table holds: it is flushed (after a synchronisation) and refilled
-        view = big[16 + i * small.size: 16 + (i + 1) * small.size].view(small.shape)
+        view = big[i * small.size: (i + 1) * small.size].view(small.shape)
+        assert view.data_ptr() % align == 0
         view.copy_(torch.from_numpy(small))
         res = pipe2.run_frames(view)
         if i in (0, 1, 63, 64, 65, 69):
