@@ -323,6 +323,33 @@ int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weig
                              int batch, float *orient_host, float *line_end_host, int64_t *points_host,
                              int64_t capacity, int64_t *count_host, silent_stream stream);
 
+/* ---- binary16 outputs ---------------------------------------------------------------------------------------------
+ * The five calls below are their float32 counterparts above with orient and line_end stored as IEEE binary16: each
+ * output holds the bit patterns (uint16_t) of the float32 value the counterpart computes, rounded once to nearest even
+ * (subnormals kept, overflow to +-inf, NaN stays NaN with an unspecified payload) -- what torch's Tensor.half() does to
+ * the float32 result. Everything else is computed from the float32 values exactly as by the counterpart: gray (still
+ * float32), the regulator's early-out, and the feature points, which are bit-identical to the counterpart's. Output
+ * bytes halve. Arguments, checks (all on the host, before any CUDA call) and status codes are those of the counterpart.
+ * uint8 frames through the three-orientation stack stay far inside binary16's range (orient <= ~5.7e3, line_end <= 255),
+ * with 11 significant bits (steps of 0.125 just below 255). */
+int silent_stack_fused_f16(const float *pyramid_dev, int n, int h, int w, const silent_stack_weights *weights_host,
+                           uint16_t *orient_dev, uint16_t *line_end_dev, float *gray_dev, void *workspace_dev,
+                           size_t workspace_bytes, silent_stream stream);
+int silent_stack_bank_f16(const float *pyramid_dev, int n, int h, int w, const silent_orientation_bank *bank_host,
+                          uint16_t *orient_dev, uint16_t *line_end_dev, float *gray_dev, void *workspace_dev,
+                          size_t workspace_bytes, silent_stream stream);
+int silent_pipeline_run_f16(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_dev, int batch,
+                            float *pyramid_dev, uint16_t *orient_dev, uint16_t *line_end_dev, int64_t *points_dev,
+                            int64_t capacity, int64_t *count_dev, silent_stream stream);
+int silent_pipeline_run_orientations_f16(silent_plan *plan, const silent_orientation_bank *bank_host,
+                                         const void *frames_dev, int batch, uint16_t *orient_dev, uint16_t *line_end_dev,
+                                         int64_t *points_dev, int64_t capacity, int64_t *count_dev, silent_stream stream);
+/* The host-buffer call with binary16 outputs: its pinned staging mirrors and its device-to-host copies are half the
+ * bytes of silent_pipeline_run_host's. */
+int silent_pipeline_run_host_f16(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_host,
+                                 int batch, uint16_t *orient_host, uint16_t *line_end_host, int64_t *points_host,
+                                 int64_t capacity, int64_t *count_host, silent_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

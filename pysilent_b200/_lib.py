@@ -27,6 +27,8 @@ SYMBOLS = (
     "silent_pipeline_run_host", "silent_pipeline_run_bank", "silent_pipeline_run_orientations", "silent_stack_bank", "silent_get_centroids", "silent_resize_nearest", "silent_get_boosting", "silent_pointwise", "silent_display_tensors",
     "silent_display_sequence_scratch_bytes", "silent_display_sequence", "silent_pack_points",
     "silent_comm_unique_id", "silent_comm_create", "silent_comm_destroy", "silent_comm_check", "silent_gather_points",
+    "silent_stack_fused_f16", "silent_stack_bank_f16", "silent_pipeline_run_f16", "silent_pipeline_run_orientations_f16",
+    "silent_pipeline_run_host_f16",
 )
 
 
@@ -109,6 +111,12 @@ def lib():
         "silent_pipeline_run_bank": (i, [p, ctypes.POINTER(SilentBankWeights), p, i, p, p, p, i64, p, p]),
         "silent_pipeline_run_orientations": (i, [p, ctypes.POINTER(SilentOrientationBank), p, i, p, p, p, i64, p, p]),
         "silent_stack_bank": (i, [p, i, i, i, ctypes.POINTER(SilentOrientationBank), p, p, p, p, sz, p]),
+        # binary16 outputs: the same arguments, orient / line_end as uint16_t bit patterns (np.float16, torch.float16)
+        "silent_stack_fused_f16": (i, [p, i, i, i, ctypes.POINTER(SilentStackWeights), p, p, p, p, sz, p]),
+        "silent_stack_bank_f16": (i, [p, i, i, i, ctypes.POINTER(SilentOrientationBank), p, p, p, p, sz, p]),
+        "silent_pipeline_run_f16": (i, [p, ctypes.POINTER(SilentStackWeights), p, i, p, p, p, p, i64, p, p]),
+        "silent_pipeline_run_orientations_f16": (i, [p, ctypes.POINTER(SilentOrientationBank), p, i, p, p, p, i64, p, p]),
+        "silent_pipeline_run_host_f16": (i, [p, ctypes.POINTER(SilentStackWeights), p, i, p, p, p, i64, p, p]),
         "silent_get_centroids": (i, [p, i, i, i, i, i, p, p, p, p]),
         "silent_resize_nearest": (i, [p, i, i, i, i, i, i, p, p]),
         "silent_get_boosting": (i, [p, p, i, i, i, f, f, i, p, p, p]),

@@ -279,15 +279,23 @@ def display_sequence_scratch_bytes(steps, n, h, w, region_h, region_w):
                                                                 int(region_w)))
 
 
-def _stack(symbol, noun, pyramid, weights, channels, want_orient, want_line_end, want_gray):
+# output dtypes of the fused stacks: float32, or binary16 through the entry points named <symbol>_f16
+OUT_DTYPES = (torch.float32, torch.float16)
+
+
+def _stack(symbol, noun, pyramid, weights, channels, want_orient, want_line_end, want_gray, out_dtype):
+    if out_dtype not in OUT_DTYPES:
+        raise ValueError("%s writes float32 or float16 outputs, not %s" % (noun, out_dtype))
     x = as_device_tensor(pyramid)
     n, h, w, c = _nhwc(x, symbol[len("silent_"):])
     if c != 3:
         raise ValueError("%s needs 3-channel pyramids" % noun)
-    mk = lambda ch: torch.empty((n, h, w, ch), dtype=torch.float32, device=x.device)  # noqa: E731
-    orient = mk(channels) if want_orient else None
-    line_end = mk(channels) if want_line_end else None
-    gray = mk(1) if want_gray else None
+    if out_dtype == torch.float16:
+        symbol += "_f16"
+    mk = lambda ch, dt: torch.empty((n, h, w, ch), dtype=dt, device=x.device)  # noqa: E731
+    orient = mk(channels, out_dtype) if want_orient else None
+    line_end = mk(channels, out_dtype) if want_line_end else None
+    gray = mk(1, torch.float32) if want_gray else None
     nbytes = _lib.lib().silent_stack_workspace_bytes(n, h, w)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
     with torch.cuda.device(x.device):
@@ -296,12 +304,16 @@ def _stack(symbol, noun, pyramid, weights, channels, want_orient, want_line_end,
     return orient, line_end, gray
 
 
-def stack_fused(pyramid, weights, want_orient=True, want_line_end=True, want_gray=True):
-    return _stack("silent_stack_fused", "the fused stack", pyramid, weights, 3, want_orient, want_line_end, want_gray)
+def stack_fused(pyramid, weights, want_orient=True, want_line_end=True, want_gray=True, out_dtype=torch.float32):
+    """The fused three-orientation stack (``silent_stack_fused``, or ``silent_stack_fused_f16`` for float16 outputs) on a
+    finite NHWC pyramid: orient and padded_line_end ``[n, h, w, 3]`` of ``out_dtype``, gray ``[n, h, w, 1]`` float32."""
+    return _stack("silent_stack_fused", "the fused stack", pyramid, weights, 3, want_orient, want_line_end, want_gray,
+                  out_dtype)
 
 
-def stack_bank(pyramid, bank, want_orient=True, want_line_end=True, want_gray=True):
-    """The orientation bank's stack (``silent_stack_bank``) on a finite NHWC pyramid ``[n, h, w, 3]``: returns orient and
-    padded_line_end ``[n, h, w, bank.orientations]`` and gray ``[n, h, w, 1]``."""
+def stack_bank(pyramid, bank, want_orient=True, want_line_end=True, want_gray=True, out_dtype=torch.float32):
+    """The orientation bank's stack (``silent_stack_bank``, or ``silent_stack_bank_f16`` for float16 outputs) on a finite
+    NHWC pyramid ``[n, h, w, 3]``: returns orient and padded_line_end ``[n, h, w, bank.orientations]`` of ``out_dtype``
+    and gray ``[n, h, w, 1]`` float32."""
     return _stack("silent_stack_bank", "the fused orientation bank", pyramid, bank, int(bank.orientations), want_orient,
-                  want_line_end, want_gray)
+                  want_line_end, want_gray, out_dtype)

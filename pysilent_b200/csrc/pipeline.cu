@@ -140,10 +140,12 @@ static TileMaxima tile_maxima(const silent_plan *plan)
 // K1 + K2 for frames [frame0, frame0 + nb) of a batch: the outputs, gray and the region maxima of these frames land at
 // their place in the whole-batch tensors, so that the emit stage can run once over the batch afterwards. frame0 must be
 // even on the frame-pair path (pairs never straddle a chunk). K2 is the three-orientation stack (W) or, when bank is set,
-// the orientation bank's stack (frame-pair path only; no tile flags, geo must be null).
+// the orientation bank's stack (frame-pair path only; no tile flags, geo must be null). orient_dev / line_end_dev hold
+// float32, or binary16 when half_out.
 static int run_stack_stages(silent_plan *plan, const silent_stack_weights *W, const silent_orientation_bank *bank,
-                            const void *frames_dev, int frame0, int nb, float *pyramid_dev, float *orient_dev,
-                            float *line_end_dev, const WindowGeom *geo, cudaStream_t s, const PairClear *also_clear = nullptr)
+                            const void *frames_dev, int frame0, int nb, float *pyramid_dev, void *orient_dev,
+                            void *line_end_dev, bool half_out, const WindowGeom *geo, cudaStream_t s,
+                            const PairClear *also_clear = nullptr)
 {
     Workspace &ws = plan->ws;
     const bool pair_path = pyramid_pair_supported(plan);
@@ -183,14 +185,15 @@ static int run_stack_stages(silent_plan *plan, const silent_stack_weights *W, co
                                 : (const void *)(pyramid_dev ? pyramid_dev + img0 * level_elems * 3 : ws.d_pyramid);
     if (plan->timing) SILENT_CUDA(cudaEventRecord(plan->ev[1], s));
     const size_t ch = bank ? bank->orientations : 3;
-    float *orient = orient_dev ? orient_dev + img0 * level_elems * ch : nullptr;
-    float *line_end = line_end_dev ? line_end_dev + img0 * level_elems * ch : nullptr;
+    const size_t out_offset = img0 * level_elems * ch * (half_out ? 2 : sizeof(float));   // bytes
+    void *orient = orient_dev ? (char *)orient_dev + out_offset : nullptr;
+    void *line_end = line_end_dev ? (char *)line_end_dev + out_offset : nullptr;
     cudaEvent_t mid = plan->timing ? plan->ev_mid : nullptr;
     if (bank)
-        return stack_bank(pyr, n, plan->h, plan->w, plan->levels, bank, orient, line_end, ws.d_gray + img0 * level_elems,
-                          ws.d_stack, ws.stack_bytes, s, mid);
+        return stack_bank(pyr, n, plan->h, plan->w, plan->levels, bank, orient, line_end, half_out,
+                          ws.d_gray + img0 * level_elems, ws.d_stack, ws.stack_bytes, s, mid);
     const TileMaxima tm = tile_maxima(plan);
-    return stack_fused(pyr, n, plan->h, plan->w, pair_path ? plan->levels : 0, W, orient, line_end,
+    return stack_fused(pyr, n, plan->h, plan->w, pair_path ? plan->levels : 0, W, orient, line_end, half_out,
                        ws.d_gray + img0 * level_elems, ws.d_stack, ws.stack_bytes, geo,
                        geo ? ws.d_winmax + img0 * geo->count : nullptr, ws.d_tilemax + img0 * tm.nty * tm.ntx, s, mid, true);
 }
@@ -209,10 +212,11 @@ static int check_pipeline_args(const char *who, const silent_plan *plan, const v
 }
 
 // pyramid -> stack -> emit of a batch resident in HBM, with the three-orientation stack (W) or an orientation bank
-// (bank). The bank's kernel reduces neither region nor tile maxima: its emit scans gray on its own.
+// (bank). The bank's kernel reduces neither region nor tile maxima: its emit scans gray on its own. Outputs in float32,
+// or binary16 when half_out.
 static int run_pipeline(silent_plan *plan, const silent_stack_weights *W, const silent_orientation_bank *bank,
-                        const void *frames_dev, int batch, float *pyramid_dev, float *orient_dev, float *line_end_dev,
-                        int64_t *points_dev, int64_t capacity, int64_t *count_dev, cudaStream_t s)
+                        const void *frames_dev, int batch, float *pyramid_dev, void *orient_dev, void *line_end_dev,
+                        bool half_out, int64_t *points_dev, int64_t capacity, int64_t *count_dev, cudaStream_t s)
 {
     Workspace &ws = plan->ws;
     if (ws.batch < batch)
@@ -224,7 +228,7 @@ static int run_pipeline(silent_plan *plan, const silent_stack_weights *W, const 
     const bool fuse_windows = !bank && count_dev && window_geometry(plan->h, plan->w, plan->h / 2, plan->w / 2, &geo);
     PairClear winmax_clear;   // the region maxima start at 0: cleared together with the tile flags (see run_stack_stages)
     if (fuse_windows) winmax_clear.b = ws.d_winmax, winmax_clear.b_bytes = (size_t)n * geo.count * sizeof(int);
-    int rc = run_stack_stages(plan, W, bank, frames_dev, 0, batch, pyramid_dev, orient_dev, line_end_dev,
+    int rc = run_stack_stages(plan, W, bank, frames_dev, 0, batch, pyramid_dev, orient_dev, line_end_dev, half_out,
                               fuse_windows ? &geo : nullptr, s, &winmax_clear);
     if (rc != SILENT_OK) return rc;
     if (timing) SILENT_CUDA(cudaEventRecord(plan->ev[2], s));
@@ -239,13 +243,45 @@ static int run_pipeline(silent_plan *plan, const silent_stack_weights *W, const 
     return rc;
 }
 
+// shared body of silent_pipeline_run and silent_pipeline_run_f16
+static int pipeline_run_entry(const char *who, silent_plan *plan, const silent_stack_weights *weights_host,
+                              const void *frames_dev, int batch, float *pyramid_dev, void *orient_dev, void *line_end_dev,
+                              bool half_out, int64_t *points_dev, int64_t capacity, int64_t *count_dev, silent_stream stream)
+{
+    const int rc = check_pipeline_args(who, plan, weights_host, frames_dev, batch);
+    if (rc != SILENT_OK) return rc;
+    return run_pipeline(plan, weights_host, nullptr, frames_dev, batch, pyramid_dev, orient_dev, line_end_dev, half_out,
+                        points_dev, capacity, count_dev, (cudaStream_t)stream);
+}
+
 int silent_pipeline_run(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_dev, int batch,
                         float *pyramid_dev, float *orient_dev, float *line_end_dev, int64_t *points_dev,
                         int64_t capacity, int64_t *count_dev, silent_stream stream)
 {
-    const int rc = check_pipeline_args("silent_pipeline_run", plan, weights_host, frames_dev, batch);
+    return pipeline_run_entry("silent_pipeline_run", plan, weights_host, frames_dev, batch, pyramid_dev, orient_dev,
+                              line_end_dev, false, points_dev, capacity, count_dev, stream);
+}
+
+int silent_pipeline_run_f16(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_dev, int batch,
+                            float *pyramid_dev, uint16_t *orient_dev, uint16_t *line_end_dev, int64_t *points_dev,
+                            int64_t capacity, int64_t *count_dev, silent_stream stream)
+{
+    return pipeline_run_entry("silent_pipeline_run_f16", plan, weights_host, frames_dev, batch, pyramid_dev, orient_dev,
+                              line_end_dev, true, points_dev, capacity, count_dev, stream);
+}
+
+// shared body of silent_pipeline_run_orientations and silent_pipeline_run_orientations_f16
+static int pipeline_run_orientations_entry(const char *who, silent_plan *plan, const silent_orientation_bank *bank_host,
+                                           const void *frames_dev, int batch, void *orient_dev, void *line_end_dev,
+                                           bool half_out, int64_t *points_dev, int64_t capacity, int64_t *count_dev,
+                                           silent_stream stream)
+{
+    int rc = check_bank(bank_host, who);
+    if (rc == SILENT_OK) rc = check_pipeline_args(who, plan, bank_host, frames_dev, batch);
     if (rc != SILENT_OK) return rc;
-    return run_pipeline(plan, weights_host, nullptr, frames_dev, batch, pyramid_dev, orient_dev, line_end_dev, points_dev,
+    if (!pyramid_pair_supported(plan))
+        return fail(SILENT_E_SHAPE, "the fused orientation bank needs uint8 frames with 3 colours (frame-pair pyramid path)");
+    return run_pipeline(plan, nullptr, bank_host, frames_dev, batch, nullptr, orient_dev, line_end_dev, half_out, points_dev,
                         capacity, count_dev, (cudaStream_t)stream);
 }
 
@@ -253,14 +289,16 @@ int silent_pipeline_run_orientations(silent_plan *plan, const silent_orientation
                                      int batch, float *orient_dev, float *line_end_dev, int64_t *points_dev,
                                      int64_t capacity, int64_t *count_dev, silent_stream stream)
 {
-    const char *who = "silent_pipeline_run_orientations";
-    int rc = check_bank(bank_host, who);
-    if (rc == SILENT_OK) rc = check_pipeline_args(who, plan, bank_host, frames_dev, batch);
-    if (rc != SILENT_OK) return rc;
-    if (!pyramid_pair_supported(plan))
-        return fail(SILENT_E_SHAPE, "the fused orientation bank needs uint8 frames with 3 colours (frame-pair pyramid path)");
-    return run_pipeline(plan, nullptr, bank_host, frames_dev, batch, nullptr, orient_dev, line_end_dev, points_dev, capacity,
-                        count_dev, (cudaStream_t)stream);
+    return pipeline_run_orientations_entry("silent_pipeline_run_orientations", plan, bank_host, frames_dev, batch,
+                                           orient_dev, line_end_dev, false, points_dev, capacity, count_dev, stream);
+}
+
+int silent_pipeline_run_orientations_f16(silent_plan *plan, const silent_orientation_bank *bank_host,
+                                         const void *frames_dev, int batch, uint16_t *orient_dev, uint16_t *line_end_dev,
+                                         int64_t *points_dev, int64_t capacity, int64_t *count_dev, silent_stream stream)
+{
+    return pipeline_run_orientations_entry("silent_pipeline_run_orientations_f16", plan, bank_host, frames_dev, batch,
+                                           orient_dev, line_end_dev, true, points_dev, capacity, count_dev, stream);
 }
 
 int silent_pipeline_run_bank(silent_plan *plan, const silent_bank_weights *weights_host, const void *frames_dev, int batch,
@@ -324,11 +362,12 @@ int silent_plan_stack_split_ms(silent_plan *plan, float *stack_a_ms, float *stac
     return SILENT_OK;
 }
 
-int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_host,
-                             int batch, float *orient_host, float *line_end_host, int64_t *points_host,
-                             int64_t capacity, int64_t *count_host, silent_stream stream)
+// shared body of silent_pipeline_run_host and silent_pipeline_run_host_f16: outputs of float32, or binary16 when half_out
+static int pipeline_run_host(const char *who, silent_plan *plan, const silent_stack_weights *weights_host,
+                             const void *frames_host, int batch, void *orient_host, void *line_end_host, bool half_out,
+                             int64_t *points_host, int64_t capacity, int64_t *count_host, silent_stream stream)
 {
-    int rc = check_pipeline_args("silent_pipeline_run_host", plan, weights_host, frames_host, batch);
+    int rc = check_pipeline_args(who, plan, weights_host, frames_host, batch);
     if (rc != SILENT_OK) return rc;
     if (capacity < 0) return fail(SILENT_E_INVAL, "capacity must be >= 0");
     rc = silent_plan_reserve(plan, batch);
@@ -337,7 +376,7 @@ int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weig
     cudaStream_t s = (cudaStream_t)stream;
     const size_t fbytes = frame_bytes(plan);
     const size_t n = (size_t)batch * plan->levels;
-    const size_t image_bytes = (size_t)plan->h * plan->w * 3 * sizeof(float);
+    const size_t image_bytes = (size_t)plan->h * plan->w * 3 * (half_out ? 2 : sizeof(float));   // one output level
     const size_t cap_tensor_bytes = (size_t)ws.batch * plan->levels * image_bytes;
 
     // Three queues: s_in (host -> HBM), the caller's stream (kernels), s_out (HBM -> host). The batch is cut into chunks
@@ -353,9 +392,19 @@ int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weig
     const bool orient_direct = orient_host && is_pinned(orient_host, n * image_bytes);
     const bool line_end_direct = line_end_host && is_pinned(line_end_host, n * image_bytes);
     if (!frames_direct && !ws.h_frames) SILENT_CUDA(cudaMallocHost(&ws.h_frames, fbytes * ws.batch));
-    if (orient_host && !orient_direct && !ws.h_orient) SILENT_CUDA(cudaMallocHost(&ws.h_orient, cap_tensor_bytes));
-    if (line_end_host && !line_end_direct && !ws.h_line_end)
-        SILENT_CUDA(cudaMallocHost(&ws.h_line_end, cap_tensor_bytes));
+    // the mirrors are sized for this call's element type; a later call with wider elements replaces them (nothing is
+    // in flight on them between calls: every call drains its queues before it returns)
+    auto mirror = [&](void *&buf, size_t &bytes) -> int {
+        if (buf && bytes >= cap_tensor_bytes) return SILENT_OK;
+        cudaFreeHost(buf);
+        buf = nullptr, bytes = 0;
+        SILENT_CUDA(cudaMallocHost(&buf, cap_tensor_bytes));
+        bytes = cap_tensor_bytes;
+        return SILENT_OK;
+    };
+    if (orient_host && !orient_direct) rc = mirror(ws.h_orient, ws.h_orient_bytes);
+    if (rc == SILENT_OK && line_end_host && !line_end_direct) rc = mirror(ws.h_line_end, ws.h_line_end_bytes);
+    if (rc != SILENT_OK) return rc;
     char *orient_dst = (char *)(orient_direct ? orient_host : ws.h_orient);
     char *line_end_dst = (char *)(line_end_direct ? line_end_host : ws.h_line_end);
 
@@ -397,7 +446,7 @@ int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weig
             SILENT_CUDA(cudaStreamWaitEvent(s, ws.ev_in[chunk], 0));
             const int rcs = run_stack_stages(plan, weights_host, nullptr, ws.d_frames, f0, nb, nullptr,
                                              orient_host ? ws.d_orient : nullptr, line_end_host ? ws.d_line_end : nullptr,
-                                             fuse_windows ? &geo : nullptr, s);
+                                             half_out, fuse_windows ? &geo : nullptr, s);
             if (rcs != SILENT_OK) return rcs;
             SILENT_CUDA(cudaEventRecord(ws.ev_done[chunk], s));
             SILENT_CUDA(cudaStreamWaitEvent(ws.s_out, ws.ev_done[chunk], 0));
@@ -423,7 +472,7 @@ int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weig
     if (rc != SILENT_OK) return rc;
     {
         const cudaError_t late = cudaGetLastError();   // an asynchronous failure surfaces at the synchronisation
-        if (late != cudaSuccess) return fail(SILENT_E_CUDA, "silent_pipeline_run_host: %s", cudaGetErrorString(late));
+        if (late != cudaSuccess) return fail(SILENT_E_CUDA, "%s: %s", who, cudaGetErrorString(late));
     }
     const size_t tensor_bytes = n * image_bytes;
     if (orient_host && !orient_direct) std::memcpy(orient_host, ws.h_orient, tensor_bytes);
@@ -435,6 +484,22 @@ int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weig
         std::memcpy(points_host, ws.h_points, rows * 4 * sizeof(int64_t));
     }
     return SILENT_OK;
+}
+
+int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_host,
+                             int batch, float *orient_host, float *line_end_host, int64_t *points_host,
+                             int64_t capacity, int64_t *count_host, silent_stream stream)
+{
+    return pipeline_run_host("silent_pipeline_run_host", plan, weights_host, frames_host, batch, orient_host, line_end_host,
+                             false, points_host, capacity, count_host, stream);
+}
+
+int silent_pipeline_run_host_f16(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_host,
+                                 int batch, uint16_t *orient_host, uint16_t *line_end_host, int64_t *points_host,
+                                 int64_t capacity, int64_t *count_host, silent_stream stream)
+{
+    return pipeline_run_host("silent_pipeline_run_host_f16", plan, weights_host, frames_host, batch, orient_host,
+                             line_end_host, true, points_host, capacity, count_host, stream);
 }
 
 }  // extern "C"

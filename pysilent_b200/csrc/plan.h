@@ -43,8 +43,9 @@ struct Workspace {
     int64_t points_capacity = 0;
     int64_t *d_count = nullptr;
     void *h_frames = nullptr;      // pinned mirrors
-    float *h_orient = nullptr;
-    float *h_line_end = nullptr;
+    void *h_orient = nullptr;      // ... of h_orient_bytes / h_line_end_bytes (sized by the output element type)
+    void *h_line_end = nullptr;
+    size_t h_orient_bytes = 0, h_line_end_bytes = 0;
     int64_t *h_points = nullptr;
     int64_t *h_count = nullptr;
     // silent_pipeline_run_host: upload / download queues and per-chunk events (chunked, overlapped transfers)

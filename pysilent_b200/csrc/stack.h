@@ -14,8 +14,9 @@ struct WindowGeom {
 };
 
 size_t stack_workspace_bytes(int n, int h, int w);
-int stack_fused(const void *pyr, int n, int h, int w, int pair_levels, const silent_stack_weights *W, float *orient,
-                float *line_end, float *gray, void *workspace, size_t workspace_bytes, const WindowGeom *geo,
+// orient / line_end: float32 outputs, or binary16 (uint16_t bit patterns) when half_out; gray is float32 either way
+int stack_fused(const void *pyr, int n, int h, int w, int pair_levels, const silent_stack_weights *W, void *orient,
+                void *line_end, bool half_out, float *gray, void *workspace, size_t workspace_bytes, const WindowGeom *geo,
                 int *winmax, int *tilemax, cudaStream_t stream, cudaEvent_t between_kernels = nullptr,
                 bool flags_clean = false);
 int stack_clear_flags(void *workspace, int n, int h, int w, cudaStream_t stream);
@@ -30,9 +31,10 @@ struct TileMaxima {
 
 // orientation bank of W->orientations = 4, 8, 12 or 16 (config C4: 8): pyr -> orient / line_end [n,h,w,nb], gray [n,h,w].
 // pyr as in stack_fused: NHWC [n][h][w][3] when pair_levels == 0, else the pyramid_pair_kernel layout. between_kernels
-// (optional) is recorded between stack_a and stack_bank_kernel. The caller has passed W through check_bank.
-int stack_bank(const void *pyr, int n, int h, int w, int pair_levels, const silent_orientation_bank *W, float *orient,
-               float *line_end, float *gray, void *workspace, size_t workspace_bytes, cudaStream_t stream,
+// (optional) is recorded between stack_a and stack_bank_kernel. The caller has passed W through check_bank. Output
+// types as in stack_fused.
+int stack_bank(const void *pyr, int n, int h, int w, int pair_levels, const silent_orientation_bank *W, void *orient,
+               void *line_end, bool half_out, float *gray, void *workspace, size_t workspace_bytes, cudaStream_t stream,
                cudaEvent_t between_kernels = nullptr);
 // width (SILENT_E_SHAPE) and structure (SILENT_E_STRUCTURE) checks of a bank; host only, no CUDA call
 int check_bank(const silent_orientation_bank *W, const char *who);

@@ -25,6 +25,7 @@
 // bit-identical to it. Tensor cores do not apply (3-channel fp32 stencils); measured, the path is bound by packed-fp32
 // issue and shared-memory bandwidth rather than HBM (DESIGN.md section 4).
 #include <cuda.h>
+#include <cuda_fp16.h>
 
 #include <algorithm>
 #include <cmath>
@@ -153,29 +154,83 @@ __device__ __forceinline__ void store_nhwc8(float *__restrict__ dst, const f2 (&
     }
 }
 
-// Write a staged tile ([2 images][TH][TW*CH (+4 pad)] floats, NHWC) to global memory with coalesced 128-bit stores.
-template <int TH, int TW, int CH, int NT>
-__device__ __forceinline__ void copy_out_tile(const float *__restrict__ stage, float *__restrict__ out, int img0, int img1,
+// two floats rounded to binary16 (nearest even, subnormals kept, overflow to inf) and packed, lo at the lower address
+__device__ __forceinline__ uint32_t pack_half2(float lo, float hi)
+{
+    uint32_t r;
+    asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    return r;
+}
+
+// the same run as binary16 outputs: three 128-bit stores (48 contiguous bytes)
+template <int LANE>
+__device__ __forceinline__ void store_nhwc8(__half *__restrict__ dst, const f2 (&v)[kPX][3], bool vec_ok, int valid_px)
+{
+    float vals[kPX * 3];
+#pragma unroll
+    for (int p = 0; p < kPX; ++p)
+#pragma unroll
+        for (int co = 0; co < 3; ++co) vals[3 * p + co] = LANE ? v[p][co].y : v[p][co].x;
+    if (vec_ok) {
+#pragma unroll
+        for (int q = 0; q < kPX * 3 / 8; ++q)
+            reinterpret_cast<uint4 *>(dst)[q] = make_uint4(pack_half2(vals[8 * q], vals[8 * q + 1]), pack_half2(vals[8 * q + 2], vals[8 * q + 3]),
+                                                           pack_half2(vals[8 * q + 4], vals[8 * q + 5]), pack_half2(vals[8 * q + 6], vals[8 * q + 7]));
+    } else {
+#pragma unroll
+        for (int e = 0; e < kPX * 3; ++e)
+            if (e / 3 < valid_px) dst[e] = __float2half_rn(vals[e]);
+    }
+}
+
+// four consecutive outputs (one group of 4 orientations of one pixel): one 128-bit store of floats, or 64 bits of binary16
+__device__ __forceinline__ void store_quad(float *dst, float a, float b, float c, float d)
+{
+    *reinterpret_cast<float4 *>(dst) = make_float4(a, b, c, d);
+}
+__device__ __forceinline__ void store_quad(__half *dst, float a, float b, float c, float d)
+{
+    *reinterpret_cast<uint2 *>(dst) = make_uint2(pack_half2(a, b), pack_half2(c, d));
+}
+
+// Write a staged tile ([2 images][TH][TW*CH (+16 bytes of pad)] elements of T = float or __half, NHWC) to global
+// memory with coalesced 128-bit stores (VEC elements each) where the rows are 16-byte aligned.
+template <int TH, int TW, int CH, int NT, typename T>
+__device__ __forceinline__ void copy_out_tile(const T *__restrict__ stage, T *__restrict__ out, int img0, int img1,
                                               bool has_b, int ty0, int tx0, int h, int w, int tid)
 {
     if (!out) return;
-    constexpr int QUADS = TW * CH / 4, PITCH = TW * CH + 4;
+    constexpr int VEC = 16 / sizeof(T);
+    constexpr int QUADS = TW * CH / VEC, PITCH = TW * CH + VEC;
     const int valid_floats = min(TW, w - tx0) * CH;
-    const bool vec_ok = (w % 4) == 0;
+    const bool vec_ok = sizeof(T) == 4 ? (w % 4) == 0 : (w * CH) % VEC == 0;
     for (int i = tid; i < 2 * TH * QUADS; i += NT) {
         const int q = i % QUADS, rest = i / QUADS;
         const int r = rest % TH, lane = rest / TH;
         const int gy = ty0 + r;
-        if (gy >= h || (lane == 1 && !has_b) || 4 * q >= valid_floats) continue;
-        const float4 v = *reinterpret_cast<const float4 *>(stage + (size_t)(lane * TH + r) * PITCH + 4 * q);
-        float *dst = out + (((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * CH + 4 * q;
-        if (vec_ok && 4 * q + 4 <= valid_floats) {
-            *reinterpret_cast<float4 *>(dst) = v;
-        } else {
-            const float vals[4] = {v.x, v.y, v.z, v.w};
+        if (gy >= h || (lane == 1 && !has_b) || VEC * q >= valid_floats) continue;
+        if constexpr (sizeof(T) == 4) {
+            const float4 v = *reinterpret_cast<const float4 *>(stage + (size_t)(lane * TH + r) * PITCH + 4 * q);
+            float *dst = out + (((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * CH + 4 * q;
+            if (vec_ok && 4 * q + 4 <= valid_floats) {
+                *reinterpret_cast<float4 *>(dst) = v;
+            } else {
+                const float vals[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
-            for (int e = 0; e < 4; ++e)
-                if (4 * q + e < valid_floats) dst[e] = vals[e];
+                for (int e = 0; e < 4; ++e)
+                    if (4 * q + e < valid_floats) dst[e] = vals[e];
+            }
+        } else {
+            const uint4 v = *reinterpret_cast<const uint4 *>(stage + (size_t)(lane * TH + r) * PITCH + VEC * q);
+            T *dst = out + (((size_t)(lane ? img1 : img0) * h + gy) * w + tx0) * CH + VEC * q;
+            if (vec_ok && VEC * q + VEC <= valid_floats) {
+                *reinterpret_cast<uint4 *>(dst) = v;
+            } else {
+                const T *vals = reinterpret_cast<const T *>(&v);
+#pragma unroll
+                for (int e = 0; e < VEC; ++e)
+                    if (VEC * q + e < valid_floats) dst[e] = vals[e];
+            }
         }
     }
 }
@@ -183,11 +238,11 @@ __device__ __forceinline__ void copy_out_tile(const float *__restrict__ stage, f
 // Same tile through the TMA unit: ONE bulk store per staged row (needs 16-byte aligned rows). The `rows` staged rows
 // (2 * TH: image A's rows, then image B's) are dealt in contiguous blocks to the warps [warp0, warp0 + nwarps); lane 0 of
 // each warp issues its block in a loop whose trip count and addresses are warp-uniform (a per-lane deal made the compiler
-// serialise the lanes around the uniform-operand UBLKCP: ~20 instructions per store). row_floats: floats per global row
-// of one image (w * channels); tile_floats: floats this tile covers of a row. The caller fences + barriers before; the
-// issuing lane commits its group and must bulk_wait_read() before the staging buffer is reused.
-template <int TH>
-__device__ __forceinline__ bool bulk_rows(const float *__restrict__ stage, int stage_pitch, float *__restrict__ out,
+// serialise the lanes around the uniform-operand UBLKCP: ~20 instructions per store). row_floats: elements (of T) per
+// global row of one image (w * channels); tile_floats: elements this tile covers of a row. The caller fences + barriers
+// before; the issuing lane commits its group and must bulk_wait_read() before the staging buffer is reused.
+template <int TH, typename T>
+__device__ __forceinline__ bool bulk_rows(const T *__restrict__ stage, int stage_pitch, T *__restrict__ out,
                                           int img0, int img1, bool has_b, int ty0, int h, size_t row_floats, size_t col0,
                                           uint32_t tile_floats, int warp, int warp0, int nwarps, bool leader)
 {
@@ -195,14 +250,14 @@ __device__ __forceinline__ bool bulk_rows(const float *__restrict__ stage, int s
     if (wi < 0 || wi >= nwarps) return false;
     const int per_warp = (2 * TH + nwarps - 1) / nwarps;
     const int first = wi * per_warp, last = min(first + per_warp, 2 * TH);
-    const uint32_t bytes = tile_floats * (uint32_t)sizeof(float);
+    const uint32_t bytes = tile_floats * (uint32_t)sizeof(T);
 #pragma unroll
     for (int lane = 0; lane < 2; ++lane) {   // this warp's rows of image A, then of image B: pointers step by one row
         const int r0 = max(first, lane * TH) - lane * TH;
         const int r1 = min(min(last, (lane + 1) * TH) - lane * TH, h - ty0);
         if (r0 >= r1 || (lane == 1 && !has_b)) continue;
-        float *dst = out + ((size_t)(lane ? img1 : img0) * h + ty0 + r0) * row_floats + col0;
-        const float *src = stage + (size_t)(lane * TH + r0) * stage_pitch;
+        T *dst = out + ((size_t)(lane ? img1 : img0) * h + ty0 + r0) * row_floats + col0;
+        const T *src = stage + (size_t)(lane * TH + r0) * stage_pitch;
 #pragma unroll 1
         for (int r = r0; r < r1; ++r, dst += row_floats, src += stage_pitch)
             if (leader) bulk_store(dst, src, bytes);
@@ -211,10 +266,10 @@ __device__ __forceinline__ bool bulk_rows(const float *__restrict__ stage, int s
     return leader;
 }
 
-// the staged rows of a tile ([2][TH][pitch] floats: image A's rows, then image B's) as TMA tile stores of kTileStoreRows rows
+// the staged rows of a tile ([2][TH][pitch] elements: image A's rows, then image B's) as TMA tile stores of kTileStoreRows rows
 constexpr int kTileStoreRows = 16;
-template <int TH>
-__device__ __forceinline__ void tile_store_images(const CUtensorMap *map, const float *stage, int pitch, int bx, int ty0, int h,
+template <int TH, typename T>
+__device__ __forceinline__ void tile_store_images(const CUtensorMap *map, const T *stage, int pitch, int bx, int ty0, int h,
                                                   int img0, int img1, bool has_b)
 {
     static_assert(TH % kTileStoreRows == 0, "tiles are whole multiples of the store box");
@@ -227,13 +282,13 @@ __device__ __forceinline__ void tile_store_images(const CUtensorMap *map, const 
     }
 }
 
-// A staged tile ([2][TH][pitch] floats: image A's rows, then image B's; CH floats per pixel) leaves shared memory by one
-// of three routes: TMA tile stores issued by thread `issuer` (tile_store), one bulk copy per row from the warps of the
-// threads [first, first + NTHREADS) (bulk_ok: 16-byte aligned global rows), or coalesced element-wise copies by those
-// threads. The caller fences and synchronises the participants before. Returns true for a thread that issued bulk
-// copies: it must bulk_wait_read() before the staging buffer is reused.
-template <int TH, int TW, int CH, int NTHREADS>
-__device__ __forceinline__ bool store_staged_tile(const CUtensorMap *map, const float *stage, int pitch, float *out,
+// A staged tile ([2][TH][pitch] elements of T = float or __half: image A's rows, then image B's; CH per pixel) leaves
+// shared memory by one of three routes: TMA tile stores issued by thread `issuer` (tile_store), one bulk copy per row
+// from the warps of the threads [first, first + NTHREADS) (bulk_ok: 16-byte aligned global rows), or coalesced
+// element-wise copies by those threads. The caller fences and synchronises the participants before. Returns true for a
+// thread that issued bulk copies: it must bulk_wait_read() before the staging buffer is reused.
+template <int TH, int TW, int CH, int NTHREADS, typename T>
+__device__ __forceinline__ bool store_staged_tile(const CUtensorMap *map, const T *stage, int pitch, T *out,
                                                   bool tile_store, bool bulk_ok, int tid, int issuer, int first, int warp,
                                                   bool leader, int bx, int ty0, int tx0, int h, int w, int img0, int img1,
                                                   bool has_b)
@@ -645,8 +700,8 @@ struct ParamsB {
 // 7x7 halo at all: the stripe stage covers the tile + 1 (what the end filter needs), the blur is never evaluated, and a
 // tile in which ANY run fails the test is left untouched and flagged for the full variant (launched right after on the
 // flagged tiles only). Less shared memory (68 KB instead of 92 KB for 24-row tiles: 3 CTAs per SM) and a third of the
-// halo arithmetic.
-template <int TH, int TW, bool LITE>
+// halo arithmetic. OutT: element type of the staged orient / line_end rows (float, or __half for binary16 outputs).
+template <int TH, int TW, bool LITE, typename OutT = float>
 struct TileB {
     static constexpr int HALO_C = LITE ? 1 : 4;                   // rows of stripe output around the tile
     static constexpr int C_RUNS = (TW + 8) / kPX;                 // S3 runs start at column -4 (TW % 8 == 0)
@@ -660,9 +715,10 @@ struct TileB {
                                                                                        : kPX * (E_RUNS - 1) + 10);  // -1
     static constexpr int B_PLANE = B_ROWS * B_PITCH, CS_PLANE = LITE ? 0 : CS_ROWS * CS_PITCH, CD_PLANE = CD_ROWS * CD_PITCH;
     // output staging (NHWC rows of one tile for both images), overlaid on sB + sCs once S4 is done. The row pitch is
-    // an odd multiple of 16 B: the run-per-lane 128-bit stores AND the linear copy-out loads are conflict-free.
-    static constexpr int ST_PITCH = TW * 3 + 4;                       // floats per staged row
-    static constexpr int STAGE_F2 = 2 * TH * ST_PITCH / 2;            // float2 slots
+    // an odd multiple of 16 B (TW * 3 elements are an even multiple for TW % 16 == 0, plus 16 bytes): the run-per-lane
+    // 128-bit stores AND the linear copy-out loads are conflict-free.
+    static constexpr int ST_PITCH = TW * 3 + 16 / sizeof(OutT);       // elements per staged row
+    static constexpr int STAGE_F2 = 2 * TH * ST_PITCH * sizeof(OutT) / sizeof(f2);   // float2 slots
     static constexpr int G_PITCH = TW + 4;                            // floats per staged gray row (odd multiple of 16 B)
     static constexpr int FRONT_F2 = B_PLANE + CS_PLANE > STAGE_F2 ? B_PLANE + CS_PLANE : STAGE_F2;
     // sums of the stripe channel sum over aligned groups of 4 columns ("quads", origin -4): the S4 early-out reads
@@ -675,6 +731,7 @@ struct TileB {
     static constexpr int Q_OFFSET = Q_IN_FRONT ? B_PLANE + CS_PLANE : FRONT_F2 + 3 * CD_PLANE;
     static constexpr size_t kSmemBytes = (size_t)(FRONT_F2 + 3 * CD_PLANE + (Q_IN_FRONT ? 0 : Q_PLANE) + 8) * sizeof(f2) + 64;
     static_assert(TW % kPX == 0, "tile width must be a multiple of the run length");
+    static_assert(ST_PITCH * sizeof(OutT) % 32 == 16, "staging pitch: an odd multiple of 16 bytes");
 };
 
 // STRUCTURED, both of:
@@ -685,15 +742,16 @@ struct TileB {
 // Both orders are part of the canonical FUSED evaluation order (oracle/silent_oracle.c: so_line_end_stack_fused).
 // tile_flag [pairs][tile rows][tile cols] bytes: the LITE variant sets the flag of a tile it could not finish; the
 // full variant, given the flags, only works on flagged tiles (null: every tile).
-// One tile (bx, by) of image pair bz in a grid of nbx x nby tiles per pair.
-template <int TH, int TW, int NT, bool STRUCTURED, bool LITE>
+// One tile (bx, by) of image pair bz in a grid of nbx x nby tiles per pair. orient and line_end are stored as OutT
+// (float, or __half: each float32 result rounded once to binary16 when it is staged); gray stays float.
+template <int TH, int TW, int NT, bool STRUCTURED, bool LITE, typename OutT>
 __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const int bz, const int nbx, const int nby,
                                              const f2 *__restrict__ bsum2, const ParamsB &P, const CUtensorMap &tmap,
-                                             const StoreMaps &M, float *__restrict__ orient, float *__restrict__ line_end,
+                                             const StoreMaps &M, OutT *__restrict__ orient, OutT *__restrict__ line_end,
                                              float *__restrict__ gray, int *__restrict__ winmax, int *__restrict__ tilemax,
                                              unsigned char *__restrict__ tile_flag, const int tm_split)
 {
-    using T = TileB<TH, TW, LITE>;
+    using T = TileB<TH, TW, LITE, OutT>;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t tma_bar;
     const size_t tile_id = ((size_t)bz * nby + by) * nbx + bx;
@@ -701,7 +759,7 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
     f2 *sCs = sB + T::B_PLANE;                   // [CS_ROWS][CS_PITCH]     stripe channel sum, origin (-4, -4)
     f2 *sCD = sB + T::FRONT_F2;                  // [3][CD_ROWS][CD_PITCH]  stripe, regulated in place, origin (-1, -1)
     f2 *sQ = sB + T::Q_OFFSET;                   // [CS_ROWS][Q_PITCH]      quad sums of the stripe sum, origin (-4, -4)
-    float *sStage = reinterpret_cast<float *>(sB);   // [2][TH][ST_PITCH] NHWC staging, valid after the S4 barrier
+    OutT *sStage = reinterpret_cast<OutT *>(sB);     // [2][TH][ST_PITCH] NHWC staging, valid after the S4 barrier
     int *sWin = reinterpret_cast<int *>(sB + T::FRONT_F2 + 3 * T::CD_PLANE + (T::Q_IN_FRONT ? 0 : T::Q_PLANE));   // 10 ints
     float *sGray = reinterpret_cast<float *>(sCD);                // [2][TH][G_PITCH] gray staging, valid after the S5 barrier
 
@@ -988,9 +1046,11 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
     //      the rows to the TMA unit. When the CTA has at least two warps WITHOUT an S5 task (S5 has the fewest tasks of
     //      the three phases) they do all of this on their own, synchronised by a named barrier, while the S5 warps start
     //      the end filter at once; the copy drains while S5 computes ---------------------------------------------
-    const bool bulk_ok = (w % 4) == 0;   // staged rows start and end on 16-byte boundaries of the global tensors
+    // staged rows start and end on 16-byte boundaries of the global tensors: gray (float) and the outputs (OutT)
+    const bool gray_bulk_ok = (w % 4) == 0;
+    const bool bulk_ok = sizeof(OutT) == 4 ? gray_bulk_ok : (w % 8) == 0;
     // TMA tile stores need 128-byte aligned shared-memory sources: every 16-row part of the staging buffers must be one
-    constexpr bool kStageTileStore = (kTileStoreRows * T::ST_PITCH * 4) % 128 == 0;
+    constexpr bool kStageTileStore = (kTileStoreRows * T::ST_PITCH * sizeof(OutT)) % 128 == 0;
     constexpr bool kGrayTileStore = ((size_t)T::FRONT_F2 * sizeof(f2)) % 128 == 0 && (kTileStoreRows * T::G_PITCH * 4) % 128 == 0;
     const bool tile_store = kStageTileStore && P.tma_store != 0;   // (the host checked w % TW == 0 and built the maps)
     constexpr int kS5Warps = (TH * T::E_RUNS + 31) / 32, kIdleWarps = NT / 32 - kS5Warps;
@@ -1114,7 +1174,7 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
         store_nhwc8<0>(sStage + (size_t)r5 * T::ST_PITCH + 3 * kPX * k5, acc, true, kPX);
         store_nhwc8<1>(sStage + (size_t)(TH + r5) * T::ST_PITCH + 3 * kPX * k5, acc, true, kPX);
         if (gray) {
-            if (bulk_ok) {   // staged over the (now dead) CD planes: rows of TW floats, written by bulk stores below
+            if (gray_bulk_ok) {   // staged over the (now dead) CD planes: rows of TW floats, written by bulk stores below
                 float4 *ga = reinterpret_cast<float4 *>(sGray + (size_t)r5 * T::G_PITCH + kPX * k5);
                 float4 *gb = reinterpret_cast<float4 *>(sGray + (size_t)(TH + r5) * T::G_PITCH + kPX * k5);
                 ga[0] = make_float4(g[0].x, g[1].x, g[2].x, g[3].x);
@@ -1172,7 +1232,7 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
     fence_async_smem();
     __syncthreads();
     const bool gray_tile_store = tile_store && kGrayTileStore;
-    if (gray && (gray_tile_store || bulk_ok))   // (without bulk_ok, gray left straight from registers in S5)
+    if (gray && (gray_tile_store || gray_bulk_ok))   // (otherwise gray left straight from registers in S5)
         issued_line_end |= store_staged_tile<TH, TW, 1, NT>(&M.gray, sGray, T::G_PITCH, gray, gray_tile_store, true, tid, 32,
                                                             0, warp_u, leader, bx, ty0, tx0, h, w, img0, img1, has_b);
     if (line_end)
@@ -1200,10 +1260,10 @@ __device__ __forceinline__ void stack_b_tile(const int bx, const int by, const i
 // finish. The full variant without flags works on every tile (one CTA per tile); WITH flags it is the fix-up pass: a
 // small 1-D grid of CTAs walks the tile list and redoes the flagged tiles (none on textured input: the pass then costs
 // a few microseconds instead of a full grid of early exits).
-template <int TH, int TW, int NT, bool STRUCTURED, bool LITE>
+template <int TH, int TW, int NT, bool STRUCTURED, bool LITE, typename OutT>
 __global__ void __launch_bounds__(NT, LITE ? (TH <= 16 ? 5 : 3) : 2)
 stack_b_kernel(const f2 *__restrict__ bsum2, const __grid_constant__ ParamsB P, const __grid_constant__ CUtensorMap tmap,
-               const __grid_constant__ StoreMaps M, float *__restrict__ orient, float *__restrict__ line_end, float *__restrict__ gray, int *__restrict__ winmax,
+               const __grid_constant__ StoreMaps M, OutT *__restrict__ orient, OutT *__restrict__ line_end, float *__restrict__ gray, int *__restrict__ winmax,
                int *__restrict__ tilemax, unsigned char *__restrict__ tile_flag, int nbx, int nby, int pairs, int tm_split)
 {
     pdl_enter();
@@ -1238,13 +1298,13 @@ stack_b_kernel(const f2 *__restrict__ bsum2, const __grid_constant__ ParamsB P, 
                 const int bz = t / per_pair, rest = t - bz * per_pair;
                 if (again) __syncthreads();   // every thread is done with the previous tile's shared memory
                 again = true;
-                stack_b_tile<TH, TW, NT, STRUCTURED, LITE>(rest % nbx, rest / nbx, bz, nbx, nby, bsum2, P, tmap, M, orient,
+                stack_b_tile<TH, TW, NT, STRUCTURED, LITE, OutT>(rest % nbx, rest / nbx, bz, nbx, nby, bsum2, P, tmap, M, orient,
                                                        line_end, gray, winmax, tilemax, tile_flag, tm_split);
             }
             again = true;
         }
     } else {
-        stack_b_tile<TH, TW, NT, STRUCTURED, LITE>(blockIdx.x, blockIdx.y, blockIdx.z, gridDim.x, gridDim.y, bsum2, P, tmap,
+        stack_b_tile<TH, TW, NT, STRUCTURED, LITE, OutT>(blockIdx.x, blockIdx.y, blockIdx.z, gridDim.x, gridDim.y, bsum2, P, tmap,
                                                M, orient, line_end, gray, winmax, tilemax, tile_flag, tm_split);
     }
 }
@@ -1277,7 +1337,7 @@ struct ParamsBank {
     int tma_store;   // orient / line_end leave as TMA tile stores (StoreMaps valid)
 };
 
-template <int NB, int TH, int TW>
+template <int NB, int TH, int TW, typename OutT = float>
 struct TileBank {
     static constexpr int C_RUNS = (TW + 9 + kRun - 1) / kRun;   // stripe runs start at column -5 (need -4 .. TW + 3)
     static constexpr int D_RUNS = (TW + 2 + kRun - 1) / kRun;   // regulator runs start at column -1
@@ -1290,11 +1350,12 @@ struct TileBank {
                                                                                        : kRun * (E_RUNS - 1) + 6);   // -1
     static constexpr int Q_PITCH = C_RUNS | 1;                                     // one quad sum per stripe run
     static constexpr int B_PLANE = B_ROWS * B_PITCH, CS_PLANE = CS_ROWS * CS_PITCH, CD_PLANE = CD_ROWS * CD_PITCH;
-    static constexpr int ST_PITCH = TW * NB + 4;                    // floats per staged NHWC row (odd multiple of 16 B)
-    static constexpr int STAGE_F2 = 2 * TH * ST_PITCH / 2;
+    static constexpr int ST_PITCH = TW * NB + 16 / sizeof(OutT);   // elements per staged NHWC row (odd multiple of 16 B)
+    static constexpr int STAGE_F2 = 2 * TH * ST_PITCH * sizeof(OutT) / sizeof(f2);
     static constexpr int FRONT_F2 = B_PLANE + CS_PLANE > STAGE_F2 ? B_PLANE + CS_PLANE : STAGE_F2;
     static constexpr size_t kSmemBytes = (size_t)(FRONT_F2 + NB * CD_PLANE + CS_ROWS * Q_PITCH) * sizeof(f2) + 64;
     static_assert(TW % kRun == 0 && TW % 4 == 0, "tile width must be a multiple of the run length");
+    static_assert(ST_PITCH * sizeof(OutT) % 32 == 16, "staging pitch: an odd multiple of 16 bytes");
 };
 
 __device__ __forceinline__ void store_cols4(f2 *__restrict__ dst, const f2 (&v)[kRun])
@@ -1304,12 +1365,13 @@ __device__ __forceinline__ void store_cols4(f2 *__restrict__ dst, const f2 (&v)[
     p[1] = make_float4(v[2].x, v[2].y, v[3].x, v[3].y);
 }
 
-template <int NB, int TH, int TW, int NT>
+// OutT: element type of orient / line_end (float, or __half: rounded once to binary16 when staged); gray stays float.
+template <int NB, int TH, int TW, int NT, typename OutT>
 __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict__ bsum2, const __grid_constant__ ParamsBank<NB> P,
-                                                           const __grid_constant__ StoreMaps M, float *__restrict__ orient, float *__restrict__ line_end,
+                                                           const __grid_constant__ StoreMaps M, OutT *__restrict__ orient, OutT *__restrict__ line_end,
                                                            float *__restrict__ gray)
 {
-    using T = TileBank<NB, TH, TW>;
+    using T = TileBank<NB, TH, TW, OutT>;
     // loops over the orientations, unrolled whole up to 8 orientations. Wider banks walk them in chunks (4 orientations
     // in S3 / S4, one group of 4 in the restage and S5) that are not unrolled into each other: unrolled whole, the
     // compiler hoists every orientation's weights into registers and spills.
@@ -1320,7 +1382,7 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
     f2 *sCs = sB + T::B_PLANE;                   // [CS_ROWS][CS_PITCH]    sum of the stripe bank, origin (-4, -5)
     f2 *sCD = sB + T::FRONT_F2;                  // [NB][CD_ROWS][CD_PITCH] stripe bank, regulated in place, origin (-1, -1)
     f2 *sQ = sCD + NB * T::CD_PLANE;            // [CS_ROWS][Q_PITCH]     quad sums of sCs
-    float *sStage = reinterpret_cast<float *>(sB);   // [2][TH][ST_PITCH] NHWC staging, valid after the S4 barrier
+    OutT *sStage = reinterpret_cast<OutT *>(sB);     // [2][TH][ST_PITCH] NHWC staging, valid after the S4 barrier
 
     const int tid = threadIdx.x;
     const int warp_u = __shfl_sync(0xffffffffu, tid >> 5, 0);
@@ -1435,8 +1497,10 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
     __syncthreads();
 
     // ---- orient = d: centre rows of the planes, restaged NHWC (4 orientations = one 128-bit chunk per pixel and image) --
-    const bool bulk_ok = (w % 4) == 0;
-    constexpr bool kStageTileStore = (kTileStoreRows * T::ST_PITCH * 4) % 128 == 0;
+    // 16-byte aligned global rows: gray (float) and the outputs (OutT)
+    const bool gray_vec_ok = (w % 4) == 0;
+    const bool bulk_ok = sizeof(OutT) == 4 ? gray_vec_ok : (w * NB) % 8 == 0;
+    constexpr bool kStageTileStore = (kTileStoreRows * T::ST_PITCH * sizeof(OutT)) % 128 == 0;
     const bool tile_store = kStageTileStore && P.tma_store != 0;
     bool issued = false;
     if (orient) {
@@ -1451,10 +1515,10 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
                 for (int oo = 0; oo < 4; ++oo) load_cols<3>(sCD + (4 * g + oo) * T::CD_PLANE + (r + 1) * T::CD_PITCH + kRun * k, d[oo]);
 #pragma unroll
                 for (int p = 0; p < kRun; ++p) {
-                    float *a = sStage + (size_t)r * T::ST_PITCH + (kRun * k + p) * NB + 4 * g;
-                    float *b = sStage + (size_t)(TH + r) * T::ST_PITCH + (kRun * k + p) * NB + 4 * g;
-                    *reinterpret_cast<float4 *>(a) = make_float4(d[0][p + 1].x, d[1][p + 1].x, d[2][p + 1].x, d[3][p + 1].x);
-                    *reinterpret_cast<float4 *>(b) = make_float4(d[0][p + 1].y, d[1][p + 1].y, d[2][p + 1].y, d[3][p + 1].y);
+                    OutT *a = sStage + (size_t)r * T::ST_PITCH + (kRun * k + p) * NB + 4 * g;
+                    OutT *b = sStage + (size_t)(TH + r) * T::ST_PITCH + (kRun * k + p) * NB + 4 * g;
+                    store_quad(a, d[0][p + 1].x, d[1][p + 1].x, d[2][p + 1].x, d[3][p + 1].x);
+                    store_quad(b, d[0][p + 1].y, d[1][p + 1].y, d[2][p + 1].y, d[3][p + 1].y);
                 }
             }
         }
@@ -1504,16 +1568,16 @@ __global__ void __launch_bounds__(NT, 2) stack_bank_kernel(const f2 *__restrict_
             }
 #pragma unroll
             for (int p = 0; p < kRun; ++p) {
-                float *a = sStage + (size_t)r * T::ST_PITCH + (kRun * k + p) * NB + 4 * gq;
-                float *b = sStage + (size_t)(TH + r) * T::ST_PITCH + (kRun * k + p) * NB + 4 * gq;
-                *reinterpret_cast<float4 *>(a) = make_float4(e[0][p].x, e[1][p].x, e[2][p].x, e[3][p].x);
-                *reinterpret_cast<float4 *>(b) = make_float4(e[0][p].y, e[1][p].y, e[2][p].y, e[3][p].y);
+                OutT *a = sStage + (size_t)r * T::ST_PITCH + (kRun * k + p) * NB + 4 * gq;
+                OutT *b = sStage + (size_t)(TH + r) * T::ST_PITCH + (kRun * k + p) * NB + 4 * gq;
+                store_quad(a, e[0][p].x, e[1][p].x, e[2][p].x, e[3][p].x);
+                store_quad(b, e[0][p].y, e[1][p].y, e[2][p].y, e[3][p].y);
             }
         }
 #pragma unroll
         for (int p = 0; p < kRun; ++p) g[p] = mul2(g[p], make_float2(inv_nb, inv_nb));
         if (gray) {   // few bytes: written straight from registers (4 consecutive floats per image)
-            if (bulk_ok && gx0 + kRun <= w && gy < h) {
+            if (gray_vec_ok && gx0 + kRun <= w && gy < h) {
                 *reinterpret_cast<float4 *>(gray + ((size_t)img0 * h + gy) * w + gx0) = make_float4(g[0].x, g[1].x, g[2].x, g[3].x);
                 if (has_b)
                     *reinterpret_cast<float4 *>(gray + ((size_t)img1 * h + gy) * w + gx0) = make_float4(g[0].y, g[1].y, g[2].y, g[3].y);
@@ -1576,23 +1640,27 @@ static bool make_pair_map(CUtensorMap *map, const void *base, int w, int rows, l
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-// Store view of an NHWC float32 output [n][h][w][ch] for TMA tile stores (see tma_store_tile): dims (floats of a tile row,
-// tiles per row, rows, images), box (tile row + pad, 1, box_rows, 1). False if the geometry does not allow it.
+// Store view of an NHWC output [n][h][w][ch] of value_bytes per value (4: float32, 2: binary16) for TMA tile stores (see
+// tma_store_tile): dims (elements of a tile row, tiles per row, rows, images), box (tile row + pad values, 1, box_rows, 1).
+// The map's elements are map_bytes wide: value_bytes, or 8 for tile rows longer than a box's 256 elements. False if
+// the geometry does not allow it.
 static bool make_tile_store_map(CUtensorMap *map, const void *base, int n, int h, int w, int ch, int tw, int pad, int box_rows,
-                                int elem_floats = 1)   // 2: 8-byte elements (tile rows of more than 252 floats: boxes hold <= 256 elements)
+                                int value_bytes, int map_bytes)
 {
     const EncodeTiledFn encode = encode_tiled();
     if (!encode) return false;
-    const int tile_floats = tw * ch;
-    if (!base || ((uintptr_t)base & 15) != 0 || w % tw != 0 || tile_floats % 4 != 0 || (tile_floats + pad) % 4 != 0 ||
-        (tile_floats + pad) / elem_floats > 256 || box_rows > 256)
+    const int tile_bytes = tw * ch * value_bytes, box_bytes = (tw * ch + pad) * value_bytes;
+    if (!base || ((uintptr_t)base & 15) != 0 || w % tw != 0 || tile_bytes % 16 != 0 || box_bytes % 16 != 0 ||
+        box_bytes / map_bytes > 256 || box_rows > 256)
         return false;
-    const cuuint64_t row_bytes = (cuuint64_t)w * ch * 4;
-    const cuuint64_t dims[4] = {(cuuint64_t)(tile_floats / elem_floats), (cuuint64_t)(w / tw), (cuuint64_t)h, (cuuint64_t)n};
-    const cuuint64_t strides[3] = {(cuuint64_t)tile_floats * 4, row_bytes, row_bytes * h};
-    const cuuint32_t box[4] = {(cuuint32_t)((tile_floats + pad) / elem_floats), 1, (cuuint32_t)box_rows, 1};
+    const cuuint64_t row_bytes = (cuuint64_t)w * ch * value_bytes;
+    const cuuint64_t dims[4] = {(cuuint64_t)(tile_bytes / map_bytes), (cuuint64_t)(w / tw), (cuuint64_t)h, (cuuint64_t)n};
+    const cuuint64_t strides[3] = {(cuuint64_t)tile_bytes, row_bytes, row_bytes * h};
+    const cuuint32_t box[4] = {(cuuint32_t)(box_bytes / map_bytes), 1, (cuuint32_t)box_rows, 1};
     const cuuint32_t estr[4] = {1, 1, 1, 1};
-    return encode(map, elem_floats == 2 ? CU_TENSOR_MAP_DATA_TYPE_UINT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<void *>(base), dims, strides, box, estr,
+    const CUtensorMapDataType type = map_bytes == 8 ? CU_TENSOR_MAP_DATA_TYPE_UINT64
+                                     : map_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+    return encode(map, type, 4, const_cast<void *>(base), dims, strides, box, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -1810,24 +1878,25 @@ static size_t stack_flag_bytes(int n, int h, int w)
 static size_t stack_plane_bytes(int n, int h, int w) { return ((size_t)(n / 2 + 8) * h * (w + 2) * sizeof(f2) + 255) / 256 * 256; }
 size_t stack_workspace_bytes(int n, int h, int w) { return stack_plane_bytes(n, h, w) + stack_flag_bytes(n, h, w) + 256; }
 
-template <int TH, int TW, bool STRUCTURED, bool LITE>
-static int launch_b(StackPlanHost &S, int pairs, f2 *bsum2, float *orient, float *line_end, float *gray, int *winmax,
+template <int TH, int TW, bool STRUCTURED, bool LITE, typename OutT>
+static int launch_b(StackPlanHost &S, int pairs, f2 *bsum2, OutT *orient, OutT *line_end, float *gray, int *winmax,
                     int *tilemax, unsigned char *tile_flag, cudaStream_t stream)
 {
     const int h = S.b.h, w = S.b.w;
     CUtensorMap map_b;
     std::memset(&map_b, 0, sizeof(map_b));
-    using TB = TileB<TH, TW, LITE>;
+    using TB = TileB<TH, TW, LITE, OutT>;
     constexpr int NT = ThreadsB<TH, TW, LITE>::value;
-    auto kern = stack_b_kernel<TH, TW, NT, STRUCTURED, LITE>;
+    constexpr int V = sizeof(OutT);
+    auto kern = stack_b_kernel<TH, TW, NT, STRUCTURED, LITE, OutT>;
     SILENT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TB::kSmemBytes));
     S.b.use_tma = (w % 2) == 0 && make_pair_map(&map_b, bsum2, w + 2, h, pairs, TB::B_PITCH, TB::B_ROWS, 1);
     // outputs as TMA tile stores (one per 16 rows and image instead of one bulk copy per row) when every tile is whole in x
     StoreMaps maps;
     std::memset(&maps, 0, sizeof(maps));
-    S.b.tma_store = (!orient || make_tile_store_map(&maps.orient, orient, S.b.n, h, w, 3, TW, TB::ST_PITCH - 3 * TW, kTileStoreRows)) &&
-                    (!line_end || make_tile_store_map(&maps.line_end, line_end, S.b.n, h, w, 3, TW, TB::ST_PITCH - 3 * TW, kTileStoreRows)) &&
-                    (!gray || make_tile_store_map(&maps.gray, gray, S.b.n, h, w, 1, TW, TB::G_PITCH - TW, kTileStoreRows));
+    S.b.tma_store = (!orient || make_tile_store_map(&maps.orient, orient, S.b.n, h, w, 3, TW, TB::ST_PITCH - 3 * TW, kTileStoreRows, V, V)) &&
+                    (!line_end || make_tile_store_map(&maps.line_end, line_end, S.b.n, h, w, 3, TW, TB::ST_PITCH - 3 * TW, kTileStoreRows, V, V)) &&
+                    (!gray || make_tile_store_map(&maps.gray, gray, S.b.n, h, w, 1, TW, TB::G_PITCH - TW, kTileStoreRows, 4, 4));
     S.b.pairs = pairs;
     S.b.prefetch_pairs = 4;   // measured: 2 / 4 / 8 alike (-5 % on the quick pass against 0 = off)
     const int nbx = ceil_div(w, TW), nby = ceil_div(h, TH);
@@ -1858,34 +1927,34 @@ static int launch_stack_a(const void *pyr, StackPlanHost &S, bool paired_in, int
                      : launch_a<TWA, false, false>(pyr, S.a, map_x, bsum2, pairs, stream);
 }
 
-template <int TW>
-static int launch_stack(const void *pyr, StackPlanHost &S, bool paired_in, int pairs, f2 *bsum2, float *orient,
-                        float *line_end, float *gray, int *winmax, int *tilemax, unsigned char *tile_flag, bool flags_clean,
+template <int TW, typename OutT>
+static int launch_stack(const void *pyr, StackPlanHost &S, bool paired_in, int pairs, f2 *bsum2, OutT *orient,
+                        OutT *line_end, float *gray, int *winmax, int *tilemax, unsigned char *tile_flag, bool flags_clean,
                         cudaStream_t stream, cudaEvent_t between_kernels)
 {
     int rc = launch_stack_a<TW>(pyr, S, paired_in, pairs, bsum2, stream);   // (96-wide stack_a tiles: measured 8 % slower)
     if (rc != SILENT_OK) return rc;
     if (between_kernels) SILENT_CUDA(cudaEventRecord(between_kernels, stream));   // stage timing hook
     if (!S.b_structured)
-        return launch_b<kTileHB, TW, false, false>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, nullptr, stream);
+        return launch_b<kTileHB, TW, false, false, OutT>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, nullptr, stream);
     // a grid that fits the device in about one wave (single frames, config C2) gains nothing from the quick variant's
     // higher occupancy and would pay for a second launch: the full variant does it alone
     const int sms = sm_count();
     const long long tiles = (long long)pairs * ceil_div(S.b.h, kTileHB) * ceil_div(S.b.w, TW);
     if (tiles <= 3LL * sms && (S.b.h % (2 * kTileHB)) == 0)   // ... on tiles twice as tall (half as many CTAs, one wave)
-        return launch_b<2 * kTileHB, TW, true, false>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, nullptr, stream);
+        return launch_b<2 * kTileHB, TW, true, false, OutT>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, nullptr, stream);
     if (!(S.b.quick_thr > 0.0f && tile_flag) || tiles <= 3LL * sms)
-        return launch_b<kTileHB, TW, true, false>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, nullptr, stream);
+        return launch_b<kTileHB, TW, true, false, OutT>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, nullptr, stream);
     // quick variant on every tile, then the full variant on the tiles it flagged (none on textured input)
     if (!flags_clean) {   // (the pipeline clears them before the pyramid launch, so that no memset sits between kernels)
         const size_t flags = (size_t)pairs * ceil_div(S.b.h, kTileHB) * ceil_div(S.b.w, TW);
         SILENT_CUDA(cudaMemsetAsync(tile_flag - 16, 0, flags + 16, stream));   // flags and the counter in front of them
     }
-    rc = launch_b<kTileHB, TW, true, true>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, tile_flag, stream);
+    rc = launch_b<kTileHB, TW, true, true, OutT>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, tile_flag, stream);
     if (rc != SILENT_OK) return rc;
     if ((S.b.h % (2 * kTileHB)) == 0)   // fix-up on tiles twice as tall: a third less halo arithmetic per redone row
-        return launch_b<2 * kTileHB, TW, true, false>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, tile_flag, stream);
-    return launch_b<kTileHB, TW, true, false>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, tile_flag, stream);
+        return launch_b<2 * kTileHB, TW, true, false, OutT>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, tile_flag, stream);
+    return launch_b<kTileHB, TW, true, false, OutT>(S, pairs, bsum2, orient, line_end, gray, winmax, tilemax, tile_flag, stream);
 }
 
 // Tile grid of stack_b for a level shape (the emit stage reads the per-tile maxima it writes).
@@ -1918,8 +1987,8 @@ int stack_clear_flags(void *workspace, int n, int h, int w, cudaStream_t stream)
 
 // Argument checks shared by the stack entry points (`who` names the entry point in the messages); *pairs: the image
 // pairs of n images with pair_levels levels per frame (0: NHWC input, images paired (2p, 2p + 1)).
-static int check_stack_args(const char *who, const void *pyr, int n, int h, int w, int pair_levels, const float *orient,
-                            const float *line_end, const float *gray, const void *workspace, size_t workspace_bytes,
+static int check_stack_args(const char *who, const void *pyr, int n, int h, int w, int pair_levels, const void *orient,
+                            const void *line_end, const float *gray, const void *workspace, size_t workspace_bytes,
                             int *pairs)
 {
     if (!pyr) return fail(SILENT_E_INVAL, "%s: null pyramid", who);
@@ -1936,12 +2005,13 @@ static int check_stack_args(const char *who, const void *pyr, int n, int h, int 
     return SILENT_OK;
 }
 
-int stack_fused(const void *pyr, int n, int h, int w, int pair_levels, const silent_stack_weights *W, float *orient,
-                float *line_end, float *gray, void *workspace, size_t workspace_bytes, const WindowGeom *geo,
+// Both output types share this body; the element type only picks the kernels' instantiations.
+int stack_fused(const void *pyr, int n, int h, int w, int pair_levels, const silent_stack_weights *W, void *orient,
+                void *line_end, bool half_out, float *gray, void *workspace, size_t workspace_bytes, const WindowGeom *geo,
                 int *winmax, int *tilemax, cudaStream_t stream, cudaEvent_t between_kernels, bool flags_clean)
 {
     int pairs = 0;
-    int rc = check_stack_args("silent_stack_fused", pyr, n, h, w, pair_levels, orient, line_end, gray, workspace,
+    int rc = check_stack_args(half_out ? "silent_stack_fused_f16" : "silent_stack_fused", pyr, n, h, w, pair_levels, orient, line_end, gray, workspace,
                               workspace_bytes, &pairs);
     if (rc != SILENT_OK) return rc;
     StackPlanHost S;
@@ -1953,11 +2023,16 @@ int stack_fused(const void *pyr, int n, int h, int w, int pair_levels, const sil
     S.a.pair_levels = S.b.pair_levels = pack_pair_levels(paired_in ? pair_levels : 1);
     f2 *bsum2 = reinterpret_cast<f2 *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
     unsigned char *tile_flag = reinterpret_cast<unsigned char *>(bsum2) + stack_plane_bytes(n, h, w) + 16;   // [-4]: counter
-    if (pick_tile_w(w) == 48)
-        return launch_stack<48>(pyr, S, paired_in, pairs, bsum2, orient, line_end, gray, winmax, tilemax, tile_flag,
-                                flags_clean, stream, between_kernels);
-    return launch_stack<64>(pyr, S, paired_in, pairs, bsum2, orient, line_end, gray, winmax, tilemax, tile_flag, flags_clean,
-                            stream, between_kernels);
+    auto launch = [&](auto out_type) {
+        using OutT = decltype(out_type);
+        OutT *o = static_cast<OutT *>(orient), *e = static_cast<OutT *>(line_end);
+        if (pick_tile_w(w) == 48)
+            return launch_stack<48>(pyr, S, paired_in, pairs, bsum2, o, e, gray, winmax, tilemax, tile_flag, flags_clean,
+                                    stream, between_kernels);
+        return launch_stack<64>(pyr, S, paired_in, pairs, bsum2, o, e, gray, winmax, tilemax, tile_flag, flags_clean,
+                                stream, between_kernels);
+    };
+    return half_out ? launch(__half()) : launch(float());
 }
 
 
@@ -2001,9 +2076,9 @@ int check_bank(const silent_orientation_bank *W, const char *who)
     return SILENT_OK;
 }
 
-template <int NB>
+template <int NB, typename OutT>
 static int launch_bank(const silent_orientation_bank *W, int n, int h, int w, int levels, int pairs, const f2 *bsum2,
-                       float *orient, float *line_end, float *gray, cudaStream_t stream)
+                       OutT *orient, OutT *line_end, float *gray, cudaStream_t stream)
 {
     ParamsBank<NB> B;
     for (int t = 0; t < 49; ++t) B.wb[t] = dup(W->blur[t * NB * NB]);
@@ -2017,22 +2092,22 @@ static int launch_bank(const silent_orientation_bank *W, int n, int h, int w, in
     B.h = h, B.w = w, B.n = n, B.pair_levels = pack_pair_levels(levels);
 
     using Tile = BankTile<NB>;
-    using T = typename Tile::T;
-    auto kern = stack_bank_kernel<NB, Tile::TH, Tile::TW, Tile::NT>;
+    using T = TileBank<NB, Tile::TH, Tile::TW, OutT>;
+    auto kern = stack_bank_kernel<NB, Tile::TH, Tile::TW, Tile::NT, OutT>;
     SILENT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T::kSmemBytes));
     const dim3 grid(ceil_div(w, Tile::TW), ceil_div(h, Tile::TH), pairs);
-    StoreMaps maps;   // tile rows of up to 388 floats: described in 8-byte elements (a box holds at most 256 of them)
+    StoreMaps maps;   // tile rows of up to 388 floats (264 halves): described in 8-byte elements (a box holds at most 256)
     std::memset(&maps, 0, sizeof(maps));
-    const int pad = T::ST_PITCH - NB * Tile::TW;
-    B.tma_store = (!orient || make_tile_store_map(&maps.orient, orient, n, h, w, NB, Tile::TW, pad, kTileStoreRows, 2)) &&
-                  (!line_end || make_tile_store_map(&maps.line_end, line_end, n, h, w, NB, Tile::TW, pad, kTileStoreRows, 2));
+    const int pad = T::ST_PITCH - NB * Tile::TW, V = sizeof(OutT);
+    B.tma_store = (!orient || make_tile_store_map(&maps.orient, orient, n, h, w, NB, Tile::TW, pad, kTileStoreRows, V, 8)) &&
+                  (!line_end || make_tile_store_map(&maps.line_end, line_end, n, h, w, NB, Tile::TW, pad, kTileStoreRows, V, 8));
     SILENT_CUDA(launch_dependent(kern, grid, dim3(Tile::NT), T::kSmemBytes, stream, bsum2, B, maps, orient, line_end, gray));
     SILENT_LAUNCH_CHECK("stack_bank_kernel");
     return SILENT_OK;
 }
 
-int stack_bank(const void *pyr, int n, int h, int w, int pair_levels, const silent_orientation_bank *W, float *orient,
-               float *line_end, float *gray, void *workspace, size_t workspace_bytes, cudaStream_t stream,
+int stack_bank(const void *pyr, int n, int h, int w, int pair_levels, const silent_orientation_bank *W, void *orient,
+               void *line_end, bool half_out, float *gray, void *workspace, size_t workspace_bytes, cudaStream_t stream,
                cudaEvent_t between_kernels)
 {
     int pairs = 0;
@@ -2051,12 +2126,17 @@ int stack_bank(const void *pyr, int n, int h, int w, int pair_levels, const sile
                               : launch_stack_a<64>(pyr, S, paired_in, pairs, bsum2, stream);
     if (rc != SILENT_OK) return rc;
     if (between_kernels) SILENT_CUDA(cudaEventRecord(between_kernels, stream));   // stage timing hook
-    switch (W->orientations) {
-    case 4: return launch_bank<4>(W, n, h, w, levels, pairs, bsum2, orient, line_end, gray, stream);
-    case 8: return launch_bank<8>(W, n, h, w, levels, pairs, bsum2, orient, line_end, gray, stream);
-    case 12: return launch_bank<12>(W, n, h, w, levels, pairs, bsum2, orient, line_end, gray, stream);
-    default: return launch_bank<16>(W, n, h, w, levels, pairs, bsum2, orient, line_end, gray, stream);
-    }
+    auto launch = [&](auto out_type) {
+        using OutT = decltype(out_type);
+        OutT *o = static_cast<OutT *>(orient), *e = static_cast<OutT *>(line_end);
+        switch (W->orientations) {
+        case 4: return launch_bank<4>(W, n, h, w, levels, pairs, bsum2, o, e, gray, stream);
+        case 8: return launch_bank<8>(W, n, h, w, levels, pairs, bsum2, o, e, gray, stream);
+        case 12: return launch_bank<12>(W, n, h, w, levels, pairs, bsum2, o, e, gray, stream);
+        default: return launch_bank<16>(W, n, h, w, levels, pairs, bsum2, o, e, gray, stream);
+        }
+    };
+    return half_out ? launch(__half()) : launch(float());
 }
 
 }  // namespace silent
@@ -2073,18 +2153,45 @@ int silent_stack_fused(const float *pyramid_dev, int n, int h, int w, const sile
                        float *orient_dev, float *line_end_dev, float *gray_dev, void *workspace_dev,
                        size_t workspace_bytes, silent_stream stream)
 {
-    return silent::stack_fused(pyramid_dev, n, h, w, 0, weights_host, orient_dev, line_end_dev, gray_dev, workspace_dev,
-                               workspace_bytes, nullptr, nullptr, nullptr, (cudaStream_t)stream, nullptr, false);
+    return silent::stack_fused(pyramid_dev, n, h, w, 0, weights_host, orient_dev, line_end_dev, false, gray_dev,
+                               workspace_dev, workspace_bytes, nullptr, nullptr, nullptr, (cudaStream_t)stream, nullptr,
+                               false);
+}
+
+int silent_stack_fused_f16(const float *pyramid_dev, int n, int h, int w, const silent_stack_weights *weights_host,
+                           uint16_t *orient_dev, uint16_t *line_end_dev, float *gray_dev, void *workspace_dev,
+                           size_t workspace_bytes, silent_stream stream)
+{
+    return silent::stack_fused(pyramid_dev, n, h, w, 0, weights_host, orient_dev, line_end_dev, true, gray_dev,
+                               workspace_dev, workspace_bytes, nullptr, nullptr, nullptr, (cudaStream_t)stream, nullptr,
+                               false);
+}
+
+// shared body of silent_stack_bank and silent_stack_bank_f16
+static int stack_bank_entry(const char *who, const float *pyramid_dev, int n, int h, int w,
+                            const silent_orientation_bank *bank_host, void *orient_dev, void *line_end_dev, bool half_out,
+                            float *gray_dev, void *workspace_dev, size_t workspace_bytes, silent_stream stream)
+{
+    const int rc = silent::check_bank(bank_host, who);
+    if (rc != SILENT_OK) return rc;
+    return silent::stack_bank(pyramid_dev, n, h, w, 0, bank_host, orient_dev, line_end_dev, half_out, gray_dev,
+                              workspace_dev, workspace_bytes, (cudaStream_t)stream);
 }
 
 int silent_stack_bank(const float *pyramid_dev, int n, int h, int w, const silent_orientation_bank *bank_host,
                       float *orient_dev, float *line_end_dev, float *gray_dev, void *workspace_dev, size_t workspace_bytes,
                       silent_stream stream)
 {
-    const int rc = silent::check_bank(bank_host, "silent_stack_bank");
-    if (rc != SILENT_OK) return rc;
-    return silent::stack_bank(pyramid_dev, n, h, w, 0, bank_host, orient_dev, line_end_dev, gray_dev, workspace_dev,
-                              workspace_bytes, (cudaStream_t)stream);
+    return stack_bank_entry("silent_stack_bank", pyramid_dev, n, h, w, bank_host, orient_dev, line_end_dev, false, gray_dev,
+                            workspace_dev, workspace_bytes, stream);
+}
+
+int silent_stack_bank_f16(const float *pyramid_dev, int n, int h, int w, const silent_orientation_bank *bank_host,
+                          uint16_t *orient_dev, uint16_t *line_end_dev, float *gray_dev, void *workspace_dev,
+                          size_t workspace_bytes, silent_stream stream)
+{
+    return stack_bank_entry("silent_stack_bank_f16", pyramid_dev, n, h, w, bank_host, orient_dev, line_end_dev, true,
+                            gray_dev, workspace_dev, workspace_bytes, stream);
 }
 
 }  // extern "C"

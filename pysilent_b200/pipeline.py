@@ -47,10 +47,18 @@ class LineEndPipeline:
 
     Constructor keywords follow ``PyramidDisplayer.__init__`` (``pyramid_displayer.py:22``): ``output_size`` is
     ``(w, h)`` of every pyramid level, ``zoom_ratio`` the scale between levels.
+
+    ``out_dtype`` is the dtype of ``orient`` and ``padded_line_end`` on every entry point: ``torch.float32`` (default) or
+    ``torch.float16``. With float16 each value is the float32 result rounded once to nearest even, as ``.half()`` rounds
+    it; the fused kernels store it that way (half the output bytes, on the device and over the host link), the other
+    paths cast their float32 result once. ``gray`` stays float32, and the feature points are the float32 call's.
     """
 
     def __init__(self, n_dimensions=2, output_size=(288, 192), output_colors=3, zoom_ratio=math.e ** .5, device=None,
-                 orientations=None):
+                 orientations=None, out_dtype=torch.float32):
+        if out_dtype not in _ops.OUT_DTYPES:
+            raise ValueError("out_dtype must be torch.float32 or torch.float16, got %r" % (out_dtype,))
+        self.out_dtype = out_dtype
         # None: the reference's 3 simplex orientations; n: a bank of n orientations (config C4: 8). Fused kernels for n = 4,
         # 8, 12 and 16; other n up to 8 run operator by operator
         self.orientations = orientations
@@ -86,6 +94,15 @@ class LineEndPipeline:
         _ops._require_cuda()
         return self.device if self.device is not None else torch.device("cuda", torch.cuda.current_device())
 
+    def _half(self):
+        return self.out_dtype == torch.float16
+
+    def _cast(self, res):
+        """A float32 result in ``out_dtype``: orient and padded_line_end rounded once (``.half()``), gray and points kept."""
+        if not self._half():
+            return res
+        return res._replace(orient=res.orient.half(), padded_line_end=res.padded_line_end.half())
+
     def _region(self):
         rh, rw = self.region_shape[1], self.region_shape[2]
         if int(rh) != rh or int(rw) != rw:
@@ -104,7 +121,7 @@ class LineEndPipeline:
         # finite input only (include/silent_b200.h). NaN / Inf / huge values go operator by operator, like the graph.
         if not _ops.fused_input_ok(x):
             return self.run_unfused(x, want_points)
-        orient, line_end, gray = _ops.stack_fused(x, self.stack_weights())
+        orient, line_end, gray = _ops.stack_fused(x, self.stack_weights(), out_dtype=self.out_dtype)
         points = None
         if want_points:
             rh, rw = self._region()
@@ -122,7 +139,7 @@ class LineEndPipeline:
         padded = pad_inwards(line_end, [[0, 0], [2, 2], [2, 2], [0, 0]])
         gray = get_value_from_color(padded)
         points = max_value_indices_region(padded, self.region_shape, gray) if want_points else None
-        return LineEndResult(orient, padded, gray, points)
+        return self._cast(LineEndResult(orient, padded, gray, points))
 
     def bank_filters(self):
         if self._bank is None:
@@ -158,7 +175,7 @@ class LineEndPipeline:
             if not _ops.fused_input_ok(x):
                 raise ValueError("a pyramid with NaN, Inf or values beyond 1e30 goes operator by operator, which supports "
                                  "at most 8 orientations (got %d)" % nb)
-            orient, padded, gray = _ops.stack_bank(x, self.orientation_bank())
+            orient, padded, gray = _ops.stack_bank(x, self.orientation_bank(), out_dtype=self.out_dtype)
             points = max_value_indices_region(padded, region, gray) if want_points else None
             return LineEndResult(orient, padded, gray, points)
         f = self.bank_filters()
@@ -168,7 +185,7 @@ class LineEndPipeline:
         padded = pad_inwards(line_end, [[0, 0], [2, 2], [2, 2], [0, 0]])
         gray = get_value_from_color(padded)
         points = max_value_indices_region(padded, region, gray) if want_points else None
-        return LineEndResult(orient, padded, gray, points)
+        return self._cast(LineEndResult(orient, padded, gray, points))
 
     # -- frames resident in HBM ---------------------------------------------------------------------------------------
     def _plan(self, frame_shape, frame_dtype, device):
@@ -191,9 +208,13 @@ class LineEndPipeline:
 
         ``out`` may carry preallocated ``(orient, padded_line_end, points, count)`` tensors to avoid allocation in a
         steady-state loop; ``points`` then holds ``count`` valid rows (no host sync is performed in that case). With
-        ``orientations`` set, orient and padded_line_end have ``orientations`` channels instead of 3.
+        ``orientations`` set, orient and padded_line_end have ``orientations`` channels instead of 3. Both are of
+        ``out_dtype``, and so must be the ``out`` buffers.
         """
         nb = self._bank_width() if self.orientations is not None else None
+        if out is not None and (out[0].dtype != self.out_dtype or out[1].dtype != self.out_dtype):
+            raise ValueError("run_frames(out=...) needs orient and padded_line_end buffers of %s, got %s and %s"
+                             % (self.out_dtype, out[0].dtype, out[1].dtype))
         frames = frames if frames.dim() == 4 else frames.unsqueeze(0)
         frames = frames.contiguous()
         if nb is not None and not (nb in _lib.FUSED_BANK_WIDTHS and frames.dtype == torch.uint8 and frames.shape[3] >= 3
@@ -208,7 +229,7 @@ class LineEndPipeline:
         n = b * plan.levels
         dev = frames.device
         if out is None:
-            orient = torch.empty((n, plan.h, plan.w, nb or 3), dtype=torch.float32, device=dev)
+            orient = torch.empty((n, plan.h, plan.w, nb or 3), dtype=self.out_dtype, device=dev)
             line_end = torch.empty_like(orient)
             cap = int(points_capacity) if points_capacity else max(64 * n, 1024)
             points = torch.empty((cap, 4), dtype=torch.int64, device=dev)
@@ -222,6 +243,8 @@ class LineEndPipeline:
             name, args = "silent_pipeline_run", (ctypes.byref(self.stack_weights()), _ops.ptr(frames), b, None)
         else:
             name, args = "silent_pipeline_run_orientations", (ctypes.byref(self.orientation_bank()), _ops.ptr(frames), b)
+        if self._half():
+            name += "_f16"
         with torch.cuda.device(dev):
             _lib.check(getattr(_lib.lib(), name)(
                 plan.handle, *args, _ops.ptr(orient), _ops.ptr(line_end), _ops.ptr(points), cap,
@@ -238,9 +261,14 @@ class LineEndPipeline:
     # -- host buffers on both sides (LineEndDisplayer.callback) -----------------------------------------------------------
     def run_host(self, frames, orient_out=None, line_end_out=None, points_capacity=4096):
         """frames: host numpy ``[B, H, W, 3]`` (ideally page-locked) -> host numpy results via the C-ABI host call (with
-        ``orientations`` set: through ``run_frames`` and page-locked buffers, results ``[B * L, h, w, orientations]``)."""
+        ``orientations`` set: through ``run_frames`` and page-locked buffers, results ``[B * L, h, w, orientations]``).
+        With ``out_dtype=torch.float16`` the results are ``np.float16``, and so must be ``orient_out`` / ``line_end_out``."""
         if self.orientations is not None:
             self._bank_width()
+        if self._half():
+            for name, arr in (("orient_out", orient_out), ("line_end_out", line_end_out)):
+                if arr is not None and arr.dtype != np.float16:
+                    raise ValueError("%s must be a np.float16 array for out_dtype=torch.float16, got %s" % (name, arr.dtype))
         frames = np.ascontiguousarray(frames)
         if frames.ndim == 3:
             frames = frames[np.newaxis]
@@ -253,17 +281,19 @@ class LineEndPipeline:
         plan = self._plan(frames.shape[1:], tdtype, dev)
         b = frames.shape[0]
         n = b * plan.levels
+        out_np = np.float16 if self._half() else np.float32
         if orient_out is None:
-            orient_out = np.empty((n, plan.h, plan.w, 3), np.float32)
+            orient_out = np.empty((n, plan.h, plan.w, 3), out_np)
         if line_end_out is None:
-            line_end_out = np.empty((n, plan.h, plan.w, 3), np.float32)
+            line_end_out = np.empty((n, plan.h, plan.w, 3), out_np)
         points = np.empty((points_capacity, 4), np.int64)
         count = ctypes.c_int64(0)
+        name = "silent_pipeline_run_host_f16" if self._half() else "silent_pipeline_run_host"
         with torch.cuda.device(dev):
-            _lib.check(_lib.lib().silent_pipeline_run_host(
+            _lib.check(getattr(_lib.lib(), name)(
                 plan.handle, ctypes.byref(self.stack_weights()), frames.ctypes.data, b, orient_out.ctypes.data,
                 line_end_out.ctypes.data, points.ctypes.data, points_capacity, ctypes.byref(count),
-                _ops.stream_ptr()), "silent_pipeline_run_host")
+                _ops.stream_ptr()), name)
         if count.value > points_capacity:
             # rare (an all-zero level emits every pixel, top_value_points.py:42-44): redo with room for every point, as
             # run_frames does -- feature points are never silently truncated

@@ -28,6 +28,9 @@ class LineEndDisplayer(LineEndPipeline):
         """Line-end ("end-stopped") detector stage on top of the pyramid pipeline; same constructor attributes as the
         reference's ``LineEndDisplayer.__init__`` (``recognition_testing.py:22-43``)."""
         super(LineEndDisplayer, self).__init__(n_dimensions, **argv)
+        if self.out_dtype != torch.float32:   # the display chain reads float32 padded_line_end
+            raise ValueError("LineEndDisplayer computes its display images from float32 outputs; out_dtype must be "
+                             "torch.float32, got %s" % (self.out_dtype,))
         self.tensor_return_type = [torch.Tensor]
         self.precompile_list = []
         self.constant_recovery = True
