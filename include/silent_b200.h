@@ -39,7 +39,13 @@ typedef enum silent_status {
     SILENT_E_NCCL = -6       /* NCCL could not be loaded, or reported an error (also asynchronously) */
 } silent_status;
 
-typedef enum silent_dtype { SILENT_U8 = 0, SILENT_F32 = 1 } silent_dtype;
+/* SILENT_NV12: 4:2:0 frames as video decoders (NVDEC) and cv2 lay them out, one contiguous [H * 3 / 2, W] uint8 array per
+ * frame: H rows of Y, then H / 2 rows of interleaved (U, V) pairs, one pair per 2 x 2 block, U first. A plan of this
+ * dtype needs frame_c = num_colors = 3 and even H and W. Every entry point that accepts it computes exactly what it
+ * computes on the BGR frame cv2.cvtColor(frame, cv2.COLOR_YUV2BGR_NV12) returns (BT.601 limited range, see
+ * silent_nv12_to_bgr): the frames are converted on the GPU first, into a plan-owned buffer, and then take the uint8
+ * BGR path. The plan's geometry (levels, level info, tap tables) is the BGR plan's for the same H x W. */
+typedef enum silent_dtype { SILENT_U8 = 0, SILENT_F32 = 1, SILENT_NV12 = 2 } silent_dtype;
 
 typedef void *silent_stream; /* cudaStream_t */
 typedef struct silent_plan silent_plan;
@@ -51,7 +57,7 @@ typedef struct silent_params {
     int32_t num_colors;                /* channels 0..num_colors-1 go into the pyramid (from_image.py:54) */
     int32_t center_w, center_h;        /* center_dimensions, (w, h) order as the reference passes it (from_image.py:44) */
     double scale;                      /* zoom_ratio > 1 (from_image.py:38) */
-    int32_t frame_dtype;               /* silent_dtype of the frames: SILENT_U8 (camera) or SILENT_F32 */
+    int32_t frame_dtype;               /* silent_dtype of the frames: SILENT_U8 (camera), SILENT_F32 or SILENT_NV12 */
     int32_t reserved;
 } silent_params;
 
@@ -113,7 +119,8 @@ int silent_device_count(void);
 int silent_plan_create(const silent_params *params, silent_plan **out_plan);
 void silent_plan_destroy(silent_plan *plan);
 /* Pre-size the plan-owned workspace / pinned staging buffers for up to max_batch frames (needed by *_host calls and
- * silent_pipeline_run). May be called again with a larger batch. */
+ * silent_pipeline_run, and by silent_pyramid_build on an SILENT_NV12 plan, whose converted frames live in it). May be
+ * called again with a larger batch. */
 int silent_plan_reserve(silent_plan *plan, int max_batch);
 
 int silent_plan_levels(const silent_plan *plan);                 /* num_scales, from_image.py:45-46 */
@@ -125,14 +132,15 @@ int silent_plan_level_info(const silent_plan *plan, int level, int *y0, int *y1,
  * output row/column that is defined as 0. */
 int silent_plan_level_tables(const silent_plan *plan, int level, int32_t *idx_y, float *w_y, int32_t *idx_x,
                              float *w_x);
-/* Algorithmic HBM bytes of one frame through silent_pipeline_run (SURVEY.md 8(d)): union crop read + two output
- * tensors; feature points excluded. */
+/* Algorithmic HBM bytes of one frame through silent_pipeline_run (SURVEY.md 8(d)): union crop read (1.5 bytes per pixel
+ * for SILENT_NV12) + two output tensors; feature points excluded. */
 int64_t silent_plan_algorithmic_bytes(const silent_plan *plan);
 
 /* ---- per-operator entry points ----------------------------------------------------------------------------------- */
 
 /* zoom.from_image (util/zoom/from_image.py:10-69) for a batch: frames_dev [batch, H, W, frame_c] of params.frame_dtype
- * -> pyramid_dev [batch * L, h, w, num_colors] float32. Rows/columns the reference leaves uninitialised are 0. */
+ * -> pyramid_dev [batch * L, h, w, num_colors] float32. Rows/columns the reference leaves uninitialised are 0.
+ * SILENT_NV12 plans take frames_dev [batch, H * 3 / 2, W] and need silent_plan_reserve(plan, batch) first. */
 int silent_pyramid_build(const silent_plan *plan, const void *frames_dev, int batch, float *pyramid_dev,
                          silent_stream stream);
 
@@ -168,6 +176,15 @@ int silent_max_value_indices_region(const float *value_dev, int n, int h, int w,
 int silent_top_value_points(const float *color_dev, const float *value_dev, int n, int h, int w, int c,
                             double top_percent, float *out_dev, void *workspace_dev, size_t workspace_bytes,
                             silent_stream stream);
+
+/* cv2.cvtColor(frame, cv2.COLOR_YUV2BGR_NV12) for a batch on the GPU: nv12_dev [batch, h * 3 / 2, w] uint8 (layout at
+ * SILENT_NV12) -> bgr_dev [batch, h, w, 3] uint8, both contiguous. h and w even. BT.601 limited range in 20-bit fixed
+ * point, bit-identical to OpenCV's integer code: with u = U - 128, v = V - 128 of the pixel's 2 x 2 block and
+ * y = max(0, Y - 16) * 1220542,
+ *   B = sat8((y + 2^19 + 2116026 u) >> 20), G = sat8((y + 2^19 - 852492 v - 409993 u) >> 20),
+ *   R = sat8((y + 2^19 + 1673527 v) >> 20)   (arithmetic shift; every sum fits in int32).
+ * The same device routine converts the frames of a SILENT_NV12 plan. Argument checks run before any CUDA call. */
+int silent_nv12_to_bgr(const uint8_t *nv12_dev, int batch, int h, int w, uint8_t *bgr_dev, silent_stream stream);
 
 /* ---- display tensors that follow gray_line_end_tensor (recognition_testing.py:79-100) --------------------------------- */
 
@@ -316,7 +333,8 @@ int silent_plan_stage_ms(silent_plan *plan, float *pyramid_ms, float *stack_ms, 
 int silent_plan_stack_split_ms(silent_plan *plan, float *stack_a_ms, float *stack_b_ms);
 
 /* Same, with HOST buffers on both sides: the drop-in for LineEndDisplayer.callback (recognition_testing.py:136-144):
- * frames_host [batch,H,W,frame_c] -> orient_host, line_end_host [batch*L,h,w,3], points_host [capacity][4], *count_host.
+ * frames_host [batch,H,W,frame_c] ([batch,H*3/2,W] on a SILENT_NV12 plan: half the upload of BGR) -> orient_host,
+ * line_end_host [batch*L,h,w,3], points_host [capacity][4], *count_host.
  * Copies go through plan-owned pinned staging buffers; synchronises `stream` before returning. Output pointers may be
  * NULL to skip the corresponding device->host copy. */
 int silent_pipeline_run_host(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_host,

@@ -12,7 +12,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libsilent_b200.so")
 
-SILENT_U8, SILENT_F32 = 0, 1
+SILENT_U8, SILENT_F32, SILENT_NV12 = 0, 1, 2
 POST_NONE, POST_RELU, POST_RELU_CLIP = 0, 1, 2
 PW_DIV255, PW_INVERT255, PW_IMPORTANCE, PW_MUL255, PW_ENERGY_DISPLAY, PW_PRODUCT = range(6)
 
@@ -28,7 +28,7 @@ SYMBOLS = (
     "silent_display_sequence_scratch_bytes", "silent_display_sequence", "silent_pack_points",
     "silent_comm_unique_id", "silent_comm_create", "silent_comm_destroy", "silent_comm_check", "silent_gather_points",
     "silent_stack_fused_f16", "silent_stack_bank_f16", "silent_pipeline_run_f16", "silent_pipeline_run_orientations_f16",
-    "silent_pipeline_run_host_f16",
+    "silent_pipeline_run_host_f16", "silent_nv12_to_bgr",
 )
 
 
@@ -117,6 +117,7 @@ def lib():
         "silent_pipeline_run_f16": (i, [p, ctypes.POINTER(SilentStackWeights), p, i, p, p, p, p, i64, p, p]),
         "silent_pipeline_run_orientations_f16": (i, [p, ctypes.POINTER(SilentOrientationBank), p, i, p, p, p, i64, p, p]),
         "silent_pipeline_run_host_f16": (i, [p, ctypes.POINTER(SilentStackWeights), p, i, p, p, p, i64, p, p]),
+        "silent_nv12_to_bgr": (i, [p, i, i, i, p, p]),
         "silent_get_centroids": (i, [p, i, i, i, i, i, p, p, p, p]),
         "silent_resize_nearest": (i, [p, i, i, i, i, i, i, p, p]),
         "silent_get_boosting": (i, [p, p, i, i, i, f, f, i, p, p, p]),

@@ -279,6 +279,39 @@ def display_sequence_scratch_bytes(steps, n, h, w, region_h, region_w):
                                                                 int(region_w)))
 
 
+# frame layouts LineEndPipeline(frame_format=...) takes: interleaved [H, W, 3] BGR, or NV12 (include/silent_b200.h)
+FRAME_FORMATS = ("bgr", "nv12")
+
+
+def nv12_frame_hw(shape, dtype, ranks=(2, 3), what="NV12 frames"):
+    """``(H, W)`` of NV12 frames of ``shape`` (a uint8 ``[H * 3 / 2, W]`` array per frame, in an array of one of the
+    ``ranks``); ``ValueError`` for another dtype, rank or an odd frame size."""
+    if dtype not in (np.uint8, torch.uint8):
+        raise ValueError("%s are uint8, got %s" % (what, dtype))
+    shape = tuple(int(v) for v in shape)
+    if len(shape) not in ranks or min(shape, default=0) < 1:
+        raise ValueError("%s need rank %s with no empty axis ([..., H * 3 / 2, W]), got shape %s"
+                         % (what, " or ".join(str(r) for r in ranks), shape))
+    rows, w = shape[-2:]
+    if rows % 3 or w % 2:
+        raise ValueError("%s need even height and width: %d rows of %d is not [H * 3 / 2, W] with H, W even"
+                         % (what, rows, w))
+    return 2 * rows // 3, w
+
+
+def nv12_to_bgr(frames):
+    """``silent_nv12_to_bgr``: NV12 frames ``[B, H * 3 / 2, W]`` (or one ``[H * 3 / 2, W]``), uint8, on the GPU ->
+    contiguous BGR ``[B, H, W, 3]`` uint8 on the same device, bit for bit ``cv2.cvtColor(frame, COLOR_YUV2BGR_NV12)``."""
+    h, w = nv12_frame_hw(frames.shape, frames.dtype)
+    x = as_device_tensor(frames, torch.uint8)
+    x = x if x.dim() == 3 else x.unsqueeze(0)
+    b = int(x.shape[0])
+    out = torch.empty((b, h, w, 3), dtype=torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().silent_nv12_to_bgr(ptr(x), b, h, w, ptr(out), stream_ptr()), "silent_nv12_to_bgr")
+    return out
+
+
 # output dtypes of the fused stacks: float32, or binary16 through the entry points named <symbol>_f16
 OUT_DTYPES = (torch.float32, torch.float16)
 

@@ -21,6 +21,7 @@ struct StageRange {
 static void release(Workspace &ws)
 {
     cudaFree(ws.d_frames);
+    cudaFree(ws.d_bgr);
     cudaFree(ws.d_pyramid);
     cudaFree(ws.d_orient);
     cudaFree(ws.d_line_end);
@@ -62,9 +63,11 @@ static bool is_pinned(const void *p, size_t bytes)
     return p && bytes > 0 && is_pinned_at(p) && is_pinned_at((const char *)p + bytes - 1);
 }
 
+// bytes of one frame as the caller passes it
 static size_t frame_bytes(const silent_plan *plan)
 {
     const silent_params &p = plan->params;
+    if (p.frame_dtype == SILENT_NV12) return (size_t)p.frame_h * p.frame_w * 3 / 2;
     return (size_t)p.frame_h * p.frame_w * p.frame_c * (p.frame_dtype == SILENT_U8 ? 1 : 4);
 }
 
@@ -106,6 +109,7 @@ int silent_plan_reserve(silent_plan *plan, int max_batch)
     ws.select_bytes = silent_selection_workspace_bytes((int)n, plan->h, plan->w);
     ws.points_capacity = (int64_t)n * 64;
     SILENT_CUDA(cudaMalloc(&ws.d_frames, frame_bytes(plan) * max_batch));
+    if (plan->params.frame_dtype == SILENT_NV12) SILENT_CUDA(cudaMalloc(&ws.d_bgr, (size_t)plan->frame_stride * max_batch));
     SILENT_CUDA(cudaMalloc(&ws.d_pyramid, pyr_bytes));
     SILENT_CUDA(cudaMalloc(&ws.d_orient, tensor_bytes));
     SILENT_CUDA(cudaMalloc(&ws.d_line_end, tensor_bytes));
@@ -141,7 +145,8 @@ static TileMaxima tile_maxima(const silent_plan *plan)
 // their place in the whole-batch tensors, so that the emit stage can run once over the batch afterwards. frame0 must be
 // even on the frame-pair path (pairs never straddle a chunk). K2 is the three-orientation stack (W) or, when bank is set,
 // the orientation bank's stack (frame-pair path only; no tile flags, geo must be null). orient_dev / line_end_dev hold
-// float32, or binary16 when half_out.
+// float32, or binary16 when half_out. NV12 frames are converted into ws.d_bgr first (these frames only), and the pyramid
+// reads them there.
 static int run_stack_stages(silent_plan *plan, const silent_stack_weights *W, const silent_orientation_bank *bank,
                             const void *frames_dev, int frame0, int nb, float *pyramid_dev, void *orient_dev,
                             void *line_end_dev, bool half_out, const WindowGeom *geo, cudaStream_t s,
@@ -153,10 +158,16 @@ static int run_stack_stages(silent_plan *plan, const silent_stack_weights *W, co
     const size_t img0 = (size_t)frame0 * plan->levels;
     const int n = nb * plan->levels;
     const unsigned char *frames = (const unsigned char *)frames_dev + frame_bytes(plan) * frame0;
+    int rc = SILENT_OK;
+    if (plan->params.frame_dtype == SILENT_NV12) {
+        StageRange range("silent:nv12");
+        rc = nv12_convert(plan, frames_dev, frame0, nb, s);
+        if (rc != SILENT_OK) return rc;
+        frames = ws.d_bgr + (size_t)plan->frame_stride * frame0;
+    }
     // stack_b's tile flags must be zero before it runs: the frame-pair pyramid kernel clears them on its way (and what
     // the caller adds in also_clear), so that no memset sits between the previous step's last kernel and this launch;
     // without that kernel a memset ahead of the launches does it
-    int rc = SILENT_OK;
     PairClear clear;   // (the bank's kernel keeps no tile flags: nothing to clear)
     if (!bank && pair_path) {
         stack_flag_region(ws.d_stack, n, plan->h, plan->w, &clear.a, &clear.a_bytes);

@@ -108,14 +108,21 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
     if (p->num_colors > p->frame_c || p->num_colors > kMaxChannels)
         return fail(SILENT_E_SHAPE, "num_colors=%d must be <= frame channels (%d) and <= %d", p->num_colors, p->frame_c,
                     kMaxChannels);
-    if (p->frame_dtype != SILENT_U8 && p->frame_dtype != SILENT_F32)
-        return fail(SILENT_E_INVAL, "frame_dtype must be SILENT_U8 or SILENT_F32");
+    if (p->frame_dtype != SILENT_U8 && p->frame_dtype != SILENT_F32 && p->frame_dtype != SILENT_NV12)
+        return fail(SILENT_E_INVAL, "frame_dtype must be SILENT_U8, SILENT_F32 or SILENT_NV12");
+    const bool nv12 = p->frame_dtype == SILENT_NV12;
+    if (nv12 && (p->frame_c != 3 || p->num_colors != 3))
+        return fail(SILENT_E_SHAPE, "NV12 frames convert to 3 colours: frame_c and num_colors must be 3, got %d and %d",
+                    p->frame_c, p->num_colors);
+    if (nv12 && (p->frame_h % 2 || p->frame_w % 2))
+        return fail(SILENT_E_SHAPE, "NV12 frames need even height and width, got %dx%d", p->frame_h, p->frame_w);
 
     silent_plan *plan = new (std::nothrow) silent_plan();
     if (!plan) return fail(SILENT_E_CAPACITY, "out of host memory");
     plan->params = *p;
     plan->h = p->center_h;
     plan->w = p->center_w;
+    plan->frame_pitch = nv12 ? ((int64_t)p->frame_w * 3 + 15) / 16 * 16 : (int64_t)p->frame_w * p->frame_c;
     const int dims_img[2] = {p->frame_h, p->frame_w};
     const int dims_ctr[2] = {p->center_h, p->center_w};
 
@@ -163,6 +170,21 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
         plan->union_w = std::max(plan->union_w, li.x1 - li.x0);
     }
 
+    // NV12: the frame rows and columns any tap reads, rounded out to row pairs and 16-pixel runs (the converter's unit)
+    if (nv12) {
+        int y0 = p->frame_h, y1 = 0, x0 = p->frame_w, x1 = 0;
+        for (size_t o = 0; o < plan->idx_y.size(); o += kTaps)
+            if (plan->idx_y[o] >= 0)
+                for (int t = 0; t < kTaps; ++t) y0 = std::min(y0, plan->idx_y[o + t]), y1 = std::max(y1, plan->idx_y[o + t] + 1);
+        for (size_t o = 0; o < plan->idx_x.size(); o += kTaps)
+            if (plan->idx_x[o] >= 0)
+                for (int t = 0; t < kTaps; ++t) x0 = std::min(x0, plan->idx_x[o + t]), x1 = std::max(x1, plan->idx_x[o + t] + 1);
+        if (y1 > y0 && x1 > x0) {
+            plan->nv12_y0 = y0 & ~1, plan->nv12_y1 = std::min(p->frame_h, (y1 + 1) & ~1);
+            plan->nv12_x0 = x0 & ~15, plan->nv12_x1 = std::min(p->frame_w, (x1 + 15) & ~15);
+        }
+    }
+
     // geometry of the frame-pair pyramid kernel: per level and x tile, the span of frame-row words its x-taps touch
     plan->pair.assign(L, PairLevel());
     // tile width: the widest one (<= 85 columns = 255 phase-H threads) that wastes the fewest columns of the last tile
@@ -174,7 +196,7 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
     }
     plan->pair_tile_w = kPairTileW;
     plan->pair_ok = L > 0 && L <= kPairMaxLevels && ceil_div(w, kPairTileW) <= kPairMaxTiles && p->frame_c >= 3 &&
-                    (int64_t)p->frame_h * p->frame_w * p->frame_c < INT32_MAX;   // row offsets inside a frame are 32-bit
+                    (int64_t)p->frame_h * plan->frame_pitch < INT32_MAX;   // row offsets inside a frame are 32-bit
     for (int s = 0; s < L && plan->pair_ok; ++s) {
         PairLevel &pl = plan->pair[s];
         pl.ntx = ceil_div(w, kPairTileW);
@@ -281,7 +303,7 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
                 // frame's row pitch in bytes and a task needs the first TWO 128-bit words only; else STEP = -(offset of
                 // tap row 5) - 1 and the third word holds the other four offsets.
                 std::vector<int32_t> ytab((size_t)L * h * 12, 0);
-                const int64_t row_bytes = (int64_t)p->frame_w * p->frame_c;
+                const int64_t row_bytes = plan->frame_pitch;
                 for (int s = 0; s < L; ++s)
                     for (int oy = 0; oy < h; ++oy) {
                         const int32_t *ty = &plan->idx_y[((size_t)s * h + oy) * kTaps];
@@ -329,6 +351,10 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
             plan->on_device = true;
         }
     }
+    // NV12: converted frames start at the texture alignment (512 B on B200), so every frame pair and every chunk of the
+    // host-buffer path can take the frame-pair kernel's texture route
+    const int64_t frame_align = nv12 ? std::max(plan->texture_alignment, 512) : 1;
+    plan->frame_stride = ((int64_t)p->frame_h * plan->frame_pitch + frame_align - 1) / frame_align * frame_align;
     *out_plan = plan;
     return SILENT_OK;
 }
@@ -375,8 +401,9 @@ int silent_plan_level_tables(const silent_plan *plan, int level, int32_t *idx_y,
 int64_t silent_plan_algorithmic_bytes(const silent_plan *plan)
 {
     if (!plan) return fail(SILENT_E_INVAL, "null plan");
-    const int64_t elem = plan->params.frame_dtype == SILENT_U8 ? 1 : 4;
-    const int64_t in_bytes = (int64_t)plan->union_h * plan->union_w * plan->params.frame_c * elem;
+    const int64_t px = (int64_t)plan->union_h * plan->union_w;
+    const int dtype = plan->params.frame_dtype;
+    const int64_t in_bytes = dtype == SILENT_NV12 ? px * 3 / 2 : px * plan->params.frame_c * (dtype == SILENT_U8 ? 1 : 4);
     const int64_t out_bytes = 2LL * plan->levels * plan->h * plan->w * plan->params.num_colors * 4;
     return in_bytes + out_bytes;
 }

@@ -28,7 +28,8 @@ constexpr int kMaxChunks = 16;   // chunks per silent_pipeline_run_host call
 // Plan-owned device scratch, sized by silent_plan_reserve(max_batch).
 struct Workspace {
     int batch = 0;
-    void *d_frames = nullptr;      // [B,H,W,FC] staging for *_host calls
+    void *d_frames = nullptr;      // [B,H,W,FC] staging for *_host calls ([B,H*3/2,W] on an NV12 plan)
+    uint8_t *d_bgr = nullptr;      // NV12 plans only: the converted frames the pyramid reads, [B][frame_stride] bytes
     float *d_pyramid = nullptr;    // [B*L,h,w,C] (NHWC path) or [ceil(B/2)*L][3][h][w] float2 (frame-pair path)
     float *d_orient = nullptr;     // [B*L,h,w,3] staging for *_host calls
     float *d_line_end = nullptr;
@@ -60,6 +61,11 @@ struct silent_plan {
     int levels = 0, h = 0, w = 0;
     int union_h = 0, union_w = 0;
     bool on_device = false;
+    // the frames the pyramid kernels read: row pitch and frame stride in bytes (frame elements for SILENT_F32). BGR and
+    // float frames are read in place (W * FC and H * W * FC). NV12 frames are converted first into ws.d_bgr, whose rows
+    // are padded to 16 bytes and whose frames to the texture alignment, so every frame takes the frame-pair path
+    int64_t frame_pitch = 0, frame_stride = 0;
+    int nv12_y0 = 0, nv12_y1 = 0, nv12_x0 = 0, nv12_x1 = 0;   // NV12: rows / columns converted (all tap rows / columns)
     std::vector<silent::LevelInfo> info;
     std::vector<int32_t> idx_y, idx_x;   // [L][h|w][6], absolute frame row / column, idx[.][0] = -1 => sample is 0
     std::vector<float> w_y, w_x;

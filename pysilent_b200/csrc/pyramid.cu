@@ -6,7 +6,7 @@
 //
 // Two kernels:
 //  * pyramid_kernel      one thread per output pixel, NHWC float32 output: the stand-alone from_image operator, any
-//                        channel count / frame dtype.
+//                        channel count / frame dtype. Frames are read at the plan's row pitch and frame stride.
 //  * pyramid_pair_kernel the pipeline's producer. One CTA = one tile of one level for TWO frames in lockstep (float2
 //                        lanes, like the stack kernels). Phase V walks ALIGNED 128-bit words of the uint8 frame down the
 //                        6 tap rows (coalesced, 16 byte-columns per load), converts with PRMT + FADD2 (the I2F pipe is
@@ -39,7 +39,7 @@ template <typename T, int NC>
 __global__ void __launch_bounds__(256) pyramid_kernel(const T *__restrict__ frames, float *__restrict__ out,
                                                       const int32_t *__restrict__ idx_y, const float *__restrict__ w_y,
                                                       const int32_t *__restrict__ idx_x, const float *__restrict__ w_x,
-                                                      int L, int h, int w, int H, int W, int FC)
+                                                      int L, int h, int w, size_t frame_stride, int row_pitch, int FC)
 {
     const int ox = blockIdx.x * blockDim.x + threadIdx.x;
     const int oy = blockIdx.y * blockDim.y + threadIdx.y;
@@ -57,12 +57,12 @@ __global__ void __launch_bounds__(256) pyramid_kernel(const T *__restrict__ fram
     for (int c = 0; c < NC; ++c) acc[c] = 0.0f;
 
     if (__ldg(ty) >= 0 && __ldg(tx) >= 0) {
-        const T *frame = frames + (size_t)b * H * W * FC;
+        const T *frame = frames + (size_t)b * frame_stride;
         size_t row_off[kTaps];
         float wy[kTaps];
 #pragma unroll
         for (int j = 0; j < kTaps; ++j) {
-            row_off[j] = (size_t)__ldg(ty + j) * W * FC;
+            row_off[j] = (size_t)__ldg(ty + j) * row_pitch;
             wy[j] = __ldg(gy + j);
         }
 #pragma unroll
@@ -95,7 +95,8 @@ static int launch_pyramid(const silent_plan *plan, const T *frames, int batch, f
 #define SILENT_PYR_CASE(NC)                                                                                           \
     case NC:                                                                                                          \
         pyramid_kernel<T, NC><<<grid, block, 0, stream>>>(frames, out, plan->d_idx_y, plan->d_w_y, plan->d_idx_x,     \
-                                                          plan->d_w_x, L, h, w, p.frame_h, p.frame_w, p.frame_c);     \
+                                                          plan->d_w_x, L, h, w, (size_t)plan->frame_stride,           \
+                                                          (int)plan->frame_pitch, p.frame_c);                         \
         break;
     switch (p.num_colors) {
         SILENT_PYR_CASE(1)
@@ -121,7 +122,7 @@ int pyramid_build(const silent_plan *plan, const void *frames_dev, int batch, fl
     if (plan->levels == 0) return SILENT_OK;
     if (!plan->on_device) return fail(SILENT_E_CUDA, "plan was created without a CUDA device; no CPU fallback exists");
     if ((long long)batch * plan->levels > 65535) return fail(SILENT_E_SHAPE, "batch * levels must be <= 65535");
-    if (plan->params.frame_dtype == SILENT_U8)
+    if (plan->params.frame_dtype != SILENT_F32)   // uint8 BGR frames, or NV12 frames converted to them
         return launch_pyramid<uint8_t>(plan, (const uint8_t *)frames_dev, batch, pyramid_dev, stream);
     return launch_pyramid<float>(plan, (const float *)frames_dev, batch, pyramid_dev, stream);
 }
@@ -306,12 +307,13 @@ __global__ void __launch_bounds__(kPairThreads, 768 / kPairThreads) pyramid_pair
     }
 }
 
-// Can the pair kernel serve this plan? (uint8 frames, 3 colours, word-aligned rows, table of tiles fits)
+// Can the pair kernel serve this plan? (uint8 frames, or NV12 frames converted to them, 3 colours, 16-byte aligned rows,
+// table of tiles fits)
 bool pyramid_pair_supported(const silent_plan *plan)
 {
     const silent_params &p = plan->params;
-    return plan->on_device && p.frame_dtype == SILENT_U8 && p.num_colors == 3 && (p.frame_w * p.frame_c) % 16 == 0 &&
-           plan->pair_ok;
+    return plan->on_device && (p.frame_dtype == SILENT_U8 || p.frame_dtype == SILENT_NV12) && p.num_colors == 3 &&
+           plan->frame_pitch % 16 == 0 && plan->pair_ok;
 }
 
 size_t pyramid_pair_bytes(const silent_plan *plan, int batch)
@@ -324,14 +326,13 @@ int pyramid_pair_build(const silent_plan *plan, const void *frames_dev, int batc
 {
     if (!pyramid_pair_supported(plan)) return fail(SILENT_E_SHAPE, "frame-pair pyramid kernel does not support this plan");
     if (((uintptr_t)frames_dev & 15) != 0) return fail(SILENT_E_INVAL, "frames must be 16-byte aligned");
-    const silent_params &p = plan->params;
     const int pairs = (batch + 1) / 2;
     if (pairs > 65535) return fail(SILENT_E_SHAPE, "at most 131070 frames per call");
     // frames as a texture of 128-bit texels (cached per plan: same pointer and size -> same object). The texture variant
     // needs a pointer at the device's texture alignment (CUDA requires it of a linear texture's devPtr), fewer than 2^27
     // texels (1-D linear textures; the texel index is a 32-bit int) and the phase-H table's texture; any other buffer
     // takes the LDG variant, which computes the same bits
-    const size_t total_bytes = (size_t)batch * p.frame_h * p.frame_w * p.frame_c;
+    const size_t total_bytes = (size_t)batch * plan->frame_stride;
     bool use_tex = plan->texture_alignment > 0 && (uintptr_t)frames_dev % (uintptr_t)plan->texture_alignment == 0 &&
                    (total_bytes >> 4) < ((size_t)1 << 27) && plan->htab_tex != 0;
     cudaTextureObject_t tex = 0;
@@ -377,7 +378,7 @@ int pyramid_pair_build(const silent_plan *plan, const void *frames_dev, int batc
     P.ytab = reinterpret_cast<const int4 *>(plan->d_pair_ytab);
     P.words = reinterpret_cast<const int4 *>(plan->d_pair_words);
     P.htab = reinterpret_cast<const int4 *>(plan->d_pair_htab);
-    P.frame_bytes = (size_t)p.frame_h * p.frame_w * p.frame_c;
+    P.frame_bytes = (size_t)plan->frame_stride;
     P.h = plan->h, P.w = plan->w, P.L = plan->levels, P.B = batch;
     P.tile_w = plan->pair_tile_w;
     P.clear_a = clear ? (uint4 *)clear->a : nullptr, P.clear_n16 = clear && clear->a ? (unsigned)(clear->a_bytes / 16) : 0u;
@@ -406,5 +407,16 @@ int pyramid_pair_build(const silent_plan *plan, const void *frames_dev, int batc
 extern "C" int silent_pyramid_build(const silent_plan *plan, const void *frames_dev, int batch, float *pyramid_dev,
                                     silent_stream stream)
 {
-    return silent::pyramid_build(plan, frames_dev, batch, pyramid_dev, (cudaStream_t)stream);
+    using namespace silent;
+    // NV12 frames are converted into the plan's buffer first; pyramid_build reads them there
+    if (plan && frames_dev && pyramid_dev && batch > 0 && plan->levels > 0 && plan->params.frame_dtype == SILENT_NV12) {
+        if (!plan->on_device) return fail(SILENT_E_CUDA, "plan was created without a CUDA device; no CPU fallback exists");
+        if (plan->ws.batch < batch)
+            return fail(SILENT_E_CAPACITY, "NV12 plan holds converted frames for %d frames, need %d: call silent_plan_reserve",
+                        plan->ws.batch, batch);
+        const int rc = nv12_convert(plan, frames_dev, 0, batch, (cudaStream_t)stream);
+        if (rc != SILENT_OK) return rc;
+        frames_dev = plan->ws.d_bgr;
+    }
+    return pyramid_build(plan, frames_dev, batch, pyramid_dev, (cudaStream_t)stream);
 }

@@ -55,6 +55,10 @@ struct PairClear {
 int pyramid_pair_build(const silent_plan *plan, const void *frames_dev, int batch, void *xpair_dev, cudaStream_t stream,
                        const PairClear *clear = nullptr);
 
+// nv12.cu: frames [frame0, frame0 + nb) of an NV12 batch (nv12_dev: frame 0) -> the same frames of plan->ws.d_bgr, at
+// the plan's frame pitch and stride; only the rows and columns the pyramid's taps read (plan->nv12_*)
+int nv12_convert(const silent_plan *plan, const void *nv12_dev, int frame0, int nb, cudaStream_t stream);
+
 // emit.cu
 bool window_geometry(int h, int w, int region_h, int region_w, WindowGeom *geo);
 int max_value_indices_region(const float *value, int n, int h, int w, int region_h, int region_w, int64_t *points,

@@ -52,13 +52,22 @@ class LineEndPipeline:
     ``torch.float16``. With float16 each value is the float32 result rounded once to nearest even, as ``.half()`` rounds
     it; the fused kernels store it that way (half the output bytes, on the device and over the host link), the other
     paths cast their float32 result once. ``gray`` stays float32, and the feature points are the float32 call's.
+
+    ``frame_format`` is the layout of the frames every entry point takes: ``"bgr"`` (default), ``[H, W, 3]`` per frame,
+    or ``"nv12"``, the 4:2:0 layout video decoders produce: one uint8 ``[H * 3 / 2, W]`` array per frame (H rows of Y,
+    then H / 2 rows of interleaved U, V), H and W even. An NV12 call returns exactly what the same call returns on the
+    frames ``cv2.cvtColor(frame, cv2.COLOR_YUV2BGR_NV12)`` makes of them; the conversion runs on the GPU, in front of the
+    pyramid, and only the bytes of the NV12 frames cross the host link.
     """
 
     def __init__(self, n_dimensions=2, output_size=(288, 192), output_colors=3, zoom_ratio=math.e ** .5, device=None,
-                 orientations=None, out_dtype=torch.float32):
+                 orientations=None, out_dtype=torch.float32, frame_format="bgr"):
         if out_dtype not in _ops.OUT_DTYPES:
             raise ValueError("out_dtype must be torch.float32 or torch.float16, got %r" % (out_dtype,))
+        if not isinstance(frame_format, str) or frame_format not in _ops.FRAME_FORMATS:
+            raise ValueError("frame_format must be one of %s, got %r" % (", ".join(_ops.FRAME_FORMATS), frame_format))
         self.out_dtype = out_dtype
+        self.frame_format = frame_format
         # None: the reference's 3 simplex orientations; n: a bank of n orientations (config C4: 8). Fused kernels for n = 4,
         # 8, 12 and 16; other n up to 8 run operator by operator
         self.orientations = orientations
@@ -96,6 +105,17 @@ class LineEndPipeline:
 
     def _half(self):
         return self.out_dtype == torch.float16
+
+    def _nv12(self):
+        return self.frame_format == "nv12"
+
+    def _nv12_fused(self, nb, w):
+        """Whether NV12 frames of width ``w`` go through an NV12 plan (conversion kernel, then the fused path) rather
+        than ``_ops.nv12_to_bgr`` and the BGR route: the routes a BGR frame of that width takes fused. A bank needs
+        16-byte BGR rows there (``run_frames``), the three-orientation stack computes the same bits either way."""
+        if self.blur_size != 7 or self.output_colors != 3:
+            return False
+        return nb is None or (nb in _lib.FUSED_BANK_WIDTHS and (3 * w) % 16 == 0)
 
     def _cast(self, res):
         """A float32 result in ``out_dtype``: orient and padded_line_end rounded once (``.half()``), gray and points kept."""
@@ -188,23 +208,30 @@ class LineEndPipeline:
         return self._cast(LineEndResult(orient, padded, gray, points))
 
     # -- frames resident in HBM ---------------------------------------------------------------------------------------
-    def _plan(self, frame_shape, frame_dtype, device):
+    def _plan(self, frame_shape, frame_dtype, device, frame_format="bgr"):
         """Plan cache keyed like the reference's per-shape session (``recognition_testing.py:108-118``). The cache is
-        per pipeline: use one ``LineEndPipeline`` per camera thread, as the reference uses one displayer per camera."""
-        key = (tuple(int(v) for v in frame_shape), frame_dtype, self.output_colors, self.output_size,
+        per pipeline: use one ``LineEndPipeline`` per camera thread, as the reference uses one displayer per camera.
+        NV12 plans take ``frame_shape`` ``(H, W, 3)`` of the image."""
+        key = (tuple(int(v) for v in frame_shape), frame_dtype, frame_format, self.output_colors, self.output_size,
                float(self.zoom_ratio), str(device))
         plan = self._plans.get(key)
         if plan is None:
             with torch.cuda.device(device):
-                plan = PyramidPlan(frame_shape, frame_dtype, self.output_colors, self.output_size, self.zoom_ratio)
+                plan = PyramidPlan(frame_shape, frame_dtype, self.output_colors, self.output_size, self.zoom_ratio,
+                                   frame_format)
             self._plans[key] = plan
         return plan
 
     def plan_for(self, frames):
+        """The plan of a batch of frames in the pipeline's ``frame_format``."""
+        if self._nv12():
+            h, w = _ops.nv12_frame_hw(frames.shape, frames.dtype)
+            return self._plan((h, w, 3), torch.uint8, frames.device, "nv12")
         return self._plan(frames.shape[1:], frames.dtype, frames.device)
 
     def run_frames(self, frames, want_points=True, points_capacity=None, out=None):
-        """frames: CUDA ``[B, H, W, 3]`` uint8/float32 -> LineEndResult over ``B * L`` levels (pyramid + S1-S8).
+        """frames: CUDA ``[B, H, W, 3]`` uint8/float32 (``frame_format="nv12"``: ``[B, H * 3 / 2, W]`` uint8) ->
+        LineEndResult over ``B * L`` levels (pyramid + S1-S8). A single frame may come without its batch axis.
 
         ``out`` may carry preallocated ``(orient, padded_line_end, points, count)`` tensors to avoid allocation in a
         steady-state loop; ``points`` then holds ``count`` valid rows (no host sync is performed in that case). With
@@ -215,15 +242,28 @@ class LineEndPipeline:
         if out is not None and (out[0].dtype != self.out_dtype or out[1].dtype != self.out_dtype):
             raise ValueError("run_frames(out=...) needs orient and padded_line_end buffers of %s, got %s and %s"
                              % (self.out_dtype, out[0].dtype, out[1].dtype))
+        if self._nv12():
+            h, w = _ops.nv12_frame_hw(frames.shape, frames.dtype)
+            frames = (frames if frames.dim() == 3 else frames.unsqueeze(0)).contiguous()
+            if not self._nv12_fused(nb, w):   # routes without an NV12 plan: convert, then the BGR route
+                return self._run_frames(_ops.nv12_to_bgr(frames), nb, want_points, points_capacity, out)
+            return self._run_frames(frames, nb, want_points, points_capacity, out, (h, w))
         frames = frames if frames.dim() == 4 else frames.unsqueeze(0)
-        frames = frames.contiguous()
-        if nb is not None and not (nb in _lib.FUSED_BANK_WIDTHS and frames.dtype == torch.uint8 and frames.shape[3] >= 3
-                                   and self.blur_size == 7 and self.output_colors == 3
-                                   and (frames.shape[2] * frames.shape[3]) % 16 == 0):
+        return self._run_frames(frames.contiguous(), nb, want_points, points_capacity, out)
+
+    def _run_frames(self, frames, nb, want_points, points_capacity, out, nv12_hw=None):
+        """run_frames on a contiguous batch: BGR / float ``[B, H, W, C]``, or NV12 ``[B, H * 3 / 2, W]`` of an
+        ``nv12_hw`` = ``(H, W)`` image through an NV12 plan."""
+        if nv12_hw is None and nb is not None and not (
+                nb in _lib.FUSED_BANK_WIDTHS and frames.dtype == torch.uint8 and frames.shape[3] >= 3
+                and self.blur_size == 7 and self.output_colors == 3 and (frames.shape[2] * frames.shape[3]) % 16 == 0):
             from .util.zoom.from_image import image_to_zoom_tensor   # other frames: pyramid, then run_bank
             return self.run_bank(image_to_zoom_tensor(frames, self.output_colors, self.output_size, self.zoom_ratio),
                                  want_points)
-        plan = self.plan_for(frames)
+        if nv12_hw is None:
+            plan = self._plan(frames.shape[1:], frames.dtype, frames.device)
+        else:
+            plan = self._plan(nv12_hw + (3,), torch.uint8, frames.device, "nv12")
         b = int(frames.shape[0])
         plan.reserve(b)
         n = b * plan.levels
@@ -255,30 +295,35 @@ class LineEndPipeline:
             return LineEndResult(orient, line_end, None, None)
         total = int(count.item())
         if total > cap:   # rare (e.g. an all-black level emits every pixel): redo the emit with room for everything
-            return self.run_frames(frames, want_points, points_capacity=total)
+            return self._run_frames(frames, nb, want_points, total, None, nv12_hw)
         return LineEndResult(orient, line_end, None, points[:total])
 
     # -- host buffers on both sides (LineEndDisplayer.callback) -----------------------------------------------------------
     def run_host(self, frames, orient_out=None, line_end_out=None, points_capacity=4096):
-        """frames: host numpy ``[B, H, W, 3]`` (ideally page-locked) -> host numpy results via the C-ABI host call (with
-        ``orientations`` set: through ``run_frames`` and page-locked buffers, results ``[B * L, h, w, orientations]``).
-        With ``out_dtype=torch.float16`` the results are ``np.float16``, and so must be ``orient_out`` / ``line_end_out``."""
-        if self.orientations is not None:
-            self._bank_width()
+        """frames: host numpy ``[B, H, W, 3]`` (``frame_format="nv12"``: ``[B, H * 3 / 2, W]`` uint8; ideally page-locked)
+        -> host numpy results via the C-ABI host call (with ``orientations`` set: through ``run_frames`` and page-locked
+        buffers, results ``[B * L, h, w, orientations]``). With ``out_dtype=torch.float16`` the results are
+        ``np.float16``, and so must be ``orient_out`` / ``line_end_out``."""
+        nb = self._bank_width() if self.orientations is not None else None
         if self._half():
             for name, arr in (("orient_out", orient_out), ("line_end_out", line_end_out)):
                 if arr is not None and arr.dtype != np.float16:
                     raise ValueError("%s must be a np.float16 array for out_dtype=torch.float16, got %s" % (name, arr.dtype))
+        frames = np.asarray(frames)
+        nv12_hw = _ops.nv12_frame_hw(frames.shape, frames.dtype) if self._nv12() else None
         frames = np.ascontiguousarray(frames)
-        if frames.ndim == 3:
+        if frames.ndim == (2 if nv12_hw else 3):
             frames = frames[np.newaxis]
         if frames.dtype != np.uint8:
             frames = frames.astype(np.float32)
         dev = self._device()
-        if self.orientations is not None:
+        if nb is not None or (nv12_hw and not self._nv12_fused(nb, nv12_hw[1])):
             return self._run_host_bank(frames, dev, orient_out, line_end_out, points_capacity)
         tdtype = torch.uint8 if frames.dtype == np.uint8 else torch.float32
-        plan = self._plan(frames.shape[1:], tdtype, dev)
+        if nv12_hw:
+            plan = self._plan(nv12_hw + (3,), tdtype, dev, "nv12")
+        else:
+            plan = self._plan(frames.shape[1:], tdtype, dev)
         b = frames.shape[0]
         n = b * plan.levels
         out_np = np.float16 if self._half() else np.float32
@@ -301,8 +346,9 @@ class LineEndPipeline:
         return LineEndResult(orient_out, line_end_out, None, points[:count.value])
 
     def _run_host_bank(self, frames, dev, orient_out, line_end_out, points_capacity):
-        """run_host for a bank: the frames go up from a page-locked copy, and the results come back with asynchronous
-        copies into page-locked buffers and one synchronisation, as ``LineEndDisplayer.callback`` does."""
+        """run_host for a bank (and for NV12 frames on a route without an NV12 plan): the frames go up from a page-locked
+        copy, and the results come back with asynchronous copies into page-locked buffers and one synchronisation, as
+        ``LineEndDisplayer.callback`` does."""
         staged = torch.from_numpy(frames).pin_memory()
         with torch.cuda.device(dev):
             res = self.run_frames(staged.to(dev, non_blocking=True), points_capacity=points_capacity)
@@ -326,7 +372,7 @@ class LineEndPipeline:
 
         Returns ``[frame, [orient level images...], [padded_line_end level images...], points]``: the two result
         tensors on the north-star path as per-level host images, plus the feature points the reference builds but never
-        fetches.
+        fetches. ``frame`` is the frame as given (an NV12 array with ``frame_format="nv12"``).
         """
         res = self.run_host(np.asarray(frame))
         return [frame, [res.orient[i] for i in range(res.orient.shape[0])],

@@ -100,16 +100,19 @@ class LineEndDisplayer(LineEndPipeline):
     def run_clip(self, frames):
         """A clip of consecutive frames resident in HBM -> the six display tensors on the device, in the order of
         ``run_frames_display``. ``frames`` is ``[T, H, W, 3]`` (one camera) or ``[T, S, H, W, 3]`` (S cameras),
-        time-major; step t's images are ``[t * S * L, (t + 1) * S * L)`` and equal, bit for bit, what
+        time-major (``frame_format="nv12"``: ``[T, H * 3 / 2, W]`` or ``[T, S, H * 3 / 2, W]``); step t's images are ``[t * S * L, (t + 1) * S * L)`` and equal, bit for bit, what
         ``run_frames_display(frames[t])`` returns when called for t = 0 ... T-1 in turn. ``energy_values`` ends where
         those calls leave it, so ``callback``, ``run_clip`` and ``callback`` on one camera continue one state. The
         pipeline runs once over all T * S frames, and the boosting recurrence over the whole clip in one launch."""
         rank = frames.dim() if isinstance(frames, torch.Tensor) else np.ndim(frames)
-        if rank not in (4, 5) or frames.shape[0] < 1:
+        frame_rank = 2 if self._nv12() else 3
+        if self._nv12():
+            _ops.nv12_frame_hw(frames.shape, frames.dtype, ranks=(3, 4), what="NV12 clips")
+        if rank not in (frame_rank + 1, frame_rank + 2) or frames.shape[0] < 1:
             raise ValueError("run_clip takes frames [T, H, W, 3] or [T, S, H, W, 3] with T >= 1, got shape %s"
                              % (tuple(frames.shape),))
         steps = int(frames.shape[0])
-        res = self.run_frames(frames.reshape((-1,) + tuple(frames.shape[-3:])), want_points=False)
+        res = self.run_frames(frames.reshape((-1,) + tuple(frames.shape[-frame_rank:])), want_points=False)
         orient, padded = res.orient, res.padded_line_end
         gray = get_value_from_color(padded)                                                       # :77
         step_shape = (orient.shape[0] // steps,) + tuple(orient.shape[1:])
@@ -120,13 +123,16 @@ class LineEndDisplayer(LineEndPipeline):
         return [orient, cent, cent2, fired, update, padded]
 
     def callback_clip(self, frames, cam_id=None):
-        """``callback`` over a host clip ``[T, H, W, 3]`` of one camera: a list of T results, each
+        """``callback`` over a host clip ``[T, H, W, 3]`` (``frame_format="nv12"``: ``[T, H * 3 / 2, W]``) of one
+        camera: a list of T results, each
         ``[frames[t]] + six lists of per-level images`` like ``callback``'s, with the state carried from step to step.
         The clip goes up through a page-locked buffer, runs through ``run_clip`` and comes back with asynchronous
         copies and one synchronisation. The arrays handed out stay untouched for the next ``host_slots - 1`` calls of
         ``callback`` or ``callback_clip``."""
         z = np.asarray(frames)
-        if z.ndim != 4 or z.shape[0] < 1:
+        if self._nv12():
+            _ops.nv12_frame_hw(z.shape, z.dtype, ranks=(3,), what="NV12 clips")
+        elif z.ndim != 4 or z.shape[0] < 1:
             raise ValueError("callback_clip takes host frames [T, H, W, 3] with T >= 1, got shape %s" % (z.shape,))
         if self.orientations is not None:
             self._bank_width()
@@ -147,10 +153,13 @@ class LineEndDisplayer(LineEndPipeline):
         return [[frames[t]] + [[outs[x][t * L + y] for y in range(L)] for x in range(6)] for t in range(z.shape[0])]
 
     def callback(self, frame, cam_id=None, depth=2):
-        """``recognition_testing.py:136-144``: ``[frame] + [[tensors[x][y] for y in levels] for x in range(6)]``."""
+        """``recognition_testing.py:136-144``: ``[frame] + [[tensors[x][y] for y in levels] for x in range(6)]``. With
+        ``frame_format="nv12"`` the frame is one NV12 array ``[H * 3 / 2, W]``, and comes back as given."""
         if self.orientations is not None:
             self._bank_width()
         z = np.asarray(frame)
+        if self._nv12():
+            _ops.nv12_frame_hw(z.shape, z.dtype, ranks=(2,))
         z = np.ascontiguousarray(z if z.dtype == np.uint8 else z.astype(np.float32))
         dev = self._device()
         self._slot = (self._slot + 1) % self.host_slots

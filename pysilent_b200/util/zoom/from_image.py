@@ -9,13 +9,18 @@ from ... import _lib, _ops
 
 
 class PyramidPlan:
-    """Owns a ``silent_plan`` (level geometry + order-5 spline tap tables, uploaded once)."""
+    """Owns a ``silent_plan`` (level geometry + order-5 spline tap tables, uploaded once). ``frame_shape`` is
+    ``(H, W, C)``; with ``frame_format="nv12"`` the frames are NV12 ``[H * 3 / 2, W]`` uint8 arrays of an H x W x 3
+    image (``C`` = 3), converted on the GPU before the pyramid reads them."""
 
-    def __init__(self, frame_shape, frame_dtype, num_colors, center_dimensions, scale):
+    def __init__(self, frame_shape, frame_dtype, num_colors, center_dimensions, scale, frame_format="bgr"):
         h, w, c = (int(v) for v in frame_shape)
+        if frame_format == "nv12":
+            dtype = _lib.SILENT_NV12
+        else:
+            dtype = _lib.SILENT_U8 if frame_dtype == torch.uint8 else _lib.SILENT_F32
         self.params = _lib.SilentParams(h, w, c, int(num_colors), int(center_dimensions[0]), int(center_dimensions[1]),
-                                        float(scale), _lib.SILENT_U8 if frame_dtype == torch.uint8 else _lib.SILENT_F32,
-                                        0)
+                                        float(scale), dtype, 0)
         self.handle = ctypes.c_void_p()
         _lib.check(_lib.lib().silent_plan_create(ctypes.byref(self.params), ctypes.byref(self.handle)),
                    "silent_plan_create")
@@ -23,6 +28,7 @@ class PyramidPlan:
         self.h, self.w = int(center_dimensions[1]), int(center_dimensions[0])
         self.num_colors = int(num_colors)
         self.frame_dtype = frame_dtype
+        self.frame_format = frame_format
 
     def level_info(self, level):
         vals = [ctypes.c_int() for _ in range(6)]
@@ -46,10 +52,13 @@ class PyramidPlan:
         _lib.check(_lib.lib().silent_plan_reserve(self.handle, int(batch)), "silent_plan_reserve")
 
     def build(self, frames):
-        """``frames`` CUDA ``[B, H, W, C]`` of the plan's dtype -> ``[B * L, h, w, num_colors]`` float32."""
+        """``frames`` CUDA ``[B, H, W, C]`` of the plan's dtype (NV12 plans: ``[B, H * 3 / 2, W]`` uint8) ->
+        ``[B * L, h, w, num_colors]`` float32."""
         b = int(frames.shape[0])
         out = torch.empty((b * self.levels, self.h, self.w, self.num_colors), dtype=torch.float32, device=frames.device)
         if self.levels > 0:
+            if self.frame_format == "nv12":
+                self.reserve(b)   # the converted frames live in the plan's workspace
             with torch.cuda.device(frames.device):
                 _lib.check(_lib.lib().silent_pyramid_build(self.handle, _ops.ptr(frames), b, _ops.ptr(out),
                                                            _ops.stream_ptr()), "silent_pyramid_build")
