@@ -86,7 +86,8 @@ __global__ void __launch_bounds__(256) window_max_kernel(const float *__restrict
 }
 
 // One warp per row (level, y). Pass 0 counts hits, pass 1 writes them at row_offset in x order.
-// COUNT pass: one warp per row (level, y); 128-bit loads when the row length allows; writes the row's hit count.
+// COUNT pass: one warp per row (level, y); 128-bit loads when the row length and the tensor's address allow (a contiguous
+// caller tensor may start 4 bytes past a 16-byte boundary); writes the row's hit count.
 __global__ void __launch_bounds__(256) count_rows_kernel(const float *__restrict__ value, int rows, int h, int w, PoolGeom g,
                                                          const float *__restrict__ pooled, int *__restrict__ row_count)
 {
@@ -98,7 +99,7 @@ __global__ void __launch_bounds__(256) count_rows_kernel(const float *__restrict
     const float *v = value + (size_t)row * w;
     const float *pool_row = pooled + ((size_t)n * g.oh + nearest_src(y, g.sy, g.oh)) * g.ow;
     int hits = 0;
-    if ((w & 3) == 0) {
+    if ((w & 3) == 0 && (reinterpret_cast<uintptr_t>(value) & 15) == 0) {
         for (int q = lane; q < (w >> 2); q += 32) {
             const float4 f = __ldg(reinterpret_cast<const float4 *>(v) + q);
             const int x = 4 * q;
