@@ -18,7 +18,7 @@ from .constant_convolutions.center_surround import midget_rgc, rgby_3
 from .constant_convolutions.edge_orientation_detector import rgb_2d_stripe_tensors
 from .constant_convolutions.gaussian_blur.gaussian_blur import blur_tensor
 from .constant_convolutions.oriented_end_detector import rgb_2d_end_tensors
-from .util.zoom.from_image import PyramidPlan
+from .util.zoom.from_image import PyramidPlan, image_to_zoom_tensor
 
 def orientation_bank_filters(n_orient=8):
     """Filters of BASELINE config C4 (SURVEY 8(d)): ``n_orient`` orientations at ``k * 360 / n_orient`` degrees built
@@ -36,6 +36,23 @@ def orientation_bank_filters(n_orient=8):
     return dict(rgc=midget_rgc(2), rgby=rgby_3(2), stripe=np.ascontiguousarray(stripe[:, :, :3, :]),
                 blur=blur_tensor(2, 7, channels_in=n_orient, channels_out=n_orient), end=end)
 
+
+def host_round_trip(staged, device, run, pinned):
+    """``run`` on a copy of the page-locked host tensor ``staged`` on ``device``; returns the tensors it returns as numpy
+    arrays. The upload and every download are asynchronous, result i into the page-locked ``pinned(i, shape, dtype)``,
+    and the stream is synchronised once for all of them."""
+    with torch.cuda.device(device):
+        outs = []
+        for i, t in enumerate(run(staged.to(device, non_blocking=True))):
+            host = pinned(i, tuple(t.shape), t.dtype)
+            host.copy_(t, non_blocking=True)
+            outs.append(host.numpy())
+        torch.cuda.current_stream().synchronize()
+    return outs
+
+
+# routes of frames (LineEndPipeline._frame_route)
+PLAN, CONVERT, PYRAMID = "plan", "convert", "pyramid"
 
 LineEndResult = collections.namedtuple("LineEndResult", "orient padded_line_end gray points")
 LineEndResult.__doc__ = """orient: ``orient_tensor`` [N,h,w,3]; padded_line_end: ``padded_line_end_tensor`` [N,h,w,3];
@@ -109,57 +126,65 @@ class LineEndPipeline:
     def _nv12(self):
         return self.frame_format == "nv12"
 
-    def _nv12_fused(self, nb, w):
-        """Whether NV12 frames of width ``w`` go through an NV12 plan (conversion kernel, then the fused path) rather
-        than ``_ops.nv12_to_bgr`` and the BGR route: the routes a BGR frame of that width takes fused. A bank needs
-        16-byte BGR rows there (``run_frames``), the three-orientation stack computes the same bits either way."""
-        if self.blur_size != 7 or self.output_colors != 3:
-            return False
-        return nb is None or (nb in _lib.FUSED_BANK_WIDTHS and (3 * w) % 16 == 0)
-
-    def _cast(self, res):
-        """A float32 result in ``out_dtype``: orient and padded_line_end rounded once (``.half()``), gray and points kept."""
-        if not self._half():
-            return res
-        return res._replace(orient=res.orient.half(), padded_line_end=res.padded_line_end.half())
-
-    def _region(self):
+    def _points(self, gray):
+        """Feature points of ``gray``: the maxima of the reference's region windows (``recognition_testing.py:40``)."""
         rh, rw = self.region_shape[1], self.region_shape[2]
         if int(rh) != rh or int(rw) != rw:
             raise ValueError("Ambiguous dimension: %s" % ([rh, rw],))
-        return int(rh), int(rw)
+        return _ops.max_value_indices_region(gray, int(rh), int(rw))
 
     # -- graph on a pyramid (LineEndDisplayer.run) --------------------------------------------------------------------
     def run(self, pyramid_tensor, want_points=True):
         """S1-S8 on a pyramid ``[N, h, w, 3]`` (numpy or CUDA tensor). One fused kernel + the emit kernels."""
         if self.orientations is not None:
             return self.run_bank(pyramid_tensor, want_points)
-        if self.blur_size != 7:
-            return self.run_unfused(pyramid_tensor, want_points)
+        return self._run_pyramid(pyramid_tensor, None, want_points)
+
+    def run_unfused(self, pyramid_tensor, want_points=True):
+        """The same graph through the per-operator kernels (any filter structure, any blur size)."""
+        return self._run_operators(pyramid_tensor, self.filters, want_points)
+
+    def run_bank(self, pyramid_tensor, want_points=True):
+        """Config C4: S1-S2 on 3 channels, S3-S7 on an ``orientations``-channel bank (same composition as ``compile()``,
+        ``recognition_testing.py:69-77``), on the route ``_run_pyramid`` gives."""
+        return self._run_pyramid(pyramid_tensor, self._bank_width(), want_points)
+
+    def _run_pyramid(self, pyramid_tensor, nb, want_points):
+        """``run`` and ``run_bank`` with ``nb`` orientations (None: the reference's three). A finite pyramid goes through
+        the fused stack without a bank at blur size 7 (``silent_stack_fused``), and through the fused bank stack with 12
+        or 16 orientations (``silent_stack_bank``; a non-finite one raises ValueError). All else goes operator by
+        operator, banks of 4 and 8 included: their results are pinned to the operators' order, not the fused one."""
+        fused = self.blur_size == 7 if nb is None else nb > 8
+        if not fused:
+            return self._run_operators(pyramid_tensor, self.filters if nb is None else self.bank_filters, want_points)
         x = _ops.as_device_tensor(pyramid_tensor)
         # the fused kernels skip exact-zero weights and shortcut the regulator where the blur is provably >= 1: valid for
         # finite input only (include/silent_b200.h). NaN / Inf / huge values go operator by operator, like the graph.
         if not _ops.fused_input_ok(x):
-            return self.run_unfused(x, want_points)
-        orient, line_end, gray = _ops.stack_fused(x, self.stack_weights(), out_dtype=self.out_dtype)
-        points = None
-        if want_points:
-            rh, rw = self._region()
-            points = _ops.max_value_indices_region(gray, rh, rw)
-        return LineEndResult(orient, line_end, gray, points)
+            if nb is not None:
+                raise ValueError("a pyramid with NaN, Inf or values beyond 1e30 goes operator by operator, which "
+                                 "supports at most 8 orientations (got %d)" % nb)
+            return self._run_operators(x, self.filters, want_points)
+        if nb is None:
+            orient, line_end, gray = _ops.stack_fused(x, self.stack_weights(), out_dtype=self.out_dtype)
+        else:
+            orient, line_end, gray = _ops.stack_bank(x, self.orientation_bank(), out_dtype=self.out_dtype)
+        return LineEndResult(orient, line_end, gray, self._points(gray) if want_points else None)
 
-    def run_unfused(self, pyramid_tensor, want_points=True):
-        """The same graph through the per-operator kernels (any filter structure, any blur size)."""
-        from .filters import rgc_filter, rgby_filter, orientation_filter
-        from .util.selection import pad_inwards, max_value_indices_region
-        from .util.color import get_value_from_color
+    def _run_operators(self, pyramid_tensor, filters, want_points):
+        """The graph of ``compile()`` (``recognition_testing.py:69-77``) one operator kernel at a time, on the HWIO
+        filters ``filters()`` returns (``self.filters`` or ``self.bank_filters``)."""
         x = _ops.as_device_tensor(pyramid_tensor)
-        orient = orientation_filter(rgby_filter(rgc_filter(x)), self.blur_size)
-        line_end = _ops.conv2d(orient, self.simplex_end_stop, post=_lib.POST_RELU_CLIP, clip_max=255.0)
-        padded = pad_inwards(line_end, [[0, 0], [2, 2], [2, 2], [0, 0]])
-        gray = get_value_from_color(padded)
-        points = max_value_indices_region(padded, self.region_shape, gray) if want_points else None
-        return self._cast(LineEndResult(orient, padded, gray, points))
+        f = filters()
+        x = _ops.conv2d(_ops.conv2d(x, f["rgc"], post=_lib.POST_RELU), f["rgby"], post=_lib.POST_RELU)
+        orient = _ops.regulate(_ops.conv2d(x, f["stripe"], post=_lib.POST_RELU), f["blur"], 1.0, .1)
+        line_end = _ops.conv2d(orient, f["end"], post=_lib.POST_RELU_CLIP, clip_max=255.0)
+        padded = _ops.pad_inwards(line_end, 2, 2, 2, 2)
+        gray = _ops.value_from_color(padded)
+        points = self._points(gray) if want_points else None
+        if self._half():   # the float32 result in out_dtype: orient and padded_line_end rounded once, gray and points kept
+            orient, padded = orient.half(), padded.half()
+        return LineEndResult(orient, padded, gray, points)
 
     def bank_filters(self):
         if self._bank is None:
@@ -180,32 +205,6 @@ class LineEndPipeline:
             f = self.bank_filters()
             self._bank_weights = _lib.make_orientation_bank(f["rgc"], f["rgby"], f["stripe"], f["blur"], f["end"])
         return self._bank_weights
-
-    def run_bank(self, pyramid_tensor, want_points=True):
-        """Config C4: S1-S2 on 3 channels, S3-S7 on an ``orientations``-channel bank (same composition as ``compile()``,
-        ``recognition_testing.py:69-77``). Up to 8 orientations through the per-operator kernels; 12 and 16 through the
-        fused bank stack (``silent_stack_bank``), which needs a finite pyramid."""
-        from .util.selection import pad_inwards, max_value_indices_region
-        from .util.color import get_value_from_color
-        from .util.regulator import regulate_tensor
-        nb = self._bank_width()
-        x = _ops.as_device_tensor(pyramid_tensor)
-        region = [1, self.region_shape[1], self.region_shape[2], nb]
-        if nb > 8:
-            if not _ops.fused_input_ok(x):
-                raise ValueError("a pyramid with NaN, Inf or values beyond 1e30 goes operator by operator, which supports "
-                                 "at most 8 orientations (got %d)" % nb)
-            orient, padded, gray = _ops.stack_bank(x, self.orientation_bank(), out_dtype=self.out_dtype)
-            points = max_value_indices_region(padded, region, gray) if want_points else None
-            return LineEndResult(orient, padded, gray, points)
-        f = self.bank_filters()
-        x = _ops.conv2d(_ops.conv2d(x, f["rgc"], post=_lib.POST_RELU), f["rgby"], post=_lib.POST_RELU)
-        orient = regulate_tensor(_ops.conv2d(x, f["stripe"], post=_lib.POST_RELU), f["blur"], 1.0, .1)
-        line_end = _ops.conv2d(orient, f["end"], post=_lib.POST_RELU_CLIP, clip_max=255.0)
-        padded = pad_inwards(line_end, [[0, 0], [2, 2], [2, 2], [0, 0]])
-        gray = get_value_from_color(padded)
-        points = max_value_indices_region(padded, region, gray) if want_points else None
-        return self._cast(LineEndResult(orient, padded, gray, points))
 
     # -- frames resident in HBM ---------------------------------------------------------------------------------------
     def _plan(self, frame_shape, frame_dtype, device, frame_format="bgr"):
@@ -229,6 +228,34 @@ class LineEndPipeline:
             return self._plan((h, w, 3), torch.uint8, frames.device, "nv12")
         return self._plan(frames.shape[1:], frames.dtype, frames.device)
 
+    def _frame_route(self, nb, frame_format, dtype, frame_shape):
+        """How ``run_frames`` and ``run_host`` compute on frames of ``frame_format``, torch ``dtype`` and a shape ending
+        in ``[W, C]`` (NV12: ``[W]``) with ``nb`` orientations (None: the reference's three):
+        - ``PLAN``: a plan of the frames' format and the fused pipeline, ``silent_pipeline_run[_f16]`` (a bank:
+          ``silent_pipeline_run_orientations[_f16]``);
+        - ``CONVERT``: ``_ops.nv12_to_bgr``, then the route of the BGR frames;
+        - ``PYRAMID``: ``image_to_zoom_tensor``, then ``run_bank``.
+
+        BGR frames without a bank take ``PLAN``; with a bank they take it where the fused bank kernels serve them, else
+        ``PYRAMID``. NV12 frames take ``PLAN`` where the BGR frames they convert to would, with blur size 7 and
+        ``output_colors`` 3; else ``CONVERT``. Quirks kept as they are:
+        - ``PYRAMID`` ignores ``out=`` and ``points_capacity``: it returns new tensors, ``gray`` and every point;
+        - on ``PYRAMID`` a bank of 12 or 16 raises ValueError for non-finite frames, and a bank of 4 or 8 runs operator
+          by operator, in the operators' order;
+        - a blur size other than 7 sends a bank to ``PYRAMID``, though a bank's filters blur with 7 taps at any size;
+        - without a bank, a blur size other than 7 raises in ``make_stack_weights`` and ``output_colors`` other than 3
+          in the C argument check, on NV12 frames after ``CONVERT``."""
+        fusable = self.blur_size == 7 and self.output_colors == 3
+        if frame_format == "nv12":   # the BGR frames they convert to are uint8 [.., W, 3]
+            return PLAN if fusable and self._frame_route(nb, "bgr", torch.uint8, (frame_shape[-1], 3)) == PLAN else CONVERT
+        w, c = frame_shape[-2:]
+        # a bank's pyramid is the frame-pair kernel, which reads rows of whole 16-byte words of uint8 frames (the C
+        # condition is pyramid_pair_supported, csrc/pyramid.cu)
+        if nb is None or (nb in _lib.FUSED_BANK_WIDTHS and dtype == torch.uint8 and c >= 3 and fusable
+                          and (w * c) % 16 == 0):
+            return PLAN
+        return PYRAMID
+
     def run_frames(self, frames, want_points=True, points_capacity=None, out=None):
         """frames: CUDA ``[B, H, W, 3]`` uint8/float32 (``frame_format="nv12"``: ``[B, H * 3 / 2, W]`` uint8) ->
         LineEndResult over ``B * L`` levels (pyramid + S1-S8). A single frame may come without its batch axis.
@@ -242,24 +269,20 @@ class LineEndPipeline:
         if out is not None and (out[0].dtype != self.out_dtype or out[1].dtype != self.out_dtype):
             raise ValueError("run_frames(out=...) needs orient and padded_line_end buffers of %s, got %s and %s"
                              % (self.out_dtype, out[0].dtype, out[1].dtype))
-        if self._nv12():
-            h, w = _ops.nv12_frame_hw(frames.shape, frames.dtype)
-            frames = (frames if frames.dim() == 3 else frames.unsqueeze(0)).contiguous()
-            if not self._nv12_fused(nb, w):   # routes without an NV12 plan: convert, then the BGR route
-                return self._run_frames(_ops.nv12_to_bgr(frames), nb, want_points, points_capacity, out)
-            return self._run_frames(frames, nb, want_points, points_capacity, out, (h, w))
-        frames = frames if frames.dim() == 4 else frames.unsqueeze(0)
-        return self._run_frames(frames.contiguous(), nb, want_points, points_capacity, out)
-
-    def _run_frames(self, frames, nb, want_points, points_capacity, out, nv12_hw=None):
-        """run_frames on a contiguous batch: BGR / float ``[B, H, W, C]``, or NV12 ``[B, H * 3 / 2, W]`` of an
-        ``nv12_hw`` = ``(H, W)`` image through an NV12 plan."""
-        if nv12_hw is None and nb is not None and not (
-                nb in _lib.FUSED_BANK_WIDTHS and frames.dtype == torch.uint8 and frames.shape[3] >= 3
-                and self.blur_size == 7 and self.output_colors == 3 and (frames.shape[2] * frames.shape[3]) % 16 == 0):
-            from .util.zoom.from_image import image_to_zoom_tensor   # other frames: pyramid, then run_bank
+        nv12_hw = _ops.nv12_frame_hw(frames.shape, frames.dtype) if self._nv12() else None
+        frames = (frames if frames.dim() == (3 if nv12_hw else 4) else frames.unsqueeze(0)).contiguous()
+        route = self._frame_route(nb, self.frame_format, frames.dtype, frames.shape)
+        if route == CONVERT:
+            frames, nv12_hw = _ops.nv12_to_bgr(frames), None
+            route = self._frame_route(nb, "bgr", frames.dtype, frames.shape)
+        if route == PYRAMID:
             return self.run_bank(image_to_zoom_tensor(frames, self.output_colors, self.output_size, self.zoom_ratio),
                                  want_points)
+        return self._run_plan(frames, nb, want_points, points_capacity, out, nv12_hw)
+
+    def _run_plan(self, frames, nb, want_points, points_capacity, out, nv12_hw):
+        """The ``PLAN`` route on a contiguous batch: BGR / float ``[B, H, W, C]``, or NV12 ``[B, H * 3 / 2, W]`` of an
+        ``nv12_hw`` = ``(H, W)`` image."""
         if nv12_hw is None:
             plan = self._plan(frames.shape[1:], frames.dtype, frames.device)
         else:
@@ -295,15 +318,15 @@ class LineEndPipeline:
             return LineEndResult(orient, line_end, None, None)
         total = int(count.item())
         if total > cap:   # rare (e.g. an all-black level emits every pixel): redo the emit with room for everything
-            return self._run_frames(frames, nb, want_points, total, None, nv12_hw)
+            return self._run_plan(frames, nb, want_points, total, None, nv12_hw)
         return LineEndResult(orient, line_end, None, points[:total])
 
     # -- host buffers on both sides (LineEndDisplayer.callback) -----------------------------------------------------------
     def run_host(self, frames, orient_out=None, line_end_out=None, points_capacity=4096):
         """frames: host numpy ``[B, H, W, 3]`` (``frame_format="nv12"``: ``[B, H * 3 / 2, W]`` uint8; ideally page-locked)
-        -> host numpy results via the C-ABI host call (with ``orientations`` set: through ``run_frames`` and page-locked
-        buffers, results ``[B * L, h, w, orientations]``). With ``out_dtype=torch.float16`` the results are
-        ``np.float16``, and so must be ``orient_out`` / ``line_end_out``."""
+        -> host numpy results via the C-ABI host call (with ``orientations`` set, or off the ``PLAN`` route: through
+        ``run_frames`` and page-locked buffers, results ``[B * L, h, w, orientations]``). With
+        ``out_dtype=torch.float16`` the results are ``np.float16``, and so must be ``orient_out`` / ``line_end_out``."""
         nb = self._bank_width() if self.orientations is not None else None
         if self._half():
             for name, arr in (("orient_out", orient_out), ("line_end_out", line_end_out)):
@@ -317,9 +340,20 @@ class LineEndPipeline:
         if frames.dtype != np.uint8:
             frames = frames.astype(np.float32)
         dev = self._device()
-        if nb is not None or (nv12_hw and not self._nv12_fused(nb, nv12_hw[1])):
-            return self._run_host_bank(frames, dev, orient_out, line_end_out, points_capacity)
         tdtype = torch.uint8 if frames.dtype == np.uint8 else torch.float32
+        if nb is not None or self._frame_route(nb, self.frame_format, tdtype, frames.shape) != PLAN:
+            def run(x):   # through run_frames: the frames in and the results out through new page-locked buffers
+                res = self.run_frames(x, points_capacity=points_capacity)
+                return res.orient, res.padded_line_end, res.points
+            orient, line_end, points = host_round_trip(torch.from_numpy(frames).pin_memory(), dev, run,
+                                                       lambda i, shape, dtype: torch.empty(shape, dtype=dtype).pin_memory())
+            if orient_out is not None:
+                orient_out[...] = orient
+                orient = orient_out
+            if line_end_out is not None:
+                line_end_out[...] = line_end
+                line_end = line_end_out
+            return LineEndResult(orient, line_end, None, points)
         if nv12_hw:
             plan = self._plan(nv12_hw + (3,), tdtype, dev, "nv12")
         else:
@@ -344,28 +378,6 @@ class LineEndPipeline:
             # run_frames does -- feature points are never silently truncated
             return self.run_host(frames, orient_out, line_end_out, points_capacity=int(count.value))
         return LineEndResult(orient_out, line_end_out, None, points[:count.value])
-
-    def _run_host_bank(self, frames, dev, orient_out, line_end_out, points_capacity):
-        """run_host for a bank (and for NV12 frames on a route without an NV12 plan): the frames go up from a page-locked
-        copy, and the results come back with asynchronous copies into page-locked buffers and one synchronisation, as
-        ``LineEndDisplayer.callback`` does."""
-        staged = torch.from_numpy(frames).pin_memory()
-        with torch.cuda.device(dev):
-            res = self.run_frames(staged.to(dev, non_blocking=True), points_capacity=points_capacity)
-            host = []
-            for t in (res.orient, res.padded_line_end, res.points):
-                h = torch.empty(tuple(t.shape), dtype=t.dtype).pin_memory()
-                h.copy_(t, non_blocking=True)
-                host.append(h)
-            torch.cuda.current_stream().synchronize()
-        orient, line_end, points = (h.numpy() for h in host)
-        if orient_out is not None:
-            orient_out[...] = orient
-            orient = orient_out
-        if line_end_out is not None:
-            line_end_out[...] = line_end
-            line_end = line_end_out
-        return LineEndResult(orient, line_end, None, points)
 
     def callback(self, frame, cam_id=None, depth=2):
         """Per-frame entry point with the reference's signature (``recognition_testing.py:136-144``).

@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from . import _lib, _ops
-from .pipeline import LineEndPipeline
+from .pipeline import LineEndPipeline, host_round_trip
 from .util.centroids import get_centroids, _region as region_dims
 from .util.color import get_value_from_color
 from .util.energy.boosting import get_boosting, initialize_boosting
@@ -136,19 +136,7 @@ class LineEndDisplayer(LineEndPipeline):
             raise ValueError("callback_clip takes host frames [T, H, W, 3] with T >= 1, got shape %s" % (z.shape,))
         if self.orientations is not None:
             self._bank_width()
-        z = np.ascontiguousarray(z if z.dtype == np.uint8 else z.astype(np.float32))
-        dev = self._device()
-        self._slot = (self._slot + 1) % self.host_slots
-        staged = self._host_buffer(("clip", self._slot), z.shape, torch.uint8 if z.dtype == np.uint8 else torch.float32)
-        staged.numpy()[...] = z
-        with torch.cuda.device(dev):
-            tensors = self.run_clip(staged.to(dev, non_blocking=True))
-            outs = []
-            for i, t in enumerate(tensors):
-                host = self._host_buffer(("clip_out", self._slot, i), tuple(t.shape), t.dtype)
-                host.copy_(t, non_blocking=True)
-                outs.append(host.numpy())
-            torch.cuda.current_stream().synchronize()
+        outs = self._round_trip("clip", z, self.run_clip)
         L = outs[0].shape[0] // z.shape[0]
         return [[frames[t]] + [[outs[x][t * L + y] for y in range(L)] for x in range(6)] for t in range(z.shape[0])]
 
@@ -160,22 +148,18 @@ class LineEndDisplayer(LineEndPipeline):
         z = np.asarray(frame)
         if self._nv12():
             _ops.nv12_frame_hw(z.shape, z.dtype, ranks=(2,))
+        outs = self._round_trip("frame", z, lambda x: self.run_frames_display(x.unsqueeze(0)))
+        return [frame] + [[outs[x][y] for y in range(len(outs[x]))] for x in range(6)]
+
+    def _round_trip(self, kind, z, run):
+        """``host_round_trip`` of the frames ``z`` through the next slot of the page-locked buffer ring: one
+        synchronisation instead of a pageable upload and six blocking ``.cpu()`` calls."""
         z = np.ascontiguousarray(z if z.dtype == np.uint8 else z.astype(np.float32))
         dev = self._device()
-        self._slot = (self._slot + 1) % self.host_slots
-        # frame in through a page-locked buffer (asynchronous H2D), the six tensors out into page-locked buffers with
-        # asynchronous copies and ONE synchronisation -- instead of a pageable upload and six blocking .cpu() calls
-        staged = self._host_buffer(("frame", self._slot), z.shape, torch.uint8 if z.dtype == np.uint8 else torch.float32)
+        self._slot = slot = (self._slot + 1) % self.host_slots
+        staged = self._host_buffer((kind, slot), z.shape, torch.uint8 if z.dtype == np.uint8 else torch.float32)
         staged.numpy()[...] = z
-        with torch.cuda.device(dev):
-            tensors = self.run_frames_display(staged.to(dev, non_blocking=True).unsqueeze(0))
-            outs = []
-            for i, t in enumerate(tensors):
-                host = self._host_buffer(("out", self._slot, i), tuple(t.shape), t.dtype)
-                host.copy_(t, non_blocking=True)
-                outs.append(host.numpy())
-            torch.cuda.current_stream().synchronize()
-        return [frame] + [[outs[x][y] for y in range(len(outs[x]))] for x in range(6)]
+        return host_round_trip(staged, dev, run, lambda i, shape, dtype: self._host_buffer((kind, slot, i), shape, dtype))
 
     def _host_buffer(self, key, shape, dtype):
         buf = self._pinned.get(key)
