@@ -132,6 +132,12 @@ int silent_plan_level_info(const silent_plan *plan, int level, int *y0, int *y1,
  * output row/column that is defined as 0. */
 int silent_plan_level_tables(const silent_plan *plan, int level, int32_t *idx_y, float *w_y, int32_t *idx_x,
                              float *w_x);
+/* Frame position of every row and column of `level`: frame_y [h], frame_x [w] (either may be NULL). Along each axis the
+ * value is offset + o * (n_in - 1) / (n_out - 1) (scipy.ndimage.zoom's sample position; the factor is 1 when n_out <= 1),
+ * computed in float64 when the plan is created and rounded once to float32; offset is the crop's y0 / x0, n_in its
+ * height / width and n_out the zoomed size. NaN where silent_plan_level_tables marks the row / column as 0 (o >= valid_h /
+ * valid_w, or the position outside [0, n_in - 1]). These are the tables silent_point_records reads. */
+int silent_plan_level_coords(const silent_plan *plan, int level, float *frame_y, float *frame_x);
 /* Algorithmic HBM bytes of one frame through silent_pipeline_run (SURVEY.md 8(d)): union crop read (1.5 bytes per pixel
  * for SILENT_NV12) + two output tensors; feature points excluded. */
 int64_t silent_plan_algorithmic_bytes(const silent_plan *plan);
@@ -367,6 +373,32 @@ int silent_pipeline_run_orientations_f16(silent_plan *plan, const silent_orienta
 int silent_pipeline_run_host_f16(silent_plan *plan, const silent_stack_weights *weights_host, const void *frames_host,
                                  int batch, uint16_t *orient_host, uint16_t *line_end_host, int64_t *points_host,
                                  int64_t capacity, int64_t *count_host, silent_stream stream);
+
+/* ---- feature-point records ---------------------------------------------------------------------------------------------
+ * One record per emitted point, gathered on the device, so that a caller who wants points and what fired there needs
+ * neither the host round trip for the count nor the whole output tensors. Reads the first min(*count_dev, capacity) rows
+ * (level, y, x, 0) of points_dev (as written by silent_pipeline_run* / silent_max_value_indices_region, level =
+ * frame * L + l) and writes, for row i:
+ *   coords_dev [capacity][2]: (frame_y, frame_x) of the point, from silent_plan_level_coords (NaN on an axis whose row /
+ *     column the level defines as 0);
+ *   values_dev [capacity][1 + 2 * channels]: gray, orient[channels], line_end[channels] at (level, y, x), as float32.
+ *     orient_dev / line_end_dev are [batch * L, h, w, channels], float32, or binary16 (uint16_t bits) when half = 1,
+ *     widened exactly; channels is 3 or an orientation bank's width (4, 8, 12, 16). gray_dev is [batch * L, h, w].
+ *   frame_offsets_dev [batch + 1]: int64, the rows of frame b are [frame_offsets[b], frame_offsets[b + 1]) among the
+ *     written rows (frame_offsets[batch] = min(count, capacity)).
+ * Nothing is written past row `capacity`; *count_dev may exceed it (the emit's total), the records then stop at capacity.
+ * gray_dev = NULL reads the plan's own gray: that of the latest silent_pipeline_run* / silent_pipeline_run_host* call on
+ * this plan, valid until the next such call on it, or a silent_plan_reserve that grows it (or silent_plan_destroy), and
+ * ordered by `stream` (pass the stream of that call, or order the two yourself); batch must not exceed the batch
+ * reserved. A row whose (level, y, x) lies outside [batch * L, h, w] gets NaN records. One kernel, launched as a
+ * programmatic dependent launch on `stream`: it may start while the emit drains. Argument checks (all on the host,
+ * before any CUDA call): null pointers (points, coords and values may be NULL when capacity is 0) or capacity < 0 or half
+ * not 0 / 1 or batch <= 0 -> SILENT_E_INVAL; channels not 3, 4, 8, 12, 16 or a plan of 0 levels -> SILENT_E_SHAPE;
+ * gray_dev = NULL with batch above the plan's reserve -> SILENT_E_CAPACITY. */
+int silent_point_records(const silent_plan *plan, int batch, const int64_t *points_dev, const int64_t *count_dev,
+                         int64_t capacity, const void *orient_dev, const void *line_end_dev, int channels, int half,
+                         const float *gray_dev, int64_t *frame_offsets_dev, float *coords_dev, float *values_dev,
+                         silent_stream stream);
 
 #ifdef __cplusplus
 }

@@ -28,7 +28,7 @@ SYMBOLS = (
     "silent_display_sequence_scratch_bytes", "silent_display_sequence", "silent_pack_points",
     "silent_comm_unique_id", "silent_comm_create", "silent_comm_destroy", "silent_comm_check", "silent_gather_points",
     "silent_stack_fused_f16", "silent_stack_bank_f16", "silent_pipeline_run_f16", "silent_pipeline_run_orientations_f16",
-    "silent_pipeline_run_host_f16", "silent_nv12_to_bgr",
+    "silent_pipeline_run_host_f16", "silent_nv12_to_bgr", "silent_plan_level_coords", "silent_point_records",
 )
 
 
@@ -54,6 +54,7 @@ class SilentBankWeights(ctypes.Structure):
 
 BANK_MAX = 16                  # SILENT_BANK_MAX
 FUSED_BANK_WIDTHS = (4, 8, 12, 16)   # orientation counts with fused kernels (silent_pipeline_run_orientations)
+RECORD_CHANNELS = (3,) + FUSED_BANK_WIDTHS   # output channel counts silent_point_records reads
 
 
 class SilentOrientationBank(ctypes.Structure):
@@ -95,6 +96,7 @@ def lib():
         "silent_plan_level_hw": (i, [p, ip, ip]),
         "silent_plan_level_info": (i, [p, i, ip, ip, ip, ip, ip, ip]),
         "silent_plan_level_tables": (i, [p, i, p, p, p, p]),
+        "silent_plan_level_coords": (i, [p, i, p, p]),
         "silent_plan_algorithmic_bytes": (i64, [p]),
         "silent_pyramid_build": (i, [p, p, i, p, p]),
         "silent_conv2d": (i, [p, i, i, i, i, p, i, i, i, f, p, p]),
@@ -118,6 +120,7 @@ def lib():
         "silent_pipeline_run_orientations_f16": (i, [p, ctypes.POINTER(SilentOrientationBank), p, i, p, p, p, i64, p, p]),
         "silent_pipeline_run_host_f16": (i, [p, ctypes.POINTER(SilentStackWeights), p, i, p, p, p, i64, p, p]),
         "silent_nv12_to_bgr": (i, [p, i, i, i, p, p]),
+        "silent_point_records": (i, [p, i, p, p, i64, p, p, i, i, p, p, p, p, p]),
         "silent_get_centroids": (i, [p, i, i, i, i, i, p, p, p, p]),
         "silent_resize_nearest": (i, [p, i, i, i, i, i, i, p, p]),
         "silent_get_boosting": (i, [p, p, i, i, i, f, f, i, p, p, p]),

@@ -350,3 +350,53 @@ def stack_bank(pyramid, bank, want_orient=True, want_line_end=True, want_gray=Tr
     and gray ``[n, h, w, 1]`` float32."""
     return _stack("silent_stack_bank", "the fused orientation bank", pyramid, bank, int(bank.orientations), want_orient,
                   want_line_end, want_gray, out_dtype)
+
+
+def point_records(plan, batch, points, count, orient, line_end, gray=None, frame_offsets=None, frame_yx=None,
+                  values=None):
+    """``silent_point_records``: the records of the first ``min(count, capacity)`` rows of ``points`` ``[capacity, 4]``
+    int64 (``count``: an int64 device scalar, the emit's total). ``orient`` and ``line_end`` are the call's
+    ``[batch * L, h, w, C]`` outputs (float32 or float16, C = 3, 4, 8, 12 or 16); ``gray`` ``[batch * L, h, w, 1]``
+    float32, or None for the plan's own gray of its latest pipeline call. Returns ``(frame_offsets [batch + 1] int64,
+    frame_yx [capacity, 2] float32, values [capacity, 1 + 2C] float32)``, into the given buffers where passed; no host
+    synchronisation. Shapes, dtypes and devices are checked first (ValueError)."""
+    batch = int(batch)
+    if batch <= 0:
+        raise ValueError("point_records needs a positive batch, got %d" % batch)
+    n = batch * plan.levels
+    if orient.dim() != 4 or orient.shape[:3] != (n, plan.h, plan.w) or line_end.shape != orient.shape:
+        raise ValueError("point_records needs orient and line_end of shape [%d, %d, %d, C], got %s and %s"
+                         % (n, plan.h, plan.w, tuple(orient.shape), tuple(line_end.shape)))
+    c = int(orient.shape[3])
+    if c not in _lib.RECORD_CHANNELS:
+        raise ValueError("point_records reads 3, 4, 8, 12 or 16 channels, got %d" % c)
+    if orient.dtype not in OUT_DTYPES or line_end.dtype != orient.dtype:
+        raise ValueError("orient and line_end must both be float32 or both float16, got %s and %s"
+                         % (orient.dtype, line_end.dtype))
+    if points.dim() != 2 or points.shape[1] != 4 or points.dtype != torch.int64:
+        raise ValueError("points must be int64 [capacity, 4], got %s %s" % (points.dtype, tuple(points.shape)))
+    cap = int(points.shape[0])
+    if count.dtype != torch.int64 or count.numel() < 1:
+        raise ValueError("count must be an int64 tensor of at least one element")
+    if gray is not None and (gray.dtype != torch.float32 or tuple(gray.shape) != (n, plan.h, plan.w, 1)):
+        raise ValueError("gray must be float32 [%d, %d, %d, 1], got %s %s" % (n, plan.h, plan.w, gray.dtype,
+                                                                            tuple(gray.shape)))
+    dev = points.device
+    mk = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)  # noqa: E731
+    frame_offsets = mk((batch + 1,), torch.int64) if frame_offsets is None else frame_offsets
+    frame_yx = mk((cap, 2), torch.float32) if frame_yx is None else frame_yx
+    values = mk((cap, 1 + 2 * c), torch.float32) if values is None else values
+    for name, t, dt, shape in (("frame_offsets", frame_offsets, torch.int64, (batch + 1,)),
+                               ("frame_yx", frame_yx, torch.float32, (cap, 2)),
+                               ("values", values, torch.float32, (cap, 1 + 2 * c))):
+        if t.dtype != dt or tuple(t.shape) != shape:
+            raise ValueError("%s must be %s %s, got %s %s" % (name, dt, shape, t.dtype, tuple(t.shape)))
+    tensors = [points, count, orient, line_end, frame_offsets, frame_yx, values] + ([gray] if gray is not None else [])
+    if any(not t.is_cuda or t.device != dev or not t.is_contiguous() for t in tensors):
+        raise ValueError("point_records needs contiguous CUDA tensors on one device")
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().silent_point_records(
+            plan.handle, batch, ptr(points), ptr(count), cap, ptr(orient), ptr(line_end), c,
+            int(orient.dtype == torch.float16), ptr(gray), ptr(frame_offsets), ptr(frame_yx), ptr(values),
+            stream_ptr()), "silent_point_records")
+    return frame_offsets, frame_yx, values

@@ -50,13 +50,15 @@ static double bspline5(double x)
 }
 
 // One axis of scipy's zoom: cc = o * (n_in - 1) / (n_out - 1); taps floor(cc)-2 .. +3, mirror-reflected; cc outside
-// [0, n_in - 1] -> the output sample is cval = 0 (idx[0] = -1 marks it).
-static void axis_table(int n_in, int n_out, int n_keep, int offset, int32_t *idx, float *wts)
+// [0, n_in - 1] -> the output sample is cval = 0 (idx[0] = -1 marks it). coord[o] = the sample's frame position
+// offset + cc, rounded once to float32 (left NaN where the sample is 0).
+static void axis_table(int n_in, int n_out, int n_keep, int offset, int32_t *idx, float *wts, float *coord)
 {
     const double factor = n_out > 1 ? (double)(n_in - 1) / (double)(n_out - 1) : 1.0;
     for (int o = 0; o < n_keep; ++o) {
         const double cc = (double)o * factor;
         if (cc < 0 || cc > n_in - 1) continue;
+        coord[o] = (float)((double)offset + cc);
         const int base = (int)std::floor(cc) - 2;
         for (int t = 0; t < kTaps; ++t) {
             int src = base + t;
@@ -139,6 +141,8 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
     plan->w_y.assign((size_t)L * h * kTaps, 0.0f);
     plan->idx_x.assign((size_t)L * w * kTaps, -1);
     plan->w_x.assign((size_t)L * w * kTaps, 0.0f);
+    plan->coord_y.assign((size_t)L * h, NAN);
+    plan->coord_x.assign((size_t)L * w, NAN);
     plan->union_h = plan->union_w = 0;
     for (int s = 0; s < L; ++s) {
         const double grow = std::pow(p->scale, (double)s);    // scale ** s
@@ -160,9 +164,9 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
         li.valid_w = std::min(w, std::max(out_w, 0));
         if (li.y1 > li.y0 && li.x1 > li.x0) {
             axis_table(li.y1 - li.y0, out_h, li.valid_h, li.y0, &plan->idx_y[(size_t)s * h * kTaps],
-                       &plan->w_y[(size_t)s * h * kTaps]);
+                       &plan->w_y[(size_t)s * h * kTaps], &plan->coord_y[(size_t)s * h]);
             axis_table(li.x1 - li.x0, out_w, li.valid_w, li.x0, &plan->idx_x[(size_t)s * w * kTaps],
-                       &plan->w_x[(size_t)s * w * kTaps]);
+                       &plan->w_x[(size_t)s * w * kTaps], &plan->coord_x[(size_t)s * w]);
         } else {
             li.valid_h = li.valid_w = 0;
         }
@@ -239,7 +243,8 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
             plan->on_device = false;   // geometry-only plan (host queries still work; compute calls fail loudly)
         } else {
             const size_t by = plan->idx_y.size(), bx = plan->idx_x.size();
-            cudaError_t e = cudaMalloc(&plan->d_tables, (by + bx) * (sizeof(int32_t) + sizeof(float)));
+            const size_t cy = plan->coord_y.size(), cx = plan->coord_x.size();
+            cudaError_t e = cudaMalloc(&plan->d_tables, (by + bx) * (sizeof(int32_t) + sizeof(float)) + (cy + cx) * sizeof(float));
             if (e != cudaSuccess) {
                 delete plan;
                 return fail(SILENT_E_CUDA, "cudaMalloc(tap tables) failed: %s", cudaGetErrorString(e));
@@ -249,10 +254,14 @@ int silent_plan_create(const silent_params *p, silent_plan **out_plan)
             plan->d_idx_x = plan->d_idx_y + by;
             plan->d_w_y = (float *)(plan->d_idx_x + bx);
             plan->d_w_x = plan->d_w_y + by;
+            plan->d_coord_y = plan->d_w_x + bx;
+            plan->d_coord_x = plan->d_coord_y + cy;
             e = cudaMemcpy(plan->d_idx_y, plan->idx_y.data(), by * 4, cudaMemcpyHostToDevice);
             if (e == cudaSuccess) e = cudaMemcpy(plan->d_idx_x, plan->idx_x.data(), bx * 4, cudaMemcpyHostToDevice);
             if (e == cudaSuccess) e = cudaMemcpy(plan->d_w_y, plan->w_y.data(), by * 4, cudaMemcpyHostToDevice);
             if (e == cudaSuccess) e = cudaMemcpy(plan->d_w_x, plan->w_x.data(), bx * 4, cudaMemcpyHostToDevice);
+            if (e == cudaSuccess) e = cudaMemcpy(plan->d_coord_y, plan->coord_y.data(), cy * 4, cudaMemcpyHostToDevice);
+            if (e == cudaSuccess) e = cudaMemcpy(plan->d_coord_x, plan->coord_x.data(), cx * 4, cudaMemcpyHostToDevice);
             if (e != cudaSuccess) {
                 delete plan;
                 return fail(SILENT_E_CUDA, "upload of tap tables failed: %s", cudaGetErrorString(e));
@@ -395,6 +404,15 @@ int silent_plan_level_tables(const silent_plan *plan, int level, int32_t *idx_y,
     if (w_y) std::memcpy(w_y, &plan->w_y[level * ny], ny * 4);
     if (idx_x) std::memcpy(idx_x, &plan->idx_x[level * nx], nx * 4);
     if (w_x) std::memcpy(w_x, &plan->w_x[level * nx], nx * 4);
+    return SILENT_OK;
+}
+
+int silent_plan_level_coords(const silent_plan *plan, int level, float *frame_y, float *frame_x)
+{
+    if (!plan) return fail(SILENT_E_INVAL, "null plan");
+    if (level < 0 || level >= plan->levels) return fail(SILENT_E_INVAL, "level %d out of range [0,%d)", level, plan->levels);
+    if (frame_y) std::memcpy(frame_y, &plan->coord_y[(size_t)level * plan->h], (size_t)plan->h * sizeof(float));
+    if (frame_x) std::memcpy(frame_x, &plan->coord_x[(size_t)level * plan->w], (size_t)plan->w * sizeof(float));
     return SILENT_OK;
 }
 

@@ -69,6 +69,9 @@ struct silent_plan {
     std::vector<silent::LevelInfo> info;
     std::vector<int32_t> idx_y, idx_x;   // [L][h|w][6], absolute frame row / column, idx[.][0] = -1 => sample is 0
     std::vector<float> w_y, w_x;
+    // [L][h|w]: frame row / column of each level row / column, float32(offset + o * (n_in - 1) / (n_out - 1)) from the
+    // float64 of axis_table; NaN where idx[.][0] < 0 (the sample is defined as 0). Read by point_records_kernel
+    std::vector<float> coord_y, coord_x;
     std::vector<silent::PairLevel> pair;   // per level
     bool pair_ok = false;
     int pair_tile_w = 64;                  // output columns per tile of the frame-pair pyramid kernel (see plan.cu)
@@ -89,6 +92,7 @@ struct silent_plan {
     void *d_tables = nullptr;
     int32_t *d_idx_y = nullptr, *d_idx_x = nullptr;
     float *d_w_y = nullptr, *d_w_x = nullptr;
+    float *d_coord_y = nullptr, *d_coord_x = nullptr;   // coord_y / coord_x, in the d_tables allocation
     silent::Workspace ws;
     bool timing = false;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};   // before pyramid / stack / emit, after emit

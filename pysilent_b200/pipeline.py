@@ -18,7 +18,7 @@ from .constant_convolutions.center_surround import midget_rgc, rgby_3
 from .constant_convolutions.edge_orientation_detector import rgb_2d_stripe_tensors
 from .constant_convolutions.gaussian_blur.gaussian_blur import blur_tensor
 from .constant_convolutions.oriented_end_detector import rgb_2d_end_tensors
-from .util.zoom.from_image import PyramidPlan, image_to_zoom_tensor
+from .util.zoom.from_image import PyramidPlan, image_to_zoom_tensor, zoom_frames_and_plan
 
 def orientation_bank_filters(n_orient=8):
     """Filters of BASELINE config C4 (SURVEY 8(d)): ``n_orient`` orientations at ``k * 360 / n_orient`` degrees built
@@ -57,6 +57,14 @@ PLAN, CONVERT, PYRAMID = "plan", "convert", "pyramid"
 LineEndResult = collections.namedtuple("LineEndResult", "orient padded_line_end gray points")
 LineEndResult.__doc__ = """orient: ``orient_tensor`` [N,h,w,3]; padded_line_end: ``padded_line_end_tensor`` [N,h,w,3];
 gray: ``gray_line_end_tensor`` [N,h,w,1] (or None); points: int64 [K,4] rows (level, y, x, 0) (``top_percent_points``)."""
+
+PointRecords = collections.namedtuple("PointRecords", "points frame_offsets frame_yx gray orient line_end")
+PointRecords.__doc__ = """The feature points of a batch of B frames with what fired at each (``silent_point_records``):
+points: int64 [K,4] rows (level, y, x, 0) as ``LineEndResult.points``, level = frame * L + l; frame_offsets: int64
+[B+1], the rows of frame b are ``points[frame_offsets[b]:frame_offsets[b + 1]]``; frame_yx: float32 [K,2], the
+point's (row, column) in its frame, ``y0 + y * (n_in - 1) / (n_out - 1)`` per axis (``PyramidPlan.level_coords``; NaN
+on an axis the level defines as 0); gray: float32 [K], orient and line_end: float32 [K,C], the values of ``gray``,
+``orient`` and ``padded_line_end`` at the point (float16 outputs widened exactly)."""
 
 
 class LineEndPipeline:
@@ -280,13 +288,16 @@ class LineEndPipeline:
                                  want_points)
         return self._run_plan(frames, nb, want_points, points_capacity, out, nv12_hw)
 
+    def _plan_of(self, frames, nv12_hw):
+        """The plan of a contiguous batch on the ``PLAN`` route (see ``_run_plan``)."""
+        if nv12_hw is None:
+            return self._plan(frames.shape[1:], frames.dtype, frames.device)
+        return self._plan(nv12_hw + (3,), torch.uint8, frames.device, "nv12")
+
     def _run_plan(self, frames, nb, want_points, points_capacity, out, nv12_hw):
         """The ``PLAN`` route on a contiguous batch: BGR / float ``[B, H, W, C]``, or NV12 ``[B, H * 3 / 2, W]`` of an
         ``nv12_hw`` = ``(H, W)`` image."""
-        if nv12_hw is None:
-            plan = self._plan(frames.shape[1:], frames.dtype, frames.device)
-        else:
-            plan = self._plan(nv12_hw + (3,), torch.uint8, frames.device, "nv12")
+        plan = self._plan_of(frames, nv12_hw)
         b = int(frames.shape[0])
         plan.reserve(b)
         n = b * plan.levels
@@ -320,6 +331,103 @@ class LineEndPipeline:
         if total > cap:   # rare (e.g. an all-black level emits every pixel): redo the emit with room for everything
             return self._run_plan(frames, nb, want_points, total, None, nv12_hw)
         return LineEndResult(orient, line_end, None, points[:total])
+
+    # -- feature-point records ------------------------------------------------------------------------------------------
+    def run_frames_records(self, frames, points_capacity=None, out=None):
+        """``run_frames`` on the same frames and route, returning the feature points with their frame coordinates and
+        the responses at each (``PointRecords`` of CUDA tensors) instead of the whole output tensors.
+
+        ``out`` may carry preallocated ``(orient, padded_line_end, points, count, frame_offsets, frame_yx, values)``
+        buffers: the first four as for ``run_frames(out=...)``, then int64 ``[B + 1]``, float32 ``[capacity, 2]`` and
+        float32 ``[capacity, 1 + 2 * C]`` (C = 3 or ``orientations``). No host synchronisation is performed then, and
+        the result's tensors are views of those buffers over the whole capacity: the first ``min(count, capacity)`` rows
+        are written and ``frame_offsets`` counts only those. Without ``out`` the call synchronises once to trim to the
+        points found, and redoes the call with room for all of them when they exceed ``points_capacity``.
+
+        The records are those of every route ``run_frames`` takes; like there, the ``PYRAMID`` route ignores ``out`` and
+        ``points_capacity`` and returns every point in new tensors. Banks of widths other than 4, 8, 12 and 16 raise
+        ValueError."""
+        return self._records(*self._record_rows(frames, points_capacity, out))
+
+    def _record_rows(self, frames, points_capacity, out):
+        """``run_frames_records`` as ``(points, frame_offsets, frame_yx, values [K, 1 + 2C])``."""
+        nb = self._bank_width() if self.orientations is not None else None
+        c = nb or 3
+        if c not in _lib.RECORD_CHANNELS:
+            raise ValueError("feature-point records need 3 orientations or a bank of 4, 8, 12 or 16, got %d" % c)
+        if points_capacity is not None and int(points_capacity) < 0:
+            raise ValueError("points_capacity must be >= 0, got %d" % int(points_capacity))
+        if out is not None:
+            if len(out) != 7:
+                raise ValueError("run_frames_records(out=...) takes (orient, padded_line_end, points, count, "
+                                 "frame_offsets, frame_yx, values), got %d buffers" % len(out))
+            if out[0].dtype != self.out_dtype or out[1].dtype != self.out_dtype:
+                raise ValueError("run_frames_records(out=...) needs orient and padded_line_end buffers of %s, got %s "
+                                 "and %s" % (self.out_dtype, out[0].dtype, out[1].dtype))
+        nv12_hw = _ops.nv12_frame_hw(frames.shape, frames.dtype) if self._nv12() else None
+        frames = (frames if frames.dim() == (3 if nv12_hw else 4) else frames.unsqueeze(0)).contiguous()
+        route = self._frame_route(nb, self.frame_format, frames.dtype, frames.shape)
+        if route == CONVERT:
+            frames, nv12_hw = _ops.nv12_to_bgr(frames), None
+            route = self._frame_route(nb, "bgr", frames.dtype, frames.shape)
+        if route == PYRAMID:
+            zframes, zplan = zoom_frames_and_plan(frames, self.output_colors, self.output_size, self.zoom_ratio)
+            res = self.run_bank(zplan.build(zframes), True)
+            count = torch.full((1,), len(res.points), dtype=torch.int64, device=res.points.device)
+            recs = _ops.point_records(zplan, zframes.shape[0], res.points, count, res.orient, res.padded_line_end,
+                                      res.gray)
+            return (res.points,) + recs
+        return self._run_plan_records(frames, nb, points_capacity, out, nv12_hw)
+
+    def _run_plan_records(self, frames, nb, points_capacity, out, nv12_hw):
+        plan = self._plan_of(frames, nv12_hw)
+        b = int(frames.shape[0])
+        if out is None:
+            dev = frames.device
+            cap = int(points_capacity) if points_capacity is not None else max(64 * b * plan.levels, 1024)
+            orient = torch.empty((b * plan.levels, plan.h, plan.w, nb or 3), dtype=self.out_dtype, device=dev)
+            run_out = (orient, torch.empty_like(orient), torch.empty((cap, 4), dtype=torch.int64, device=dev),
+                       torch.zeros(1, dtype=torch.int64, device=dev))
+            bufs = (None, None, None)
+        else:
+            run_out, bufs = tuple(out[:4]), tuple(out[4:])
+        orient, line_end, points, count = run_out
+        self._run_plan(frames, nb, True, None, run_out, nv12_hw)
+        # gray: the plan's own, written by the call above on this stream
+        recs = _ops.point_records(plan, b, points, count, orient, line_end, None, *bufs)
+        if out is not None:
+            return (points,) + recs
+        total = int(count.item())
+        if total > points.shape[0]:   # as run_frames: redo with room for every point
+            return self._run_plan_records(frames, nb, total, None, nv12_hw)
+        frame_offsets, frame_yx, values = recs
+        return points[:total], frame_offsets, frame_yx[:total], values[:total]
+
+    @staticmethod
+    def _records(points, frame_offsets, frame_yx, values):
+        """``PointRecords`` of the rows ``_record_rows`` returns (gray, orient and line_end are views of ``values``)."""
+        c = (values.shape[1] - 1) // 2
+        return PointRecords(points, frame_offsets, frame_yx, values[:, 0], values[:, 1:1 + c], values[:, 1 + c:])
+
+    def run_host_records(self, frames, points_capacity=4096):
+        """``run_frames_records`` on host frames: numpy ``[B, H, W, 3]`` (``frame_format="nv12"``: ``[B, H * 3 / 2, W]``
+        uint8), pageable or page-locked. The frames go up once and only the records come back (``PointRecords`` of
+        numpy arrays): ``orient`` and ``padded_line_end`` never cross the host link. ``points_capacity`` sizes the first
+        attempt; every point is returned."""
+        frames = np.asarray(frames)
+        nv12_hw = _ops.nv12_frame_hw(frames.shape, frames.dtype) if self._nv12() else None
+        frames = np.ascontiguousarray(frames)
+        if frames.ndim == (2 if nv12_hw else 3):
+            frames = frames[np.newaxis]
+        if frames.dtype != np.uint8:
+            frames = frames.astype(np.float32)
+        dev = self._device()
+        staged = torch.from_numpy(frames)
+        if not staged.is_pinned():   # page-locked frames (e.g. views of pinned tensors) go up in place
+            staged = staged.pin_memory()
+        rows = host_round_trip(staged, dev, lambda x: self._record_rows(x, points_capacity, None),
+                               lambda i, shape, dtype: torch.empty(shape, dtype=dtype, pin_memory=True))
+        return self._records(*rows)
 
     # -- host buffers on both sides (LineEndDisplayer.callback) -----------------------------------------------------------
     def run_host(self, frames, orient_out=None, line_end_out=None, points_capacity=4096):

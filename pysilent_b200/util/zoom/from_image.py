@@ -44,6 +44,14 @@ class PyramidPlan:
                                                        ix.ctypes.data, wx.ctypes.data))
         return iy, wy, ix, wx
 
+    def level_coords(self, level):
+        """``(frame_y [h], frame_x [w])`` float32: the frame position of every row and column of ``level``, NaN where
+        the level defines the row or column as 0 (``silent_plan_level_coords``)."""
+        fy = np.empty(self.h, np.float32)
+        fx = np.empty(self.w, np.float32)
+        _lib.check(_lib.lib().silent_plan_level_coords(self.handle, level, fy.ctypes.data, fx.ctypes.data))
+        return fy, fx
+
     @property
     def algorithmic_bytes(self):
         return int(_lib.lib().silent_plan_algorithmic_bytes(self.handle))
@@ -104,6 +112,13 @@ def image_to_zoom_tensor(image, num_colors, center_dimensions, scale):
     :return: CUDA float32 ``[L, h, w, num_colors]`` (``[B * L, ...]`` for a batch). Rows/columns the reference leaves
         uninitialised (``np.empty``) are 0.
     """
+    frames, plan = zoom_frames_and_plan(image, num_colors, center_dimensions, scale)
+    return plan.build(frames)
+
+
+def zoom_frames_and_plan(image, num_colors, center_dimensions, scale):
+    """The batch ``[B, H, W, C]`` (CUDA, uint8 or float32) that ``image_to_zoom_tensor`` builds its pyramid from, and
+    the cached ``PyramidPlan`` it builds it with (whose geometry places each level's pixels in the frame)."""
     assert scale > 1, "Scale must be greater than one."
     assert num_colors > 0, "Number of colors must be greater than zero."
     for d in center_dimensions:
@@ -123,4 +138,4 @@ def image_to_zoom_tensor(image, num_colors, center_dimensions, scale):
     plan = get_plan(frames.shape[1:], frames.dtype, num_colors, center_dimensions, scale, frames.device)
     if plan.levels < 0:
         raise ValueError("negative dimensions are not allowed")
-    return plan.build(frames)
+    return frames, plan
