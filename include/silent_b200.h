@@ -400,6 +400,22 @@ int silent_point_records(const silent_plan *plan, int batch, const int64_t *poin
                          const float *gray_dev, int64_t *frame_offsets_dev, float *coords_dev, float *values_dev,
                          silent_stream stream);
 
+/* ---- feature-point patches ---------------------------------------------------------------------------------------------
+ * silent_point_records with the square neighbourhood of side P = 2 * radius + 1 around each point instead of its one
+ * pixel, for descriptors, sub-pixel refinement or orientation histograms built from the raw responses. Everything is as
+ * for silent_point_records (the rows read, coords_dev, frame_offsets_dev, gray_dev = NULL, the capacity and the launch)
+ * except values_dev, which is [capacity][P][P][1 + 2 * channels] float32: pixel (y + dy, x + dx) of the point's level,
+ * dy, dx in [-radius, radius], at [radius + dy][radius + dx], holding gray, orient[channels], line_end[channels] there.
+ * A patch pixel outside the level's [0, h) x [0, w) is +0.0 in every value (what the stack's SAME zero padding reads
+ * there); a row outside [batch * L, h, w] gets NaN in its whole patch. radius = 0 is silent_point_records, bit for bit.
+ * Argument checks (all on the host, before any CUDA call): those of silent_point_records, and radius < 0 or radius >
+ * SILENT_PATCH_RADIUS_MAX -> SILENT_E_SHAPE. */
+#define SILENT_PATCH_RADIUS_MAX 31
+int silent_point_patches(const silent_plan *plan, int batch, const int64_t *points_dev, const int64_t *count_dev,
+                         int64_t capacity, const void *orient_dev, const void *line_end_dev, int channels, int half,
+                         const float *gray_dev, int radius, int64_t *frame_offsets_dev, float *coords_dev,
+                         float *values_dev, silent_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -29,6 +29,7 @@ SYMBOLS = (
     "silent_comm_unique_id", "silent_comm_create", "silent_comm_destroy", "silent_comm_check", "silent_gather_points",
     "silent_stack_fused_f16", "silent_stack_bank_f16", "silent_pipeline_run_f16", "silent_pipeline_run_orientations_f16",
     "silent_pipeline_run_host_f16", "silent_nv12_to_bgr", "silent_plan_level_coords", "silent_point_records",
+    "silent_point_patches",
 )
 
 
@@ -55,6 +56,7 @@ class SilentBankWeights(ctypes.Structure):
 BANK_MAX = 16                  # SILENT_BANK_MAX
 FUSED_BANK_WIDTHS = (4, 8, 12, 16)   # orientation counts with fused kernels (silent_pipeline_run_orientations)
 RECORD_CHANNELS = (3,) + FUSED_BANK_WIDTHS   # output channel counts silent_point_records reads
+PATCH_RADIUS_MAX = 31          # SILENT_PATCH_RADIUS_MAX: largest radius silent_point_patches takes
 
 
 class SilentOrientationBank(ctypes.Structure):
@@ -121,6 +123,7 @@ def lib():
         "silent_pipeline_run_host_f16": (i, [p, ctypes.POINTER(SilentStackWeights), p, i, p, p, p, i64, p, p]),
         "silent_nv12_to_bgr": (i, [p, i, i, i, p, p]),
         "silent_point_records": (i, [p, i, p, p, i64, p, p, i, i, p, p, p, p, p]),
+        "silent_point_patches": (i, [p, i, p, p, i64, p, p, i, i, p, i, p, p, p, p]),
         "silent_get_centroids": (i, [p, i, i, i, i, i, p, p, p, p]),
         "silent_resize_nearest": (i, [p, i, i, i, i, i, i, p, p]),
         "silent_get_boosting": (i, [p, p, i, i, i, f, f, i, p, p, p]),

@@ -352,14 +352,48 @@ def stack_bank(pyramid, bank, want_orient=True, want_line_end=True, want_gray=Tr
                   want_line_end, want_gray, out_dtype)
 
 
+def patch_radius(radius):
+    """``radius`` as an int in ``[0, PATCH_RADIUS_MAX]``, or None for None; anything else (a bool, a float, a value out
+    of range) raises ValueError."""
+    if radius is None:
+        return None
+    if isinstance(radius, bool) or not isinstance(radius, (int, np.integer)):
+        raise ValueError("patch radius must be an int, got %r" % (radius,))
+    if not 0 <= radius <= _lib.PATCH_RADIUS_MAX:
+        raise ValueError("patch radius must be in [0, %d], got %d" % (_lib.PATCH_RADIUS_MAX, radius))
+    return int(radius)
+
+
+def record_values_shape(capacity, channels, radius=None):
+    """Shape of the float32 ``values`` of ``capacity`` records of ``channels`` channels: ``[capacity, 1 + 2C]``, or
+    ``[capacity, P, P, 1 + 2C]`` with a patch of radius ``radius`` (P = 2 * radius + 1)."""
+    v = 1 + 2 * channels
+    return (capacity, v) if radius is None else (capacity, 2 * radius + 1, 2 * radius + 1, v)
+
+
+def check_record_buffers(batch, capacity, channels, radius, frame_offsets, frame_yx, values):
+    """ValueError unless ``frame_offsets``, ``frame_yx`` and ``values`` are the int64 / float32 / float32 tensors that
+    ``capacity`` records of ``batch`` frames with ``channels`` channels (and a patch of ``radius``) fill."""
+    for name, t, dt, shape in (("frame_offsets", frame_offsets, torch.int64, (batch + 1,)),
+                               ("frame_yx", frame_yx, torch.float32, (capacity, 2)),
+                               ("values", values, torch.float32, record_values_shape(capacity, channels, radius))):
+        if not isinstance(t, torch.Tensor):
+            raise ValueError("%s must be %s %s, got %s" % (name, dt, shape, type(t).__name__))
+        if t.dtype != dt or tuple(t.shape) != shape:
+            raise ValueError("%s must be %s %s, got %s %s" % (name, dt, shape, t.dtype, tuple(t.shape)))
+
+
 def point_records(plan, batch, points, count, orient, line_end, gray=None, frame_offsets=None, frame_yx=None,
-                  values=None):
+                  values=None, radius=None):
     """``silent_point_records``: the records of the first ``min(count, capacity)`` rows of ``points`` ``[capacity, 4]``
     int64 (``count``: an int64 device scalar, the emit's total). ``orient`` and ``line_end`` are the call's
     ``[batch * L, h, w, C]`` outputs (float32 or float16, C = 3, 4, 8, 12 or 16); ``gray`` ``[batch * L, h, w, 1]``
     float32, or None for the plan's own gray of its latest pipeline call. Returns ``(frame_offsets [batch + 1] int64,
     frame_yx [capacity, 2] float32, values [capacity, 1 + 2C] float32)``, into the given buffers where passed; no host
-    synchronisation. Shapes, dtypes and devices are checked first (ValueError)."""
+    synchronisation. With an int ``radius`` (``silent_point_patches``) ``values`` is ``[capacity, P, P, 1 + 2C]``, the
+    patch of side P = 2 * radius + 1 around each point, +0.0 outside the level. Shapes, dtypes, devices and the radius
+    are checked first (ValueError)."""
+    radius = patch_radius(radius)
     batch = int(batch)
     if batch <= 0:
         raise ValueError("point_records needs a positive batch, got %d" % batch)
@@ -385,18 +419,19 @@ def point_records(plan, batch, points, count, orient, line_end, gray=None, frame
     mk = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)  # noqa: E731
     frame_offsets = mk((batch + 1,), torch.int64) if frame_offsets is None else frame_offsets
     frame_yx = mk((cap, 2), torch.float32) if frame_yx is None else frame_yx
-    values = mk((cap, 1 + 2 * c), torch.float32) if values is None else values
-    for name, t, dt, shape in (("frame_offsets", frame_offsets, torch.int64, (batch + 1,)),
-                               ("frame_yx", frame_yx, torch.float32, (cap, 2)),
-                               ("values", values, torch.float32, (cap, 1 + 2 * c))):
-        if t.dtype != dt or tuple(t.shape) != shape:
-            raise ValueError("%s must be %s %s, got %s %s" % (name, dt, shape, t.dtype, tuple(t.shape)))
+    values = mk(record_values_shape(cap, c, radius), torch.float32) if values is None else values
+    check_record_buffers(batch, cap, c, radius, frame_offsets, frame_yx, values)
     tensors = [points, count, orient, line_end, frame_offsets, frame_yx, values] + ([gray] if gray is not None else [])
     if any(not t.is_cuda or t.device != dev or not t.is_contiguous() for t in tensors):
         raise ValueError("point_records needs contiguous CUDA tensors on one device")
+    half = int(orient.dtype == torch.float16)
     with torch.cuda.device(dev):
-        _lib.check(_lib.lib().silent_point_records(
-            plan.handle, batch, ptr(points), ptr(count), cap, ptr(orient), ptr(line_end), c,
-            int(orient.dtype == torch.float16), ptr(gray), ptr(frame_offsets), ptr(frame_yx), ptr(values),
-            stream_ptr()), "silent_point_records")
+        if radius is None:
+            _lib.check(_lib.lib().silent_point_records(
+                plan.handle, batch, ptr(points), ptr(count), cap, ptr(orient), ptr(line_end), c, half, ptr(gray),
+                ptr(frame_offsets), ptr(frame_yx), ptr(values), stream_ptr()), "silent_point_records")
+        else:
+            _lib.check(_lib.lib().silent_point_patches(
+                plan.handle, batch, ptr(points), ptr(count), cap, ptr(orient), ptr(line_end), c, half, ptr(gray),
+                radius, ptr(frame_offsets), ptr(frame_yx), ptr(values), stream_ptr()), "silent_point_patches")
     return frame_offsets, frame_yx, values

@@ -64,7 +64,13 @@ points: int64 [K,4] rows (level, y, x, 0) as ``LineEndResult.points``, level = f
 [B+1], the rows of frame b are ``points[frame_offsets[b]:frame_offsets[b + 1]]``; frame_yx: float32 [K,2], the
 point's (row, column) in its frame, ``y0 + y * (n_in - 1) / (n_out - 1)`` per axis (``PyramidPlan.level_coords``; NaN
 on an axis the level defines as 0); gray: float32 [K], orient and line_end: float32 [K,C], the values of ``gray``,
-``orient`` and ``padded_line_end`` at the point (float16 outputs widened exactly)."""
+``orient`` and ``padded_line_end`` at the point (float16 outputs widened exactly).
+
+With a patch radius r (``patch_radius=r`` of ``run_frames_records`` / ``run_host_records``, ``silent_point_patches``)
+gray is float32 [K,P,P], orient and line_end float32 [K,P,P,C], P = 2r + 1: the values at pixel (y + dy, x + dx) of the
+point's level, dy and dx in [-r, r], at [r + dy, r + dx]; +0.0 where that pixel leaves the level (what the stack's
+SAME zero padding reads there). points, frame_offsets and frame_yx stay one per point. gray, orient and line_end are
+views of one float32 values tensor [K,1 + 2C] ([K,P,P,1 + 2C] with a patch)."""
 
 
 class LineEndPipeline:
@@ -333,7 +339,7 @@ class LineEndPipeline:
         return LineEndResult(orient, line_end, None, points[:total])
 
     # -- feature-point records ------------------------------------------------------------------------------------------
-    def run_frames_records(self, frames, points_capacity=None, out=None):
+    def run_frames_records(self, frames, points_capacity=None, out=None, patch_radius=None):
         """``run_frames`` on the same frames and route, returning the feature points with their frame coordinates and
         the responses at each (``PointRecords`` of CUDA tensors) instead of the whole output tensors.
 
@@ -344,13 +350,18 @@ class LineEndPipeline:
         are written and ``frame_offsets`` counts only those. Without ``out`` the call synchronises once to trim to the
         points found, and redoes the call with room for all of them when they exceed ``points_capacity``.
 
-        The records are those of every route ``run_frames`` takes; like there, the ``PYRAMID`` route ignores ``out`` and
-        ``points_capacity`` and returns every point in new tensors. Banks of widths other than 4, 8, 12 and 16 raise
-        ValueError."""
-        return self._records(*self._record_rows(frames, points_capacity, out))
+        With an int ``patch_radius`` r in [0, 31] each record carries the patch of side P = 2r + 1 around its point
+        (see ``PointRecords``); ``out``'s ``values`` is then float32 ``[capacity, P, P, 1 + 2 * C]``. Without ``out``
+        the call synchronises once on the count first and sizes the patches by the points found, not by the capacity.
 
-    def _record_rows(self, frames, points_capacity, out):
-        """``run_frames_records`` as ``(points, frame_offsets, frame_yx, values [K, 1 + 2C])``."""
+        The records are those of every route ``run_frames`` takes; like there, the ``PYRAMID`` route ignores ``out`` and
+        ``points_capacity`` and returns every point in new tensors. Banks of widths other than 4, 8, 12 and 16, and a
+        ``patch_radius`` that is not an int in [0, 31], raise ValueError."""
+        return self._records(*self._record_rows(frames, points_capacity, out, patch_radius))
+
+    def _record_rows(self, frames, points_capacity, out, radius=None):
+        """``run_frames_records`` as ``(points, frame_offsets, frame_yx, values [K, 1 + 2C] or [K, P, P, 1 + 2C])``."""
+        radius = _ops.patch_radius(radius)
         nb = self._bank_width() if self.orientations is not None else None
         c = nb or 3
         if c not in _lib.RECORD_CHANNELS:
@@ -366,6 +377,8 @@ class LineEndPipeline:
                                  "and %s" % (self.out_dtype, out[0].dtype, out[1].dtype))
         nv12_hw = _ops.nv12_frame_hw(frames.shape, frames.dtype) if self._nv12() else None
         frames = (frames if frames.dim() == (3 if nv12_hw else 4) else frames.unsqueeze(0)).contiguous()
+        if out is not None and radius is not None:
+            _ops.check_record_buffers(int(frames.shape[0]), int(out[2].shape[0]), c, radius, *out[4:])
         route = self._frame_route(nb, self.frame_format, frames.dtype, frames.shape)
         if route == CONVERT:
             frames, nv12_hw = _ops.nv12_to_bgr(frames), None
@@ -375,11 +388,11 @@ class LineEndPipeline:
             res = self.run_bank(zplan.build(zframes), True)
             count = torch.full((1,), len(res.points), dtype=torch.int64, device=res.points.device)
             recs = _ops.point_records(zplan, zframes.shape[0], res.points, count, res.orient, res.padded_line_end,
-                                      res.gray)
+                                      res.gray, radius=radius)
             return (res.points,) + recs
-        return self._run_plan_records(frames, nb, points_capacity, out, nv12_hw)
+        return self._run_plan_records(frames, nb, points_capacity, out, nv12_hw, radius)
 
-    def _run_plan_records(self, frames, nb, points_capacity, out, nv12_hw):
+    def _run_plan_records(self, frames, nb, points_capacity, out, nv12_hw, radius=None):
         plan = self._plan_of(frames, nv12_hw)
         b = int(frames.shape[0])
         if out is None:
@@ -394,7 +407,14 @@ class LineEndPipeline:
         orient, line_end, points, count = run_out
         self._run_plan(frames, nb, True, None, run_out, nv12_hw)
         # gray: the plan's own, written by the call above on this stream
-        recs = _ops.point_records(plan, b, points, count, orient, line_end, None, *bufs)
+        if out is None and radius is not None:
+            # patches for the whole default capacity could take GBs: size them by the points found
+            total = int(count.item())
+            if total > points.shape[0]:
+                return self._run_plan_records(frames, nb, total, None, nv12_hw, radius)
+            points = points[:total]
+            return (points,) + _ops.point_records(plan, b, points, count, orient, line_end, None, radius=radius)
+        recs = _ops.point_records(plan, b, points, count, orient, line_end, None, *bufs, radius=radius)
         if out is not None:
             return (points,) + recs
         total = int(count.item())
@@ -406,14 +426,15 @@ class LineEndPipeline:
     @staticmethod
     def _records(points, frame_offsets, frame_yx, values):
         """``PointRecords`` of the rows ``_record_rows`` returns (gray, orient and line_end are views of ``values``)."""
-        c = (values.shape[1] - 1) // 2
-        return PointRecords(points, frame_offsets, frame_yx, values[:, 0], values[:, 1:1 + c], values[:, 1 + c:])
+        c = (values.shape[-1] - 1) // 2
+        return PointRecords(points, frame_offsets, frame_yx, values[..., 0], values[..., 1:1 + c], values[..., 1 + c:])
 
-    def run_host_records(self, frames, points_capacity=4096):
+    def run_host_records(self, frames, points_capacity=4096, patch_radius=None):
         """``run_frames_records`` on host frames: numpy ``[B, H, W, 3]`` (``frame_format="nv12"``: ``[B, H * 3 / 2, W]``
         uint8), pageable or page-locked. The frames go up once and only the records come back (``PointRecords`` of
         numpy arrays): ``orient`` and ``padded_line_end`` never cross the host link. ``points_capacity`` sizes the first
-        attempt; every point is returned."""
+        attempt; every point is returned. ``patch_radius`` as for ``run_frames_records`` (checked before the upload)."""
+        radius = _ops.patch_radius(patch_radius)
         frames = np.asarray(frames)
         nv12_hw = _ops.nv12_frame_hw(frames.shape, frames.dtype) if self._nv12() else None
         frames = np.ascontiguousarray(frames)
@@ -425,7 +446,7 @@ class LineEndPipeline:
         staged = torch.from_numpy(frames)
         if not staged.is_pinned():   # page-locked frames (e.g. views of pinned tensors) go up in place
             staged = staged.pin_memory()
-        rows = host_round_trip(staged, dev, lambda x: self._record_rows(x, points_capacity, None),
+        rows = host_round_trip(staged, dev, lambda x: self._record_rows(x, points_capacity, None, radius),
                                lambda i, shape, dtype: torch.empty(shape, dtype=dtype, pin_memory=True))
         return self._records(*rows)
 
