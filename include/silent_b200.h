@@ -183,6 +183,37 @@ int silent_top_value_points(const float *color_dev, const float *value_dev, int 
                             double top_percent, float *out_dev, void *workspace_dev, size_t workspace_bytes,
                             silent_stream stream);
 
+/* Peak feature points: every 3 x 3 local maximum of a level above its top-percent threshold. This project's composition
+ * of two reference operators, not a reference function: the per-level threshold of top_value_points (above) and the 3 x 3
+ * max-pool equality get_boosting uses as its non-max (util/energy/boosting.py:18-22). For each level v of value_dev
+ * [n,h,w,1] and p = top_percent in [0, 1]:
+ *   thr = float32(1 - p) * max(v) + float32(p) * min(v), in float32 without FMA (as silent_top_value_points; a NaN
+ *     anywhere in the level makes thr NaN);
+ *   pixel (y, x) fires iff v[y,x] > 0 and v[y,x] >= thr and v[y,x] >= the NaN-propagating maximum of the 3 x 3 window
+ *     around it, the pixel included and neighbours outside the level ignored (tf.nn.max_pool SAME).
+ * So a plateau fires on every one of its pixels (equality, as in the reference's non-max), a level holding a NaN emits
+ * nothing, and an all-zero level emits nothing (the v > 0 term: pad_inwards's zero border and the rows a level defines
+ * as 0 would otherwise fire wherever thr is 0, e.g. at p = 1). Output and capacity contract as for
+ * silent_max_value_indices_region: int64 rows (level, y, x, 0) in row-major order to points_dev[capacity][4], the TOTAL
+ * in *count_dev, only the first min(total, capacity) rows written, nothing past capacity. The rows feed
+ * silent_point_records / silent_point_patches and silent_pack_points unchanged. Workspace: silent_selection_workspace_bytes.
+ * Five kernels on `stream` (the threshold, then four programmatic dependent launches). Argument checks (all on the host,
+ * before any CUDA call): null pointers (points_dev may be NULL when capacity is 0), n, h or w <= 0, capacity < 0, or
+ * top_percent NaN or outside [0, 1] -> SILENT_E_INVAL; more than 65535 levels or levels of 2^30 pixels or more ->
+ * SILENT_E_SHAPE; a short workspace -> SILENT_E_CAPACITY. */
+int silent_peak_points(const float *value_dev, int n, int h, int w, double top_percent, int64_t *points_dev,
+                       int64_t capacity, int64_t *count_dev, void *workspace_dev, size_t workspace_bytes,
+                       silent_stream stream);
+
+/* silent_peak_points on the plan's own gray, [batch * L, h, w], with the plan's own workspace: the gray of the latest
+ * silent_pipeline_run* / silent_pipeline_run_host* call on this plan, with the validity and stream rules of gray_dev =
+ * NULL in silent_point_records. A caller runs silent_pipeline_run* with count_dev = NULL (no region emit) and then this,
+ * and when *count_dev exceeds the capacity redoes only this call with a larger buffer. Argument checks (all on the host,
+ * before any CUDA call): those of silent_peak_points (batch <= 0 -> SILENT_E_INVAL; a plan of 0 levels or more than 65535
+ * levels in batch * L -> SILENT_E_SHAPE), and batch above the plan's reserve -> SILENT_E_CAPACITY. */
+int silent_plan_peak_points(silent_plan *plan, int batch, double top_percent, int64_t *points_dev, int64_t capacity,
+                            int64_t *count_dev, silent_stream stream);
+
 /* cv2.cvtColor(frame, cv2.COLOR_YUV2BGR_NV12) for a batch on the GPU: nv12_dev [batch, h * 3 / 2, w] uint8 (layout at
  * SILENT_NV12) -> bgr_dev [batch, h, w, 3] uint8, both contiguous. h and w even. BT.601 limited range in 20-bit fixed
  * point, bit-identical to OpenCV's integer code: with u = U - 128, v = V - 128 of the pixel's 2 x 2 block and

@@ -29,7 +29,7 @@ SYMBOLS = (
     "silent_comm_unique_id", "silent_comm_create", "silent_comm_destroy", "silent_comm_check", "silent_gather_points",
     "silent_stack_fused_f16", "silent_stack_bank_f16", "silent_pipeline_run_f16", "silent_pipeline_run_orientations_f16",
     "silent_pipeline_run_host_f16", "silent_nv12_to_bgr", "silent_plan_level_coords", "silent_point_records",
-    "silent_point_patches",
+    "silent_point_patches", "silent_peak_points", "silent_plan_peak_points",
 )
 
 
@@ -108,6 +108,8 @@ def lib():
         "silent_selection_workspace_bytes": (sz, [i, i, i]),
         "silent_max_value_indices_region": (i, [p, i, i, i, i, i, p, i64, p, p, sz, p]),
         "silent_top_value_points": (i, [p, p, i, i, i, i, d, p, p, sz, p]),
+        "silent_peak_points": (i, [p, i, i, i, d, p, i64, p, p, sz, p]),
+        "silent_plan_peak_points": (i, [p, i, d, p, i64, p, p]),
         "silent_stack_workspace_bytes": (sz, [i, i, i]),
         "silent_stack_fused": (i, [p, i, i, i, ctypes.POINTER(SilentStackWeights), p, p, p, p, sz, p]),
         "silent_pipeline_run": (i, [p, ctypes.POINTER(SilentStackWeights), p, i, p, p, p, p, i64, p, p]),

@@ -4,6 +4,7 @@ Tensors are contiguous float32 NHWC ``[levels, h, w, C]`` on a CUDA device (the 
 ``recognition_testing.py:62``); numpy inputs are uploaded to the current CUDA device.
 """
 import ctypes
+import numbers
 import threading
 
 import numpy as np
@@ -144,6 +145,50 @@ def max_value_indices_region(value, region_h, region_w, capacity=None):
             if total <= cap or capacity is not None:
                 return pts[:min(total, cap)]
             cap = total
+
+
+def peak_percent(top_percent):
+    """``top_percent`` of the peak emit as a float in [0, 1]; anything else (a bool, a non-number, NaN, a value out of
+    range) raises ValueError."""
+    if isinstance(top_percent, (bool, np.bool_)) or not isinstance(top_percent, numbers.Real):
+        raise ValueError("peaks (top_percent) must be a real number in [0, 1], got %r" % (top_percent,))
+    p = float(top_percent)
+    if not 0.0 <= p <= 1.0:
+        raise ValueError("peaks (top_percent) must be in [0, 1], got %r" % (top_percent,))
+    return p
+
+
+def peak_points(value, top_percent, capacity=None):
+    """``silent_peak_points``: int64 rows ``(level, y, x, 0)`` of every 3 x 3 local maximum of ``value``
+    ``[n, h, w, 1]`` that is > 0 and >= its level's top-percent threshold, in row-major order. Without ``capacity``
+    every point is returned (one host synchronisation, and a second emit when they exceed the first buffer); with it, at
+    most ``capacity`` rows."""
+    p = peak_percent(top_percent)
+    v = as_device_tensor(value)
+    n, h, w, c = _nhwc(v, "peak_points")
+    if c != 1:
+        raise ValueError("value tensor must have one channel")
+    ws, nbytes = _selection_workspace(n, h, w, v.device)
+    cap = int(capacity) if capacity is not None else max(64 * n, 1024)
+    count = torch.zeros(1, dtype=torch.int64, device=v.device)
+    with torch.cuda.device(v.device):
+        while True:
+            pts = torch.empty((cap, 4), dtype=torch.int64, device=v.device)
+            _lib.check(_lib.lib().silent_peak_points(ptr(v), n, h, w, p, ptr(pts), cap, ptr(count), ptr(ws), nbytes,
+                                                     stream_ptr()), "silent_peak_points")
+            total = int(count.item())
+            if total <= cap or capacity is not None:
+                return pts[:min(total, cap)]
+            cap = total
+
+
+def plan_peak_points(plan, batch, top_percent, points, count):
+    """``silent_plan_peak_points``: the peak emit on the plan's own gray of its latest pipeline call (``batch`` frames)
+    into ``points`` ``[capacity, 4]`` int64 and the int64 device scalar ``count``; no host synchronisation."""
+    with torch.cuda.device(points.device):
+        _lib.check(_lib.lib().silent_plan_peak_points(plan.handle, int(batch), float(top_percent), ptr(points),
+                                                      int(points.shape[0]), ptr(count), stream_ptr()),
+                   "silent_plan_peak_points")
 
 
 def top_value_points(color, value, top_percent):

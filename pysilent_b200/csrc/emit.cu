@@ -463,6 +463,177 @@ __global__ void apply_threshold_kernel(const float *__restrict__ color, const fl
     out[i] = color[i] * keep;
 }
 
+// ---- peak emit: every 3x3 local maximum of a level above its top-percent threshold -------------------------------------
+// Pixel (y, x) of level v fires iff v > 0, v >= thr (level_threshold_kernel) and v >= the NaN-propagating maximum of the
+// 3x3 window around it (TF max_pool SAME: neighbours outside the level are ignored). Rows of (level, y, x, 0) in row-major
+// order: peak_count_kernel counts each row's hits, scan_level_kernel turns the counts into offsets within the level,
+// peak_base_kernel scans the level totals into each level's first row (and the grand total), peak_write_kernel writes
+// each row's hits in x order at its level base + row offset. The hit test reads rows y - 1, y and y + 1.
+
+__device__ __forceinline__ float max_nan(float a, float b)
+{
+    float r;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+    return r;
+}
+
+// V = 4: the run of pixels x .. x + 3 as one 128-bit load (the row length is a multiple of 4 and the tensor 16-byte
+// aligned); V = 1: pixel x. Out of the level (row null, or x >= w): -inf, which every comparison below ignores.
+template <int V>
+__device__ __forceinline__ void load_run(const float *row, int x, int w, float (&f)[V])
+{
+    if (V == 4) {
+        float4 q = make_float4(kNegInf, kNegInf, kNegInf, kNegInf);
+        if (row && x < w) q = __ldg(reinterpret_cast<const float4 *>(row + x));
+        f[0] = q.x, f[1] = q.y, f[2] = q.z, f[3] = q.w;
+    } else {
+        f[0] = row && x < w ? __ldg(row + x) : kNegInf;
+    }
+}
+
+__device__ __forceinline__ float column_max(const float *up, const float *mid, const float *down, int x)
+{
+    const float a = up ? __ldg(up + x) : kNegInf, c = down ? __ldg(down + x) : kNegInf;
+    return max_nan(max_nan(a, __ldg(mid + x)), c);
+}
+
+// Hit mask (bit i: pixel x + i) of the lane's run in row `mid`; every lane of the warp calls it (the columns next to the
+// run come from the neighbouring lanes; lanes 0 and 31 read theirs). x >= w: no hits.
+template <int V>
+__device__ __forceinline__ unsigned peak_bits(const float *up, const float *mid, const float *down, int x, int w,
+                                              float thr, int lane)
+{
+    float a[V], v[V], c[V], col[V];
+    load_run<V>(up, x, w, a);
+    load_run<V>(mid, x, w, v);
+    load_run<V>(down, x, w, c);
+#pragma unroll
+    for (int i = 0; i < V; ++i) col[i] = max_nan(max_nan(a[i], v[i]), c[i]);
+    float left = __shfl_up_sync(0xffffffffu, col[V - 1], 1);
+    float right = __shfl_down_sync(0xffffffffu, col[0], 1);
+    if (lane == 0) left = x > 0 && x < w ? column_max(up, mid, down, x - 1) : kNegInf;
+    if (x + V >= w) right = kNegInf;
+    else if (lane == 31) right = column_max(up, mid, down, x + V);
+    unsigned bits = 0;
+#pragma unroll
+    for (int i = 0; i < V; ++i) {
+        const float m = max_nan(max_nan(i == 0 ? left : col[i - 1], col[i]), i == V - 1 ? right : col[i + 1]);
+        if (x + i < w && v[i] > 0.0f && v[i] >= thr && v[i] >= m) bits |= 1u << i;
+    }
+    return bits;
+}
+
+struct PeakRow {
+    const float *up, *mid, *down;
+    float thr;
+};
+
+__device__ __forceinline__ PeakRow peak_row(const float *value, int row, int h, int w, const float *thr)
+{
+    const int n = row / h, y = row - n * h;
+    const float *mid = value + (size_t)row * w;
+    return PeakRow{y > 0 ? mid - w : nullptr, mid, y + 1 < h ? mid + w : nullptr, __ldg(thr + n)};
+}
+
+// COUNT pass: one warp per row (level, y); 128-bit loads under count_rows_kernel's condition; writes the row's hit count.
+__global__ void __launch_bounds__(256) peak_count_kernel(const float *__restrict__ value, int rows, int h, int w,
+                                                         const float *__restrict__ thr, int *__restrict__ row_count)
+{
+    pdl_enter();
+    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= rows) return;
+    const PeakRow r = peak_row(value, row, h, w, thr);
+    int hits = 0;
+    if ((w & 3) == 0 && (reinterpret_cast<uintptr_t>(value) & 15) == 0) {
+        for (int x0 = 0; x0 < w; x0 += 128) hits += __popc(peak_bits<4>(r.up, r.mid, r.down, x0 + 4 * lane, w, r.thr, lane));
+    } else {
+        for (int x0 = 0; x0 < w; x0 += 32) hits += __popc(peak_bits<1>(r.up, r.mid, r.down, x0 + lane, w, r.thr, lane));
+    }
+    hits = __reduce_add_sync(0xffffffffu, hits);
+    if (lane == 0) row_count[row] = hits;
+}
+
+// One CTA: exclusive scan of the level totals -> level_base (the first row of each level), and the grand total. Replaces
+// write_rows_kernel's per-row sum over the levels before, which dense output (most rows with hits) would pay per row.
+__global__ void __launch_bounds__(1024) peak_base_kernel(const int *__restrict__ level_total, int levels,
+                                                         long long *__restrict__ level_base, long long *__restrict__ total)
+{
+    pdl_enter();
+    __shared__ long long s_warp[32];
+    __shared__ long long s_carry;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x == 0) s_carry = 0;
+    __syncthreads();
+    for (int base = 0; base < levels; base += 1024) {
+        const int i = base + threadIdx.x;
+        const long long mine = i < levels ? __ldg(level_total + i) : 0;
+        long long incl = mine;
+        for (int o = 1; o < 32; o <<= 1) {
+            const long long up = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += up;
+        }
+        if (lane == 31) s_warp[warp] = incl;
+        __syncthreads();
+        long long before = s_carry + incl - mine;
+        for (int k = 0; k < warp; ++k) before += s_warp[k];
+        if (i < levels) level_base[i] = before;
+        __syncthreads();
+        if (threadIdx.x == 1023) s_carry = before + mine;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *total = s_carry;
+}
+
+// WRITE pass: one warp per row with hits; each lane's hits go at the row's slot + the hits of the lanes before it (a warp
+// scan of the per-lane counts), so the rows come out in x order without a pass per hit.
+template <int V>
+__device__ __forceinline__ void write_peak_row(const PeakRow &r, int n, int y, int w, long long slot, int lane,
+                                               long long *__restrict__ points, long long capacity)
+{
+    for (int x0 = 0; x0 < w; x0 += 32 * V) {
+        const int x = x0 + V * lane;
+        unsigned bits = peak_bits<V>(r.up, r.mid, r.down, x, w, r.thr, lane);
+        const int mine = __popc(bits);
+        int incl = mine;
+        for (int o = 1; o < 32; o <<= 1) {
+            const int up = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += up;
+        }
+        long long at = slot + incl - mine;
+        while (bits) {
+            const int i = __ffs(bits) - 1;
+            bits &= bits - 1;
+            if (at < capacity) {
+                reinterpret_cast<longlong2 *>(points)[at * 2] = make_longlong2(n, y);
+                reinterpret_cast<longlong2 *>(points)[at * 2 + 1] = make_longlong2(x + i, 0);
+            }
+            ++at;
+        }
+        slot += __shfl_sync(0xffffffffu, incl, 31);
+    }
+}
+
+__global__ void __launch_bounds__(256) peak_write_kernel(const float *__restrict__ value, int rows, int h, int w,
+                                                         const float *__restrict__ thr,
+                                                         const int *__restrict__ row_offset,
+                                                         const long long *__restrict__ level_base,
+                                                         long long *__restrict__ points, long long capacity)
+{
+    pdl_enter();
+    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= rows || capacity <= 0) return;
+    const int packed = __ldg(row_offset + row);
+    if (!(packed & 0x40000000)) return;
+    const int n = row / h, y = row - n * h;
+    const long long slot = __ldg(level_base + n) + (packed & 0x3fffffff);
+    if (slot >= capacity) return;
+    const PeakRow r = peak_row(value, row, h, w, thr);
+    if ((w & 3) == 0 && (reinterpret_cast<uintptr_t>(value) & 15) == 0) write_peak_row<4>(r, n, y, w, slot, lane, points, capacity);
+    else write_peak_row<1>(r, n, y, w, slot, lane, points, capacity);
+}
+
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 size_t selection_bytes(int n, int h, int w)
@@ -559,6 +730,54 @@ int max_value_indices_region(const float *value, int n, int h, int w, int region
     return SILENT_OK;
 }
 
+// Host-side checks of the peak emit's shape and top_percent (`who` prefixes the messages); SILENT_OK or the status.
+static int check_peaks(const char *who, int64_t n, int h, int w, double top_percent, int64_t capacity)
+{
+    if (n <= 0 || h <= 0 || w <= 0) return fail(SILENT_E_INVAL, "%s: bad shape", who);
+    if (capacity < 0) return fail(SILENT_E_INVAL, "%s: capacity must be >= 0", who);
+    if (!(top_percent >= 0.0 && top_percent <= 1.0))   // (NaN fails both)
+        return fail(SILENT_E_INVAL, "%s: top_percent must be in [0, 1], got %g", who, top_percent);
+    if (n > 65535) return fail(SILENT_E_SHAPE, "%s: at most 65535 levels per call, got %lld", who, (long long)n);
+    if ((long long)h * w >= (1 << 30)) return fail(SILENT_E_SHAPE, "%s: levels of 2^30 pixels or more are not supported", who);
+    if (n * h > INT32_MAX - 255) return fail(SILENT_E_SHAPE, "%s: %lld rows are too many for one call", who, (long long)(n * h));
+    return SILENT_OK;
+}
+
+// The peak emit on checked arguments: level_threshold_kernel, then the four row kernels (programmatic dependent
+// launches). Workspace: thr in the window-maxima area, level_base in the reserved words, row_offset and level_total as
+// for max_value_indices_region.
+static int peak_points(const float *value, int n, int h, int w, double top_percent, int64_t *points, int64_t capacity,
+                       int64_t *count, void *workspace, cudaStream_t stream)
+{
+    const int rows = n * h;
+    char *ws = (char *)workspace;
+    float *thr = (float *)ws;
+    ws += align_up((size_t)n * 4096 * sizeof(float), 256);
+    int *row_offset = (int *)ws;
+    ws += align_up((size_t)rows * sizeof(int), 256);
+    long long *level_base = (long long *)ws;
+    ws += align_up((size_t)n * sizeof(long long), 256);
+    int *level_total = (int *)ws;
+    // the constants of silent_top_value_points: (1.0 - p) and p rounded to float32
+    const float keep_max = (float)(1.0 - top_percent), keep_min = (float)top_percent;
+    level_threshold_kernel<<<n, 256, 0, stream>>>(value, h * w, keep_max, keep_min, thr);
+    SILENT_LAUNCH_CHECK("level_threshold_kernel");
+    const unsigned blocks = (unsigned)ceil_div(rows, 8);
+    SILENT_CUDA(launch_dependent(peak_count_kernel, dim3(blocks), dim3(256), 0, stream, value, rows, h, w,
+                                 (const float *)thr, row_offset));
+    SILENT_LAUNCH_CHECK("peak_count_kernel");
+    SILENT_CUDA(launch_dependent(scan_level_kernel, dim3(n), dim3(256), 0, stream, row_offset, h, level_total));
+    SILENT_LAUNCH_CHECK("scan_level_kernel");
+    SILENT_CUDA(launch_dependent(peak_base_kernel, dim3(1), dim3(1024), 0, stream, (const int *)level_total, n, level_base,
+                                 (long long *)count));
+    SILENT_LAUNCH_CHECK("peak_base_kernel");
+    SILENT_CUDA(launch_dependent(peak_write_kernel, dim3(blocks), dim3(256), 0, stream, value, rows, h, w,
+                                 (const float *)thr, (const int *)row_offset, (const long long *)level_base,
+                                 (long long *)points, (long long)capacity));
+    SILENT_LAUNCH_CHECK("peak_write_kernel");
+    return SILENT_OK;
+}
+
 }  // namespace silent
 
 using namespace silent;
@@ -577,6 +796,39 @@ int silent_max_value_indices_region(const float *value_dev, int n, int h, int w,
 {
     return max_value_indices_region(value_dev, n, h, w, region_h, region_w, points_dev, capacity, count_dev,
                                     workspace_dev, workspace_bytes, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+int silent_peak_points(const float *value_dev, int n, int h, int w, double top_percent, int64_t *points_dev,
+                       int64_t capacity, int64_t *count_dev, void *workspace_dev, size_t workspace_bytes,
+                       silent_stream stream)
+{
+    if (!value_dev || !count_dev || !workspace_dev || (!points_dev && capacity > 0))
+        return fail(SILENT_E_INVAL, "silent_peak_points: null argument");
+    const int rc = check_peaks("silent_peak_points", n, h, w, top_percent, capacity);
+    if (rc != SILENT_OK) return rc;
+    if (workspace_bytes < selection_bytes(n, h, w))
+        return fail(SILENT_E_CAPACITY, "silent_peak_points: selection workspace too small: %zu < %zu", workspace_bytes,
+                    selection_bytes(n, h, w));
+    return peak_points(value_dev, n, h, w, top_percent, points_dev, capacity, count_dev, workspace_dev,
+                       (cudaStream_t)stream);
+}
+
+int silent_plan_peak_points(silent_plan *plan, int batch, double top_percent, int64_t *points_dev, int64_t capacity,
+                            int64_t *count_dev, silent_stream stream)
+{
+    if (!plan || !count_dev || (!points_dev && capacity > 0))
+        return fail(SILENT_E_INVAL, "silent_plan_peak_points: null argument");
+    if (batch <= 0) return fail(SILENT_E_INVAL, "silent_plan_peak_points: batch must be positive");
+    if (plan->levels == 0) return fail(SILENT_E_SHAPE, "frame is not larger than the pyramid centre: 0 levels");
+    const int rc = check_peaks("silent_plan_peak_points", (int64_t)batch * plan->levels, plan->h, plan->w, top_percent,
+                               capacity);
+    if (rc != SILENT_OK) return rc;
+    if (batch > plan->ws.batch)
+        return fail(SILENT_E_CAPACITY, "silent_plan_peak_points: the plan's gray holds %d frames (silent_plan_reserve), "
+                    "need %d", plan->ws.batch, batch);
+    if (!plan->on_device) return fail(SILENT_E_CUDA, "plan was created without a CUDA device; no CPU fallback exists");
+    return peak_points(plan->ws.d_gray, batch * plan->levels, plan->h, plan->w, top_percent, points_dev, capacity,
+                       count_dev, plan->ws.d_select, (cudaStream_t)stream);
 }
 
 int silent_top_value_points(const float *color_dev, const float *value_dev, int n, int h, int w, int c,

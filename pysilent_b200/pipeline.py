@@ -89,10 +89,18 @@ class LineEndPipeline:
     then H / 2 rows of interleaved U, V), H and W even. An NV12 call returns exactly what the same call returns on the
     frames ``cv2.cvtColor(frame, cv2.COLOR_YUV2BGR_NV12)`` makes of them; the conversion runs on the GPU, in front of the
     pyramid, and only the bytes of the NV12 frames cross the host link.
+
+    ``peaks`` chooses the feature points of every entry point. ``None`` (default) keeps the reference's region maxima
+    (``max_value_indices_region``, one to four points per level). A real number p in [0, 1] emits the peaks of every
+    level instead (``silent_peak_points``): each pixel that is > 0, >= the level's top-percent threshold
+    ``float32(1 - p) * max + float32(p) * min`` (``top_value_points``) and >= every pixel of its 3 x 3 neighbourhood. A
+    plateau fires on every pixel, and a level holding a NaN or only zeros emits nothing. The rows keep the format and
+    order of the region maxima, so records, patches and the point gathers take them as they are.
     """
 
     def __init__(self, n_dimensions=2, output_size=(288, 192), output_colors=3, zoom_ratio=math.e ** .5, device=None,
-                 orientations=None, out_dtype=torch.float32, frame_format="bgr"):
+                 orientations=None, out_dtype=torch.float32, frame_format="bgr", peaks=None):
+        self.peaks = _ops.peak_percent(peaks) if peaks is not None else None
         if out_dtype not in _ops.OUT_DTYPES:
             raise ValueError("out_dtype must be torch.float32 or torch.float16, got %r" % (out_dtype,))
         if not isinstance(frame_format, str) or frame_format not in _ops.FRAME_FORMATS:
@@ -141,7 +149,10 @@ class LineEndPipeline:
         return self.frame_format == "nv12"
 
     def _points(self, gray):
-        """Feature points of ``gray``: the maxima of the reference's region windows (``recognition_testing.py:40``)."""
+        """Feature points of ``gray``: the maxima of the reference's region windows (``recognition_testing.py:40``), or
+        its peaks with ``peaks`` set."""
+        if self.peaks is not None:
+            return _ops.peak_points(gray, self.peaks)
         rh, rw = self.region_shape[1], self.region_shape[2]
         if int(rh) != rh or int(rw) != rw:
             raise ValueError("Ambiguous dimension: %s" % ([rh, rw],))
@@ -325,18 +336,30 @@ class LineEndPipeline:
             name, args = "silent_pipeline_run_orientations", (ctypes.byref(self.orientation_bank()), _ops.ptr(frames), b)
         if self._half():
             name += "_f16"
+        # the emit step: the region maxima inside the pipeline call, or the peaks after it on the plan's own gray
+        peaks = want_points and self.peaks is not None
         with torch.cuda.device(dev):
             _lib.check(getattr(_lib.lib(), name)(
                 plan.handle, *args, _ops.ptr(orient), _ops.ptr(line_end), _ops.ptr(points), cap,
-                _ops.ptr(count) if want_points else None, _ops.stream_ptr()), name)
+                _ops.ptr(count) if want_points and not peaks else None, _ops.stream_ptr()), name)
+        if peaks:
+            _ops.plan_peak_points(plan, b, self.peaks, points, count)
         if out is not None:
             return LineEndResult(orient, line_end, None, points)
         if not want_points:
             return LineEndResult(orient, line_end, None, None)
         total = int(count.item())
-        if total > cap:   # rare (e.g. an all-black level emits every pixel): redo the emit with room for everything
+        if total > cap and peaks:   # only the emit again, on the plan's gray of this call
+            points = self._plan_peaks(plan, b, total, count)
+        elif total > cap:   # rare (e.g. an all-black level emits every pixel): redo the emit with room for everything
             return self._run_plan(frames, nb, want_points, total, None, nv12_hw)
         return LineEndResult(orient, line_end, None, points[:total])
+
+    def _plan_peaks(self, plan, b, capacity, count):
+        """The peaks of the plan's gray of its latest call (``b`` frames) into new points of ``capacity`` rows."""
+        points = torch.empty((capacity, 4), dtype=torch.int64, device=count.device)
+        _ops.plan_peak_points(plan, b, self.peaks, points, count)
+        return points
 
     # -- feature-point records ------------------------------------------------------------------------------------------
     def run_frames_records(self, frames, points_capacity=None, out=None, patch_radius=None):
@@ -410,7 +433,9 @@ class LineEndPipeline:
         if out is None and radius is not None:
             # patches for the whole default capacity could take GBs: size them by the points found
             total = int(count.item())
-            if total > points.shape[0]:
+            if total > points.shape[0] and self.peaks is not None:   # only the emit again, as run_frames
+                points = self._plan_peaks(plan, b, total, count)
+            elif total > points.shape[0]:
                 return self._run_plan_records(frames, nb, total, None, nv12_hw, radius)
             points = points[:total]
             return (points,) + _ops.point_records(plan, b, points, count, orient, line_end, None, radius=radius)
@@ -418,7 +443,10 @@ class LineEndPipeline:
         if out is not None:
             return (points,) + recs
         total = int(count.item())
-        if total > points.shape[0]:   # as run_frames: redo with room for every point
+        if total > points.shape[0] and self.peaks is not None:   # only the emit again, then the records of every point
+            points = self._plan_peaks(plan, b, total, count)
+            recs = _ops.point_records(plan, b, points, count, orient, line_end, None)
+        elif total > points.shape[0]:   # as run_frames: redo with room for every point
             return self._run_plan_records(frames, nb, total, None, nv12_hw)
         frame_offsets, frame_yx, values = recs
         return points[:total], frame_offsets, frame_yx[:total], values[:total]
@@ -453,8 +481,8 @@ class LineEndPipeline:
     # -- host buffers on both sides (LineEndDisplayer.callback) -----------------------------------------------------------
     def run_host(self, frames, orient_out=None, line_end_out=None, points_capacity=4096):
         """frames: host numpy ``[B, H, W, 3]`` (``frame_format="nv12"``: ``[B, H * 3 / 2, W]`` uint8; ideally page-locked)
-        -> host numpy results via the C-ABI host call (with ``orientations`` set, or off the ``PLAN`` route: through
-        ``run_frames`` and page-locked buffers, results ``[B * L, h, w, orientations]``). With
+        -> host numpy results via the C-ABI host call (with ``orientations`` or ``peaks`` set, or off the ``PLAN``
+        route: through ``run_frames`` and page-locked buffers, results ``[B * L, h, w, orientations]``). With
         ``out_dtype=torch.float16`` the results are ``np.float16``, and so must be ``orient_out`` / ``line_end_out``."""
         nb = self._bank_width() if self.orientations is not None else None
         if self._half():
@@ -470,7 +498,9 @@ class LineEndPipeline:
             frames = frames.astype(np.float32)
         dev = self._device()
         tdtype = torch.uint8 if frames.dtype == np.uint8 else torch.float32
-        if nb is not None or self._frame_route(nb, self.frame_format, tdtype, frames.shape) != PLAN:
+        # banks, peaks and the routes off PLAN go through run_frames (the C host-buffer call emits region maxima only)
+        if nb is not None or self.peaks is not None or self._frame_route(nb, self.frame_format, tdtype,
+                                                                          frames.shape) != PLAN:
             def run(x):   # through run_frames: the frames in and the results out through new page-locked buffers
                 res = self.run_frames(x, points_capacity=points_capacity)
                 return res.orient, res.padded_line_end, res.points
