@@ -447,6 +447,33 @@ int silent_point_patches(const silent_plan *plan, int batch, const int64_t *poin
                          const float *gray_dev, int radius, int64_t *frame_offsets_dev, float *coords_dev,
                          float *values_dev, silent_stream stream);
 
+/* ---- feature-point matches ---------------------------------------------------------------------------------------------
+ * Links between the points of consecutive frames of one batch, computed on the device from the records, so that a
+ * tracker needs a few bytes per point instead of the patches. Reads the first rows = clamp(*count_dev, 0, capacity) rows
+ * (level, y, x, 0) of points_dev [capacity][4] (level = frame * levels + l, sorted by (level, y, x) as every emit writes
+ * them; the order is not checked, but nothing outside [0, rows) is read) and their descriptors values_dev
+ * [capacity][row_elems] float32 (a record's values, P * P * (1 + 2C) with a patch). Level n of frame f pairs with level
+ * n + levels of frame f + 1:
+ *   candidates of row i in the next frame: rows j of level_i + levels with |y_j - y_i| <= search_radius and
+ *     |x_j - x_i| <= search_radius (level pixels); in the previous frame the same with level_i - levels;
+ *   SSD(i, j): for k = 0..31, s_k = +0.0, then for e = k, k + 32, ... < row_elems: d = a_e - b_e, s_k = s_k + d * d;
+ *     then for m = 16, 8, 4, 2, 1: s_k = s_k + s_(k xor m); SSD = s_0. Float32, every operation rounded to nearest, no
+ *     fused products. Symmetric in i and j bit for bit. A candidate whose SSD is NaN is ignored;
+ *   raw link of i in one direction: the candidate of smallest SSD d1 (ties to the smaller row), kept iff
+ *     d1 <= float32(max_ratio) * d2 (rounded), d2 the smallest SSD over the other candidates (+inf without any);
+ *     max_ratio = 1 turns the test off, and it applies to SSD (Lowe's 0.8 on distances is 0.64 here);
+ *   accepted match i -> j: j is i's raw link in the next frame and i is j's raw link in the previous frame.
+ * Outputs, over the whole capacity: next_dev [capacity] int64, j or -1; prev_dev [capacity] int64, i for the j above or
+ * -1; distance_dev [capacity] float32, SSD(i, next[i]) or NaN where next is -1. Rows at or past `rows` get -1 / -1 / NaN.
+ * Matches never span calls: a stream processed in batches keeps one frame of overlap. No plan and no workspace. Two
+ * kernels, launched as programmatic dependent launches on `stream`; capacity 0 launches nothing. Argument checks (all
+ * on the host, before any CUDA call): a null count_dev, capacity < 0, a null points, values or output pointer with
+ * capacity > 0, or max_ratio NaN, <= 0 or > 1 -> SILENT_E_INVAL; row_elems < 1, levels < 1 or search_radius < 0 ->
+ * SILENT_E_SHAPE; no CUDA device -> SILENT_E_CUDA. */
+int silent_match_points(const int64_t *points_dev, const int64_t *count_dev, int64_t capacity, const float *values_dev,
+                        int64_t row_elems, int levels, int search_radius, float max_ratio, int64_t *next_dev,
+                        int64_t *prev_dev, float *distance_dev, silent_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -29,7 +29,7 @@ SYMBOLS = (
     "silent_comm_unique_id", "silent_comm_create", "silent_comm_destroy", "silent_comm_check", "silent_gather_points",
     "silent_stack_fused_f16", "silent_stack_bank_f16", "silent_pipeline_run_f16", "silent_pipeline_run_orientations_f16",
     "silent_pipeline_run_host_f16", "silent_nv12_to_bgr", "silent_plan_level_coords", "silent_point_records",
-    "silent_point_patches", "silent_peak_points", "silent_plan_peak_points",
+    "silent_point_patches", "silent_peak_points", "silent_plan_peak_points", "silent_match_points",
 )
 
 
@@ -126,6 +126,7 @@ def lib():
         "silent_nv12_to_bgr": (i, [p, i, i, i, p, p]),
         "silent_point_records": (i, [p, i, p, p, i64, p, p, i, i, p, p, p, p, p]),
         "silent_point_patches": (i, [p, i, p, p, i64, p, p, i, i, p, i, p, p, p, p]),
+        "silent_match_points": (i, [p, p, i64, p, i64, i, i, f, p, p, p, p]),
         "silent_get_centroids": (i, [p, i, i, i, i, i, p, p, p, p]),
         "silent_resize_nearest": (i, [p, i, i, i, i, i, i, p, p]),
         "silent_get_boosting": (i, [p, p, i, i, i, f, f, i, p, p, p]),

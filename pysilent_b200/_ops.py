@@ -480,3 +480,66 @@ def point_records(plan, batch, points, count, orient, line_end, gray=None, frame
                 plan.handle, batch, ptr(points), ptr(count), cap, ptr(orient), ptr(line_end), c, half, ptr(gray),
                 radius, ptr(frame_offsets), ptr(frame_yx), ptr(values), stream_ptr()), "silent_point_patches")
     return frame_offsets, frame_yx, values
+
+
+def match_radius(radius):
+    """``radius`` of the match search window as an int in ``[0, 2^31 - 1]``; anything else (a bool, a float, a str, a
+    negative value) raises ValueError."""
+    if isinstance(radius, (bool, np.bool_)) or not isinstance(radius, (int, np.integer)):
+        raise ValueError("search radius must be an int, got %r" % (radius,))
+    if not 0 <= radius <= 2 ** 31 - 1:
+        raise ValueError("search radius must be in [0, 2^31 - 1], got %d" % radius)
+    return int(radius)
+
+
+def match_ratio(max_ratio):
+    """``max_ratio`` of the match ratio test as a float in (0, 1]; anything else (a bool, a non-number, NaN, a value out
+    of range) raises ValueError."""
+    if isinstance(max_ratio, (bool, np.bool_)) or not isinstance(max_ratio, numbers.Real):
+        raise ValueError("max_ratio must be a real number in (0, 1], got %r" % (max_ratio,))
+    m = float(max_ratio)
+    if not 0.0 < m <= 1.0 or not 0.0 < float(np.float32(m)) <= 1.0:
+        raise ValueError("max_ratio must be in (0, 1], got %r" % (max_ratio,))
+    return m
+
+
+def match_points(points, count, values, levels, search_radius, max_ratio=1.0, next=None, prev=None, distance=None):
+    """``silent_match_points``: mutual nearest descriptors between consecutive frames. ``points`` ``[capacity, 4]``
+    int64 rows ``(level, y, x, 0)`` sorted by (level, y, x), level = frame * ``levels`` + l; ``count`` an int64 device
+    scalar (the rows used are the first ``clamp(count, 0, capacity)``); ``values`` float32 ``[capacity, ...]``, each
+    row's descriptor of E = the product of the trailing shape elements. Returns ``(next, prev, distance)``: int64, int64
+    and float32 ``[capacity]`` (see ``pipeline.PointMatches``), into the given buffers where passed; no host
+    synchronisation. Shapes, dtypes, devices, contiguity and the arguments are checked first (ValueError)."""
+    radius = match_radius(search_radius)
+    ratio = match_ratio(max_ratio)
+    if isinstance(levels, (bool, np.bool_)) or not isinstance(levels, (int, np.integer)) or not 1 <= levels < 2 ** 31:
+        raise ValueError("match_points needs levels as an int >= 1, got %r" % (levels,))
+    for name, t in (("points", points), ("count", count), ("values", values)):
+        if not isinstance(t, torch.Tensor):
+            raise ValueError("%s must be a torch.Tensor, got %s" % (name, type(t).__name__))
+    if points.dim() != 2 or points.shape[1] != 4 or points.dtype != torch.int64:
+        raise ValueError("points must be int64 [capacity, 4], got %s %s" % (points.dtype, tuple(points.shape)))
+    cap = int(points.shape[0])
+    if count.dtype != torch.int64 or count.numel() < 1:
+        raise ValueError("count must be an int64 tensor of at least one element")
+    if values.dtype != torch.float32 or values.dim() < 1 or int(values.shape[0]) != cap:
+        raise ValueError("values must be float32 [%d, ...], got %s %s" % (cap, values.dtype, tuple(values.shape)))
+    elems = int(np.prod(values.shape[1:], dtype=np.int64))
+    if elems < 1:
+        raise ValueError("values must hold at least one element per row, got %s" % (tuple(values.shape),))
+    dev = points.device
+    mk = lambda dt: torch.empty((cap,), dtype=dt, device=dev)  # noqa: E731
+    next = mk(torch.int64) if next is None else next
+    prev = mk(torch.int64) if prev is None else prev
+    distance = mk(torch.float32) if distance is None else distance
+    for name, t, dt in (("next", next, torch.int64), ("prev", prev, torch.int64), ("distance", distance, torch.float32)):
+        if not isinstance(t, torch.Tensor) or t.dtype != dt or tuple(t.shape) != (cap,):
+            raise ValueError("%s must be %s [%d], got %s" % (name, dt, cap, getattr(t, "dtype", type(t).__name__)))
+    tensors = (points, count, values, next, prev, distance)
+    if any(not t.is_cuda or t.device != dev or not t.is_contiguous() for t in tensors):
+        raise ValueError("match_points needs contiguous CUDA tensors on one device")
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().silent_match_points(
+            ptr(points), ptr(count), cap, ptr(values), elems, int(levels), radius, ratio, ptr(next), ptr(prev),
+            ptr(distance), stream_ptr()), "silent_match_points")
+    return next, prev, distance

@@ -72,6 +72,25 @@ point's level, dy and dx in [-r, r], at [r + dy, r + dx]; +0.0 where that pixel 
 SAME zero padding reads there). points, frame_offsets and frame_yx stay one per point. gray, orient and line_end are
 views of one float32 values tensor [K,1 + 2C] ([K,P,P,1 + 2C] with a patch)."""
 
+PointMatches = collections.namedtuple("PointMatches", "next prev distance")
+PointMatches.__doc__ = """Links between the feature points of consecutive frames of one batch (``silent_match_points``),
+over the K rows of the ``PointRecords`` they come with: next: int64 [K], the row j of frame f + 1 that row i of frame f
+matches, or -1; prev: int64 [K], the row i for that j, or -1; distance: float32 [K], SSD(i, next[i]), or NaN where next
+is -1. next and prev are consistent (``prev[next[i]] == i``), so following next gives a track through the batch.
+
+Level n of frame f (n = f * L + l) pairs with level n + L of frame f + 1. The candidates of row i in the next frame are
+the rows j of that level with |y_j - y_i| <= R and |x_j - x_i| <= R in level pixels (R = ``search_radius``); in the
+previous frame the same with n - L. The distance of two rows is the float32 SSD of their descriptors, the record's
+values flattened (E = P * P * (1 + 2C) with a patch, 1 + 2C without), in a fixed order: lane k = 0..31 sums
+``d = a_e - b_e; s_k = s_k + d * d`` over e = k, k + 32, ... from +0.0, then ``s_k = s_k + s_(k xor m)`` for m = 16, 8, 4,
+2, 1 gives SSD = s_0; every operation rounded to nearest, no fused products, symmetric in the two rows bit for bit. A
+candidate of NaN SSD is ignored, so a row of NaN values matches nothing. In each direction d1 is the smallest SSD over
+the candidates (ties to the smaller row) and d2 the smallest over the others (+inf without any); the best candidate is
+the raw link iff ``d1 <= float32(max_ratio) * d2`` (rounded). ``max_ratio`` = 1 turns the test off; it applies to SSD,
+so Lowe's 0.8 on distances is 0.64 here. i -> j is accepted iff j is i's raw link in the next frame and i is j's in the
+previous one. Rows of the last frame have next = -1 and rows of frame 0 prev = -1: matches never span calls, so a stream
+processed in batches keeps one frame of overlap between consecutive batches to link them."""
+
 
 class LineEndPipeline:
     """Drop-in for the compute half of ``LineEndDisplayer`` (camera / window handling is out of scope).
@@ -380,10 +399,11 @@ class LineEndPipeline:
         The records are those of every route ``run_frames`` takes; like there, the ``PYRAMID`` route ignores ``out`` and
         ``points_capacity`` and returns every point in new tensors. Banks of widths other than 4, 8, 12 and 16, and a
         ``patch_radius`` that is not an int in [0, 31], raise ValueError."""
-        return self._records(*self._record_rows(frames, points_capacity, out, patch_radius))
+        return self._records(*self._record_rows(frames, points_capacity, out, patch_radius)[1])
 
     def _record_rows(self, frames, points_capacity, out, radius=None):
-        """``run_frames_records`` as ``(points, frame_offsets, frame_yx, values [K, 1 + 2C] or [K, P, P, 1 + 2C])``."""
+        """``run_frames_records`` as ``(L, (points, frame_offsets, frame_yx, values [K, 1 + 2C] or [K, P, P, 1 + 2C]))``,
+        L the levels per frame of the route's plan."""
         radius = _ops.patch_radius(radius)
         nb = self._bank_width() if self.orientations is not None else None
         c = nb or 3
@@ -412,8 +432,9 @@ class LineEndPipeline:
             count = torch.full((1,), len(res.points), dtype=torch.int64, device=res.points.device)
             recs = _ops.point_records(zplan, zframes.shape[0], res.points, count, res.orient, res.padded_line_end,
                                       res.gray, radius=radius)
-            return (res.points,) + recs
-        return self._run_plan_records(frames, nb, points_capacity, out, nv12_hw, radius)
+            return zplan.levels, (res.points,) + recs
+        levels = self._plan_of(frames, nv12_hw).levels
+        return levels, self._run_plan_records(frames, nb, points_capacity, out, nv12_hw, radius)
 
     def _run_plan_records(self, frames, nb, points_capacity, out, nv12_hw, radius=None):
         plan = self._plan_of(frames, nv12_hw)
@@ -463,6 +484,13 @@ class LineEndPipeline:
         numpy arrays): ``orient`` and ``padded_line_end`` never cross the host link. ``points_capacity`` sizes the first
         attempt; every point is returned. ``patch_radius`` as for ``run_frames_records`` (checked before the upload)."""
         radius = _ops.patch_radius(patch_radius)
+        staged, dev = self._stage_host(frames)
+        rows = host_round_trip(staged, dev, lambda x: self._record_rows(x, points_capacity, None, radius)[1],
+                               lambda i, shape, dtype: torch.empty(shape, dtype=dtype, pin_memory=True))
+        return self._records(*rows)
+
+    def _stage_host(self, frames):
+        """Host frames of ``run_host_records`` / ``run_host_matches`` as a batched page-locked tensor, and the device."""
         frames = np.asarray(frames)
         nv12_hw = _ops.nv12_frame_hw(frames.shape, frames.dtype) if self._nv12() else None
         frames = np.ascontiguousarray(frames)
@@ -474,9 +502,47 @@ class LineEndPipeline:
         staged = torch.from_numpy(frames)
         if not staged.is_pinned():   # page-locked frames (e.g. views of pinned tensors) go up in place
             staged = staged.pin_memory()
-        rows = host_round_trip(staged, dev, lambda x: self._record_rows(x, points_capacity, None, radius),
-                               lambda i, shape, dtype: torch.empty(shape, dtype=dtype, pin_memory=True))
-        return self._records(*rows)
+        return staged, dev
+
+    # -- feature-point matches ------------------------------------------------------------------------------------------
+    def run_frames_matches(self, frames, patch_radius, search_radius, max_ratio=1.0, points_capacity=None):
+        """The records of ``run_frames_records(frames, points_capacity, patch_radius=patch_radius)`` and the links between
+        the points of consecutive frames (``PointRecords``, ``PointMatches``), all CUDA tensors. Each point's descriptor
+        is its record's values: the patch of radius ``patch_radius`` (an int in [0, 31], or None for the one pixel).
+        ``search_radius`` R (an int >= 0) bounds the window in level pixels and ``max_ratio`` (in (0, 1]) is the ratio
+        test on SSD; see ``PointMatches``. Runs on every route, bank, ``out_dtype`` and ``peaks`` the records serve.
+        The three arguments are checked before any GPU work (ValueError)."""
+        radius, r, ratio = self._match_args(patch_radius, search_radius, max_ratio)
+        levels, rows = self._record_rows(frames, points_capacity, None, radius)
+        return self._records(*rows), self._matches(levels, rows, r, ratio)
+
+    @staticmethod
+    def _match_args(patch_radius, search_radius, max_ratio):
+        return _ops.patch_radius(patch_radius), _ops.match_radius(search_radius), _ops.match_ratio(max_ratio)
+
+    @staticmethod
+    def _matches(levels, rows, search_radius, max_ratio):
+        """``PointMatches`` of the rows ``_record_rows`` returns (every row found; its count is known on the host)."""
+        points, values = rows[0], rows[3]
+        count = torch.full((1,), points.shape[0], dtype=torch.int64, device=points.device)
+        return PointMatches(*_ops.match_points(points, count, values, levels, search_radius, max_ratio))
+
+    def run_host_matches(self, frames, patch_radius, search_radius, max_ratio=1.0, points_capacity=4096):
+        """``run_frames_matches`` on host frames, as ``run_host_records`` takes them: numpy ``(PointRecords,
+        PointMatches)``. The patches are matched on the device and never cross the host link: the records come without
+        them, their values are the patch centres (the records of ``run_host_records`` without a patch, bit for bit).
+        ``points_capacity`` sizes the first attempt; every point is returned. The arguments are checked before the
+        upload."""
+        radius, r, ratio = self._match_args(patch_radius, search_radius, max_ratio)
+        staged, dev = self._stage_host(frames)
+
+        def run(x):
+            levels, rows = self._record_rows(x, points_capacity, None, radius)
+            links = self._matches(levels, rows, r, ratio)
+            values = rows[3] if radius is None else rows[3][:, radius, radius].contiguous()
+            return rows[:3] + (values,) + tuple(links)
+        outs = host_round_trip(staged, dev, run, lambda i, shape, dtype: torch.empty(shape, dtype=dtype, pin_memory=True))
+        return self._records(*outs[:4]), PointMatches(*outs[4:])
 
     # -- host buffers on both sides (LineEndDisplayer.callback) -----------------------------------------------------------
     def run_host(self, frames, orient_out=None, line_end_out=None, points_capacity=4096):
