@@ -474,6 +474,60 @@ int silent_match_points(const int64_t *points_dev, const int64_t *count_dev, int
                         int64_t row_elems, int levels, int search_radius, float max_ratio, int64_t *next_dev,
                         int64_t *prev_dev, float *distance_dev, silent_stream stream);
 
+/* ---- frame-to-frame motion ---------------------------------------------------------------------------------------------
+ * How the camera moved between consecutive frames of one batch, and which matches agree with that motion: a 2-D affine
+ * map per frame pair, found by a seeded RANSAC on the device from the records and matches, so that only 48 bytes per
+ * pair and one byte per point come back. Reads the first rows = clamp(*count_dev, 0, capacity) rows, the batch + 1
+ * entries of frame_offsets_dev (the rows of frame f are [lo, hi) = [clamp(frame_offsets[f], 0, rows),
+ * clamp(frame_offsets[f + 1], lo, rows)), as silent_point_records writes them), frame_yx_dev [capacity][2] float32 (a
+ * record's frame coordinates, 8-byte aligned) and next_dev [capacity] int64 (silent_match_points' links). For each pair
+ * f = 0 .. batch - 2:
+ *   correspondences: the rows i of frame f, in row order, with 0 <= next[i] < rows and frame_yx[i], frame_yx[next[i]]
+ *     all finite (a level that defines an axis as 0 has NaN coordinates, so its rows never take part); M_f of them,
+ *     c_k = (y0, x0, y1, x1), k = 0 .. M_f - 1;
+ *   model: [y1, x1] = T[:, :2] @ [y0, x0] + T[:, 2] in frame pixels, T float64 [2][3] = (a, b, c; d, e, g);
+ *   hypothesis h = 0 .. hypotheses - 1: draws k_d = mulhi64(u_d, M_f) (the high 64 bits of the 128-bit product), d = 0,
+ *     1, 2, u_d = splitmix64(seed ^ splitmix64((f << 32) | (h << 2) | d)), splitmix64(z): z += 0x9e3779b97f4a7c15,
+ *     z = (z ^ z >> 30) * 0xbf58476d1ce4e5b9, z = (z ^ z >> 27) * 0x94d049bb133111eb, z ^ z >> 31 (64-bit wrapping).
+ *     Degenerate if two draws are equal. Otherwise, in float64 and this order: with (y0, x0) = c_k0's source and
+ *     dyj = yj - y0, dxj = xj - x0 for the sources of c_k1 (j = 1) and c_k2 (j = 2), D = dy1 * dx2 - dx1 * dy2;
+ *     degenerate if !(|D| >= 1) (NaN too). Then per target u (y1, then x1): du1 = u_k1 - u_k0, du2 = u_k2 - u_k0,
+ *     a = (du1 * dx2 - dx1 * du2) / D, b = (dy1 * du2 - du1 * dy2) / D, c = u_k0 - (a * y0 + b * x0);
+ *   score of a model T: with m = float32(T) (rounded once) and t2 = float32(threshold) * float32(threshold) (rounded),
+ *     c_k is an inlier iff e_y * e_y + e_x * e_x <= t2, e_y = y1 - ((m_a * y0 + m_b * x0) + m_c), e_x likewise with
+ *     (m_d, m_e, m_g); float32, every operation rounded to nearest, no fused products. A NaN residual is no inlier;
+ *   best hypothesis: the most inliers over the hypotheses that are not degenerate, ties to the smaller h;
+ *   refit: over the inliers of the best hypothesis, with (py, px, qy, qx) = c_k0 of that hypothesis and, in float64,
+ *     Y = y0 - py, X = x0 - px, U = y1 - qy, V = x1 - qx, the 11 sums S of Y, X, YY, YX, XX, U, YU, XU, V, YV, XV (in
+ *     that order of the products' factors). Each sum in a fixed order: thread t = 0..255 adds its terms over k = t,
+ *     t + 256, ... in order from +0.0 (a correspondence that is no inlier adds nothing); then within each warp of 32
+ *     threads s_t = s_t + s_(t xor b) for b = 16, 8, 4, 2, 1; then the warps' lane-0 sums w_0 .. w_7 are added as
+ *     ((w_0 + w_1) + w_2) + ... + w_7. With n the inlier count, c00 = Sxx*n - Sx*Sx, c01 = Sx*Sy - Syx*n,
+ *     c02 = Syx*Sx - Sxx*Sy, c11 = Syy*n - Sy*Sy, c12 = Syx*Sy - Syy*Sx, c22 = Syy*Sxx - Syx*Syx,
+ *     det = (Syy*c00 + Syx*c01) + Sy*c02, and per target (r0, r1, r2, q) = (SYU, SXU, SU, qy), then (SYV, SXV, SV, qx):
+ *     a = ((c00*r0 + c01*r1) + c02*r2) / det, b = ((c01*r0 + c11*r1) + c12*r2) / det,
+ *     c' = ((c02*r0 + c12*r1) + c22*r2) / det, c = (q + c') - (a * py + b * px);
+ *   final model: the refit if its six values are finite and it scores at least as many inliers, else the best
+ *     hypothesis's T.
+ * Outputs: transform_dev [batch - 1][2][3] float64, the final T, all NaN when M_f < 3 or every hypothesis is degenerate;
+ * inlier_count_dev [batch - 1] int64, its inliers (0 then); matched_dev [batch - 1] int64, M_f; inlier_dev [capacity]
+ * uint8, 1 iff the row is a correspondence of its pair and an inlier of the final model, 0 elsewhere (every row of the
+ * last frame, and at and past `rows`). inlier_count_dev also holds each pair's winner between the kernels. No result
+ * depends on the order of atomics, the grid or the warp schedule.
+ * workspace_dev: silent_motion_workspace_bytes(capacity) bytes, 16-byte aligned. Matches never span calls, so motion
+ * never does either. Three kernels, launched as programmatic dependent launches on `stream`; capacity 0 or batch 1
+ * launches nothing and writes nothing (every pair then has M_f = 0). Argument checks (all on the host, before any CUDA
+ * call): capacity < 0, batch < 1, a null input, workspace, inlier or (with batch > 1) pair output with capacity > 0, a
+ * workspace that is not 16-byte aligned, or threshold NaN, infinite or <= 0 -> SILENT_E_INVAL; hypotheses outside
+ * [1, SILENT_MOTION_HYPOTHESES_MAX] -> SILENT_E_SHAPE; workspace_bytes short -> SILENT_E_CAPACITY; no CUDA device ->
+ * SILENT_E_CUDA. */
+#define SILENT_MOTION_HYPOTHESES_MAX 4096
+size_t silent_motion_workspace_bytes(int64_t capacity);
+int silent_estimate_motion(const int64_t *frame_offsets_dev, const float *frame_yx_dev, const int64_t *next_dev,
+                           const int64_t *count_dev, int64_t capacity, int batch, int hypotheses, float threshold,
+                           uint64_t seed, void *workspace_dev, size_t workspace_bytes, double *transform_dev,
+                           int64_t *inlier_count_dev, int64_t *matched_dev, uint8_t *inlier_dev, silent_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

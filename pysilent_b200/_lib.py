@@ -30,6 +30,7 @@ SYMBOLS = (
     "silent_stack_fused_f16", "silent_stack_bank_f16", "silent_pipeline_run_f16", "silent_pipeline_run_orientations_f16",
     "silent_pipeline_run_host_f16", "silent_nv12_to_bgr", "silent_plan_level_coords", "silent_point_records",
     "silent_point_patches", "silent_peak_points", "silent_plan_peak_points", "silent_match_points",
+    "silent_motion_workspace_bytes", "silent_estimate_motion",
 )
 
 
@@ -57,6 +58,7 @@ BANK_MAX = 16                  # SILENT_BANK_MAX
 FUSED_BANK_WIDTHS = (4, 8, 12, 16)   # orientation counts with fused kernels (silent_pipeline_run_orientations)
 RECORD_CHANNELS = (3,) + FUSED_BANK_WIDTHS   # output channel counts silent_point_records reads
 PATCH_RADIUS_MAX = 31          # SILENT_PATCH_RADIUS_MAX: largest radius silent_point_patches takes
+MOTION_HYPOTHESES_MAX = 4096   # SILENT_MOTION_HYPOTHESES_MAX: most hypotheses silent_estimate_motion takes
 
 
 class SilentOrientationBank(ctypes.Structure):
@@ -127,6 +129,8 @@ def lib():
         "silent_point_records": (i, [p, i, p, p, i64, p, p, i, i, p, p, p, p, p]),
         "silent_point_patches": (i, [p, i, p, p, i64, p, p, i, i, p, i, p, p, p, p]),
         "silent_match_points": (i, [p, p, i64, p, i64, i, i, f, p, p, p, p]),
+        "silent_motion_workspace_bytes": (sz, [i64]),
+        "silent_estimate_motion": (i, [p, p, p, p, i64, i, i, f, ctypes.c_uint64, p, sz, p, p, p, p, p]),
         "silent_get_centroids": (i, [p, i, i, i, i, i, p, p, p, p]),
         "silent_resize_nearest": (i, [p, i, i, i, i, i, i, p, p]),
         "silent_get_boosting": (i, [p, p, i, i, i, f, f, i, p, p, p]),

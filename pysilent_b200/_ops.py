@@ -4,6 +4,7 @@ Tensors are contiguous float32 NHWC ``[levels, h, w, C]`` on a CUDA device (the 
 ``recognition_testing.py:62``); numpy inputs are uploaded to the current CUDA device.
 """
 import ctypes
+import math
 import numbers
 import threading
 
@@ -543,3 +544,88 @@ def match_points(points, count, values, levels, search_radius, max_ratio=1.0, ne
             ptr(points), ptr(count), cap, ptr(values), elems, int(levels), radius, ratio, ptr(next), ptr(prev),
             ptr(distance), stream_ptr()), "silent_match_points")
     return next, prev, distance
+
+
+def motion_args(threshold, hypotheses, seed):
+    """``(threshold, hypotheses, seed)`` of ``estimate_motion`` as (float, int, int): ``threshold`` a real number whose
+    float32 value is finite and > 0 (frame pixels), ``hypotheses`` an int in ``[1, MOTION_HYPOTHESES_MAX]``, ``seed`` an
+    int in ``[0, 2^64)``; anything else (a bool, a non-number, NaN, a value out of range) raises ValueError."""
+    if isinstance(threshold, (bool, np.bool_)) or not isinstance(threshold, numbers.Real):
+        raise ValueError("threshold must be a real number > 0, got %r" % (threshold,))
+    t = float(threshold)
+    with np.errstate(over="ignore"):
+        t32 = float(np.float32(t))
+    if not (math.isfinite(t32) and t32 > 0.0):
+        raise ValueError("threshold must be finite and > 0 in float32, got %r" % (threshold,))
+    if isinstance(hypotheses, (bool, np.bool_)) or not isinstance(hypotheses, (int, np.integer)) \
+            or not 1 <= hypotheses <= _lib.MOTION_HYPOTHESES_MAX:
+        raise ValueError("hypotheses must be an int in [1, %d], got %r" % (_lib.MOTION_HYPOTHESES_MAX, hypotheses))
+    if isinstance(seed, (bool, np.bool_)) or not isinstance(seed, (int, np.integer)) or not 0 <= seed < 2 ** 64:
+        raise ValueError("seed must be an int in [0, 2^64), got %r" % (seed,))
+    return t, int(hypotheses), int(seed)
+
+
+def motion_workspace_bytes(capacity):
+    """Bytes of the ``estimate_motion`` workspace for ``capacity`` rows (``silent_motion_workspace_bytes``)."""
+    return int(_lib.lib().silent_motion_workspace_bytes(int(capacity)))
+
+
+def estimate_motion(frame_offsets, frame_yx, next, count, hypotheses, threshold, seed=0, transform=None,
+                    inlier_count=None, matched=None, inlier=None, workspace=None):
+    """``silent_estimate_motion``: a robust affine map per pair of consecutive frames from the matches. ``frame_offsets``
+    int64 ``[B + 1]`` and ``frame_yx`` float32 ``[capacity, 2]`` as ``PointRecords`` holds them, ``next`` int64
+    ``[capacity]`` as ``PointMatches`` holds it, ``count`` an int64 device scalar (the rows used are the first
+    ``clamp(count, 0, capacity)``). Returns ``(transform, inlier_count, matched, inlier)``: float64 ``[B - 1, 2, 3]``,
+    int64 ``[B - 1]``, int64 ``[B - 1]`` and uint8 ``[capacity]`` (see ``pipeline.PointMotion``), into the given buffers
+    where passed; ``workspace`` a uint8 tensor of at least ``motion_workspace_bytes(capacity)`` bytes. No host
+    synchronisation. Shapes, dtypes, devices, contiguity and the arguments are checked first (ValueError)."""
+    threshold, hypotheses, seed = motion_args(threshold, hypotheses, seed)
+    for name, t in (("frame_offsets", frame_offsets), ("frame_yx", frame_yx), ("next", next), ("count", count)):
+        if not isinstance(t, torch.Tensor):
+            raise ValueError("%s must be a torch.Tensor, got %s" % (name, type(t).__name__))
+    if frame_offsets.dim() != 1 or frame_offsets.shape[0] < 2 or frame_offsets.dtype != torch.int64:
+        raise ValueError("frame_offsets must be int64 [B + 1] with B >= 1, got %s %s"
+                         % (frame_offsets.dtype, tuple(frame_offsets.shape)))
+    batch = int(frame_offsets.shape[0]) - 1
+    if batch > 2 ** 31 - 1:
+        raise ValueError("estimate_motion takes at most 2^31 - 1 frames, got %d" % batch)
+    if frame_yx.dim() != 2 or frame_yx.shape[1] != 2 or frame_yx.dtype != torch.float32:
+        raise ValueError("frame_yx must be float32 [capacity, 2], got %s %s" % (frame_yx.dtype, tuple(frame_yx.shape)))
+    cap = int(frame_yx.shape[0])
+    if next.dtype != torch.int64 or tuple(next.shape) != (cap,):
+        raise ValueError("next must be int64 [%d], got %s %s" % (cap, next.dtype, tuple(next.shape)))
+    if count.dtype != torch.int64 or count.numel() < 1:
+        raise ValueError("count must be an int64 tensor of at least one element")
+    dev = frame_yx.device
+    pairs = batch - 1
+    transform = torch.empty((pairs, 2, 3), dtype=torch.float64, device=dev) if transform is None else transform
+    inlier_count = torch.empty((pairs,), dtype=torch.int64, device=dev) if inlier_count is None else inlier_count
+    matched = torch.empty((pairs,), dtype=torch.int64, device=dev) if matched is None else matched
+    inlier = torch.empty((cap,), dtype=torch.uint8, device=dev) if inlier is None else inlier
+    need = motion_workspace_bytes(cap)
+    workspace = torch.empty((max(need, 1),), dtype=torch.uint8, device=dev) if workspace is None else workspace
+    for name, t, dt, shape in (("transform", transform, torch.float64, (pairs, 2, 3)),
+                               ("inlier_count", inlier_count, torch.int64, (pairs,)),
+                               ("matched", matched, torch.int64, (pairs,)), ("inlier", inlier, torch.uint8, (cap,))):
+        if not isinstance(t, torch.Tensor) or t.dtype != dt or tuple(t.shape) != shape:
+            raise ValueError("%s must be %s %s, got %s %s" % (name, dt, shape, getattr(t, "dtype", type(t).__name__),
+                                                               tuple(getattr(t, "shape", ()))))
+    if not isinstance(workspace, torch.Tensor) or workspace.dtype != torch.uint8 or workspace.dim() != 1 \
+            or workspace.numel() < need:
+        raise ValueError("workspace must be a uint8 tensor of at least %d bytes" % need)
+    tensors = (frame_offsets, frame_yx, next, count, transform, inlier_count, matched, inlier, workspace)
+    if any(not t.is_cuda or t.device != dev or not t.is_contiguous() for t in tensors):
+        raise ValueError("estimate_motion needs contiguous CUDA tensors on one device")
+    if workspace.data_ptr() % 16:
+        raise ValueError("workspace must be 16-byte aligned")
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().silent_estimate_motion(
+            ptr(frame_offsets), ptr(frame_yx), ptr(next), ptr(count), cap, batch, hypotheses, threshold, seed,
+            ptr(workspace), workspace.numel(), ptr(transform), ptr(inlier_count), ptr(matched), ptr(inlier),
+            stream_ptr()), "silent_estimate_motion")
+        if cap == 0 or batch == 1:   # the library launches nothing then: no pair has a correspondence
+            transform.fill_(float("nan"))
+            inlier_count.zero_()
+            matched.zero_()
+            inlier.zero_()
+    return transform, inlier_count, matched, inlier

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsilent_b200.so")
-SOURCES = ["plan.cu", "pyramid.cu", "conv.cu", "stack_fused.cu", "emit.cu", "display.cu", "pipeline.cu", "gather.cu", "nv12.cu", "points.cu", "match.cu"]
+SOURCES = ["plan.cu", "pyramid.cu", "conv.cu", "stack_fused.cu", "emit.cu", "display.cu", "pipeline.cu", "gather.cu", "nv12.cu", "points.cu", "match.cu", "motion.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-fmad=false",                      # canonical order: every FMA in the library is an explicit fmaf()

@@ -51,6 +51,10 @@ def host_round_trip(staged, device, run, pinned):
     return outs
 
 
+# defaults of run_frames_motion / run_host_motion (profiles/motion_bench_b200.json)
+MOTION_THRESHOLD = 2.0   # frame pixels
+MOTION_HYPOTHESES = 256
+
 # routes of frames (LineEndPipeline._frame_route)
 PLAN, CONVERT, PYRAMID = "plan", "convert", "pyramid"
 
@@ -90,6 +94,39 @@ the raw link iff ``d1 <= float32(max_ratio) * d2`` (rounded). ``max_ratio`` = 1 
 so Lowe's 0.8 on distances is 0.64 here. i -> j is accepted iff j is i's raw link in the next frame and i is j's in the
 previous one. Rows of the last frame have next = -1 and rows of frame 0 prev = -1: matches never span calls, so a stream
 processed in batches keeps one frame of overlap between consecutive batches to link them."""
+
+PointMotion = collections.namedtuple("PointMotion", "transform inlier_count matched inlier")
+PointMotion.__doc__ = """How the camera moved between consecutive frames of one batch, and which matches agree with that
+motion (``silent_estimate_motion``), over the B frames and K rows of the ``PointRecords`` and ``PointMatches`` it comes
+with: transform: float64 [B - 1, 2, 3], per pair (f, f + 1) the affine map T with ``[y1, x1] = T[:, :2] @ [y0, x0] +
+T[:, 2]`` in frame pixels, (y, x) order as ``frame_yx``; all NaN when the pair has fewer than 3 correspondences or every
+hypothesis is degenerate; inlier_count: int64 [B - 1], the correspondences T keeps (0 then); matched: int64 [B - 1], the
+pair's correspondences M_f; inlier: uint8 [K], 1 iff the row is a correspondence of its pair and an inlier of T.
+
+The correspondences of pair f are the rows i of frame f (``frame_offsets[f] <= i < frame_offsets[f + 1]``), in row
+order, with ``next[i] >= 0`` and ``frame_yx[i]``, ``frame_yx[next[i]]`` all finite (rows of a level that defines an axis
+as 0 have NaN coordinates and never take part): c_k = (y0, x0, y1, x1), k = 0 .. M_f - 1.
+
+Hypothesis h = 0 .. H - 1 (H = ``hypotheses``) draws k_d = mulhi64(u_d, M_f), d = 0, 1, 2, with u_d =
+splitmix64(seed ^ splitmix64((f << 32) | (h << 2) | d)) (Vigna's splitmix64 finaliser with its 0x9e3779b97f4a7c15
+increment, 64-bit wrapping). It is degenerate if two draws are equal. Otherwise, in float64: with (y0, x0) the source of
+c_k0 and dyj = yj - y0, dxj = xj - x0 for the sources of c_k1, c_k2, D = dy1 * dx2 - dx1 * dy2, degenerate if
+``!(|D| >= 1)``; per target u (y1, then x1): du1 = u_k1 - u_k0, du2 = u_k2 - u_k0, a = (du1 * dx2 - dx1 * du2) / D,
+b = (dy1 * du2 - du1 * dy2) / D, c = u_k0 - (a * y0 + b * x0).
+
+A model T scores in float32: m = float32(T), rounded once; c_k is an inlier iff ``e_y * e_y + e_x * e_x <= t * t`` with
+t = float32(threshold), ``e_y = y1 - ((m_a * y0 + m_b * x0) + m_c)`` and e_x likewise, every operation rounded, no fused
+products. The best hypothesis has the most inliers, ties to the smaller h.
+
+Refit: one least-squares step on the inliers of the best hypothesis. With (py, px, qy, qx) = its c_k0 and Y = y0 - py,
+X = x0 - px, U = y1 - qy, V = x1 - qx in float64, the 11 sums of Y, X, YY, YX, XX, U, YU, XU, V, YV, XV are each taken in
+a fixed order: thread t = 0..255 adds its terms over k = t, t + 256, ... from +0.0; within each warp of 32 threads
+``s_t = s_t + s_(t xor b)`` for b = 16, 8, 4, 2, 1; the 8 warps' lane-0 sums w are added as ((w_0 + w_1) + ...) + w_7.
+The two 3 x 3 normal systems are solved by their adjugate (``silent_estimate_motion`` in ``silent_b200.h`` spells out
+every operation) and the translation is moved back by ``c = (q + c') - (a * py + b * px)``. The refit is kept if its six
+values are finite and it scores at least as many inliers; otherwise the best hypothesis's T is.
+
+Matches never span calls, so motion never does either; one frame (B = 1) gives empty pair outputs and inlier all 0."""
 
 
 class LineEndPipeline:
@@ -543,6 +580,48 @@ class LineEndPipeline:
             return rows[:3] + (values,) + tuple(links)
         outs = host_round_trip(staged, dev, run, lambda i, shape, dtype: torch.empty(shape, dtype=dtype, pin_memory=True))
         return self._records(*outs[:4]), PointMatches(*outs[4:])
+
+    # -- frame-to-frame motion -------------------------------------------------------------------------------------------
+    def run_frames_motion(self, frames, patch_radius, search_radius, max_ratio=1.0, threshold=MOTION_THRESHOLD,
+                          hypotheses=MOTION_HYPOTHESES, seed=0, points_capacity=None):
+        """``run_frames_matches`` and the motion between consecutive frames that its matches support
+        (``PointRecords``, ``PointMatches``, ``PointMotion``), all CUDA tensors: per frame pair an affine map in frame
+        pixels from a seeded RANSAC of ``hypotheses`` (an int in [1, 4096]) draws, inliers within ``threshold`` frame
+        pixels (a real number > 0), refined by one least-squares step; see ``PointMotion``. ``seed`` (an int in
+        [0, 2^64)) makes the draws reproducible. Runs on every route, bank, ``out_dtype``, ``frame_format`` and
+        ``peaks`` the matches serve. Every argument is checked before any GPU work (ValueError)."""
+        radius, r, ratio = self._match_args(patch_radius, search_radius, max_ratio)
+        motion_args = _ops.motion_args(threshold, hypotheses, seed)
+        levels, rows = self._record_rows(frames, points_capacity, None, radius)
+        matches = self._matches(levels, rows, r, ratio)
+        return self._records(*rows), matches, self._motion(rows, matches, *motion_args)
+
+    @staticmethod
+    def _motion(rows, matches, threshold, hypotheses, seed):
+        """``PointMotion`` of the rows ``_record_rows`` returns and their ``PointMatches``."""
+        points, frame_offsets, frame_yx = rows[:3]
+        count = torch.full((1,), points.shape[0], dtype=torch.int64, device=points.device)
+        return PointMotion(*_ops.estimate_motion(frame_offsets, frame_yx, matches.next, count, hypotheses, threshold,
+                                                 seed))
+
+    def run_host_motion(self, frames, patch_radius, search_radius, max_ratio=1.0, threshold=MOTION_THRESHOLD,
+                        hypotheses=MOTION_HYPOTHESES, seed=0, points_capacity=4096):
+        """``run_frames_motion`` on host frames, as ``run_host_matches`` takes them: numpy ``(PointRecords,
+        PointMatches, PointMotion)``. The patches stay on the device: the records' values are the patch centres.
+        ``points_capacity`` sizes the first attempt; every point is returned. The arguments are checked before the
+        upload."""
+        radius, r, ratio = self._match_args(patch_radius, search_radius, max_ratio)
+        motion_args = _ops.motion_args(threshold, hypotheses, seed)
+        staged, dev = self._stage_host(frames)
+
+        def run(x):
+            levels, rows = self._record_rows(x, points_capacity, None, radius)
+            links = self._matches(levels, rows, r, ratio)
+            motion = self._motion(rows, links, *motion_args)
+            values = rows[3] if radius is None else rows[3][:, radius, radius].contiguous()
+            return rows[:3] + (values,) + tuple(links) + tuple(motion)
+        outs = host_round_trip(staged, dev, run, lambda i, shape, dtype: torch.empty(shape, dtype=dtype, pin_memory=True))
+        return self._records(*outs[:4]), PointMatches(*outs[4:7]), PointMotion(*outs[7:])
 
     # -- host buffers on both sides (LineEndDisplayer.callback) -----------------------------------------------------------
     def run_host(self, frames, orient_out=None, line_end_out=None, points_capacity=4096):
